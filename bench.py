@@ -1,9 +1,13 @@
 #!/usr/bin/env python
 """bench.py - fp64 GMG V-cycle DOF/s (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config D|B|A|C|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config D|B|A|C|...] [--dump-outputs DIR]
 
 A "step" is one V(1,1) cycle (GMG::Cycle::apply, zero initial guess) over the whole finest level.
+
+`--dump-outputs DIR` (one GPU) writes the result u of the last timed step to DIR/u.npy (float64): all of it when it has at
+most DUMP_MAX_VALUES cells, otherwise the cells at a fixed seeded sample of indices (sorted).  The right-hand side is a
+function of the workload only, so two builds run with the same arguments can be compared output for output.
 
 Workload at EVERY N (1, 2, 4, 8): BASELINE config D as named - the >= 1 B-cell 3D uniform octree, 4uni.bin --divide 2,
 32,768 patches of 32^3 = 1,073,741,824 cells, 6 levels, trig manufactured right-hand side resident in HBM - so that the
@@ -53,6 +57,8 @@ E_WEAK = {1: ("E", None), 2: ("E", None), 4: ("E5", None), 8: ("E5", None)}
 NEUMANN = {"GMGEX": "gauss"}
 ALGO_BYTES_PER_CELL_VISIT = 48.0  # SURVEY 8(d): pre-smooth 16 + residual/restrict 16 + post-smooth 16
 CYCLE = "V(1,1), 1 coarse sweep, all levels down to the root patch"
+DUMP_MAX_VALUES = 1 << 22  # 32 MB of float64
+DUMP_SEED = 0
 DFT_CAVEAT = ("patch solver = the reference's first-party DftPatchSolver (dense n x n transform matrices through a naive dgemv_ shim): "
               "O(n) work per cell per axis, i.e. slower than the FftwPatchSolver path with a real FFTW, which is not installed here")
 
@@ -254,6 +260,16 @@ def time_cycles(env, h, f, u, opts, steps, warmup):
     launches = ctx.kernel_launches() - l0
     env.barrier()
     return env.reduce_max(ms)[0] / steps, launches, ms / steps
+
+
+def dump_outputs(out_dir, u):
+    """u of the last timed step -> out_dir/u.npy (see the module docstring)"""
+    import numpy as np
+    a = u.download()
+    if a.size > DUMP_MAX_VALUES:
+        a = a[np.sort(np.random.default_rng(DUMP_SEED).choice(a.size, DUMP_MAX_VALUES, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "u.npy"), a)
 
 
 def kernel_profile(env, h, f, u, opts, steps):
@@ -485,8 +501,9 @@ def multi_gpu_parity(env):
     return out
 
 
-def measure_config(env, cfg, steps, warmup, box_frac=None, profile=True):
-    """device-resident cycle timing of one workload -> dict (value, ms_per_step, roofline, ...)"""
+def measure_config(env, cfg, steps, warmup, box_frac=None, profile=True, dump_dir=None):
+    """device-resident cycle timing of one workload -> dict (value, ms_per_step, roofline, ...); with dump_dir, the timed
+    steps' result is written there before anything else runs on u"""
     pps = env.pps
     D, mesh_file, divide, n, _, desc = CONFIGS[cfg]
     h, mesh, part, setup_s = build_hierarchy(env, cfg, box_frac)
@@ -503,6 +520,8 @@ def measure_config(env, cfg, steps, warmup, box_frac=None, profile=True):
     if env.world > 1:
         opts.use_graph = 2  # capture the halo exchanges into the CUDA graph as well
     ms_per_step, launches, my_ms = time_cycles(env, h, f, u, opts, steps, warmup)
+    if dump_dir is not None:
+        dump_outputs(dump_dir, u)
     total_cells = int(env.reduce_sum(cells)[0])
     res = {"workload": desc if box_frac is None else desc + "; leaves with centre x < %.2f refined once more" % box_frac,
            "n_gpus": env.world, "value": total_cells / (ms_per_step * 1e-3), "unit": "DOF/s", "ms_per_step": ms_per_step,
@@ -537,7 +556,10 @@ def main():
     ap.add_argument("--cycle-only", action="store_true", help="only the device-resident V-cycle timing and its roofline")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the other BASELINE configs")
     ap.add_argument("--with-solve", action="store_true", help="with --cycle-only: also the time to 1e-10 residual")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result to DIR/u.npy (one GPU, not with --impl reference)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs works on one GPU and not with --impl reference")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -548,7 +570,7 @@ def main():
     W = max(args.warmup, 3)
     sampler = ClockSampler(env.local_rank)
     sampler.start()
-    res, state = measure_config(env, cfg, args.steps, W)
+    res, state = measure_config(env, cfg, args.steps, W, dump_dir=args.dump_outputs)
     sampler.stop_flag = True
     sampler.join()
     h, mesh, part, f, u, opts, cells, total_cells, level_cells = state

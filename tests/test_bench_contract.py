@@ -1,14 +1,19 @@
 """The JSON lines bench.py printed in the committed driver-style runs (profiles/r02_bench_*.json) carry every key of the
 measurement contract, agree with each other about the workload, and are internally consistent (value = cells / time,
-roofline.frac = achieved / peak, the reference arm ran the same config)."""
+roofline.frac = achieved / peak, the reference arm ran the same config); and what --dump-outputs writes."""
+import importlib.util
 import json
 import os
+import subprocess
+import sys
 
+import numpy as np
 import pytest
 
-from conftest import ROOT
+from conftest import MESHES, ROOT, rel_l2
 
 PROFILES = os.path.join(ROOT, "profiles")
+BENCH = os.path.join(ROOT, "bench.py")
 
 
 def load(name):
@@ -56,3 +61,52 @@ def test_scaling_curve_is_on_one_mesh_and_reference_arm_matches():
     eff = {n: lines[n]["value"] / (n * lines[1]["value"]) for n in (2, 4, 8)}
     assert eff[2] > 0.9 and eff[4] > 0.85 and eff[8] > 0.8, eff  # north star: >= 0.8 at 8 GPUs on a >= 1 B-cell mesh
     assert lines[1]["roofline"]["vcycle_frac"] >= 0.6              # north star: >= 60 % of the HBM roofline per V-cycle
+
+
+def test_dump_outputs_writes_the_whole_result_or_a_fixed_sample(tmp_path):
+    """bench.py --dump-outputs: float64, all of u up to DUMP_MAX_VALUES cells, above that the same sorted sample every run"""
+    spec = importlib.util.spec_from_file_location("bench_mod", BENCH)
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+
+    class Vec:
+        def __init__(self, n):
+            self.n = n
+
+        def download(self):
+            return np.arange(self.n, dtype=np.float64)
+
+    bench.DUMP_MAX_VALUES = 64
+    bench.dump_outputs(str(tmp_path / "whole"), Vec(64))
+    assert np.array_equal(np.load(tmp_path / "whole" / "u.npy"), np.arange(64.0))
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), Vec(1000))
+    a, b = np.load(tmp_path / "a" / "u.npy"), np.load(tmp_path / "b" / "u.npy")
+    assert a.dtype == np.float64 and a.size == 64 and np.array_equal(a, b)
+    assert np.all(np.diff(a) > 0) and a[-1] < 1000  # distinct cells in index order
+
+
+@pytest.mark.parametrize("argv,env", [(["--impl", "reference"], {}), ([], {"WORLD_SIZE": "2"})])
+def test_dump_outputs_is_refused_where_there_is_no_single_gpu_result(tmp_path, argv, env):
+    """the reference arm computes no u, and under torchrun every rank holds only its own patches"""
+    out = tmp_path / "dump"
+    res = subprocess.run([sys.executable, BENCH, "--dump-outputs", str(out)] + argv, env=dict(os.environ, **env),
+                         capture_output=True, text=True, timeout=120)
+    assert res.returncode == 2 and "--dump-outputs" in res.stderr, res.stderr
+    assert not out.exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_timed_cycles_result(tmp_path):
+    """main() hands --dump-outputs to the timed measurement: on a workload small enough to be written whole (config
+    `small`, 2,097,152 cells), u.npy is one V-cycle of the workload's right-hand side, checked against the oracle"""
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    import gmg_oracle as go
+    res = subprocess.run([sys.executable, BENCH, "--config", "small", "--cycle-only", "--no-other-configs", "--no-cpu-baseline",
+                          "--steps", "2", "--warmup", "3", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0, res.stdout + res.stderr
+    u = np.load(tmp_path / "u.npy")
+    levels = go.build_hierarchy(os.path.join(MESHES, "3uni.bin"), 3, 16, 1)
+    f, _ = go.trig_rhs(levels[0])
+    assert u.dtype == np.float64 and u.size == f.size == 2097152
+    assert rel_l2(u, go.vcycle(levels, f)) < 1e-12

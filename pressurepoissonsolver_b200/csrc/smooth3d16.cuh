@@ -29,51 +29,17 @@
 
 namespace tgpu
 {
-__device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned) __cvta_generic_to_shared(p); }
-__device__ __forceinline__ void     cp_async16(double *smem_dst, const double *gsrc)
-{
-	asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(smem_u32(smem_dst)), "l"(gsrc) : "memory");
-}
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
 
-// L2 residency hint experiment: the face buffers (50 MB on config B) are re-read by the next two kernels of the cycle, the
-// patch data streaming past them (f, u: 134 MB each) is not.  S16_L2HINT=1 stores the faces with an evict_last policy;
-// measured on configs B and C: no change (0.2242 vs 0.2251 ms, 0.5788 vs 0.5788 ms), so it stays off.
-#ifndef S16_L2HINT
-#define S16_L2HINT 0
-#endif
-__device__ __forceinline__ uint64_t l2_policy_evict_last()
-{
-	uint64_t pol;
-	asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;\n" : "=l"(pol));
-	return pol;
-}
-__device__ __forceinline__ void st_keep_l2(double *p, double v, uint64_t pol)
-{
-#if S16_L2HINT
-	asm volatile("st.global.L2::cache_hint.f64 [%0], %1, %2;\n" ::"l"(p), "d"(v), "l"(pol) : "memory");
-#else
-	*p = v;
-#endif
-}
 constexpr int    S16_BLOCK = TGPU_THREADS; // threads per CTA (the host launches with this)
 constexpr int    S16_ROW = 18, S16_PL = 290, S16_TILE = 16 * S16_PL;
-// Sweeps from a zero guess have no interface values to fold into the right-hand side, so f needs no staging:
-// it is loaded straight into the z pencils (the next patch is pulled into L2 meanwhile), one tile per CTA and
-// 64 registers per thread let four CTAs share an SM.  The other variants stage f with cp.async in a second
-// tile (the boundary cells are updated in place there) and run three CTAs per SM.
-__host__ __device__ constexpr bool   s16_direct(bool, bool src_fine) { return !src_fine; }
-#ifndef S16_GAMMA_CTAS
-#define S16_GAMMA_CTAS 3
-#endif
-__host__ __device__ constexpr int    s16_ctas_per_sm(bool zero_guess, bool src_fine, bool neu = false)
+// f is loaded straight into the z pencils (the next patch is pulled into L2 meanwhile): one tile per CTA.  Sweeps
+// from a zero guess fit 64 registers and run four CTAs per SM, the others three.
+__host__ __device__ constexpr int    s16_ctas_per_sm(bool zero_guess, bool neu = false)
 {
-	return neu ? 2 : (src_fine ? 3 : (zero_guess ? 4 : S16_GAMMA_CTAS)); // (the Neumann variant's general transforms need the registers)
+	return neu ? 2 : (zero_guess ? 4 : 3); // (the Neumann variant's general transforms need the registers)
 }
-__host__ __device__ constexpr size_t smooth3d16_smem_bytes(bool zero_guess = false, bool src_fine = false)
-{
-	return sizeof(double) * (s16_direct(zero_guess, src_fine) ? 1 : 2) * S16_TILE;
-}
+constexpr size_t smooth3d16_smem_bytes() { return sizeof(double) * S16_TILE; }
 
 // refinement-boundary sides are rare: keep their (large) code out of line
 template <bool PROLONG>
@@ -162,106 +128,6 @@ template <bool PROLONG> struct SideGamma16 {
 	}
 };
 
-// Right-hand side of a coarse patch assembled straight from the FINER level's face buffer (first sweep of a
-// level visit in the fused cycle): f_c = R r with r = -(2/h^2) E^T gamma(u_fine) living on the fine patches'
-// boundary cells (see face_residual_restrict_kernel for the identity).  Replaces that kernel's launch and the
-// round trip of f_c through memory before the sweep; the assembled f_c is still stored (the level's later
-// sweeps read it).  Same expressions and summation order as face_residual_restrict_kernel.
-template <int MODE>
-__device__ __forceinline__ double gamma_entry16(const PatchMeta &pm, int p, int s, int m, const FaceVals<3, 16, MODE> &fv)
-{
-	const int ty = pm.nbr_type[s];
-	if (ty == NBR_NONE) return 0.0;
-	if (ty == NBR_NORMAL) {
-		const double a = fv.get(p, pm.parent_idx, pm.orth_on_parent, s, m);
-		const double b = fv.get(pm.nbr_idx[s][0], pm.nbr_parent[s], pm.nbr_orth[s], s ^ 1, m);
-		return 0.5 * a + 0.5 * b;
-	}
-	return iface_gamma<3, 16, MODE>(pm, p, s, m, fv);
-}
-struct FineSrc16 {
-	const PatchMeta *fmeta;    // neighbour table of the finer level
-	const double *   fF;       // its face buffer (boundary slices of the pre-smoothed u)
-	const int32_t *  children; // [coarse patch][8]: fine patch per octant; [1] == -2: [0] is the same patch on the finer level
-	double *         fc_out;   // where f_c is stored
-};
-__device__ __forceinline__ double fine_face_block16(const PatchMeta *__restrict__ fmeta, const double *__restrict__ fF, int q, int s, int m0)
-{
-	const PatchMeta &pq   = fmeta[q];
-	const int        ty   = pq.nbr_type[s];
-	const double     cfac = 2.0 * pq.inv_h2;
-	if (ty == NBR_NONE) return 0.0;
-	double r00, r01, r10, r11;
-	if (ty == NBR_NORMAL) {
-		const double *own = fF + ((size_t) q * 6 + s) * 256 + m0;
-		const double *nbp = fF + ((size_t) pq.nbr_idx[s][0] * 6 + (s ^ 1)) * 256 + m0;
-		const double2 a0 = __ldg(reinterpret_cast<const double2 *>(own)), a1 = __ldg(reinterpret_cast<const double2 *>(own + 16));
-		const double2 b0 = __ldg(reinterpret_cast<const double2 *>(nbp)), b1 = __ldg(reinterpret_cast<const double2 *>(nbp + 16));
-		r00 = cfac * (0.5 * -a0.x + 0.5 * -b0.x);
-		r01 = cfac * (0.5 * -a0.y + 0.5 * -b0.y);
-		r10 = cfac * (0.5 * -a1.x + 0.5 * -b1.x);
-		r11 = cfac * (0.5 * -a1.y + 0.5 * -b1.y);
-	} else {
-		const FaceVals<3, 16, FV_NEG> fv{fF, nullptr, fmeta};
-		r00 = cfac * iface_gamma<3, 16, FV_NEG>(pq, q, s, m0, fv);
-		r01 = cfac * iface_gamma<3, 16, FV_NEG>(pq, q, s, m0 + 1, fv);
-		r10 = cfac * iface_gamma<3, 16, FV_NEG>(pq, q, s, m0 + 16, fv);
-		r11 = cfac * iface_gamma<3, 16, FV_NEG>(pq, q, s, m0 + 17, fv);
-	}
-	return ((r00 + r01) + (r10 + r11)) / 8.0;
-}
-// all 256 threads of the CTA; S = tile of coarse patch p; ends with a CTA barrier
-__device__ __forceinline__ void build_tile_from_fine_faces16(double *S, const FineSrc16 &src, int p, int t)
-{
-	constexpr int ROW = S16_ROW, PL = S16_PL, N = 16;
-	const int lo = t & 15, hi = t >> 4;
-	{
-		double *q = S + lo + hi * ROW;
-#pragma unroll
-		for (int k = 0; k < N; k++) q[k * PL] = 0.0;
-	}
-	__syncthreads();
-	const int32_t *ch = src.children + (size_t) p * 8;
-	if (ch[1] == -2) { // the same patch exists on the finer level: f_c = r, entry t of every side
-		const int        q    = ch[0];
-		const PatchMeta &pq   = src.fmeta[q];
-		const double     cfac = 2.0 * pq.inv_h2;
-		const FaceVals<3, 16, FV_NEG> fv{src.fF, nullptr, src.fmeta};
-		double g[6];
-#pragma unroll
-		for (int s = 0; s < 6; s++) g[s] = cfac * gamma_entry16(pq, q, s, t, fv);
-		S[lo * ROW + hi * PL] += g[0];
-		S[N - 1 + lo * ROW + hi * PL] += g[1];
-		__syncthreads();
-		S[lo + hi * PL] += g[2];
-		S[lo + (N - 1) * ROW + hi * PL] += g[3];
-		__syncthreads();
-		S[lo + hi * ROW] += g[4];
-		S[lo + hi * ROW + (N - 1) * PL] += g[5];
-		__syncthreads();
-		return;
-	}
-	const int m0 = 2 * (lo & 7) + 32 * (hi & 7); // first of the 2 x 2 fine face entries under coarse plane cell (lo, hi)
-	const int oa = lo >> 3, ob = hi >> 3;
-#pragma unroll
-	for (int ax = 0; ax < 3; ax++) {
-		double val[4];
-#pragma unroll
-		for (int pl = 0; pl < 4; pl++) {
-			const int oc = pl >> 1, s = 2 * ax + (pl & 1); // planes 0, 7, 8, 15: octant bit, lower/upper side
-			const int o  = (ax == 0) ? (oc | (oa << 1) | (ob << 2)) : (ax == 1) ? (oa | (oc << 1) | (ob << 2)) : (oa | (ob << 1) | (oc << 2));
-			val[pl]      = fine_face_block16(src.fmeta, src.fF, ch[o], s, m0);
-		}
-#pragma unroll
-		for (int pl = 0; pl < 4; pl++) {
-			const int X   = (pl >> 1) * 8 + (pl & 1) * 7;
-			const int idx = (ax == 0) ? X + lo * ROW + hi * PL : (ax == 1) ? lo + X * ROW + hi * PL : lo + hi * ROW + X * PL;
-			S[idx] += val[pl];
-		}
-		__syncthreads();
-	}
-}
-
 // tables of the general patch solve (smooth_kernel's): dense transform matrices by kind and the eigenvalue rows
 struct NeuTabs {
 	const double * mats = nullptr, *lam = nullptr;
@@ -276,22 +142,20 @@ struct NeuTabs {
 // fast form, DCT-II/III dense) and the y axis transformed and divided by the eigenvalue sums like the others instead of the
 // tridiagonal solve (whose multiplier table is the all-Dirichlet one).  Same arithmetic per patch as smooth_kernel's
 // general path (DftPatchSolver.h:173-216 with the kinds of DftPatchSolver.h:237-289).
-template <bool ZERO_GUESS, bool EMIT, bool PROLONG, bool WRITE_U, bool SRC_FINE = false, bool HALO = false, bool NEU = false>
-__global__ void __launch_bounds__(TGPU_THREADS, s16_ctas_per_sm(ZERO_GUESS, SRC_FINE, NEU))
+template <bool ZERO_GUESS, bool EMIT, bool PROLONG, bool WRITE_U, bool HALO = false, bool NEU = false>
+__global__ void __launch_bounds__(TGPU_THREADS, s16_ctas_per_sm(ZERO_GUESS, NEU))
 smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *__restrict__ f, double *__restrict__ u,
-                  const double *__restrict__ Fin, double *__restrict__ Fout, const double *__restrict__ eig,
-                  const double *__restrict__ uc, FineSrc16 src = FineSrc16{}, HaloSync hs = HaloSync{}, int skip_neumann = 0,
-                  NeuTabs nt = NeuTabs{})
+                  const double *__restrict__ Fin, double *__restrict__ Fout, const double *__restrict__ tri,
+                  const double *__restrict__ uc, HaloSync hs = HaloSync{}, int skip_neumann = 0, NeuTabs nt = NeuTabs{})
 {
-	static_assert(!NEU || (!SRC_FINE && !HALO), "the Neumann instantiation is single-GPU, right-hand side from memory");
+	static_assert(!NEU || !HALO, "the Neumann instantiation is single-GPU");
 	// skip_neumann != 0: patches with Neumann domain sides are left alone (their patch solve is not the plain Dirichlet
 	// one; the general path of smooth_kernel sweeps them in a second launch over the same range); the interface values of
 	// the next patch are still gathered while one is skipped
 	constexpr int N = 16, ROW = S16_ROW, PL = S16_PL;
 	using G = Geo<3, 16>;
 	static_assert(WRITE_U || EMIT, "a sweep must produce something");
-	static_assert(!SRC_FINE || ZERO_GUESS, "only the first sweep of a level visit takes its right-hand side from the finer level");
-	extern __shared__ __align__(16) double smem[];
+	extern __shared__ __align__(16) double S[];
 	// neighbour-table entry of the patch after the next (staged with cp.async) and the gather descriptors
 	// of the current / next patch derived from it
 	constexpr int                   MW = (int) (sizeof(PatchMeta) / sizeof(double));
@@ -305,7 +169,6 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 	auto      pid    = [&](int gg) { return NEU ? (int) __ldg(nt.list + gg) : p0 + gg; }; // patch of work item gg (CTA-uniform)
 	Mags<N> mg;
 	mg.load();
-	const uint64_t l2keep = l2_policy_evict_last();
 	pdl_launch_dependents();
 	pdl_wait();
 	if (!ZERO_GUESS) if (HALO) halo_push<3, 16>(hs, meta);
@@ -323,7 +186,6 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 		if (!ZERO_GUESS) if (HALO) halo_finish(hs);
 		return;
 	}
-	constexpr bool DIRECT = s16_direct(ZERO_GUESS, SRC_FINE); // f goes straight from memory into the z pencils, one tile
 	double gz0 = 0.0, gz1 = 0.0; // (2/h^2) gamma of entry t on the two z faces of the current patch
 	SideGamma16<PROLONG> sg;
 	if (!ZERO_GUESS) {
@@ -352,71 +214,54 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 	}
 	for (int it = 0; g < npatch; g += gridDim.x, it++) {
 		const int       b    = it & 1;
-		double *        S    = smem + (DIRECT ? 0 : b) * S16_TILE;
 		const int       p    = pid(g);
 		const int       gn   = g + gridDim.x;
 		const bool      next = gn < npatch;
 		const int       pn   = NEU ? (next ? pid(gn) : p) : p0 + gn; // patch whose gamma is gathered during this iteration
 		const int       pnn  = (gn + (int) gridDim.x < npatch) ? pid(gn + gridDim.x) : p; // the one after it
 		const GPatch16 &gp   = GD[b ^ 1]; // its descriptors
-		double          h2;
 		int             neu_p = 0; // Neumann bits of patch p
-		if (SRC_FINE) {
-			h2 = meta[p].h2;
-			build_tile_from_fine_faces16(S, src, p, t); // (tile b was last read two iterations ago)
-		} else {
-			// the previous patch's last stage has read the tile; Gs and the descriptors written during the
-			// previous iteration become visible
-			__syncthreads();
-			if (HALO && !ZERO_GUESS && next) halo_wait_cta(hs, pn, halo_ok); // gamma of patch pn is gathered during this iteration
-			h2 = ZERO_GUESS ? meta[p].h2 : GD[b].h2;
-			// table entry of the patch after the next -> metaS (read by describe() after the next barrier but one)
-			if (!ZERO_GUESS && t < MW && gn + (int) gridDim.x < npatch)
-				cp_async8(&metaS[t], reinterpret_cast<const double *>(meta + pnn) + t, true);
-			if (NEU || skip_neumann) neu_p = ZERO_GUESS ? meta[p].neumann : GD[b].neu;
-			if (NEU ? neu_p == 0 : (skip_neumann && neu_p)) { // CTA-uniform: this patch belongs to the other launch
-				if (!ZERO_GUESS) {
-					// keep the pipeline of the next patch's interface values going: all six sides at once, nothing to hide behind
-					SideGamma16<PROLONG> s6[6];
-					if (next) {
-						s6[0].template issue<0>(gp.d[0], t, lo, hi, Fin, uc);
-						s6[1].template issue<0>(gp.d[1], t, lo, hi, Fin, uc);
-						s6[2].template issue<1>(gp.d[2], t, lo, hi, Fin, uc);
-						s6[3].template issue<1>(gp.d[3], t, lo, hi, Fin, uc);
-						s6[4].template issue<2>(gp.d[4], t, lo, hi, Fin, uc);
-						s6[5].template issue<2>(gp.d[5], t, lo, hi, Fin, uc);
-					}
-					cp_async_wait_all();
-					__syncthreads(); // metaS has landed
-					if (next) {
-#pragma unroll
-						for (int s = 0; s < 4; s++) Gs[s * 256 + t] = s6[s].finish(gp, s, meta, pn, t, Fin, uc);
-						gz0 = s6[4].finish(gp, 4, meta, pn, t, Fin, uc);
-						gz1 = s6[5].finish(gp, 5, meta, pn, t, Fin, uc);
-						if (gn + (int) gridDim.x < npatch) describe(*reinterpret_cast<const PatchMeta *>(metaS), pnn, b);
-					}
+		// the previous patch's last stage has read the tile; Gs and the descriptors written during the
+		// previous iteration become visible
+		__syncthreads();
+		if (HALO && !ZERO_GUESS && next) halo_wait_cta(hs, pn, halo_ok); // gamma of patch pn is gathered during this iteration
+		const double h2 = ZERO_GUESS ? meta[p].h2 : GD[b].h2;
+		// table entry of the patch after the next -> metaS (read by describe() after the next barrier but one)
+		if (!ZERO_GUESS && t < MW && gn + (int) gridDim.x < npatch)
+			cp_async8(&metaS[t], reinterpret_cast<const double *>(meta + pnn) + t, true);
+		if (NEU || skip_neumann) neu_p = ZERO_GUESS ? meta[p].neumann : GD[b].neu;
+		if (NEU ? neu_p == 0 : (skip_neumann && neu_p)) { // CTA-uniform: this patch belongs to the other launch
+			if (!ZERO_GUESS) {
+				// keep the pipeline of the next patch's interface values going: all six sides at once, nothing to hide behind
+				SideGamma16<PROLONG> s6[6];
+				if (next) {
+					s6[0].template issue<0>(gp.d[0], t, lo, hi, Fin, uc);
+					s6[1].template issue<0>(gp.d[1], t, lo, hi, Fin, uc);
+					s6[2].template issue<1>(gp.d[2], t, lo, hi, Fin, uc);
+					s6[3].template issue<1>(gp.d[3], t, lo, hi, Fin, uc);
+					s6[4].template issue<2>(gp.d[4], t, lo, hi, Fin, uc);
+					s6[5].template issue<2>(gp.d[5], t, lo, hi, Fin, uc);
 				}
-				continue;
+				cp_async_wait_all();
+				__syncthreads(); // metaS has landed
+				if (next) {
+#pragma unroll
+					for (int s = 0; s < 4; s++) Gs[s * 256 + t] = s6[s].finish(gp, s, meta, pn, t, Fin, uc);
+					gz0 = s6[4].finish(gp, 4, meta, pn, t, Fin, uc);
+					gz1 = s6[5].finish(gp, 5, meta, pn, t, Fin, uc);
+					if (gn + (int) gridDim.x < npatch) describe(*reinterpret_cast<const PatchMeta *>(metaS), pnn, b);
+				}
 			}
+			continue;
 		}
 		double v[N];
 		{ // z forward: pencil (x, y) = (lo, hi)
-			double *q = S + lo + hi * ROW;
-			if (DIRECT) {
-				const double *fp = f + (size_t) p * G::NC + t;
+			double *      q  = S + lo + hi * ROW;
+			const double *fp = f + (size_t) p * G::NC + t;
 #pragma unroll
-				for (int k = 0; k < N; k++) v[k] = __ldcs(fp + k * G::M);
-				if (next) { // pull the next patch into L2 while this one is transformed: 256 lines of 128 bytes
-					prefetch_l2(f + (size_t) pn * G::NC + t * 16);
-				}
-			} else {
-#pragma unroll
-				for (int k = 0; k < N; k++) v[k] = q[k * PL];
-			}
-			if (SRC_FINE) { // the level's later sweeps read f_c from memory
-				double *fo = src.fc_out + (size_t) p * G::NC + t;
-#pragma unroll
-				for (int k = 0; k < N; k++) fo[k * G::M] = v[k];
+			for (int k = 0; k < N; k++) v[k] = __ldcs(fp + k * G::M);
+			if (next) { // pull the next patch into L2 while this one is transformed: 256 lines of 128 bytes
+				prefetch_l2(f + (size_t) pn * G::NC + t * 16);
 			}
 			if (!ZERO_GUESS) {
 				v[0] -= gz0;
@@ -438,7 +283,7 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 			if (NEU) {
 				general_transform<N>(nt.mats, axis_kind(neu_p, 2).fwd, v, q, PL, mg);
 			} else {
-				dst2_forward<N>(v, mg);
+				Dst2<N, N>::run(v, mg);
 #pragma unroll
 				for (int k = 0; k < N; k++) q[k * PL] = v[k];
 			}
@@ -457,7 +302,7 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 			if (NEU) {
 				general_transform<N>(nt.mats, axis_kind(neu_p, 0).fwd, v, reinterpret_cast<double *>(rowp), 1, mg);
 			} else {
-				dst2_forward<N>(v, mg);
+				Dst2<N, N>::run(v, mg);
 #pragma unroll
 				for (int j = 0; j < N / 2; j++) rowp[j] = make_double2(v[2 * j], v[2 * j + 1]);
 			}
@@ -480,15 +325,8 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 #pragma unroll
 				for (int k = 0; k < N; k++) v[k] = (singular && k == 0) ? 0.0 : q[k * ROW] * scale / (__ldg(nt.lam + ky.lam * N + k) + rest);
 			} else {
-#if TGPU_S16_TRIDIAG
 				// z and x are diagonalised: what is left per (k_x, k_z) is a tridiagonal system along y
-				TriSolve<N>::forward(v, eig + t, h2 * (4.0 / (N * N)));
-#else
-				dst2_forward<N>(v, mg);
-				const double *er = eig + t; // eig[k_y * 256 + k_x + 16 k_z] (the table is symmetric in the axes)
-#pragma unroll
-				for (int k = 0; k < N; k++) v[k] *= h2 * __ldg(er + k * G::M);
-#endif
+				TriSolve<N>::forward(v, tri + t, h2 * (4.0 / (N * N)));
 			}
 			double gx0 = 0.0, gx1 = 0.0;
 			if (!ZERO_GUESS && next) {
@@ -498,11 +336,7 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 			if (NEU) {
 				general_transform<N>(nt.mats, axis_kind(neu_p, 1).inv, v, q, ROW, mg);
 			} else {
-#if TGPU_S16_TRIDIAG
-				TriSolve<N>::backward(v, eig + t);
-#else
-				dst3_inverse<N>(v, mg);
-#endif
+				TriSolve<N>::backward(v, tri + t);
 #pragma unroll
 				for (int k = 0; k < N; k++) q[k * ROW] = v[k];
 			}
@@ -527,7 +361,7 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 			if (NEU) {
 				general_transform<N>(nt.mats, axis_kind(neu_p, 0).inv, v, reinterpret_cast<double *>(rowp), 1, mg);
 			} else {
-				dst3_inverse<N>(v, mg);
+				Dst3<N, N>::run(v, mg);
 #pragma unroll
 				for (int j = 0; j < N / 2; j++) rowp[j] = make_double2(v[2 * j], v[2 * j + 1]);
 			}
@@ -544,7 +378,7 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 #pragma unroll
 				for (int k = 0; k < N; k++) v[k] = q[k * PL];
 			} else {
-				dst3_inverse<N>(v, mg);
+				Dst3<N, N>::run(v, mg);
 			}
 			double *up = u + (size_t) p * G::NC + t;
 			if (WRITE_U) {
@@ -553,23 +387,23 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 			}
 			if (EMIT) {
 				double *Fp       = Fout + (size_t) p * G::S * G::M;
-				st_keep_l2(&Fp[4 * G::M + t], v[0], l2keep);
-				st_keep_l2(&Fp[5 * G::M + t], v[N - 1], l2keep);
+				Fp[4 * G::M + t] = v[0];
+				Fp[5 * G::M + t] = v[N - 1];
 				if (lo == 0) {
 #pragma unroll
-					for (int k = 0; k < N; k++) st_keep_l2(&Fp[0 * G::M + k * N + hi], v[k], l2keep);
+					for (int k = 0; k < N; k++) Fp[0 * G::M + k * N + hi] = v[k];
 				}
 				if (lo == N - 1) {
 #pragma unroll
-					for (int k = 0; k < N; k++) st_keep_l2(&Fp[1 * G::M + k * N + hi], v[k], l2keep);
+					for (int k = 0; k < N; k++) Fp[1 * G::M + k * N + hi] = v[k];
 				}
 				if (hi == 0) {
 #pragma unroll
-					for (int k = 0; k < N; k++) st_keep_l2(&Fp[2 * G::M + k * N + lo], v[k], l2keep);
+					for (int k = 0; k < N; k++) Fp[2 * G::M + k * N + lo] = v[k];
 				}
 				if (hi == N - 1) {
 #pragma unroll
-					for (int k = 0; k < N; k++) st_keep_l2(&Fp[3 * G::M + k * N + lo], v[k], l2keep);
+					for (int k = 0; k < N; k++) Fp[3 * G::M + k * N + lo] = v[k];
 				}
 			}
 		} else {
@@ -597,24 +431,24 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 				const double *q = S + x + y * ROW;
 #pragma unroll
 				for (int k = 0; k < N; k++) v[k] = q[k * PL];
-				dst3_inverse<N>(v, mg);
-				st_keep_l2(&Fp[4 * G::M + x + N * y], v[0], l2keep);
-				st_keep_l2(&Fp[5 * G::M + x + N * y], v[N - 1], l2keep);
+				Dst3<N, N>::run(v, mg);
+				Fp[4 * G::M + x + N * y] = v[0];
+				Fp[5 * G::M + x + N * y] = v[N - 1];
 				if (x == 0) {
 #pragma unroll
-					for (int k = 0; k < N; k++) st_keep_l2(&Fp[0 * G::M + k * N + y], v[k], l2keep);
+					for (int k = 0; k < N; k++) Fp[0 * G::M + k * N + y] = v[k];
 				}
 				if (x == N - 1) {
 #pragma unroll
-					for (int k = 0; k < N; k++) st_keep_l2(&Fp[1 * G::M + k * N + y], v[k], l2keep);
+					for (int k = 0; k < N; k++) Fp[1 * G::M + k * N + y] = v[k];
 				}
 				if (y == 0) {
 #pragma unroll
-					for (int k = 0; k < N; k++) st_keep_l2(&Fp[2 * G::M + k * N + x], v[k], l2keep);
+					for (int k = 0; k < N; k++) Fp[2 * G::M + k * N + x] = v[k];
 				}
 				if (y == N - 1) {
 #pragma unroll
-					for (int k = 0; k < N; k++) st_keep_l2(&Fp[3 * G::M + k * N + x], v[k], l2keep);
+					for (int k = 0; k < N; k++) Fp[3 * G::M + k * N + x] = v[k];
 				}
 			} else {
 				const int     idx = t - 64, x = 1 + idx % 14, y = 1 + idx / 14;
@@ -625,8 +459,9 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 					E = fma(mg.sinq(j + 1), q[j * PL], E);
 					O = fma((j + 1 == N - 1) ? 0.5 : mg.sinq(j + 2), q[(j + 1) * PL], O);
 				}
-				st_keep_l2(&Fp[4 * G::M + x + N * y], E + O, l2keep);
-				st_keep_l2(&Fp[5 * G::M + x + N * y], E - O, l2keep);
+				double *fz = &Fp[4 * G::M + x + N * y]; // z faces: entry (x, y) on side 4, then on side 5
+				*fz        = E + O;
+				fz[G::M]   = E - O;
 			}
 		}
 		if (!ZERO_GUESS && next) {

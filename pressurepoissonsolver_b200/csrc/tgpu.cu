@@ -1,6 +1,6 @@
 // tgpu.cu - C-ABI implementation (include/tgpu.h) on top of the kernels in kernels.cuh.
 // Host-side structure: context (stream, scratch), hierarchy (device neighbour tables, per-level
-// work vectors and face buffers, eigenvalue table), vectors, cycle driver with CUDA-graph replay.
+// work vectors and face buffers, tridiagonal multiplier table), vectors, cycle driver with CUDA-graph replay.
 #include <algorithm>
 #include <dlfcn.h>
 #include <nccl.h>
@@ -203,7 +203,6 @@ struct LevelDev {
 	bool       has_neumann = false;
 	int32_t *  neu_list = nullptr;          // device: owned patches with Neumann domain sides, ascending (smooth3d16_kernel<.., NEU>)
 	std::vector<int32_t> neu_host;          // the same list on the host (sub-ranges are found by binary search)
-	int32_t *  children = nullptr; // [P][8] patches of the next finer level per octant ([1] == -2: [0] is the same patch there); null: incomplete
 	// peer-to-peer halo exchange: peers' face buffers and flags mapped with CUDA IPC (see setup_p2p)
 	bool       p2p = false;
 	int32_t *  send_peer = nullptr, *send_ridx = nullptr, *peer_rank = nullptr; // device: per send face / per peer
@@ -230,7 +229,6 @@ struct tgpu_hier {
 	tgpu_ctx *            ctx = nullptr;
 	int                   D = 0, N = 0;
 	std::vector<LevelDev> levels;
-	double *              eig = nullptr; // [N^D]
 	double *              scratch32 = nullptr; // smooth3d32n_kernel (32^3 levels with Neumann sides): one 256 KB block per CTA
 	double *              cycle_faces = nullptr; // boundary slices of the last cycle's result (level 0), if it was asked to emit them
 	double *              tri = nullptr; // [N/2 + 1][N^(D-1)] tridiagonal multipliers (TriSolve)
@@ -362,11 +360,11 @@ static bool supported_dn(int D, int N)
 	return (D == 2 && (N == 4 || N == 8 || N == 16 || N == 32)) || (D == 3 && (N == 4 || N == 8 || N == 16 || N == 32));
 }
 
-template <bool Z, bool E, bool PR, bool W, bool SF = false> static int set_smem_attr_3d16()
+template <bool Z, bool E, bool PR, bool W> static int set_smem_attr_3d16()
 {
-	CU(cudaFuncSetAttribute(smooth3d16_kernel<Z, E, PR, W, SF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smooth3d16_smem_bytes(Z, SF)));
-	if (!Z && !SF) CU(cudaFuncSetAttribute(smooth3d16_kernel<Z, E, PR, W, SF, !Z && !SF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smooth3d16_smem_bytes(Z, SF)));
-	if (!SF) CU(cudaFuncSetAttribute(smooth3d16_kernel<Z, E, PR, W, false, false, !SF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smooth3d16_smem_bytes(Z, SF)));
+	CU(cudaFuncSetAttribute(smooth3d16_kernel<Z, E, PR, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smooth3d16_smem_bytes()));
+	if (!Z) CU(cudaFuncSetAttribute(smooth3d16_kernel<Z, E, PR, W, !Z>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smooth3d16_smem_bytes()));
+	CU(cudaFuncSetAttribute(smooth3d16_kernel<Z, E, PR, W, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smooth3d16_smem_bytes()));
 	return TGPU_OK;
 }
 static int set_smem_attrs_3d16()
@@ -380,9 +378,6 @@ static int set_smem_attrs_3d16()
 	TRY((set_smem_attr_3d16<false, true, true, true>()));
 	TRY((set_smem_attr_3d16<false, false, true, true>()));
 	TRY((set_smem_attr_3d16<false, true, true, false>()));
-	TRY((set_smem_attr_3d16<true, true, false, true, true>()));
-	TRY((set_smem_attr_3d16<true, false, false, true, true>()));
-	TRY((set_smem_attr_3d16<true, true, false, false, true>()));
 	return TGPU_OK;
 }
 template <bool Z, bool E, bool PR, bool W> static int set_smem_attr_2d32()
@@ -421,8 +416,6 @@ static int setup_3d32(tgpu_hier *h)
 	TRY((set_smem_attr_3d32<false, true, true, true>()));
 	TRY((set_smem_attr_3d32<false, false, true, true>()));
 	TRY((set_smem_attr_3d32<false, true, true, false>()));
-	CU(cudaFuncSetAttribute(apply3d32_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply3d32_smem_bytes()));
-	CU(cudaFuncSetAttribute(apply3d32_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply3d32_smem_bytes()));
 	CU(cudaFuncSetAttribute(apply3d32_tma_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply3d32_tma_smem_bytes()));
 	CU(cudaFuncSetAttribute(apply3d32_tma_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply3d32_tma_smem_bytes()));
 	CU(cudaFuncSetAttribute(apply3d32_tma_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply3d32_tma_smem_bytes()));
@@ -444,9 +437,6 @@ template <int D, int N> static int set_smem_attrs()
 	CU(cudaFuncSetAttribute(smooth_kernel<D, N, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sb));
 	CU(cudaFuncSetAttribute(smooth_kernel<D, N, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sb));
 	if (D == 3 && N == 16) TRY(set_smem_attrs_3d16());
-	CU(cudaFuncSetAttribute(apply_kernel<D, N, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply_smem_bytes<D, N>()));
-	CU(cudaFuncSetAttribute(apply_kernel<D, N, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply_smem_bytes<D, N>()));
-	CU(cudaFuncSetAttribute(apply_kernel<D, N, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply_smem_bytes<D, N>()));
 	CU(cudaFuncSetAttribute(apply_tma_kernel<D, N, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply_tma_smem_bytes<D, N>()));
 	CU(cudaFuncSetAttribute(apply_tma_kernel<D, N, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply_tma_smem_bytes<D, N>()));
 	CU(cudaFuncSetAttribute(apply_tma_kernel<D, N, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply_tma_smem_bytes<D, N>()));
@@ -787,65 +777,27 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 		CU(cudaMalloc(&L.Fb, L.nface * sizeof(double)));
 		h->levels.push_back(L);
 	}
-	// child tables (3D): lets a coarse sweep assemble its right-hand side from the finer level's faces (smooth3d16.cuh)
-	if (D == 3)
-		for (int l = 0; l + 1 < nlevels; l++) {
-			const TgpuLevelDesc &d  = levels[l];
-			LevelDev &           Lf = h->levels[l], &Lc = h->levels[l + 1];
-			if (!d.parent_idx || !d.orth_on_parent) continue;
-			std::vector<int32_t> ch((size_t) Lc.P * 8, -1);
-			bool                 ok = true;
-			for (int p = 0; p < Lf.P && ok; p++) {
-				const int c = d.parent_idx[p], o = d.orth_on_parent[p];
-				if (c < 0 || c >= Lc.P) ok = false; // parent is not an owned patch of the coarser level
-				else if (o < 0) ch[(size_t) c * 8] = p, ch[(size_t) c * 8 + 1] = -2;
-				else ch[(size_t) c * 8 + o] = p;
-			}
-			for (int c = 0; c < Lc.P && ok; c++) {
-				if (ch[(size_t) c * 8 + 1] == -2) continue;
-				for (int o = 0; o < 8; o++)
-					if (ch[(size_t) c * 8 + o] < 0) ok = false;
-			}
-			if (ok) TRY(dev_upload(&Lc.children, ch.data(), ch.size()));
-		}
-	// eigenvalue table: (2/n)^D / sum_axes(-4 sin^2((k+1) pi / (2n)))  [the 1/h^2 factor is applied per patch]
+	// multipliers of the two-sided tridiagonal elimination along the axis that is not transformed, for every
+	// pencil of the other axes' transform indices (TriSolve, kernels.cuh): [n/2 + 1][n^(D-1)]
 	{
-		std::vector<double> lam(n), eig(NC);
-		for (int k = 0; k < n; k++) lam[k] = -4.0 * pow(sin((k + 1) * M_PI / (2 * n)), 2);
-		const double scale = pow(2.0 / n, D);
-		for (size_t i = 0; i < NC; i++) {
-			double sum = 0;
-			size_t r   = i;
-			for (int a = 0; a < D; a++) {
-				sum += lam[r % n];
-				r /= n;
-			}
-			// transposed layout [k_x][remaining axes]: the x-pencil threads read it coalesced
-			eig[(i % n) * M + i / n] = scale / sum;
+		const int                H = n / 2;
+		std::vector<double>      tri((size_t) (H + 1) * M);
+		std::vector<long double> ll(n);
+		for (int k = 0; k < n; k++) {
+			const long double sn = sinl((k + 1) * 3.141592653589793238462643383279502884L / (2 * n));
+			ll[k]                = -4.0L * sn * sn;
 		}
-		TRY(dev_upload(&h->eig, eig.data(), eig.size()));
-		// multipliers of the two-sided tridiagonal elimination along the axis that is not transformed, for every
-		// pencil of the other axes' transform indices (TriSolve, kernels.cuh): [n/2 + 1][n^(D-1)]
-		{
-			const int                H = n / 2;
-			std::vector<double>      tri((size_t) (H + 1) * M);
-			std::vector<long double> ll(n);
-			for (int k = 0; k < n; k++) {
-				const long double sn = sinl((k + 1) * 3.141592653589793238462643383279502884L / (2 * n));
-				ll[k]                = -4.0L * sn * sn;
+		for (size_t m = 0; m < M; m++) {
+			const long double mu = (D == 2) ? ll[m] : ll[m % n] + ll[m / n];
+			long double       a  = 0.0L;
+			for (int j = 0; j < H; j++) {
+				const long double d = mu - (j == 0 ? 3.0L : 2.0L);
+				a                   = 1.0L / (d - (j == 0 ? 0.0L : a));
+				tri[(size_t) j * M + m] = (double) a;
 			}
-			for (size_t m = 0; m < M; m++) {
-				const long double mu = (D == 2) ? ll[m] : ll[m % n] + ll[m / n];
-				long double       a  = 0.0L;
-				for (int j = 0; j < H; j++) {
-					const long double d = mu - (j == 0 ? 3.0L : 2.0L);
-					a                   = 1.0L / (d - (j == 0 ? 0.0L : a));
-					tri[(size_t) j * M + m] = (double) a;
-				}
-				tri[(size_t) H * M + m] = (double) (1.0L / (1.0L - a * a));
-			}
-			TRY(dev_upload(&h->tri, tri.data(), tri.size()));
+			tri[(size_t) H * M + m] = (double) (1.0L / (1.0L - a * a));
 		}
+		TRY(dev_upload(&h->tri, tri.data(), tri.size()));
 	}
 	// general transform path (patches with Neumann domain sides): the six matrices of DftPatchSolver.h:237-289,
 	// M[k][j] such that y_k = sum_j M[k][j] x_j, order TK_*; 1-D eigenvalues -4 sin^2((k + shift) pi / 2n), shift 1, 0, 1/2
@@ -1255,7 +1207,6 @@ extern "C" int tgpu_hierarchy_destroy(tgpu_hier *h)
 	for (LevelDev &L : h->levels) {
 		cudaFree(L.meta);
 		cudaFree(L.neu_list);
-		cudaFree(L.children);
 		cudaFree(L.starts);
 		cudaFree(L.spacing);
 		if (!L.p2p) { // otherwise they live in the arena
@@ -1290,7 +1241,6 @@ extern "C" int tgpu_hierarchy_destroy(tgpu_hier *h)
 	cudaFree(h->krylov_sc);
 	cudaFree(h->mats);
 	cudaFree(h->lam);
-	cudaFree(h->eig);
 	cudaFree(h->scratch32);
 	cudaFree(h->tri);
 	delete h;
@@ -1523,11 +1473,6 @@ static int check_level_vec(const tgpu_hier *h, int level, const tgpu_vec *v, con
 	if (v->h != h || v->level != level) return fail(TGPU_ERR_ARG, std::string(what) + ": vector does not live on this level");
 	return TGPU_OK;
 }
-static int need_smoother(const tgpu_hier *h, int level)
-{
-	(void) h, (void) level; // every (D, n, closure) combination has a kernel
-	return TGPU_OK;
-}
 
 // consumer side of the hand-over for kernels that poll the DATA flags themselves and acknowledge from their last CTA
 static bool halo_in_kernel(const tgpu_hier *h, int l)
@@ -1598,15 +1543,8 @@ static int k_extract_faces(tgpu_hier *h, int l, const double *u, double *F)
 	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, extract_faces_kernel<DD, NN>, dim3(grid_for(h->ctx, L.nface)), dim3(256), 0, L.P, u, F));
 }
 // mode 0: out = A u; 1: out = f - A u; 2: coarse = R (f - A u).  F must hold the faces of u.
-// mode 3 (TMA kernels only, see apply_tma_available): out = A u with the block partial sums of out . f and out . out written to
-// ctx->d_partial ([0..nb), [MAX_PARTIAL / 2 ..)); *nb_out = number of partials
-static bool apply_tma_available()
-{
-	// TGPU_APPLY_TMA=0: the tile is staged with per-element cp.async (LDGSTS) into a ghosted tile (apply_kernel /
-	// apply3d32_kernel) instead of one TMA bulk copy per patch group (apply_tma.cuh)
-	static const bool tma = !(getenv("TGPU_APPLY_TMA") && atoi(getenv("TGPU_APPLY_TMA")) == 0);
-	return tma;
-}
+// mode 3: out = A u with the block partial sums of out . f and out . out written to ctx->d_partial ([0..nb),
+// [MAX_PARTIAL / 2 ..)); *nb_out = number of partials
 static int k_apply(tgpu_hier *h, int l, int mode, const double *u, const double *f, const double *F, double *out, double *coarse,
                    int p0 = 0, int p1 = -1, int *nb_out = nullptr)
 {
@@ -1614,11 +1552,9 @@ static int k_apply(tgpu_hier *h, int l, int mode, const double *u, const double 
 	if (p1 < 0) p1 = L.P;
 	if (p1 <= p0) return TGPU_OK;
 	Tag       tg(h->ctx, mode == 0 ? "apply" : (mode == 1 ? "residual" : (mode == 2 ? "residual_restrict" : "apply_dots")), l);
-	const bool tma = apply_tma_available();
-	if (mode == 3 && !tma) return fail(TGPU_ERR_ARG, "k_apply: the fused dot products need the TMA kernels");
 	double *const  part    = h->ctx->d_partial;
 	constexpr int  pstride = MAX_PARTIAL / 2;
-	if (tma && is_3d32(h)) {
+	if (is_3d32(h)) {
 		if (mode == 2) {
 			if (p0 != 0 || p1 != L.P) return fail(TGPU_ERR_UNSUPPORTED, "residual+restrict on a patch range is not available for 32^3 patches");
 			TRY(launch(h->ctx, apply3d32_tma_kernel<1>, dim3(std::min((p1 - p0) * 4, h->ctx->sm_count * 2)), dim3(TGPU_THREADS), apply3d32_tma_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, u, f, F, L.r, part, pstride));
@@ -1630,87 +1566,73 @@ static int k_apply(tgpu_hier *h, int l, int mode, const double *u, const double 
 		if (mode == 3) return launch(h->ctx, apply3d32_tma_kernel<3>, grid, dim3(TGPU_THREADS), apply3d32_tma_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, u, f, F, out, part, pstride);
 		return launch(h->ctx, apply3d32_tma_kernel<1>, grid, dim3(TGPU_THREADS), apply3d32_tma_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, u, f, F, out, part, pstride);
 	}
-	if (tma && !is_3d32(h)) {
-		DISPATCH_DN(h->D, h->N, {
-			using G        = Geo<DD, NN>;
-			const int nblk = (p1 - p0 + G::PPB - 1) / G::PPB;
-			const int grid = std::min(nblk, h->ctx->sm_count * 2);
-			const size_t sm = apply_tma_smem_bytes<DD, NN>();
-			if (nb_out) *nb_out = grid;
-			if (mode == 0) return launch(h->ctx, apply_tma_kernel<DD, NN, 0>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse, part, pstride);
-			if (mode == 1) return launch(h->ctx, apply_tma_kernel<DD, NN, 1>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse, part, pstride);
-			if (mode == 3) return launch(h->ctx, apply_tma_kernel<DD, NN, 3>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse, part, pstride);
-			return launch(h->ctx, apply_tma_kernel<DD, NN, 2>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse, part, pstride);
-		});
-	}
-	if (is_3d32(h)) {
-		if (mode == 2) { // no fused form for 32^3 patches: residual into the level's work vector, then restrict
-			if (p0 != 0 || p1 != L.P) return fail(TGPU_ERR_UNSUPPORTED, "residual+restrict on a patch range is not available for 32^3 patches");
-			TRY(launch(h->ctx, apply3d32_kernel<1>, dim3(std::min((p1 - p0) * 4, h->ctx->sm_count * 2)), dim3(TGPU_THREADS), apply3d32_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, u, f, F, L.r));
-			return launch(h->ctx, restrict_kernel<3, 32>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta, L.P, (const double *) L.r, coarse);
-		}
-		const dim3 grid(std::min((p1 - p0) * 4, h->ctx->sm_count * 2));
-		if (mode == 0) return launch(h->ctx, apply3d32_kernel<0>, grid, dim3(TGPU_THREADS), apply3d32_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, u, f, F, out);
-		return launch(h->ctx, apply3d32_kernel<1>, grid, dim3(TGPU_THREADS), apply3d32_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, u, f, F, out);
-	}
 	DISPATCH_DN(h->D, h->N, {
 		using G        = Geo<DD, NN>;
 		const int nblk = (p1 - p0 + G::PPB - 1) / G::PPB;
 		const int grid = std::min(nblk, h->ctx->sm_count * 2);
-		const size_t sm = apply_smem_bytes<DD, NN>();
-		if (mode == 0) return launch(h->ctx, apply_kernel<DD, NN, 0>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse);
-		if (mode == 1) return launch(h->ctx, apply_kernel<DD, NN, 1>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse);
-		return launch(h->ctx, apply_kernel<DD, NN, 2>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse);
+		const size_t sm = apply_tma_smem_bytes<DD, NN>();
+		if (nb_out) *nb_out = grid;
+		if (mode == 0) return launch(h->ctx, apply_tma_kernel<DD, NN, 0>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse, part, pstride);
+		if (mode == 1) return launch(h->ctx, apply_tma_kernel<DD, NN, 1>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse, part, pstride);
+		if (mode == 3) return launch(h->ctx, apply_tma_kernel<DD, NN, 3>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse, part, pstride);
+		return launch(h->ctx, apply_tma_kernel<DD, NN, 2>, dim3(grid), dim3(TGPU_THREADS), sm, (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse, part, pstride);
 	});
+}
+// Calls fn(Z, E, PR, W) with std::integral_constant<bool, ...> arguments for the run-time variant of a sweep: Z = zero guess,
+// E = emit the faces, PR = fused prolongation, W = write u.  These are the nine variants the smoothers are instantiated for
+// (no prolongation into a sweep from a zero guess; a sweep that emits no faces writes u).
+template <class Fn> static int smooth_variant(bool zero_guess, bool emit, bool prolong, bool write_u, Fn &&fn)
+{
+	using T = std::true_type;
+	using F = std::false_type;
+	switch ((zero_guess ? 8 : 0) | (emit ? 4 : 0) | (prolong ? 2 : 0) | (write_u ? 1 : 0)) {
+	case 8 | 4 | 1: return fn(T{}, T{}, F{}, T{});
+	case 8 | 1: return fn(T{}, F{}, F{}, T{});
+	case 8 | 4: return fn(T{}, T{}, F{}, F{});
+	case 4 | 1: return fn(F{}, T{}, F{}, T{});
+	case 1: return fn(F{}, F{}, F{}, T{});
+	case 4: return fn(F{}, T{}, F{}, F{});
+	case 4 | 2 | 1: return fn(F{}, T{}, T{}, T{});
+	case 2 | 1: return fn(F{}, F{}, T{}, T{});
+	case 4 | 2: return fn(F{}, T{}, T{}, F{});
+	default: return fail(TGPU_ERR_ARG, "k_smooth: bad variant");
+	}
 }
 // zero_guess: gamma = 0 (Fin unused); emit: write the faces of the new u to Fout;
 // uc != nullptr: face values are Fin + (P uc) on the boundary cells (fused prolongation);
 // write_u = false (needs emit): only the faces of the new u are wanted (the generic kernel still writes u)
 // neu: the instantiation for the patches with Neumann domain sides (it sweeps exactly those of the range)
-template <bool Z, bool E, bool PR, bool W, bool SF = false>
+template <bool Z, bool E, bool PR, bool W>
 static int launch_smooth3d16(tgpu_hier *h, const LevelDev &L, int p0, int p1, const double *f, double *u, const double *Fin, double *Fout,
-                             const double *uc, FineSrc16 src = FineSrc16{}, HaloSync hs = HaloSync{}, int skip_neumann = 0, bool neu = false)
+                             const double *uc, HaloSync hs = HaloSync{}, int skip_neumann = 0, bool neu = false)
 {
 	if (neu) {
-		if (SF || hs.enabled) return fail(TGPU_ERR_ARG, "smooth3d16: the Neumann instantiation is single-GPU, right-hand side from memory");
+		if (hs.enabled) return fail(TGPU_ERR_ARG, "smooth3d16: the Neumann instantiation is single-GPU");
 		// the patches of [p0, p1) with Neumann sides: a contiguous piece of the level's (ascending) list
 		const auto b0 = std::lower_bound(L.neu_host.begin(), L.neu_host.end(), p0), b1 = std::lower_bound(L.neu_host.begin(), L.neu_host.end(), p1);
 		const int  nn = (int) (b1 - b0);
 		if (nn == 0) return TGPU_OK;
-		const dim3 gridn(std::min(nn, h->ctx->sm_count * s16_ctas_per_sm(Z, false, true))), blockn(S16_BLOCK);
-		return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W, false, false, !SF>, gridn, blockn, smooth3d16_smem_bytes(Z, false), (const PatchMeta *) L.meta, p0,
-		              p1, f, u, Fin, Fout, (const double *) (TGPU_S16_TRIDIAG ? h->tri : h->eig), uc, FineSrc16{}, HaloSync{}, 0,
-		              NeuTabs{h->mats, h->lam, L.neu_list + (b0 - L.neu_host.begin()), nn});
+		const dim3 gridn(std::min(nn, h->ctx->sm_count * s16_ctas_per_sm(Z, true))), blockn(S16_BLOCK);
+		return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W, false, true>, gridn, blockn, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta, p0,
+		              p1, f, u, Fin, Fout, (const double *) h->tri, uc, HaloSync{}, 0, NeuTabs{h->mats, h->lam, L.neu_list + (b0 - L.neu_host.begin()), nn});
 	}
-	const dim3 grid(std::min(p1 - p0, h->ctx->sm_count * s16_ctas_per_sm(Z, SF))), block(S16_BLOCK);
+	const dim3 grid(std::min(p1 - p0, h->ctx->sm_count * s16_ctas_per_sm(Z))), block(S16_BLOCK);
 	if (hs.enabled) {
-		if (Z || SF) return fail(TGPU_ERR_ARG, "smooth3d16: no halo hand-over in a zero-guess sweep");
-		return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W, SF, !Z && !SF>, grid, block, smooth3d16_smem_bytes(Z, SF), (const PatchMeta *) L.meta, p0, p1, f, u,
-		              Fin, Fout, (const double *) (TGPU_S16_TRIDIAG ? h->tri : h->eig), uc, src, hs, skip_neumann, NeuTabs{});
+		if (Z) return fail(TGPU_ERR_ARG, "smooth3d16: no halo hand-over in a zero-guess sweep");
+		return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W, !Z>, grid, block, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, f, u,
+		              Fin, Fout, (const double *) h->tri, uc, hs, skip_neumann, NeuTabs{});
 	}
-	return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W, SF>, grid, block, smooth3d16_smem_bytes(Z, SF), (const PatchMeta *) L.meta, p0, p1, f, u, Fin,
-	              Fout, (const double *) (TGPU_S16_TRIDIAG ? h->tri : h->eig), uc, src, hs, skip_neumann, NeuTabs{});
-}
-// can the first (zero-guess) sweep on level lc assemble its right-hand side from level lc - 1's faces?
-// Opt-in (TGPU_FINE_SOURCE=1): measured on config B the assembly stage's dependent gathers (children -> neighbour
-// table -> faces, per axis) cost as much per patch as the separate face_residual_restrict launch they replace
-// (0.306 vs 0.279 ms per cycle), so the three-launch schedule stays the default.
-static bool can_source_from_fine(const tgpu_hier *h, int lc)
-{
-	static const bool enabled = getenv("TGPU_FINE_SOURCE") && atoi(getenv("TGPU_FINE_SOURCE")) != 0;
-	return enabled && lc >= 1 && h->D == 3 && h->N == 16 && !h->generic_kernels && h->ctx->nranks == 1 && h->levels[lc].children
-	       && !h->levels[lc].has_neumann;
+	return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W>, grid, block, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, f, u, Fin,
+	              Fout, (const double *) h->tri, uc, hs, skip_neumann, NeuTabs{});
 }
 // hsp != nullptr (multi-GPU, kernels that support it: halo_in_kernel): the launch covers interior and boundary patches and
 // does the halo hand-over itself
 static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const double *f, double *u, const double *Fin, double *Fout,
-                    const double *uc = nullptr, int p0 = 0, int p1 = -1, bool write_u = true, const double *fine_faces = nullptr,
-                    const HaloSync *hsp = nullptr)
+                    const double *uc = nullptr, int p0 = 0, int p1 = -1, bool write_u = true, const HaloSync *hsp = nullptr)
 {
 	const HaloSync hs = hsp ? *hsp : HaloSync{};
 	if (hsp && !halo_in_kernel(h, l)) return fail(TGPU_ERR_ARG, "k_smooth: in-kernel halo hand-over is not available for this level");
 	LevelDev &L = h->levels[l];
-	TRY(need_smoother(h, l));
 	if (p1 < 0) p1 = L.P;
 	if (p1 <= p0) return hs.push ? fail(TGPU_ERR_ARG, "k_smooth: a launch that pushes faces needs patches") : TGPU_OK;
 	if (!emit) write_u = true;
@@ -1722,6 +1644,21 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 	Tag tg(h->ctx, zero_guess ? (write_u ? "smooth_zero_guess" : "smooth_zero_guess_faces")
 	                          : (uc ? (write_u ? "smooth_prolong" : "smooth_prolong_faces") : (write_u ? "smooth" : "smooth_faces")),
 	       l);
+	const bool prolong = uc != nullptr;
+	const PatchMeta *meta = L.meta;
+	// smooth_kernel<DD, NN> (size-generic, the path with the general patch solve); only_neumann: sweep only the patches with
+	// Neumann domain sides of the range
+	auto generic_smooth = [&](auto dd, auto nn, int only_neumann) {
+		constexpr int DD = decltype(dd)::value, NN = decltype(nn)::value;
+		using G          = Geo<DD, NN>;
+		const int    nblk = (p1 - p0 + G::PPB - 1) / G::PPB;
+		const dim3   grid(std::min(nblk, h->ctx->sm_count * smooth_min_blocks<NN>())), block(TGPU_THREADS);
+		const size_t sm = smooth_smem_bytes<DD, NN, true>();
+		return smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto) {
+			return launch(h->ctx, smooth_kernel<DD, NN, Z, E, PR>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri, uc,
+			              (const double *) h->mats, (const double *) h->lam, h->lambda, only_neumann);
+		});
+	};
 	const bool general = L.has_neumann || h->lambda != 0.0; // patch solves that are not the plain Dirichlet Poisson solve
 	// 32^3 levels that contain patches with Neumann domain sides: the cluster kernel sweeps the Dirichlet patches of the range,
 	// the general path (smooth3d32n_kernel) exactly the others; lambda != 0 sends every patch through the general path
@@ -1738,135 +1675,45 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 	if (is_3d32(h)) {
 		// one cluster of two CTAs (two SMs) per patch, see smooth3d32c_kernel
 		const dim3   grid(2 * std::min(p1 - p0, h->ctx->sm_count / 2)), block(C32_THREADS);
-		const size_t sm  = smooth3d32c_smem_bytes();
-		const int    key = (zero_guess ? 8 : 0) | (emit ? 4 : 0) | (uc ? 2 : 0) | (write_u ? 1 : 0);
+		const size_t sm    = smooth3d32c_smem_bytes();
 		const int    skipn = mixed32 ? 1 : 0;
-#define S32_CASE(K, Z, E, PR, W) \
-	case K: return launch(h->ctx, smooth3d32c_kernel<Z, E, PR, W, !Z>, grid, block, sm, (const PatchMeta *) L.meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri, uc, hs, skipn);
-		switch (key) {
-			S32_CASE(8 | 4 | 1, true, true, false, true)
-			S32_CASE(8 | 1, true, false, false, true)
-			S32_CASE(8 | 4, true, true, false, false)
-			S32_CASE(4 | 1, false, true, false, true)
-			S32_CASE(1, false, false, false, true)
-			S32_CASE(4, false, true, false, false)
-			S32_CASE(4 | 2 | 1, false, true, true, true)
-			S32_CASE(2 | 1, false, false, true, true)
-			S32_CASE(4 | 2, false, true, true, false)
-		default: return fail(TGPU_ERR_ARG, "k_smooth: bad variant");
-		}
-#undef S32_CASE
-	}
-	if (fine_faces) { // right-hand side assembled from the finer level's faces and stored to f (see can_source_from_fine)
-		if (!zero_guess || !can_source_from_fine(h, l)) return fail(TGPU_ERR_ARG, "k_smooth: fine-face source not available");
-		Tag       tg2(h->ctx, write_u ? "smooth_zero_guess_from_fine" : "smooth_zero_guess_faces_from_fine", l);
-		FineSrc16 src{h->levels[l - 1].meta, fine_faces, L.children, const_cast<double *>(f)};
-		if (emit && write_u) return launch_smooth3d16<true, true, false, true, true>(h, L, p0, p1, f, u, Fin, Fout, uc, src);
-		if (emit) return launch_smooth3d16<true, true, false, false, true>(h, L, p0, p1, f, u, Fin, Fout, uc, src);
-		return launch_smooth3d16<true, false, false, true, true>(h, L, p0, p1, f, u, Fin, Fout, uc, src);
+		return smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto W) {
+			return launch(h->ctx, smooth3d32c_kernel<Z, E, PR, W, !Z>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri, uc, hs, skipn);
+		});
 	}
 	// 16^3 levels that contain patches with Neumann domain sides: the specialised kernel sweeps the Dirichlet patches of the
 	// range and skips the others, the general path of smooth_kernel then sweeps exactly those (two launches, disjoint patches)
 	const bool mixed16 = h->D == 3 && h->N == 16 && !h->generic_kernels && L.has_neumann && h->lambda == 0.0 && !hsp && split;
 	if (h->D == 3 && h->N == 16 && !h->generic_kernels && (!general || mixed16)) { // the generic kernel has the Neumann path
-		const int key = (zero_guess ? 8 : 0) | (emit ? 4 : 0) | (uc ? 2 : 0) | (write_u ? 1 : 0);
 		const int skipn = mixed16 ? 1 : 0;
 		// the Neumann instantiation of the same kernel first, then the plain one on the rest (TGPU_NEUMANN_FAST=0: smooth_kernel's
 		// general path instead, which always writes u)
 		static const bool neu_fast = !(getenv("TGPU_NEUMANN_FAST") && atoi(getenv("TGPU_NEUMANN_FAST")) == 0);
 		if (mixed16 && neu_fast) {
-			switch (key) {
-			case 8 | 4 | 1: TRY((launch_smooth3d16<true, true, false, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, HaloSync{}, 0, true))); break;
-			case 8 | 1: TRY((launch_smooth3d16<true, false, false, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, HaloSync{}, 0, true))); break;
-			case 8 | 4: TRY((launch_smooth3d16<true, true, false, false>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, HaloSync{}, 0, true))); break;
-			case 4 | 1: TRY((launch_smooth3d16<false, true, false, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, HaloSync{}, 0, true))); break;
-			case 1: TRY((launch_smooth3d16<false, false, false, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, HaloSync{}, 0, true))); break;
-			case 4: TRY((launch_smooth3d16<false, true, false, false>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, HaloSync{}, 0, true))); break;
-			case 4 | 2 | 1: TRY((launch_smooth3d16<false, true, true, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, HaloSync{}, 0, true))); break;
-			case 2 | 1: TRY((launch_smooth3d16<false, false, true, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, HaloSync{}, 0, true))); break;
-			case 4 | 2: TRY((launch_smooth3d16<false, true, true, false>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, HaloSync{}, 0, true))); break;
-			default: return fail(TGPU_ERR_ARG, "k_smooth: bad variant");
-			}
+			TRY(smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto W) {
+				return launch_smooth3d16<Z, E, PR, W>(h, L, p0, p1, f, u, Fin, Fout, uc, HaloSync{}, 0, true);
+			}));
 		} else if (mixed16) {
-			using G        = Geo<3, 16>;
-			const dim3 grid(std::min(p1 - p0, h->ctx->sm_count * smooth_min_blocks<16>())), block(TGPU_THREADS);
-			const size_t sm = smooth_smem_bytes<3, 16, true>();
-			const PatchMeta *meta = L.meta;
-			const double *   eig  = TGPU_S16_TRIDIAG ? h->tri : h->eig;
-			(void) sizeof(G);
-			if (zero_guess && emit) TRY(launch(h->ctx, smooth_kernel<3, 16, true, true, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-			else if (zero_guess) TRY(launch(h->ctx, smooth_kernel<3, 16, true, false, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-			else if (uc && emit) TRY(launch(h->ctx, smooth_kernel<3, 16, false, true, true>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-			else if (uc) TRY(launch(h->ctx, smooth_kernel<3, 16, false, false, true>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-			else if (emit) TRY(launch(h->ctx, smooth_kernel<3, 16, false, true, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-			else TRY(launch(h->ctx, smooth_kernel<3, 16, false, false, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
+			TRY(generic_smooth(std::integral_constant<int, 3>{}, std::integral_constant<int, 16>{}, 1));
 		}
-		switch (key) {
-		case 8 | 4 | 1: return launch_smooth3d16<true, true, false, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, hs, skipn);
-		case 8 | 1: return launch_smooth3d16<true, false, false, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, hs, skipn);
-		case 8 | 4: return launch_smooth3d16<true, true, false, false>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, hs, skipn);
-		case 4 | 1: return launch_smooth3d16<false, true, false, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, hs, skipn);
-		case 1: return launch_smooth3d16<false, false, false, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, hs, skipn);
-		case 4: return launch_smooth3d16<false, true, false, false>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, hs, skipn);
-		case 4 | 2 | 1: return launch_smooth3d16<false, true, true, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, hs, skipn);
-		case 2 | 1: return launch_smooth3d16<false, false, true, true>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, hs, skipn);
-		case 4 | 2: return launch_smooth3d16<false, true, true, false>(h, L, p0, p1, f, u, Fin, Fout, uc, FineSrc16{}, hs, skipn);
-		default: return fail(TGPU_ERR_ARG, "k_smooth: bad variant");
-		}
+		return smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto W) {
+			return launch_smooth3d16<Z, E, PR, W>(h, L, p0, p1, f, u, Fin, Fout, uc, hs, skipn);
+		});
 	}
 	const bool mixed2d = h->D == 2 && h->N == 32 && !h->generic_kernels && L.has_neumann && h->lambda == 0.0 && !hsp && split;
-	if (mixed2d) { // the general path on the patches with Neumann sides (it always writes u), then the warp-per-patch kernel on the rest
-		using G        = Geo<2, 32>;
-		const int nblk = (p1 - p0 + G::PPB - 1) / G::PPB;
-		const dim3 grid(std::min(nblk, h->ctx->sm_count * smooth_min_blocks<32>())), block(TGPU_THREADS);
-		const size_t sm = smooth_smem_bytes<2, 32, true>();
-		const PatchMeta *meta = L.meta;
-		const double *   eig  = TGPU_S16_TRIDIAG ? h->tri : h->eig;
-		if (zero_guess && emit) TRY(launch(h->ctx, smooth_kernel<2, 32, true, true, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-		else if (zero_guess) TRY(launch(h->ctx, smooth_kernel<2, 32, true, false, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-		else if (uc && emit) TRY(launch(h->ctx, smooth_kernel<2, 32, false, true, true>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-		else if (uc) TRY(launch(h->ctx, smooth_kernel<2, 32, false, false, true>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-		else if (emit) TRY(launch(h->ctx, smooth_kernel<2, 32, false, true, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-		else TRY(launch(h->ctx, smooth_kernel<2, 32, false, false, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 1));
-	}
+	if (mixed2d) // the general path on the patches with Neumann sides (it always writes u), then the warp-per-patch kernel on the rest
+		TRY(generic_smooth(std::integral_constant<int, 2>{}, std::integral_constant<int, 32>{}, 1));
 	if (h->D == 2 && h->N == 32 && !h->generic_kernels && (!general || mixed2d)) { // one warp per patch, see smooth2d32.cuh
 		const int    nblk = (p1 - p0 + Q32_WARPS - 1) / Q32_WARPS;
 		const dim3   grid(std::min(nblk, h->ctx->sm_count * 2)), block(TGPU_THREADS);
-		const size_t sm  = smooth2d32_smem_bytes();
-		const int    key = (zero_guess ? 8 : 0) | (emit ? 4 : 0) | (uc ? 2 : 0) | (write_u ? 1 : 0);
+		const size_t sm    = smooth2d32_smem_bytes();
 		const int    skipn = mixed2d ? 1 : 0;
-#define Q32_CASE(K, Z, E, PR, W) \
-	case K: \
-		if (skipn || hs.enabled) return launch(h->ctx, smooth2d32_kernel<Z, E, PR, W, true>, grid, block, sm, (const PatchMeta *) L.meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri, uc, hs, skipn); \
-		return launch(h->ctx, smooth2d32_kernel<Z, E, PR, W, false>, grid, block, sm, (const PatchMeta *) L.meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri, uc, hs, skipn);
-		switch (key) {
-			Q32_CASE(8 | 4 | 1, true, true, false, true)
-			Q32_CASE(8 | 1, true, false, false, true)
-			Q32_CASE(8 | 4, true, true, false, false)
-			Q32_CASE(4 | 1, false, true, false, true)
-			Q32_CASE(1, false, false, false, true)
-			Q32_CASE(4, false, true, false, false)
-			Q32_CASE(4 | 2 | 1, false, true, true, true)
-			Q32_CASE(2 | 1, false, false, true, true)
-			Q32_CASE(4 | 2, false, true, true, false)
-		default: return fail(TGPU_ERR_ARG, "k_smooth: bad variant");
-		}
-#undef Q32_CASE
+		return smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto W) {
+			if (skipn || hs.enabled) return launch(h->ctx, smooth2d32_kernel<Z, E, PR, W, true>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri, uc, hs, skipn);
+			return launch(h->ctx, smooth2d32_kernel<Z, E, PR, W, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri, uc, hs, skipn);
+		});
 	}
-	DISPATCH_DN(h->D, h->N, {
-		using G        = Geo<DD, NN>;
-		const int nblk = (p1 - p0 + G::PPB - 1) / G::PPB;
-		const dim3 grid(std::min(nblk, h->ctx->sm_count * smooth_min_blocks<NN>())), block(TGPU_THREADS);
-		const size_t sm = smooth_smem_bytes<DD, NN, true>();
-		const PatchMeta *meta = L.meta;
-		const double *   eig  = TGPU_S16_TRIDIAG ? h->tri : h->eig;
-		if (zero_guess && emit) return launch(h->ctx, smooth_kernel<DD, NN, true, true, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 0);
-		if (zero_guess && !emit) return launch(h->ctx, smooth_kernel<DD, NN, true, false, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 0);
-		if (uc && emit) return launch(h->ctx, smooth_kernel<DD, NN, false, true, true>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 0);
-		if (uc && !emit) return launch(h->ctx, smooth_kernel<DD, NN, false, false, true>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 0);
-		if (emit) return launch(h->ctx, smooth_kernel<DD, NN, false, true, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 0);
-		return launch(h->ctx, smooth_kernel<DD, NN, false, false, false>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, eig, uc, (const double *) h->mats, (const double *) h->lam, h->lambda, 0);
-	});
+	DISPATCH_DN(h->D, h->N, return generic_smooth(std::integral_constant<int, DD>{}, std::integral_constant<int, NN>{}, 0));
 }
 // coarse = R (f - A u) for a u that a block-Jacobi sweep has just produced: needs only the faces of the new
 // (Fnew) and, unless the sweep started from zero (Fold == nullptr), the previous (Fold) iterate
@@ -2244,10 +2091,8 @@ static int exchange_async(tgpu_hier *h, int l, double *F, const double *uc, cuda
 // (see face_residual_restrict_kernel).  So, compared with the generic schedule, the dead stores are never
 // materialised: the zero fill of u, the pre-smoothed u itself, the fine residual vector and the interior
 // of the prolonged u; only the last sweep of a level visit writes u.  opts.fused = 2 keeps the PR-1 form
-// of the middle step (residual evaluated from u and f by apply_kernel<2>) for cross-checking.
-// fine_faces != nullptr: f has not been computed; the level's first sweep assembles it from the finer level's faces
-static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double *f, double *u, bool want_faces,
-                       const double *fine_faces = nullptr)
+// of the middle step (residual evaluated from u and f by apply_tma_kernel<2>) for cross-checking.
+static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double *f, double *u, bool want_faces)
 {
 	const int last = h->last_level;
 	LevelDev &L    = h->levels[l];
@@ -2256,7 +2101,7 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 		for (int i = 0; i < o.coarse_sweeps; i++) {
 			const bool emit = (i + 1 < o.coarse_sweeps);
 			if (i > 0) TRY(k_exchange(h, l, Fcur, nullptr));
-			TRY(k_smooth(h, l, i == 0, emit, f, u, Fcur, i == 0 ? Fcur : Falt, nullptr, 0, -1, !emit, i == 0 ? fine_faces : nullptr));
+			TRY(k_smooth(h, l, i == 0, emit, f, u, Fcur, i == 0 ? Fcur : Falt, nullptr, 0, -1, !emit));
 			if (i > 0) TRY(k_exchange_done(h, l));
 			if (i > 0 && emit) std::swap(Fcur, Falt);
 		}
@@ -2266,7 +2111,7 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 	LevelDev & C          = h->levels[l + 1];
 	for (int i = 0; i < o.pre_sweeps; i++) {
 		if (i > 0) TRY(k_exchange(h, l, Fcur, nullptr));
-		TRY(k_smooth(h, l, i == 0, true, f, u, Fcur, i == 0 ? Fcur : Falt, nullptr, 0, -1, !from_faces, i == 0 ? fine_faces : nullptr));
+		TRY(k_smooth(h, l, i == 0, true, f, u, Fcur, i == 0 ? Fcur : Falt, nullptr, 0, -1, !from_faces));
 		if (i > 0) TRY(k_exchange_done(h, l));
 		if (i > 0) std::swap(Fcur, Falt);
 	}
@@ -2277,11 +2122,6 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 		if (from_faces) return k_face_residual_restrict(h, l, Fcur, Fold, C.f, p0, p1);
 		return k_apply(h, l, 2, u, f, Fcur, nullptr, C.f, p0, p1);
 	};
-	// residual + restriction fused into the coarser level's first sweep where that kernel exists
-	const bool defer = from_faces && !Fold && o.cycle_type == 0 && can_source_from_fine(h, l + 1);
-	if (defer) {
-		TRY(fused_visit(h, o, l + 1, C.f, C.u, false, Fcur));
-	} else {
 	if (crosses_replication(h, l)) TRY(k_set(h, C.f, C.ncells, 0.0));
 	if (overlap && L.p2p && from_faces && halo_in_kernel(h, l)) {
 		// the faces of the pre-smoothed u go straight into the neighbours' halo slots; theirs arrive while the patches
@@ -2308,7 +2148,6 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 	}
 	if (crosses_replication(h, l)) TRY(k_allreduce_sum(h, C.f, C.ncells));
 	TRY(fused_visit(h, o, l + 1, C.f, C.u, false));
-	}
 	if (o.cycle_type == 1) {
 		// W cycle (GMG/WCycle.h:57-63; one GPU, mid_sweeps >= 1): the second coarse-grid correction.  The iterate before the
 		// mid sweeps is u_pre + P u_c, seen only through its boundary slices: Fcur += (P u_c) on the boundary cells; every
@@ -2335,7 +2174,7 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 		if (i > 0) TRY(k_exchange(h, l, Fcur, nullptr));
 		if (i == 0 && overlap && L.p2p && halo_in_kernel(h, l)) {
 			const HaloSync hs = halo_sync(h, l, push_folded ? Fcur : nullptr, true);
-			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, C.u, 0, L.P, lastsweep, nullptr, &hs));
+			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, C.u, 0, L.P, lastsweep, &hs));
 		} else if (i == 0 && overlap) {
 			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, C.u, 0, L.n_interior, lastsweep));
 			if (L.p2p) TRY(p2p_wait(h, l, P2P_DATA, 0));
@@ -2392,7 +2231,6 @@ static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, d
 		h->last_level = l;
 	}
 	for (size_t l = 0; l <= (size_t) h->last_level; l++) {
-		TRY(need_smoother(h, (int) l));
 		const bool fused_sched = fused_schedule(o, ctx->nranks);
 		TRY(ensure_work(h, (int) l, !fused_sched || (o.fused == 2 && is_3d32(h))));
 	}
@@ -2560,21 +2398,15 @@ static int bicgstab_fused(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_ve
 	// the preconditioner's last sweep emits the boundary slices of its result, which is all A needs besides the result
 	auto M = [&](const tgpu_vec *in, tgpu_vec *out) { return cycle_ptr(h, opts, in->d, out->d, true); };
 	// out = A in for in = the vector M has just produced (its boundary slices are in h->cycle_faces), with the dot products the
-	// iteration needs next (out . dotv, out . out) formed by the same kernel where it can: *fused tells whether it did
-	auto AM = [&](const tgpu_vec *in, tgpu_vec *out, const tgpu_vec *dotv, int *nbp, bool *fused) {
-		*fused = false;
+	// iteration needs next (out . dotv, out . out) formed by the same kernel: *nbp block partials in ctx->d_partial
+	auto AM = [&](const tgpu_vec *in, tgpu_vec *out, const tgpu_vec *dotv, int *nbp) {
 		double *F = h->cycle_faces;
 		if (!F) {
 			F = h->levels[0].Fa;
 			TRY(k_extract_faces(h, 0, in->d, F));
 		}
 		TRY(k_exchange(h, 0, F, nullptr));
-		if (apply_tma_available()) {
-			TRY(k_apply(h, 0, 3, in->d, dotv->d, F, out->d, nullptr, 0, -1, nbp));
-			*fused = true;
-		} else {
-			TRY(k_apply(h, 0, 0, in->d, nullptr, F, out->d, nullptr));
-		}
+		TRY(k_apply(h, 0, 3, in->d, dotv->d, F, out->d, nullptr, 0, -1, nbp));
 		return k_exchange_done(h, 0);
 	};
 	auto finish = [&](int step, int nparts) {
@@ -2608,31 +2440,29 @@ static int bicgstab_fused(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_ve
 	int its = 0;
 	while (rn / r0_norm > tol && its < max_it) {
 		const tgpu_vec *pp = p, *ss = s;
-		bool fused_dots = false;
-		int  nparts     = nb;
+		int             nparts = nb;
 		if (prec) {
 			TRY(M(p, mp));
 			pp = mp;
-			TRY(AM(pp, ap, rhat, &nparts, &fused_dots)); // ap = A mp, ap . rhat riding along
+			TRY(AM(pp, ap, rhat, &nparts)); // ap = A mp, ap . rhat riding along
+			TRY(finish(1, nparts));         // alpha
 		} else {
 			TRY(A(pp, ap));
+			TRY(dots(rhat, ap, 1)); // alpha
 		}
-		if (fused_dots) TRY(finish(1, nparts));
-		else TRY(dots(rhat, ap, 1)); // alpha
 		{
 			Tag tg(ctx, "bicg_s", 0);
 			TRY(launch(ctx, bicg_s_kernel, dim3(grid_for(ctx, n)), dim3(256), 0, n, (const double *) resid->d, (const double *) ap->d, s->d, (const double *) sc));
 		}
-		fused_dots = false;
 		if (prec) {
 			TRY(M(s, ms));
 			ss = ms;
-			TRY(AM(ss, as, s, &nparts, &fused_dots)); // as = A ms, as . s and as . as riding along
+			TRY(AM(ss, as, s, &nparts)); // as = A ms, as . s and as . as riding along
+			TRY(finish(2, nparts));      // omega
 		} else {
 			TRY(A(ss, as));
+			TRY(dots(as, s, 2)); // omega
 		}
-		if (fused_dots) TRY(finish(2, nparts));
-		else TRY(dots(as, s, 2)); // omega
 		{
 			Tag tg(ctx, "bicg_xr", 0);
 			TRY(launch(ctx, bicg_xr_kernel, dim3(nb), dim3(256), 0, n, x->d, (const double *) pp->d, (const double *) ss->d, resid->d, (const double *) ap->d, (const double *) as->d, (const double *) rhat->d, (const double *) sc, ctx->d_partial, stride));

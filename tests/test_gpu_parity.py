@@ -363,34 +363,6 @@ def test_neumann_alternative_paths(switch):
     assert out.returncode == 0 and out.stdout.startswith("ok"), out.stdout + out.stderr
 
 
-def test_coarse_rhs_from_fine_faces_variant():
-    """TGPU_FINE_SOURCE=1 (opt-in schedule: the coarse level's first sweep assembles its right-hand side from the
-    finer level's faces) must give the default schedule's result; run in a fresh process because the switch is
-    read once."""
-    code = (
-        "import os, sys, numpy as np\n"
-        "sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
-        "import pressurepoissonsolver_b200 as pps, gmg_oracle as go\n"
-        "ctx = pps.Context(0)\n"
-        "for mesh_file, divide in (('3uni.bin', 0), ('2refine.bin', 1), ('multi_refine.bin', 0)):\n"
-        "    path = os.path.join(%r, mesh_file)\n"
-        "    mesh = pps.Mesh.load(path, 3).refine_leaves(divide)\n"
-        "    h = pps.Hierarchy.from_mesh(ctx, mesh, 16)\n"
-        "    levels = go.build_hierarchy(path, 3, 16, divide)\n"
-        "    fn = np.random.default_rng(3).standard_normal(levels[0].shape)\n"
-        "    f, u = h.new_vec(0, fn), h.new_vec(0)\n"
-        "    for graph in (0, 1):\n"
-        "        h.vcycle(f, u, pps.CycleOpts.default(use_graph=graph))\n"
-        "        ref = go.vcycle(levels, fn)\n"
-        "        err = np.linalg.norm(u.download() - ref.ravel()) / np.linalg.norm(ref)\n"
-        "        assert err < 1e-12, (mesh_file, graph, err)\n"
-        "print('ok', ctx.kernel_launches())\n"
-    ) % (ROOT, os.path.join(ROOT, "oracle"), MESHES)
-    env = dict(os.environ, TGPU_FINE_SOURCE="1")
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0 and out.stdout.startswith("ok"), out.stdout + out.stderr
-
-
 def test_blas1_and_reductions(ctx):
     h, mesh = build(ctx, "2refine.bin", 3, 8, 1)
     rng = np.random.default_rng(7)

@@ -1,6 +1,6 @@
-// tools/smooth32_bench.cu - stand-alone check + timing harness for the D = 3, n = 32 smoothers (development aid,
-// not part of the product): cluster-pair kernel (smooth3d32c_kernel) against the slab kernel (smooth3d32_kernel)
-// on a uniform G^3 grid of patches with parents on a (G/2)^3 grid and random data.
+// tools/smooth32_bench.cu - stand-alone timing harness for the D = 3, n = 32 smoother (development aid, not part of the
+// product): the cluster-pair kernel (smooth3d32c_kernel) on a uniform G^3 grid of patches with parents on a (G/2)^3
+// grid and random data.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -I pressurepoissonsolver_b200/csrc \
 //        tools/smooth32_bench.cu -o tools/smooth32_bench && tools/smooth32_bench [G=8] [reps=10]
 #include <cstdio>
@@ -60,15 +60,6 @@ template <typename F> static float time_it(const char *name, int reps, double by
 	printf("%-40s %8.2f us   %7.1f GB/s (algorithmic)\n", name, ms * 1e3, bytes / ms / 1e6);
 	return ms;
 }
-static double rel_diff(const double *a, const double *b, size_t n)
-{
-	std::vector<double> ha(n), hb(n);
-	CK(cudaMemcpy(ha.data(), a, n * 8, cudaMemcpyDeviceToHost));
-	CK(cudaMemcpy(hb.data(), b, n * 8, cudaMemcpyDeviceToHost));
-	double num = 0, den = 0;
-	for (size_t i = 0; i < n; i++) num += (ha[i] - hb[i]) * (ha[i] - hb[i]), den += hb[i] * hb[i];
-	return sqrt(num / den);
-}
 
 int main(int argc, char **argv)
 {
@@ -80,13 +71,11 @@ int main(int argc, char **argv)
 	PatchMeta *meta;
 	CK(cudaMalloc(&meta, hm.size() * sizeof(PatchMeta)));
 	CK(cudaMemcpy(meta, hm.data(), hm.size() * sizeof(PatchMeta), cudaMemcpyHostToDevice));
-	double *f, *u, *u2, *uc, *Fa, *Fb, *Fb2, *tri, *scratch;
-	CK(cudaMalloc(&f, nc * 8)); CK(cudaMalloc(&u, nc * 8)); CK(cudaMalloc(&u2, nc * 8)); CK(cudaMalloc(&uc, ncc * 8));
-	CK(cudaMalloc(&Fa, nf * 8)); CK(cudaMalloc(&Fb, nf * 8)); CK(cudaMalloc(&Fb2, nf * 8)); CK(cudaMalloc(&tri, 17 * M * 8));
+	double *f, *u, *uc, *Fa, *Fb, *tri;
+	CK(cudaMalloc(&f, nc * 8)); CK(cudaMalloc(&u, nc * 8)); CK(cudaMalloc(&uc, ncc * 8));
+	CK(cudaMalloc(&Fa, nf * 8)); CK(cudaMalloc(&Fb, nf * 8)); CK(cudaMalloc(&tri, 17 * M * 8));
 	int sms = 148;
 	cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0);
-	const int gridA = std::min(P, sms * S32_CTAS_PER_SM);
-	CK(cudaMalloc(&scratch, (size_t) gridA * NC * 8));
 	{
 		std::vector<double> h(nc);
 		for (size_t i = 0; i < nc; i++) h[i] = (double) rand() / RAND_MAX - 0.5;
@@ -109,21 +98,16 @@ int main(int argc, char **argv)
 		for (int i = 0; i <= 32; i++) mag[i] = sin(M_PI / 64.0 * i);
 		CK(cudaMemcpyToSymbol(c_mag32, mag.data(), 33 * 8));
 	}
-	const size_t smA = smooth3d32_smem_bytes(), smC = smooth3d32c_smem_bytes();
+	const size_t smC   = smooth3d32c_smem_bytes();
 	const int    gridC = 2 * std::min(P, sms / 2);
-	printf("G=%d P=%d cells=%zu slab grid=%d cluster grid=%d smem %zu / %zu\n", G, P, nc, gridA, gridC, smA, smC);
+	printf("G=%d P=%d cells=%zu cluster grid=%d smem %zu\n", G, P, nc, gridC, smC);
 	const double b16 = 16.0 * nc;
 #define VARIANT(NAME, Z, E, PR, W)                                                                                               \
 	{                                                                                                                            \
-		CK(cudaFuncSetAttribute(smooth3d32_kernel<Z, E, PR, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smA));        \
 		CK(cudaFuncSetAttribute(smooth3d32c_kernel<Z, E, PR, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smC));       \
-		CK(cudaMemset(u, 0, nc * 8)); CK(cudaMemset(u2, 0, nc * 8)); CK(cudaMemset(Fb, 0, nf * 8)); CK(cudaMemset(Fb2, 0, nf * 8)); \
-		time_it(NAME " slab", reps, b16, [&] { smooth3d32_kernel<Z, E, PR, W><<<gridA, 256, smA>>>(meta, 0, P, f, u, Fa, Fb, tri, uc, scratch); }); \
+		CK(cudaMemset(u, 0, nc * 8)); CK(cudaMemset(Fb, 0, nf * 8));                                                             \
+		time_it(NAME, reps, b16, [&] { smooth3d32c_kernel<Z, E, PR, W><<<gridC, C32_THREADS, smC>>>(meta, 0, P, f, u, Fa, Fb, tri, uc); }); \
 		CK(cudaGetLastError());                                                                                                  \
-		time_it(NAME " cluster", reps, b16, [&] { smooth3d32c_kernel<Z, E, PR, W><<<gridC, C32_THREADS, smC>>>(meta, 0, P, f, u2, Fa, Fb2, tri, uc); }); \
-		CK(cudaGetLastError());                                                                                                  \
-		if (W) printf("   u: rel diff %.3e\n", rel_diff(u2, u, nc));                                                             \
-		if (E) printf("   F: rel diff %.3e\n", rel_diff(Fb2, Fb, nf));                                                           \
 	}
 	VARIANT("zero_guess faces-only", true, true, false, false)
 	VARIANT("zero_guess write_u", true, false, false, true)

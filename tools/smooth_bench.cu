@@ -67,9 +67,9 @@ int main(int argc, char **argv)
 	PatchMeta *meta;
 	CK(cudaMalloc(&meta, hm.size() * sizeof(PatchMeta)));
 	CK(cudaMemcpy(meta, hm.data(), hm.size() * sizeof(PatchMeta), cudaMemcpyHostToDevice));
-	double *f, *u, *uc, *Fa, *Fb, *eig, *coarse;
+	double *f, *u, *uc, *Fa, *Fb, *tri, *coarse;
 	CK(cudaMalloc(&f, nc * 8)); CK(cudaMalloc(&u, nc * 8)); CK(cudaMalloc(&uc, ncc * 8)); CK(cudaMalloc(&coarse, ncc * 8));
-	CK(cudaMalloc(&Fa, nf * 8)); CK(cudaMalloc(&Fb, nf * 8)); CK(cudaMalloc(&eig, 4096 * 8));
+	CK(cudaMalloc(&Fa, nf * 8)); CK(cudaMalloc(&Fb, nf * 8)); CK(cudaMalloc(&tri, 4096 * 8));
 	{
 		std::vector<double> h(nc);
 		for (size_t i = 0; i < nc; i++) h[i] = (double) rand() / RAND_MAX - 0.5;
@@ -78,7 +78,7 @@ int main(int argc, char **argv)
 		CK(cudaMemcpy(Fa, h.data(), nf * 8, cudaMemcpyHostToDevice));
 		std::vector<double> e(4096);
 		for (int i = 0; i < 4096; i++) e[i] = -1.0 / (1 + i % 7);
-		CK(cudaMemcpy(eig, e.data(), 4096 * 8, cudaMemcpyHostToDevice));
+		CK(cudaMemcpy(tri, e.data(), 4096 * 8, cudaMemcpyHostToDevice));
 		std::vector<double> mag(17);
 		for (int i = 0; i <= 16; i++) mag[i] = sin(M_PI / 32.0 * i);
 		CK(cudaMemcpyToSymbol(c_mag16, mag.data(), 17 * 8));
@@ -92,17 +92,16 @@ int main(int argc, char **argv)
 	attr(smooth3d16_kernel<false, false, true, true>);
 	attr(smooth3d16_kernel<false, false, false, true>);
 	attr(smooth3d16_kernel<false, true, false, false>);
-	const int grid = std::min(P, sms * s16_ctas_per_sm(false, false));
+	const int grid = std::min(P, sms * s16_ctas_per_sm(false));
 	const dim3 blk(S16_BLOCK);
 	printf("G=%d P=%d cells=%zu grid=%d\n", G, P, nc, grid);
 	const double b16 = 16.0 * nc;
-	const size_t smz = smooth3d16_smem_bytes(true, false);
-	const int    gridz = std::min(P, sms * s16_ctas_per_sm(true, false));
-	time_it("zero_guess faces-only", reps, b16, [&] { smooth3d16_kernel<true, true, false, false><<<gridz, blk, smz>>>(meta, 0, P, f, u, Fa, Fb, eig, uc); });
-	time_it("zero_guess write_u", reps, b16, [&] { smooth3d16_kernel<true, false, false, true><<<gridz, blk, smz>>>(meta, 0, P, f, u, Fa, Fb, eig, uc); });
-	time_it("plain gamma write_u", reps, b16, [&] { smooth3d16_kernel<false, false, false, true><<<grid, blk, sm>>>(meta, 0, P, f, u, Fa, Fb, eig, uc); });
-	time_it("plain gamma faces-only", reps, b16, [&] { smooth3d16_kernel<false, true, false, false><<<grid, blk, sm>>>(meta, 0, P, f, u, Fa, Fb, eig, uc); });
-	if (G > 1) time_it("prolong gamma write_u", reps, b16, [&] { smooth3d16_kernel<false, false, true, true><<<grid, blk, sm>>>(meta, 0, P, f, u, Fa, Fb, eig, uc); });
+	const int    gridz = std::min(P, sms * s16_ctas_per_sm(true));
+	time_it("zero_guess faces-only", reps, b16, [&] { smooth3d16_kernel<true, true, false, false><<<gridz, blk, sm>>>(meta, 0, P, f, u, Fa, Fb, tri, uc); });
+	time_it("zero_guess write_u", reps, b16, [&] { smooth3d16_kernel<true, false, false, true><<<gridz, blk, sm>>>(meta, 0, P, f, u, Fa, Fb, tri, uc); });
+	time_it("plain gamma write_u", reps, b16, [&] { smooth3d16_kernel<false, false, false, true><<<grid, blk, sm>>>(meta, 0, P, f, u, Fa, Fb, tri, uc); });
+	time_it("plain gamma faces-only", reps, b16, [&] { smooth3d16_kernel<false, true, false, false><<<grid, blk, sm>>>(meta, 0, P, f, u, Fa, Fb, tri, uc); });
+	if (G > 1) time_it("prolong gamma write_u", reps, b16, [&] { smooth3d16_kernel<false, false, true, true><<<grid, blk, sm>>>(meta, 0, P, f, u, Fa, Fb, tri, uc); });
 	if (G > 1) time_it("face_residual_restrict", reps, b16, [&] { face_residual_restrict_kernel<3, 16, false><<<std::min(P, sms * 8), 256>>>(meta, 0, P, Fa, nullptr, coarse); });
 	if (G > 1) {
 		double *coarse2;

@@ -5,6 +5,8 @@
 //   smooth3d32c_kernel  the smoother the library uses: a thread-block cluster of two CTAs holds the whole patch in the
 //                       shared memory of two SMs; x and y are transformed, z is a two-sided tridiagonal elimination split
 //                       over the pair (see the comment above the kernel)
+//   iface_rhs32_kernel  the interface part of the right-hand side of the sweeps that do not start from zero, transformed
+//                       for smooth3d32c_kernel
 //   smooth3d32n_kernel  levels with Neumann domain sides: general dense-transform path through an L2-resident scratch block
 //   face_residual_restrict_big_kernel   residual + restriction from face data (see kernels.cuh)
 // The operator apply for 32^3 patches is apply3d32_tma_kernel (apply_tma.cuh).
@@ -41,14 +43,20 @@ __device__ __forceinline__ double gamma_entry(const PatchMeta &pm, int p, int s,
 //   transposes), the z recurrences are element-wise over the planes (two pencils per thread).
 //   f goes straight from memory into the y pencils (a warp's load = one 256-byte row) and u straight from the
 //   y pencils back to memory: HBM sees f once and u once, shared memory holds the 16 planes (136 KB).
+//   Sweeps that do not start from zero read the interface part of their right-hand side, already transformed, from the
+//   output of iface_rhs32_kernel (below).
 // Same arithmetic as smooth_kernel (SchurHelper.h:319-331, FftwPatchSolver.h:174-206).
 // ---------------------------------------------------------------------------------------------
 constexpr int    C32_THREADS = 512, C32_ROW = 34, C32_PL = 32 * C32_ROW, C32_TILE = 16 * C32_PL;
 constexpr int    C32_FV = 65; // row pitch of the face-vector staging [32][65] (faces-only sweeps, see the tail of the kernel)
-// tile + two exchange planes (double buffered) + z-face interface values + per-warp x/y-face values + x-face output staging
-// (188 KB: the next shared-memory carve-out step, 228 KB, would leave the L1 28 KB instead of 60 KB - measured 4-7 % slower)
-constexpr size_t smooth3d32c_smem_bytes() { return sizeof(double) * (C32_TILE + 2 * 1024 + 1024 + 16 * 128 + 16 * 64); }
-static_assert(32 * C32_FV <= 1024 + 16 * 128, "the face-vector staging aliases the interface-value buffers of sweeps from a zero guess");
+// tile + two exchange planes (double buffered) + x-face output staging, and for the faces-only sweeps from a zero guess the
+// face-vector staging (a 24 KB region, 188 KB in all: the carve-out step below 228 KB, which would leave the L1 28 KB instead
+// of 60 KB - measured 4-7 % slower).  The other sweeps take 160 KB and leave the L1 92 KB.
+template <bool ZERO_GUESS> constexpr size_t smooth3d32c_smem_bytes()
+{
+	return sizeof(double) * (C32_TILE + 2 * 1024 + 16 * 64 + (ZERO_GUESS ? 1024 + 16 * 128 : 0));
+}
+static_assert(32 * C32_FV <= 1024 + 16 * 128, "the face-vector staging of sweeps from a zero guess");
 __device__ __forceinline__ unsigned cluster_ctarank()
 {
 	unsigned r;
@@ -89,7 +97,6 @@ struct __align__(16) GDesc32 {
 };
 struct GPatch32 {
 	GDesc32 d[6];
-	int     neu, pad[3]; // Neumann bits of the patch (levels with Neumann patches: the cluster kernel skips them)
 };
 template <bool PROLONG>
 __device__ __forceinline__ void make_gdesc32(const PatchMeta &pm, int p, int s, GPatch32 &out)
@@ -134,136 +141,191 @@ template <bool PROLONG> struct SideGamma32 {
 			b1 = __ldg(uc + o.w + ((lo >> sb) * A + (hi >> sb) * B));
 		}
 	}
+	// the value of a side without the GD_SLOW flag
+	__device__ __forceinline__ double combine(const GDesc32 &d) const
+	{
+		return d.c * (0.5 * (a0 + a1) + 0.5 * (b0 + ((d.flags & GD_WB) ? b1 : 0.0)));
+	}
 	__device__ __forceinline__ double finish(const GDesc32 &d, const PatchMeta *__restrict__ meta, int p, int s, int m, const double *__restrict__ F,
 	                                         const double *__restrict__ uc) const
 	{
-		const double c  = d.c;
-		const int    fl = d.flags;
-		double       g  = c * (0.5 * (a0 + a1) + 0.5 * (b0 + ((fl & GD_WB) ? b1 : 0.0)));
-		if (fl & GD_SLOW) g = c * gamma_entry32<PROLONG>(meta, p, s, m, F, uc);
+		double g = combine(d);
+		if (d.flags & GD_SLOW) g = d.c * gamma_entry32<PROLONG>(meta, p, s, m, F, uc);
 		return g;
 	}
 };
 
-// HALO = false compiles the multi-GPU hand-over (HaloSync / halo_push_cta) out.  The host launches HALO = !ZERO_GUESS on
-// any number of GPUs: measured on one GPU (config D, same box, alternating runs) the post-sweep instantiation WITH the
-// hand-over code is 1 % faster than the one without (7.05 vs 7.13 ms; register allocation at the 128-register cap).
-template <bool ZERO_GUESS, bool EMIT, bool PROLONG, bool WRITE_U, bool HALO = false>
+// ---------------------------------------------------------------------------------------------
+// iface_rhs32_kernel: the interface part of the right-hand side of a 32^3 sweep that does not start from zero.
+//   A block-Jacobi sweep solves S u = f - b on each patch, b = (2/h^2) E^T gamma: non-zero on boundary cells only and a sum
+//   of six face terms.  The patch solve is linear, so each face term can enter smooth3d32c_kernel where it is uniform over the
+//   sweep's threads: the y faces before the y transform (as they are), the x faces at x = 0 / 31 of the rows of the x
+//   transform (transformed along y), the z faces at elimination step 0 (transformed along y, then x - the sweep's order).
+//   This kernel forms those terms once per patch, in the face-buffer shape G[p][6][1024]:
+//     s = 0, 1 (x faces): Dst2_y(c(., z))[k_y]       at k_y + 32 z
+//     s = 2, 3 (y faces): c(x, z)                    at x + 32 z
+//     s = 4, 5 (z faces): Dst2_x(Dst2_y(c))[k_x, k_y] at k_x + 32 k_y
+//   with c = (2/h^2) gamma from the gathers of GDesc32 / SideGamma32 (gamma_entry32 on sides with coarse / fine neighbours),
+//   so the values of c are those the sweep subtracted when it gathered them itself; only where they enter moved.
+//   One warp per patch side, one patch per CTA at a time, a padded 32 x 33 tile per warp for the transposes.  On several
+//   GPUs this kernel is the consumer of the halo hand-over of the first post-sweep (halo_push / halo_wait_cta / halo_finish,
+//   as face_residual_restrict_big_kernel): the sweep after it reads no face data.
+// ---------------------------------------------------------------------------------------------
+constexpr int    IR32_THREADS = 192, IR32_CTAS_PER_SM = 2, IR32_TP = 33;
+constexpr size_t iface_rhs32_smem_bytes() { return sizeof(double) * 6 * 32 * IR32_TP; }
+// c of side s of patch p: entry m = lane + 32 i to out[i * stride + lane]; AX = face-normal axis.  Sides with coarse / fine
+// neighbours go entry by entry through the out-of-line gamma_entry32 (SideGamma32::finish); the others keep IR32_BATCH entries'
+// loads in flight per lane and need no call, so that no in-flight load is held across one.
+constexpr int IR32_BATCH = 16;
+template <bool PROLONG, int AX>
+__device__ __forceinline__ void side_gamma32(const GDesc32 &d, const PatchMeta *__restrict__ meta, int p, int s, int lane, const double *__restrict__ F,
+                                             const double *__restrict__ uc, double *out, int stride)
+{
+	if (d.flags & GD_SLOW) { // warp-uniform
+#pragma unroll 1
+		for (int i = 0; i < 32; i++) {
+			SideGamma32<PROLONG> sg;
+			sg.template issue<AX>(d, lane + 32 * i, lane, i, F, uc);
+			out[i * stride + lane] = sg.finish(d, meta, p, s, lane + 32 * i, F, uc);
+		}
+		return;
+	}
+	constexpr int B = IR32_BATCH;
+#pragma unroll
+	for (int i0 = 0; i0 < 32; i0 += B) {
+		SideGamma32<PROLONG> sg[B];
+#pragma unroll
+		for (int j = 0; j < B; j++) sg[j].template issue<AX>(d, lane + 32 * (i0 + j), lane, i0 + j, F, uc);
+#pragma unroll
+		for (int j = 0; j < B; j++) out[(i0 + j) * stride + lane] = sg[j].combine(d);
+	}
+}
+template <bool PROLONG, bool HALO>
+__global__ void __launch_bounds__(IR32_THREADS, IR32_CTAS_PER_SM)
+iface_rhs32_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *__restrict__ Fin, const double *__restrict__ uc,
+                   double *__restrict__ Gout, HaloSync hs = HaloSync{}, int skip_neumann = 0)
+{
+	// skip_neumann != 0: patches with Neumann domain sides are left out (smooth3d32n_kernel gathers its own interface values)
+	constexpr int N = 32, M = N * N, TP = IR32_TP;
+	extern __shared__ __align__(16) double T[]; // [6 warps][32][TP]
+	__shared__ GPatch32 GD;                     // GD.d[s]: written and read by warp s only
+	const int lane = threadIdx.x & 31, s = threadIdx.x >> 5;
+	double *  tw   = T + s * N * TP;
+	Mags<N>   mg;
+	mg.load();
+	pdl_launch_dependents();
+	pdl_wait();
+	if (HALO) halo_push<3, 32>(hs, meta);
+	bool halo_ok = false;
+	for (int g = blockIdx.x; g < P - p0; g += gridDim.x) {
+		const int p = p0 + g;
+		if (skip_neumann && meta[p].neumann) continue; // CTA-uniform
+		if (HALO) halo_wait_cta(hs, p, halo_ok);
+		if (lane == 0) make_gdesc32<PROLONG>(meta[p], p, s, GD);
+		__syncwarp();
+		const GDesc32 &d  = GD.d[s];
+		double *       Gp = Gout + ((size_t) p * 6 + s) * M;
+		double         v[N];
+		if (s < 2) { // x faces: entry (y, z) = (lane, i) -> tile row z; transform along y, pencil z = lane
+			side_gamma32<PROLONG, 0>(d, meta, p, s, lane, Fin, uc, tw, TP);
+			__syncwarp();
+#pragma unroll
+			for (int k = 0; k < N; k++) v[k] = tw[lane * TP + k];
+			Dst2<N, N>::run(v, mg);
+#pragma unroll
+			for (int k = 0; k < N; k++) tw[lane * TP + k] = v[k];
+			__syncwarp();
+#pragma unroll
+			for (int i = 0; i < N; i++) Gp[lane + N * i] = tw[i * TP + lane];
+		} else if (s < 4) { // y faces: entry (x, z) = (lane, i), as they are
+			side_gamma32<PROLONG, 1>(d, meta, p, s, lane, Fin, uc, Gp, N);
+		} else { // z faces: entry (x, y) = (lane, i) -> tile row y; transform along y (pencil x = lane), then along x (pencil k_y = lane)
+			side_gamma32<PROLONG, 2>(d, meta, p, s, lane, Fin, uc, tw, TP);
+			__syncwarp();
+#pragma unroll
+			for (int k = 0; k < N; k++) v[k] = tw[k * TP + lane];
+			Dst2<N, N>::run(v, mg);
+#pragma unroll
+			for (int k = 0; k < N; k++) tw[k * TP + lane] = v[k];
+			__syncwarp();
+#pragma unroll
+			for (int k = 0; k < N; k++) v[k] = tw[lane * TP + k];
+			Dst2<N, N>::run(v, mg);
+#pragma unroll
+			for (int k = 0; k < N; k++) tw[lane * TP + k] = v[k];
+			__syncwarp();
+#pragma unroll
+			for (int i = 0; i < N; i++) Gp[lane + N * i] = tw[i * TP + lane];
+		}
+		__syncwarp(); // GD.d[s] and the tile are rewritten for the next patch
+	}
+	if (HALO) halo_finish(hs);
+}
+
+// Sweeps that do not start from zero take the interface part of the right-hand side from G (iface_rhs32_kernel, launched
+// right before over the same patches): six coalesced loads per thread and patch, issued with the loads of f.
+template <bool ZERO_GUESS, bool EMIT, bool WRITE_U>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(C32_THREADS, 1)
 smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *__restrict__ f, double *__restrict__ u,
-                   const double *__restrict__ Fin, double *__restrict__ Fout, const double *__restrict__ tri,
-                   const double *__restrict__ uc, HaloSync hs = HaloSync{}, int skip_neumann = 0)
+                   const double *__restrict__ G, double *__restrict__ Fout, const double *__restrict__ tri, int skip_neumann = 0)
 {
 	// skip_neumann != 0: patches with Neumann domain sides are left to smooth3d32n_kernel (launched over the same range
-	// with only_neumann); both CTAs of the cluster skip together and keep gathering the next patch's interface values
+	// with only_neumann); both CTAs of the cluster skip together
 	constexpr int N = 32, ROW = C32_ROW, PL = C32_PL, M = N * N, NC = N * N * N;
 	extern __shared__ __align__(16) double S[];
 	double *       X    = S + C32_TILE;  // [2][M] last eliminated plane, for the peer
-	double *       GZ   = X + 2 * M;     // [M] (2/h^2) gamma on this half's z face
-	double *       GXY  = GZ + M;        // [16 warps][4][32] x- and y-face values of a plane
-	double *       EX   = GXY + 16 * 128; // [16 warps][2][32] staging of the new x-face slices
-	double *       FV   = GZ;             // [32][C32_FV] faces-only sweeps from a zero guess (GZ and GXY are unused there): partially
-	                                      // transformed face vectors, entry j of vector i at j * C32_FV + i
+	double *       FV   = X + 2 * M;     // [32][C32_FV] faces-only sweeps from a zero guess: partially transformed face
+	                                     // vectors, entry j of vector i at j * C32_FV + i
+	double *       EX   = FV + (ZERO_GUESS ? 1024 + 16 * 128 : 0); // [16 warps][2][32] staging of the new x-face slices
 	const int      t = threadIdx.x, lane = t & 31, w = t >> 5;
 	const unsigned rank = cluster_ctarank();
 	const int      z    = rank == 0 ? w : N - 1 - w; // plane of the patch behind local plane w
 	const int      sz   = rank == 0 ? 4 : 5;         // the z side this half touches
 	const int      ncl = gridDim.x / 2, npatch = P - p0;
-	double *       gxy  = GXY + w * 128;
 	const int      mf   = lane + N * z; // x faces: entry (y, z) = (lane, z); y faces: entry (x, z) = (lane, z)
 	Mags<N>        mg;
 	mg.load();
 	pdl_launch_dependents();
 	pdl_wait();
-	if (!ZERO_GUESS) if (HALO) halo_push<3, 32>(hs, meta);
 	int g = blockIdx.x / 2;
-	// multi-GPU: each CTA polls the peers' flags itself before the first patch whose gamma needs halo faces (HaloSync)
-	bool halo_ok = false;
-	// neighbour-table entry of the patch after the next (staged with cp.async) and the gather descriptors of the next
-	// patch (GD[(it + 1) & 1]) / the one after it, resolved by lane 31 of warps 0-5
-	constexpr int                   MW = (int) (sizeof(PatchMeta) / sizeof(double));
-	__shared__ __align__(16) double metaS[MW];
-	__shared__ GPatch32             GD[2];
-	auto describe = [&](const PatchMeta &pm, int q, int slot) {
-		if (lane == 31 && w < 6) make_gdesc32<PROLONG>(pm, q, w, GD[slot]);
-		if (lane == 31 && w == 6) GD[slot].neu = pm.neumann;
-	};
-	const int zlo = t & 31, zhi = t >> 5; // z-face entries t and t + 512: (x, y) = (zlo, zhi), (zlo, zhi + 16)
-	if (!ZERO_GUESS && g < npatch) { // first patch of this cluster: nothing to hide the gathers behind
-		const int p = p0 + g;
-		if (HALO) halo_wait_cta(hs, p, halo_ok);
-		describe(meta[p], p, 0);
-		if (g + ncl < npatch) describe(meta[p + ncl], p + ncl, 1);
-		__syncthreads();
-		// all loads of the six interface values in flight at once: one memory round trip (coarse levels: one patch per cluster)
-		SideGamma32<PROLONG> g6[6];
-		g6[0].template issue<0>(GD[0].d[0], mf, lane, z, Fin, uc);
-		g6[1].template issue<0>(GD[0].d[1], mf, lane, z, Fin, uc);
-		g6[2].template issue<1>(GD[0].d[2], mf, lane, z, Fin, uc);
-		g6[3].template issue<1>(GD[0].d[3], mf, lane, z, Fin, uc);
-		g6[4].template issue<2>(GD[0].d[sz], t, zlo, zhi, Fin, uc);
-		g6[5].template issue<2>(GD[0].d[sz], t + 512, zlo, zhi + 16, Fin, uc);
-#pragma unroll
-		for (int s = 0; s < 4; s++) gxy[s * 32 + lane] = g6[s].finish(GD[0].d[s], meta, p, s, mf, Fin, uc);
-		GZ[t]       = g6[4].finish(GD[0].d[sz], meta, p, sz, t, Fin, uc);
-		GZ[t + 512] = g6[5].finish(GD[0].d[sz], meta, p, sz, t + 512, Fin, uc);
-		__syncthreads();
-	}
 	for (int it = 0; g < npatch; g += ncl, it++) {
 		const int    p    = p0 + g;
 		const bool   next = g + ncl < npatch;
 		const int    pn   = p + ncl;
 		const double h2   = meta[p].h2;
 		double       v[N];
-		// table entry of the patch after the next -> metaS (described after this iteration's first barrier)
-		if (!ZERO_GUESS && t < MW && g + 2 * ncl < npatch) cp_async8(&metaS[t], reinterpret_cast<const double *>(meta + pn + ncl) + t, true);
-		if (skip_neumann && (ZERO_GUESS ? meta[p].neumann : GD[it & 1].neu)) { // cluster-uniform: this patch belongs to the general path
-			if (!ZERO_GUESS) {
-				// keep the pipeline of the next patch's interface values going: all six at once, nothing to hide behind
-				cp_async_wait_all();
-				__syncthreads(); // metaS has landed; gxy / GZ of this (skipped) patch are free
-				const GPatch32 &gq = GD[(it + 1) & 1];
-				if (next) {
-					if (HALO) halo_wait_cta(hs, pn, halo_ok);
-					SideGamma32<PROLONG> s6[6];
-					s6[0].template issue<0>(gq.d[0], mf, lane, z, Fin, uc);
-					s6[1].template issue<0>(gq.d[1], mf, lane, z, Fin, uc);
-					s6[2].template issue<1>(gq.d[2], mf, lane, z, Fin, uc);
-					s6[3].template issue<1>(gq.d[3], mf, lane, z, Fin, uc);
-					s6[4].template issue<2>(gq.d[sz], t, zlo, zhi, Fin, uc);
-					s6[5].template issue<2>(gq.d[sz], t + 512, zlo, zhi + 16, Fin, uc);
-#pragma unroll
-					for (int s = 0; s < 4; s++) gxy[s * 32 + lane] = s6[s].finish(gq.d[s], meta, pn, s, mf, Fin, uc);
-					GZ[t]       = s6[4].finish(gq.d[sz], meta, pn, sz, t, Fin, uc);
-					GZ[t + 512] = s6[5].finish(gq.d[sz], meta, pn, sz, t + 512, Fin, uc);
-					if (g + 2 * ncl < npatch) describe(*reinterpret_cast<const PatchMeta *>(metaS), pn + ncl, it & 1);
-				}
-				__syncthreads(); // the values and descriptors are visible to the next iteration
-			}
+		if (skip_neumann && meta[p].neumann) { // cluster-uniform: this patch belongs to the general path
 			cluster_sync_all(); // keeps the pair in step: the exchange planes alternate by iteration parity
 			continue;
+		}
+		// interface terms (see iface_rhs32_kernel): y faces of pencil (x, z) = (lane, z), x faces of row (k_y, z) = (lane, z),
+		// this half's z face at pencils (k_x, k_y) = (lane, w), (lane, w + 16)
+		double gy0 = 0.0, gy1 = 0.0, gx0 = 0.0, gx1 = 0.0, gz0 = 0.0, gz1 = 0.0;
+		if (!ZERO_GUESS) {
+			const double *Gp = G + (size_t) p * 6 * M;
+			gy0              = __ldcs(Gp + 2 * M + mf);
+			gy1              = __ldcs(Gp + 3 * M + mf);
+			gx0              = __ldcs(Gp + 0 * M + mf);
+			gx1              = __ldcs(Gp + 1 * M + mf);
+			gz0              = __ldcs(Gp + sz * M + lane + N * w);
+			gz1              = __ldcs(Gp + sz * M + lane + N * (w + 16));
 		}
 		{ // y forward: pencil (x, z) = (lane, z), straight from memory
 			const double *fp = f + (size_t) p * NC + (size_t) z * M + lane;
 #pragma unroll
 			for (int k = 0; k < N; k++) v[k] = __ldcs(fp + k * N);
-			if (next) { // the same plane of the next patch -> L2 (64 lines)
+			if (next) { // the same plane of the next patch -> L2 (64 lines), and what this warp reads of its G (12 lines)
 				const double *fn = f + (size_t) pn * NC + (size_t) z * M + lane * 32;
 				prefetch_l2(fn);
 				prefetch_l2(fn + 16);
+				if (!ZERO_GUESS && lane < 12) {
+					const double *Gn = G + (size_t) pn * 6 * M + 16 * (lane & 1);
+					prefetch_l2(lane < 8 ? Gn + (lane >> 1) * M + N * z : Gn + sz * M + N * (w + 16 * ((lane >> 1) & 1)));
+				}
 			}
 			if (!ZERO_GUESS) {
-				v[0] -= gxy[64 + lane];
-				v[N - 1] -= gxy[96 + lane];
-				if (lane == 0 || lane == N - 1) {
-					const double *q = gxy + (lane ? 32 : 0);
-#pragma unroll
-					for (int k = 0; k < N; k++) v[k] -= q[k];
-				}
-				if (w == 0) {
-#pragma unroll
-					for (int k = 0; k < N; k++) v[k] -= GZ[lane + N * k];
-				}
+				v[0] -= gy0;
+				v[N - 1] -= gy1;
 			}
 			Dst2<N, N>::run(v, mg);
 			double *col = S + w * PL + lane;
@@ -279,25 +341,16 @@ smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 				v[2 * j]        = d.x;
 				v[2 * j + 1]    = d.y;
 			}
+			if (!ZERO_GUESS) {
+				v[0] -= gx0;
+				v[N - 1] -= gx1;
+			}
 			Dst2<N, N>::run(v, mg);
 #pragma unroll
 			for (int j = 0; j < N / 2; j++) rowp[j] = make_double2(v[2 * j], v[2 * j + 1]);
 		}
-		if (!ZERO_GUESS) cp_async_wait_all(); // metaS has landed (made visible by the barrier)
 		__syncthreads();
-		if (HALO && !ZERO_GUESS && next) halo_wait_cta(hs, pn, halo_ok); // gamma of patch pn is gathered from here on
-		// z: elimination step j on local plane j, in place; pencils (k_x, k_y) = (lane, w) and (lane, w + 16).
-		// The interface values of the NEXT patch are gathered around this phase (the transform registers are free here).
-		// (two batches of three: loads issued before the elimination / the back substitution, combined after it)
-		SideGamma32<PROLONG> gm[3];
-		const GPatch32 &     gp = GD[(it + 1) & 1]; // descriptors of patch pn
-		if (!ZERO_GUESS && next) {
-			gm[0].template issue<0>(gp.d[0], mf, lane, z, Fin, uc);
-			gm[1].template issue<0>(gp.d[1], mf, lane, z, Fin, uc);
-			gm[2].template issue<1>(gp.d[2], mf, lane, z, Fin, uc);
-			// descriptors of the patch after the next; GD[it & 1] (patch p) was last read during the previous iteration
-			if (g + 2 * ncl < npatch) describe(*reinterpret_cast<const PatchMeta *>(metaS), pn + ncl, it & 1);
-		}
+		// z: elimination step j on local plane j, in place; pencils (k_x, k_y) = (lane, w) and (lane, w + 16)
 		const double hsc = h2 * (4.0 / (N * N));
 		double *     Xo = X + (it & 1) * M;
 #pragma unroll
@@ -309,18 +362,12 @@ smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 #pragma unroll
 			for (int j = 0; j < 16; j++) {
 				const double a = __ldg(tb + j * M);
-				const double r = zp[j * PL] * (hsc * a);
+				const double x = (!ZERO_GUESS && j == 0) ? zp[0] - (q ? gz1 : gz0) : zp[j * PL]; // this half's z face
+				const double r = x * (hsc * a);
 				rho            = (j == 0) ? r : fma(-a, rho, r);
 				const_cast<double *>(zp)[j * PL] = rho;
 			}
 			Xo[ky * N + lane] = rho;
-		}
-		if (!ZERO_GUESS && next) { // (the buffers were consumed before this iteration's first barrier)
-#pragma unroll
-			for (int s = 0; s < 3; s++) gxy[s * 32 + lane] = gm[s].finish(gp.d[s], meta, pn, s, mf, Fin, uc);
-			gm[0].template issue<1>(gp.d[3], mf, lane, z, Fin, uc);
-			gm[1].template issue<2>(gp.d[sz], t, zlo, zhi, Fin, uc);
-			gm[2].template issue<2>(gp.d[sz], t + 512, zlo, zhi + 16, Fin, uc);
 		}
 		cluster_sync_all(); // both halves are eliminated; the peer's last plane is readable
 #pragma unroll
@@ -336,11 +383,6 @@ smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 				y          = fma(-__ldg(tb + j * M), y, zp[j * PL]);
 				zp[j * PL] = y;
 			}
-		}
-		if (!ZERO_GUESS && next) {
-			gxy[96 + lane] = gm[0].finish(gp.d[3], meta, pn, 3, mf, Fin, uc);
-			GZ[t]          = gm[1].finish(gp.d[sz], meta, pn, sz, t, Fin, uc);
-			GZ[t + 512]    = gm[2].finish(gp.d[sz], meta, pn, sz, t + 512, Fin, uc);
 		}
 		__syncthreads();
 		// faces-only sweeps from a zero guess: dot products + 60 one-dimensional transforms instead of full inverse transforms
@@ -432,7 +474,6 @@ smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 		__syncwarp();
 	}
 	cluster_sync_all(); // a CTA must not exit while its peer may still read its exchange plane
-	if (!ZERO_GUESS) if (HALO) halo_finish(hs);
 }
 
 // ---------------------------------------------------------------------------------------------

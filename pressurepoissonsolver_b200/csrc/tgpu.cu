@@ -199,6 +199,7 @@ struct LevelDev {
 	double *   starts  = nullptr;
 	double *   spacing = nullptr;
 	double *   Fa = nullptr, *Fb = nullptr; // face buffers
+	double *   G  = nullptr; // 32^3 levels: [P][6][M] interface terms of the sweeps that do not start from zero (iface_rhs32_kernel)
 	double *   u = nullptr, *f = nullptr, *r = nullptr; // cycle work vectors (lazily allocated)
 	bool       has_neumann = false;
 	int32_t *  neu_list = nullptr;          // device: owned patches with Neumann domain sides, ascending (smooth3d16_kernel<.., NEU>)
@@ -399,23 +400,41 @@ static int setup_2d32()
 	TRY((set_smem_attr_2d32<false, true, true, false>()));
 	return TGPU_OK;
 }
-template <bool Z, bool E, bool PR, bool W> static int set_smem_attr_3d32()
+template <bool Z, bool E, bool W> static int set_smem_attr_3d32()
 {
-	CU(cudaFuncSetAttribute(smooth3d32c_kernel<Z, E, PR, W, !Z>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smooth3d32c_smem_bytes()));
+	CU(cudaFuncSetAttribute(smooth3d32c_kernel<Z, E, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smooth3d32c_smem_bytes<Z>()));
+	return TGPU_OK;
+}
+// G of the 32^3 levels whose sweeps can reach smooth3d32c_kernel from a non-zero guess (iface_rhs32_kernel): lambda = 0 (a
+// shifted patch solve sends every patch through smooth3d32n_kernel) and at least one owned patch without Neumann sides.
+// Called at creation and when lambda changes (never during a graph capture); the graphs are freed before G is.
+static int update_iface_buffers(tgpu_hier *h)
+{
+	if (!is_3d32(h)) return TGPU_OK;
+	for (LevelDev &L : h->levels) {
+		const bool want = h->lambda == 0.0 && L.neu_host.size() < (size_t) L.P;
+		if (want && !L.G) CU(cudaMalloc(&L.G, (size_t) L.P * 6 * 1024 * sizeof(double)));
+		if (!want && L.G) {
+			CU(cudaDeviceSynchronize());
+			cudaFree(L.G);
+			L.G = nullptr;
+		}
+	}
 	return TGPU_OK;
 }
 // 32^3 patches: opt-in shared memory sizes
 static int setup_3d32(tgpu_hier *h)
 {
-	TRY((set_smem_attr_3d32<true, true, false, true>()));
-	TRY((set_smem_attr_3d32<true, false, false, true>()));
-	TRY((set_smem_attr_3d32<true, true, false, false>()));
-	TRY((set_smem_attr_3d32<false, true, false, true>()));
-	TRY((set_smem_attr_3d32<false, false, false, true>()));
-	TRY((set_smem_attr_3d32<false, true, false, false>()));
-	TRY((set_smem_attr_3d32<false, true, true, true>()));
-	TRY((set_smem_attr_3d32<false, false, true, true>()));
-	TRY((set_smem_attr_3d32<false, true, true, false>()));
+	TRY((set_smem_attr_3d32<true, true, true>()));
+	TRY((set_smem_attr_3d32<true, false, true>()));
+	TRY((set_smem_attr_3d32<true, true, false>()));
+	TRY((set_smem_attr_3d32<false, true, true>()));
+	TRY((set_smem_attr_3d32<false, false, true>()));
+	TRY((set_smem_attr_3d32<false, true, false>()));
+	CU(cudaFuncSetAttribute(iface_rhs32_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) iface_rhs32_smem_bytes()));
+	CU(cudaFuncSetAttribute(iface_rhs32_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) iface_rhs32_smem_bytes()));
+	CU(cudaFuncSetAttribute(iface_rhs32_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) iface_rhs32_smem_bytes()));
+	CU(cudaFuncSetAttribute(iface_rhs32_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) iface_rhs32_smem_bytes()));
 	CU(cudaFuncSetAttribute(apply3d32_tma_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply3d32_tma_smem_bytes()));
 	CU(cudaFuncSetAttribute(apply3d32_tma_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply3d32_tma_smem_bytes()));
 	CU(cudaFuncSetAttribute(apply3d32_tma_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) apply3d32_tma_smem_bytes()));
@@ -821,6 +840,7 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 	}
 	if (D == 3 && n == 32) TRY(setup_3d32(h.get()));
 	else DISPATCH_DN(D, n, TRY((set_smem_attrs<DD, NN>())));
+	TRY(update_iface_buffers(h.get()));
 	if (D == 2 && n == 32) TRY(setup_2d32());
 	*out = h.release();
 	return TGPU_OK;
@@ -1213,6 +1233,7 @@ extern "C" int tgpu_hierarchy_destroy(tgpu_hier *h)
 			cudaFree(L.Fa);
 			cudaFree(L.Fb);
 		}
+		cudaFree(L.G);
 		cudaFree(L.send_peer);
 		cudaFree(L.send_ridx);
 		cudaFree(L.peer_rank);
@@ -1293,6 +1314,7 @@ extern "C" int tgpu_hierarchy_set_lambda(tgpu_hier *h, double lambda)
 	h->lambda = lambda;
 	if (lambda != 0.0 && is_3d32(h) && !h->scratch32) CU(cudaMalloc(&h->scratch32, (size_t) h->ctx->sm_count * 2 * 32768 * sizeof(double)));
 	free_graphs(h);
+	TRY(update_iface_buffers(h));
 	return TGPU_OK;
 }
 extern "C" int tgpu_hierarchy_force_generic_kernels(tgpu_hier *h, int on)
@@ -1670,15 +1692,28 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 		TRY(launch(h->ctx, smooth3d32n_kernel, dim3(nblk), dim3(TGPU_THREADS), 0, (const PatchMeta *) L.meta, p0, p1, f, u, Fin, Fout, uc,
 		           (const double *) h->mats, (const double *) h->lam, h->scratch32, (int) zero_guess, (int) emit, (int) (uc != nullptr), (int) write_u, h->lambda,
 		           mixed32 ? 1 : 0));
-		if (!mixed32) return TGPU_OK;
+		if (!mixed32 || L.neu_host.size() == (size_t) L.P) return TGPU_OK; // (every owned patch has Neumann sides: nothing left)
 	}
 	if (is_3d32(h)) {
+		const int skipn = mixed32 ? 1 : 0;
+		if (!zero_guess) {
+			// the interface part of the right-hand side, transformed for the sweep (and the halo hand-over, which it consumes)
+			if (!L.G) return fail(TGPU_ERR_ARG, "k_smooth: interface-term buffer of the 32^3 level missing");
+			Tag          ti(h->ctx, "iface_rhs", l);
+			const dim3   gi(std::min(p1 - p0, h->ctx->sm_count * IR32_CTAS_PER_SM)), bi(IR32_THREADS);
+			const size_t si = iface_rhs32_smem_bytes();
+			if (hs.enabled && prolong) TRY(launch(h->ctx, iface_rhs32_kernel<true, true>, gi, bi, si, meta, p0, p1, Fin, uc, L.G, hs, skipn));
+			else if (hs.enabled) TRY(launch(h->ctx, iface_rhs32_kernel<false, true>, gi, bi, si, meta, p0, p1, Fin, uc, L.G, hs, skipn));
+			else if (prolong) TRY(launch(h->ctx, iface_rhs32_kernel<true, false>, gi, bi, si, meta, p0, p1, Fin, uc, L.G, hs, skipn));
+			else TRY(launch(h->ctx, iface_rhs32_kernel<false, false>, gi, bi, si, meta, p0, p1, Fin, uc, L.G, hs, skipn));
+		} else if (hs.enabled) {
+			return fail(TGPU_ERR_ARG, "smooth3d32c: no halo hand-over in a zero-guess sweep");
+		}
 		// one cluster of two CTAs (two SMs) per patch, see smooth3d32c_kernel
-		const dim3   grid(2 * std::min(p1 - p0, h->ctx->sm_count / 2)), block(C32_THREADS);
-		const size_t sm    = smooth3d32c_smem_bytes();
-		const int    skipn = mixed32 ? 1 : 0;
-		return smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto W) {
-			return launch(h->ctx, smooth3d32c_kernel<Z, E, PR, W, !Z>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri, uc, hs, skipn);
+		const dim3 grid(2 * std::min(p1 - p0, h->ctx->sm_count / 2)), block(C32_THREADS);
+		return smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto, auto W) {
+			return launch(h->ctx, smooth3d32c_kernel<Z, E, W>, grid, block, smooth3d32c_smem_bytes<Z>(), meta, p0, p1, f, u,
+			              (const double *) L.G, Fout, (const double *) h->tri, skipn);
 		});
 	}
 	// 16^3 levels that contain patches with Neumann domain sides: the specialised kernel sweeps the Dirichlet patches of the

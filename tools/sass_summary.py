@@ -19,7 +19,7 @@ for line in out.splitlines():
         kernels[kern].append(m.group(2).strip())
 demangle = subprocess.run(["c++filt"] + list(kernels), capture_output=True, text=True).stdout.splitlines()
 names = dict(zip(kernels, demangle))
-WANT = ("smooth3d16_kernel", "smooth3d32c_kernel", "smooth2d32_kernel", "apply_tma_kernel", "apply3d32_tma_kernel",
+WANT = ("smooth3d16_kernel", "smooth3d32c_kernel", "iface_rhs32_kernel", "smooth2d32_kernel", "apply_tma_kernel", "apply3d32_tma_kernel",
         "face_residual_restrict", "push_faces_kernel")
 KEYS = ("DFMA", "DADD", "DMUL", "LDS", "STS", "LDG", "STG", "LDGSTS", "UBLKCP", "SYNCS", "BAR", "SHFL", "MUFU", "LDL", "STL", "LDC", "CCTL", "MEMBAR", "ERRBAR", "ATOM", "RED")
 print("# SASS instruction mix per kernel (cuobjdump -sass %s); columns: total instructions, then the count of each opcode family" % lib)

@@ -1,6 +1,6 @@
 // tools/smooth32_bench.cu - stand-alone timing harness for the D = 3, n = 32 smoother (development aid, not part of the
-// product): the cluster-pair kernel (smooth3d32c_kernel) on a uniform G^3 grid of patches with parents on a (G/2)^3
-// grid and random data.
+// product): the cluster-pair kernel (smooth3d32c_kernel) and the interface terms of the sweeps that do not start from zero
+// (iface_rhs32_kernel) on a uniform G^3 grid of patches with parents on a (G/2)^3 grid and random data.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -I pressurepoissonsolver_b200/csrc \
 //        tools/smooth32_bench.cu -o tools/smooth32_bench && tools/smooth32_bench [G=8] [reps=10]
 #include <cstdio>
@@ -98,21 +98,38 @@ int main(int argc, char **argv)
 		for (int i = 0; i <= 32; i++) mag[i] = sin(M_PI / 64.0 * i);
 		CK(cudaMemcpyToSymbol(c_mag32, mag.data(), 33 * 8));
 	}
-	const size_t smC   = smooth3d32c_smem_bytes();
-	const int    gridC = 2 * std::min(P, sms / 2);
-	printf("G=%d P=%d cells=%zu cluster grid=%d smem %zu\n", G, P, nc, gridC, smC);
+	const size_t smZ = smooth3d32c_smem_bytes<true>(), smC = smooth3d32c_smem_bytes<false>(), smI = iface_rhs32_smem_bytes();
+	const int    gridC = 2 * std::min(P, sms / 2), gridI = std::min(P, sms * IR32_CTAS_PER_SM);
+	printf("G=%d P=%d cells=%zu cluster grid=%d smem %zu / %zu (zero guess / not), iface_rhs32 grid=%d smem %zu\n", G, P, nc, gridC, smZ, smC, gridI, smI);
 	const double b16 = 16.0 * nc;
-#define VARIANT(NAME, Z, E, PR, W)                                                                                               \
+	double *Gv;
+	CK(cudaMalloc(&Gv, nf * 8));
+	CK(cudaFuncSetAttribute(iface_rhs32_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smI));
+	CK(cudaFuncSetAttribute(iface_rhs32_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smI));
+	auto iface = [&](bool prolong) {
+		if (prolong) iface_rhs32_kernel<true, false><<<gridI, IR32_THREADS, smI>>>(meta, 0, P, Fa, uc, Gv);
+		else iface_rhs32_kernel<false, false><<<gridI, IR32_THREADS, smI>>>(meta, 0, P, Fa, uc, Gv);
+	};
+#define VARIANT(NAME, Z, E, W, PRE)                                                                                              \
 	{                                                                                                                            \
-		CK(cudaFuncSetAttribute(smooth3d32c_kernel<Z, E, PR, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smC));       \
+		const size_t sm_ = smooth3d32c_smem_bytes<Z>();                                                                          \
+		CK(cudaFuncSetAttribute(smooth3d32c_kernel<Z, E, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sm_));            \
 		CK(cudaMemset(u, 0, nc * 8)); CK(cudaMemset(Fb, 0, nf * 8));                                                             \
-		time_it(NAME, reps, b16, [&] { smooth3d32c_kernel<Z, E, PR, W><<<gridC, C32_THREADS, smC>>>(meta, 0, P, f, u, Fa, Fb, tri, uc); }); \
+		time_it(NAME, reps, b16, [&] { PRE; smooth3d32c_kernel<Z, E, W><<<gridC, C32_THREADS, sm_>>>(meta, 0, P, f, u, Gv, Fb, tri); }); \
 		CK(cudaGetLastError());                                                                                                  \
 	}
-	VARIANT("zero_guess faces-only", true, true, false, false)
-	VARIANT("zero_guess write_u", true, false, false, true)
-	VARIANT("zero_guess write_u+faces", true, true, false, true)
-	VARIANT("plain gamma write_u+faces", false, true, false, true)
-	if (G > 1) VARIANT("prolong gamma write_u", false, false, true, true)
+	VARIANT("zero_guess faces-only", true, true, false, )
+	VARIANT("zero_guess write_u", true, false, true, )
+	VARIANT("zero_guess write_u+faces", true, true, true, )
+	// sweeps that do not start from zero: the interface terms (iface_rhs32_kernel) alone, the sweep alone (reading the terms
+	// left by the previous launch), and the two back to back as the library launches them
+	time_it("iface_rhs32 plain", reps, 8.0 * nf, [&] { iface(false); });
+	VARIANT("sweep write_u+faces", false, true, true, )
+	VARIANT("iface_rhs32 plain + sweep write_u+faces", false, true, true, iface(false))
+	if (G > 1) {
+		time_it("iface_rhs32 prolong", reps, 8.0 * nf, [&] { iface(true); });
+		VARIANT("sweep write_u", false, false, true, )
+		VARIANT("iface_rhs32 prolong + sweep write_u", false, false, true, iface(true))
+	}
 	return 0;
 }

@@ -5,6 +5,9 @@
 //
 // usage: steady D mesh.bin divide n [--cycle V|W] [--plugin] [--pre k] [--post k] [--mid k] [--coarse k] [--max-levels k]
 //               [--patches-per-proc x] [--lambda x] [--out u.bin] [--neumann] [--problem trig|gauss]
+//               [--solver bicgstab|gmg] [--tol x]
+//   --solver gmg  stationary multigrid (GMGSolve, one cycle per iteration) to ||f - A u|| <= tol ||f|| (--tol, default
+//                 1e-10) from u = 0, instead of BiCGStab preconditioned by the cycle (tolerance 1e-12, relative to r0)
 //   --max-levels / --patches-per-proc   GMG::CycleOpts (GMG/CycleOpts.h:55,59, honoured as in GMG/CycleFactory3d.cpp:101-104)
 //   --lambda  the patch solver's shift (FftwPatchSolver(domain, lambda), PatchSolvers/FftwPatchSolver.h:66)
 //   --neumann Neumann domain boundaries (ThundereggDomGen(..., neumann = true), Init::initNeumann, right-hand-side mean
@@ -28,7 +31,8 @@ template <size_t D> static int run(int argc, char **argv)
 	GMG::CycleOpts    copts;
 	bool              plugin = false, neumann = false;
 	double            lambda = 0.0;
-	std::string       out, problem = "trig";
+	std::string       out, problem = "trig", solver = "bicgstab";
+	double            tol = 1e-10;
 	for (int a = 5; a < argc; a++) {
 		if (!strcmp(argv[a], "--cycle") && a + 1 < argc) copts.cycle_type = argv[++a];
 		else if (!strcmp(argv[a], "--pre") && a + 1 < argc) copts.pre_sweeps = atoi(argv[++a]);
@@ -42,7 +46,10 @@ template <size_t D> static int run(int argc, char **argv)
 		else if (!strcmp(argv[a], "--neumann")) neumann = true;
 		else if (!strcmp(argv[a], "--problem") && a + 1 < argc) problem = argv[++a];
 		else if (!strcmp(argv[a], "--out") && a + 1 < argc) out = argv[++a];
+		else if (!strcmp(argv[a], "--solver") && a + 1 < argc) solver = argv[++a];
+		else if (!strcmp(argv[a], "--tol") && a + 1 < argc) tol = atof(argv[++a]);
 	}
+	if (solver != "bicgstab" && solver != "gmg") throw Error(TGPU_ERR_ARG, "unknown solver " + solver);
 	auto ctx = std::make_shared<Context>(0);
 	Mesh mesh(mesh_file, (int) D);
 	for (int i = 0; i < divide; i++) mesh.refineLeaves();
@@ -69,7 +76,7 @@ template <size_t D> static int run(int argc, char **argv)
 
 	ctx->sync();
 	auto t0  = std::chrono::steady_clock::now();
-	int  its = BiCGStab<D>::solve(vg, A, u, f, M);
+	int  its = solver == "gmg" ? GMGSolve<D>::solve(M, u, f, tol) : BiCGStab<D>::solve(vg, A, u, f, M);
 	ctx->sync();
 	double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
 
@@ -102,7 +109,7 @@ int main(int argc, char **argv)
 {
 	if (argc < 5) {
 		std::cerr << "usage: steady D mesh.bin divide n [--cycle V|W] [--plugin] [--pre k] [--post k] [--mid k] [--coarse k] [--max-levels k] "
-		             "[--patches-per-proc x] [--lambda x] [--out u.bin] [--neumann] [--problem trig|gauss]\n";
+		             "[--patches-per-proc x] [--lambda x] [--out u.bin] [--neumann] [--problem trig|gauss] [--solver bicgstab|gmg] [--tol x]\n";
 		return 2;
 	}
 	try {

@@ -169,6 +169,19 @@ int tgpu_vcycle(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu
 /* BiCGStab with the cycle as right preconditioner (opts == NULL: unpreconditioned). */
 int tgpu_bicgstab(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu_vec *u, double tol, int max_it,
                   int *iterations, double *rel_residual);
+/* Stationary multigrid from the initial guess in u (a warm start: the previous time step's solution).  Residuals are
+ * relative to ||f||_2 (absolute if f = 0), not to the initial residual as in tgpu_bicgstab.  f aliasing u, a vector of
+ * another level or hierarchy, tol < 0 or max_it < 0 give TGPU_ERR_ARG and leave u untouched.
+ * u <- u + Cycle(f - A u): one cycle from the guess u (opts as tgpu_vcycle; NULL = defaults).  The fused schedule
+ * starts the finest level's pre-sweep from u's boundary slices; the others (fused = 0, interpolator = 1, W cycles on
+ * several GPUs, no post-sweep, one level, lambda != 0) compute the residual, a cycle from zero and the sum.
+ * rel_residual (nullable): ||f - A u_new||_2 / ||f||_2 of the result (fused: from the boundary slices, see DESIGN). */
+int tgpu_vcycle_update(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu_vec *u, double *rel_residual);
+/* cycles of tgpu_vcycle_update until ||f - A u||_2 <= tol ||f||_2 (confirmed by a full residual) or max_it cycles.
+ * iterations, rel_residual (nullable): cycles run, relative residual of the result.  history (nullable, max_it + 1
+ * doubles): the relative residual before the first cycle and after each one (iterations + 1 entries are written). */
+int tgpu_gmg_solve(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu_vec *u, double tol, int max_it,
+                   int *iterations, double *rel_residual, double *history);
 /* host-buffer convenience (the e2e path): f_host -> device, one cycle, u -> u_host */
 int tgpu_vcycle_host(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f_pinned, double *u_pinned);
 /* pipelined form for a stream of independent right-hand sides: returns once the work is enqueued; upload of

@@ -17,6 +17,7 @@
 //   GMG::CycleOpts                GMG/CycleOpts.h:51-80    GMG::CycleOpts
 //   GMG::CycleFactory{2,3}d       GMG/CycleFactory3d.cpp:69-134     GMG::CycleFactory<D>::getCycle
 //   BiCGStab<D>::solve            BiCGStab.h:45-106        BiCGStab<D>::solve (same signature; delegates to tgpu_bicgstab)
+//   (no reference counterpart)                             GMGSolve<D>::solve (stationary multigrid from a guess, tgpu_gmg_solve)
 //   Tree<D> + ThundereggDomGen<D> OctTree.h, ThundereggDomGen.h     Mesh, Hierarchy (RAII over tgpu_mesh / tgpu_hier)
 //
 // Error behaviour: the reference throws an int (`throw 3;`) on type mismatches
@@ -371,6 +372,22 @@ template <size_t D> class BiCGStab
 		}
 		int its = 0;
 		check(tgpu_bicgstab(op->h->p, cyc ? &cyc->o : nullptr, DeviceVector<D>::raw(b), DeviceVector<D>::raw(x), tolerance, max_it, &its, nullptr));
+		return its;
+	}
+};
+// Stationary multigrid u <- u + M(f - A u) from the initial guess in u until ||f - A u|| <= tol ||f|| (relative to f,
+// not to the initial residual as BiCGStab) or max_it cycles; returns the number of cycles.  M is a cycle from
+// GMG::CycleFactory on the hierarchy of u (tgpu_gmg_solve: one cycle per iteration on the fused schedule).
+template <size_t D> class GMGSolve
+{
+	public:
+	static int solve(std::shared_ptr<const Operator<D>> M, std::shared_ptr<Vector<D>> u, std::shared_ptr<const Vector<D>> f,
+	                 double tol = 1e-10, int max_it = 100)
+	{
+		auto cyc = dynamic_cast<const GMG::FusedCycle<D> *>(M.get());
+		if (cyc == nullptr) throw Error(TGPU_ERR_ARG, "GMGSolve: M must come from GMG::CycleFactory");
+		int its = 0;
+		check(tgpu_gmg_solve(cyc->h->p, &cyc->o, DeviceVector<D>::raw(f), DeviceVector<D>::raw(u), tol, max_it, &its, nullptr, nullptr));
 		return its;
 	}
 };

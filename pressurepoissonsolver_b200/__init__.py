@@ -8,7 +8,8 @@ CUDA device, or importing without the built library, raises.
 The class names mirror the reference's plugin surface (src/Thunderegg/GMG/*.h, Vector.h):
 ``Hierarchy`` ~ the Level list built by GMG::CycleFactory, ``Vec`` ~ Vector<D>,
 ``Hierarchy.apply/smooth/restrict/prolong_add/vcycle`` ~ Operator/Smoother/Restrictor/
-Interpolator/Cycle, ``Hierarchy.bicgstab`` ~ BiCGStab<D>::solve.
+Interpolator/Cycle, ``Hierarchy.bicgstab`` ~ BiCGStab<D>::solve, ``Hierarchy.vcycle_update/gmg_solve`` ~ stationary
+multigrid from an initial guess.
 """
 import ctypes as C
 import os
@@ -79,6 +80,7 @@ ABI_SYMBOLS = [
     "tgpu_comm_unique_id", "tgpu_comm_init", "tgpu_hierarchy_create_distributed",
     "tgpu_hierarchy_force_generic_kernels", "tgpu_mesh_set_neumann", "tgpu_vcycle_host_async", "tgpu_vcycle_host_wait",
     "tgpu_hierarchy_trim", "tgpu_hierarchy_set_lambda", "tgpu_prolong_add_linear", "tgpu_vec_transfer_pair",
+    "tgpu_vcycle_update", "tgpu_gmg_solve",
 ]
 
 lib.tgpu_last_error.restype = C.c_char_p
@@ -121,6 +123,9 @@ for _name, _args in {
     "tgpu_bicgstab": [_vp, C.POINTER(CycleOpts), _vp, _vp, C.c_double, C.c_int, C.POINTER(C.c_int),
                       C.POINTER(C.c_double)],
     "tgpu_vcycle_host": [_vp, C.POINTER(CycleOpts), _vp, _vp],
+    "tgpu_vcycle_update": [_vp, C.POINTER(CycleOpts), _vp, _vp, C.POINTER(C.c_double)],
+    "tgpu_gmg_solve": [_vp, C.POINTER(CycleOpts), _vp, _vp, C.c_double, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_double),
+                       C.POINTER(C.c_double)],
     "tgpu_init_trig_rhs": [_vp, _vp, _vp],
     "tgpu_init_neumann_rhs": [_vp, C.c_int, _vp, _vp],
     "tgpu_vec_integrate": [_vp, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double)],
@@ -473,6 +478,23 @@ class Hierarchy:
         its, rel = C.c_int(), C.c_double()
         check(lib.tgpu_bicgstab(self._p, C.byref(opts) if precondition else None, f._p, u._p, tol, max_it,
                                 C.byref(its), C.byref(rel)))
+        return its.value, rel.value
+
+    def vcycle_update(self, f, u, opts=None):
+        """u <- u + Cycle(f - A u) from the iterate in u; -> ||f - A u|| / ||f|| of the result"""
+        rel = C.c_double()
+        check(lib.tgpu_vcycle_update(self._p, C.byref(opts) if opts is not None else None, f._p, u._p, C.byref(rel)))
+        return rel.value
+
+    def gmg_solve(self, f, u, opts=None, tol=1e-10, max_it=100, history=False):
+        """stationary multigrid from the iterate in u until ||f - A u|| <= tol ||f||; -> (cycles, relative residual) and,
+        with history=True, the relative residual before the first cycle and after each one"""
+        its, rel = C.c_int(), C.c_double()
+        hist = (C.c_double * max(max_it + 1, 1))() if history else None
+        check(lib.tgpu_gmg_solve(self._p, C.byref(opts) if opts is not None else None, f._p, u._p, tol, max_it, C.byref(its),
+                                 C.byref(rel), hist))
+        if history:
+            return its.value, rel.value, list(hist[:its.value + 1])
         return its.value, rel.value
 
     def init_trig_rhs(self, f, exact=None):

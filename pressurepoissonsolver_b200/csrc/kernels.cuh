@@ -469,15 +469,17 @@ template <int D, int N> __device__ __forceinline__ void halo_push(const HaloSync
 // coarse vector attached (post-smoothing right after the coarse-grid correction) the piecewise
 // constant prolongation of the correction, DrctIntp.h:92-111, is added on the fly, so the
 // prolonged fine vector is never materialised: F holds the faces of the pre-smoothed u.
-enum { FV_PLAIN = 0, FV_PROLONG = 1, FV_DIFF = 2, FV_NEG = 3 };
+enum { FV_PLAIN = 0, FV_PROLONG = 1, FV_DIFF = 2, FV_NEG = 3, FV_PROLONG_DIFF = 4 };
 // FV_DIFF: F2 - F (old minus new boundary values) and FV_NEG: -F; gamma is linear in the boundary
 // values, so these give gamma(u_old) - gamma(u_new) directly (face-supported residual, see
-// face_residual_restrict_kernel).
+// face_residual_restrict_kernel).  FV_PROLONG_DIFF: (Fold + P uc) - F, the same difference when the old
+// iterate is the input of a first post-sweep (pre-smoothed u plus the prolonged correction, formed on the fly).
 template <int D, int N, int MODE> struct FaceVals {
 	using G = Geo<D, N>;
 	const double *__restrict__ F;
-	const double *__restrict__ uc; // FV_PROLONG: coarse vector; FV_DIFF: the old face buffer F2
+	const double *__restrict__ uc; // FV_PROLONG, FV_PROLONG_DIFF: coarse vector; FV_DIFF: the old face buffer F2
 	const PatchMeta *__restrict__ meta;
+	const double *__restrict__ Fold = nullptr; // FV_PROLONG_DIFF: faces of the pre-smoothed u
 	__device__ __forceinline__ double get(int q, int par, int orth, int s, int idx) const
 	{
 		const size_t o = ((size_t) q * G::S + s) * G::M + idx;
@@ -489,13 +491,22 @@ template <int D, int N, int MODE> struct FaceVals {
 			face_cell<D, N>(s, idx, c);
 			v += __ldg(uc + (size_t) par * G::NC + parent_cell<D, N>(orth, c));
 		}
+		if (MODE == FV_PROLONG_DIFF) {
+			double w = __ldg(Fold + o);
+			if (par >= 0) {
+				int c[3];
+				face_cell<D, N>(s, idx, c);
+				w += __ldg(uc + (size_t) par * G::NC + parent_cell<D, N>(orth, c));
+			}
+			v = w - v;
+		}
 		return v;
 	}
 	// slow-path variant: looks the parent of q up in the neighbour table
 	__device__ __forceinline__ double get(int q, int s, int idx) const
 	{
 		int par = 0, orth = -1;
-		if (MODE == FV_PROLONG) {
+		if (MODE == FV_PROLONG || MODE == FV_PROLONG_DIFF) {
 			par  = meta[q].parent_idx;
 			orth = meta[q].orth_on_parent;
 		}
@@ -1523,6 +1534,77 @@ template <int OP> __global__ void reduce_stage2(int nb, const double *__restrict
 		double x = threadIdx.x < (blockDim.x >> 5) ? ws[threadIdx.x] : 0.0;
 		x        = OP == 0 ? warp_sum(x) : warp_max(x);
 		if (threadIdx.x == 0) *result = x;
+	}
+}
+
+// ---------------------------------------------------------------------------------------------
+// ||f - A u_new||^2 right after a sweep, from face data: by the identity of face_residual_restrict_kernel the residual
+// is (2/h^2) E^T (gamma(u_old) - gamma(u_new)), zero away from the patch boundary cells, so only the S x M entries of
+// the sides are evaluated.  A cell on several sides (edges, corners) takes the sum of their terms in side order (as
+// frr_patch) and is counted once, by the first side it lies on.  MODE: FV_DIFF (u_old's slices in Fold) or
+// FV_PROLONG_DIFF (u_old = Fold + P uc on the boundary cells: the input of a first post-sweep).  One patch per CTA
+// iteration, [S][M] terms staged in shared memory; one partial sum per CTA in partial[blockIdx.x].
+// ---------------------------------------------------------------------------------------------
+template <int D, int N> constexpr int frn_threads()
+{
+	return 2 * D * Geo<D, N>::M >= TGPU_THREADS ? TGPU_THREADS : (2 * D * Geo<D, N>::M + 31) / 32 * 32;
+}
+template <int D, int N> constexpr size_t frn_smem_bytes() { return (size_t) 2 * D * Geo<D, N>::M * sizeof(double); }
+// index of cell c in the slice of side s (face_cell inverted)
+template <int D, int N> __device__ __forceinline__ int face_index(int s, const int (&c)[3])
+{
+	const int ax = s >> 1;
+	if (D == 2) return c[1 - ax];
+	if (ax == 0) return c[1] + N * c[2];
+	if (ax == 1) return c[0] + N * c[2];
+	return c[0] + N * c[1];
+}
+template <int D, int N, int MODE>
+__global__ void __launch_bounds__(TGPU_THREADS)
+face_residual_norm_kernel(const PatchMeta *__restrict__ meta, int P, const double *__restrict__ Fnew, const double *__restrict__ Fold,
+                          const double *__restrict__ uc, double *__restrict__ partial)
+{
+	using G = Geo<D, N>;
+	pdl_launch_dependents();
+	pdl_wait();
+	extern __shared__ double Rs[]; // [S][M]
+	const FaceVals<D, N, MODE> fv{Fnew, MODE == FV_DIFF ? Fold : uc, meta, Fold};
+	double acc = 0.0;
+	for (int p = blockIdx.x; p < P; p += gridDim.x) {
+		const PatchMeta &pm   = meta[p];
+		const double     cfac = 2.0 * pm.inv_h2;
+		for (int m = threadIdx.x; m < G::M; m += blockDim.x) {
+			int    ty[G::S];
+			double own[G::S], gm[G::S];
+			gamma_all_sides(pm, p, m, fv, ty, own, gm);
+#pragma unroll
+			for (int s = 0; s < G::S; s++) Rs[s * G::M + m] = (ty[s] == NBR_NONE) ? 0.0 : cfac * gm[s];
+		}
+		__syncthreads();
+		for (int e = threadIdx.x; e < G::S * G::M; e += blockDim.x) {
+			const int s = e / G::M;
+			int       c[3];
+			face_cell<D, N>(s, e % G::M, c);
+			double v     = 0.0;
+			int    first = -1;
+#pragma unroll
+			for (int s2 = 0; s2 < G::S; s2++) {
+				if (c[s2 >> 1] != ((s2 & 1) ? N - 1 : 0)) continue;
+				if (first < 0) first = s2;
+				v += Rs[s2 * G::M + face_index<D, N>(s2, c)];
+			}
+			if (first == s) acc = fma(v, v, acc);
+		}
+		__syncthreads();
+	}
+	__shared__ double ws[32];
+	acc = warp_sum(acc);
+	if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = acc;
+	__syncthreads();
+	if (threadIdx.x < 32) {
+		double x = threadIdx.x < (blockDim.x >> 5) ? ws[threadIdx.x] : 0.0;
+		x        = warp_sum(x);
+		if (threadIdx.x == 0) partial[blockIdx.x] = x;
 	}
 }
 

@@ -218,7 +218,9 @@ struct LevelDev {
 
 struct GraphEntry {
 	bool    want_faces = false;
+	bool    guess      = false;
 	double *faces      = nullptr;
+	const double *faces_old = nullptr, *faces_uc = nullptr;
 	const double *  f;
 	double *        u;
 	TgpuCycleOpts   opts;
@@ -232,10 +234,14 @@ struct tgpu_hier {
 	std::vector<LevelDev> levels;
 	double *              scratch32 = nullptr; // smooth3d32n_kernel (32^3 levels with Neumann sides): one 256 KB block per CTA
 	double *              cycle_faces = nullptr; // boundary slices of the last cycle's result (level 0), if it was asked to emit them
+	// ... and of the iterate before its last sweep: cycle_faces_old, plus P cycle_uc on the boundary cells if that sweep was
+	// the first post-sweep (cycle_uc == nullptr otherwise); see k_face_residual_norm
+	const double *        cycle_faces_old = nullptr, *cycle_uc = nullptr;
 	double *              tri = nullptr; // [N/2 + 1][N^(D-1)] tridiagonal multipliers (TriSolve)
 	double *              mats = nullptr, *lam = nullptr; // Neumann patches: transform matrices [6][N][N], 1-D eigenvalues [3][N]
 	std::vector<GraphEntry> graphs;
 	std::vector<tgpu_vec *> krylov_ws;
+	std::vector<tgpu_vec *> gmg_ws; // stationary solve: residual and correction of the schedules without a start from a guess
 	double *              krylov_sc = nullptr; // BiCGStab scalars on the device
 	tgpu_vec *            host_f = nullptr, *host_u = nullptr;
 	// pipelined host-buffer path (tgpu_vcycle_host_async): two slots, copy-in / copy-out streams
@@ -442,6 +448,8 @@ static int setup_3d32(tgpu_hier *h)
 	CU(cudaFuncSetAttribute(face_residual_restrict_big_kernel<3, 32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 6 * 1024 * 8));
 	CU(cudaFuncSetAttribute(face_residual_restrict_big_kernel<3, 32, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 6 * 1024 * 8));
 	CU(cudaFuncSetAttribute(face_residual_restrict_big_kernel<3, 32, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 6 * 1024 * 8));
+	CU(cudaFuncSetAttribute(face_residual_norm_kernel<3, 32, FV_DIFF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) frn_smem_bytes<3, 32>()));
+	CU(cudaFuncSetAttribute(face_residual_norm_kernel<3, 32, FV_PROLONG_DIFF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) frn_smem_bytes<3, 32>()));
 	for (const LevelDev &L : h->levels)
 		if (L.has_neumann && !h->scratch32) CU(cudaMalloc(&h->scratch32, (size_t) h->ctx->sm_count * 2 * 32768 * sizeof(double)));
 	return TGPU_OK;
@@ -1213,6 +1221,7 @@ extern "C" int tgpu_hierarchy_destroy(tgpu_hier *h)
 	cudaStreamSynchronize(h->ctx->stream);
 	free_graphs(h);
 	for (tgpu_vec *v : h->krylov_ws) tgpu_vec_destroy(v);
+	for (tgpu_vec *v : h->gmg_ws) tgpu_vec_destroy(v);
 	tgpu_vec_destroy(h->host_f);
 	tgpu_vec_destroy(h->host_u);
 	for (int k = 0; k < 2; k++) {
@@ -1282,6 +1291,8 @@ extern "C" int tgpu_hierarchy_trim(tgpu_hier *h)
 	free_graphs(h);
 	for (tgpu_vec *v : h->krylov_ws) tgpu_vec_destroy(v);
 	h->krylov_ws.clear();
+	for (tgpu_vec *v : h->gmg_ws) tgpu_vec_destroy(v);
+	h->gmg_ws.clear();
 	tgpu_vec_destroy(h->host_f), h->host_f = nullptr;
 	tgpu_vec_destroy(h->host_u), h->host_u = nullptr;
 	for (int k = 0; k < 2; k++) {
@@ -2127,7 +2138,10 @@ static int exchange_async(tgpu_hier *h, int l, double *F, const double *uc, cuda
 // materialised: the zero fill of u, the pre-smoothed u itself, the fine residual vector and the interior
 // of the prolonged u; only the last sweep of a level visit writes u.  opts.fused = 2 keeps the PR-1 form
 // of the middle step (residual evaluated from u and f by apply_tma_kernel<2>) for cross-checking.
-static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double *f, double *u, bool want_faces)
+// guess (level 0 of a cycle with coarser levels): start from the iterate in u instead of zero.  The first pre-sweep needs
+// only u's boundary slices, extracted into Fcur; from there every pre-sweep is the non-zero-guess sweep of i > 0, so
+// one cycle computes u + Cycle(f - A u) (the smoother is linear and stationary).  Coarser levels start from zero.
+static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double *f, double *u, bool want_faces, bool guess = false)
 {
 	const int last = h->last_level;
 	LevelDev &L    = h->levels[l];
@@ -2144,14 +2158,16 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 	}
 	const bool from_faces = (o.fused != 2);
 	LevelDev & C          = h->levels[l + 1];
+	if (guess) TRY(k_extract_faces(h, l, u, Fcur));
 	for (int i = 0; i < o.pre_sweeps; i++) {
-		if (i > 0) TRY(k_exchange(h, l, Fcur, nullptr));
-		TRY(k_smooth(h, l, i == 0, true, f, u, Fcur, i == 0 ? Fcur : Falt, nullptr, 0, -1, !from_faces));
-		if (i > 0) TRY(k_exchange_done(h, l));
-		if (i > 0) std::swap(Fcur, Falt);
+		const bool nonzero = guess || i > 0;
+		if (nonzero) TRY(k_exchange(h, l, Fcur, nullptr));
+		TRY(k_smooth(h, l, !nonzero, true, f, u, Fcur, nonzero ? Falt : Fcur, nullptr, 0, -1, !from_faces));
+		if (nonzero) TRY(k_exchange_done(h, l));
+		if (nonzero) std::swap(Fcur, Falt);
 	}
-	// Fcur: faces of the pre-smoothed u; Falt: faces of the iterate before the last pre-sweep (if pre_sweeps > 1)
-	const double *Fold    = o.pre_sweeps > 1 ? Falt : nullptr;
+	// Fcur: faces of the pre-smoothed u; Falt: faces of the iterate before the last pre-sweep (if it did not start from zero)
+	const double *Fold    = (guess || o.pre_sweeps > 1) ? Falt : nullptr;
 	const bool    overlap = exchanges(h, l);
 	auto residual_restrict = [&](int p0, int p1) {
 		if (from_faces) return k_face_residual_restrict(h, l, Fcur, Fold, C.f, p0, p1);
@@ -2222,7 +2238,11 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 		}
 		std::swap(Fcur, Falt);
 	}
-	if (l == 0 && want_faces) h->cycle_faces = Fcur; // the last sweep emitted the slices of u here
+	if (l == 0 && want_faces) { // the last sweep emitted the slices of u here; Falt holds those of its input
+		h->cycle_faces     = Fcur;
+		h->cycle_faces_old = Falt;
+		h->cycle_uc        = o.post_sweeps == 1 ? C.u : nullptr;
+	}
 	return TGPU_OK;
 }
 // the fused schedule covers cycles with at least one sweep everywhere and the piecewise-constant interpolator: V cycles on
@@ -2234,19 +2254,22 @@ static bool fused_schedule(const TgpuCycleOpts &o, int nranks)
 }
 // want_faces: the caller applies the operator to the result next (BiCGStab: v = A M^-1 p), so the last sweep also
 // writes the result's boundary slices (h->cycle_faces != nullptr afterwards) and no extraction pass is needed
-static int run_cycle(tgpu_hier *h, const TgpuCycleOpts &o, const double *f, double *u, bool want_faces = false)
+// guess: start from the iterate in u (guess_schedule must hold)
+static int run_cycle(tgpu_hier *h, const TgpuCycleOpts &o, const double *f, double *u, bool want_faces = false, bool guess = false)
 {
 	const bool fused = fused_schedule(o, h->ctx->nranks);
 	h->cycle_faces   = nullptr;
-	if (fused) return fused_visit(h, o, 0, f, u, want_faces && h->last_level > 0);
+	h->cycle_faces_old = h->cycle_uc = nullptr;
+	if (fused) return fused_visit(h, o, 0, f, u, want_faces && h->last_level > 0, guess);
+	if (guess) return fail(TGPU_ERR_ARG, "run_cycle: this schedule cannot start from a guess");
 	TRY(k_set(h, u, h->levels[0].ncells, 0.0)); // Cycle::apply: u->set(0)
 	return generic_visit(h, o, 0, f, u);
 }
 static bool same_opts(const TgpuCycleOpts &a, const TgpuCycleOpts &b) { return memcmp(&a, &b, sizeof(a)) == 0; }
 
-static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, double *u, bool want_faces = false)
+// the options a cycle runs with (opts == NULL: defaults), checked, and the coarsest level it visits (h->last_level)
+static int cycle_opts(tgpu_hier *h, const TgpuCycleOpts *opts, TgpuCycleOpts &o)
 {
-	TgpuCycleOpts o;
 	if (opts) o = *opts;
 	else tgpu_cycle_opts_default(&o);
 	o.reserved_ = 0;
@@ -2265,15 +2288,31 @@ static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, d
 		if ((double) h->levels[l].global_P / ctx->nranks < o.patches_per_proc) break;
 		h->last_level = l;
 	}
+	return TGPU_OK;
+}
+// the fused schedule starts from a guess on level 0 when the face identity holds for its sweeps (no shifted patch solve)
+// and there is a coarser level; cycle_opts must have run
+static bool guess_schedule(const tgpu_hier *h, const TgpuCycleOpts &o)
+{
+	return fused_schedule(o, h->ctx->nranks) && h->lambda == 0.0 && h->last_level > 0;
+}
+static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, double *u, bool want_faces = false, bool guess = false)
+{
+	TgpuCycleOpts o;
+	TRY(cycle_opts(h, opts, o));
+	tgpu_ctx *ctx = h->ctx;
+	if (guess && !guess_schedule(h, o)) return fail(TGPU_ERR_ARG, "cycle_ptr: this schedule cannot start from a guess");
 	for (size_t l = 0; l <= (size_t) h->last_level; l++) {
 		const bool fused_sched = fused_schedule(o, ctx->nranks);
 		TRY(ensure_work(h, (int) l, !fused_sched || (o.fused == 2 && is_3d32(h))));
 	}
 	for (int l = 0; l <= h->last_level; l++) TRY(ensure_push_desc(h, l));
-	if (!o.use_graph || ctx->profiling || (ctx->nranks > 1 && o.use_graph < 2)) return run_cycle(h, o, f, u, want_faces);
+	if (!o.use_graph || ctx->profiling || (ctx->nranks > 1 && o.use_graph < 2)) return run_cycle(h, o, f, u, want_faces, guess);
 	for (GraphEntry &g : h->graphs)
-		if (g.f == f && g.u == u && g.want_faces == want_faces && same_opts(g.opts, o)) {
-			h->cycle_faces = g.faces;
+		if (g.f == f && g.u == u && g.want_faces == want_faces && g.guess == guess && same_opts(g.opts, o)) {
+			h->cycle_faces     = g.faces;
+			h->cycle_faces_old = g.faces_old;
+			h->cycle_uc        = g.faces_uc;
 			CU(cudaGraphLaunch(g.exec, ctx->stream));
 			ctx->launches += g.kernels;
 			return TGPU_OK;
@@ -2283,7 +2322,7 @@ static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, d
 	ctx->capturing    = true;
 	ctx->captured     = 0;
 	CU(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-	int         rc = run_cycle(h, o, f, u, want_faces);
+	int         rc = run_cycle(h, o, f, u, want_faces, guess);
 	cudaError_t e  = cudaStreamEndCapture(ctx->stream, &graph);
 	ctx->capturing = false;
 	if (rc != TGPU_OK) {
@@ -2294,6 +2333,7 @@ static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, d
 	GraphEntry g;
 	g.f = f, g.u = u, g.opts = o, g.kernels = ctx->captured;
 	g.want_faces = want_faces, g.faces = h->cycle_faces;
+	g.guess = guess, g.faces_old = h->cycle_faces_old, g.faces_uc = h->cycle_uc;
 	CU(cudaGraphInstantiate(&g.exec, graph, 0));
 	cudaGraphDestroy(graph);
 	if (h->graphs.size() >= 8) {
@@ -2578,6 +2618,165 @@ extern "C" int tgpu_bicgstab(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu
 	}
 	if (iterations) *iterations = its;
 	if (rel_residual) *rel_residual = rn / r0_norm;
+	return TGPU_OK;
+	API_END
+}
+
+// ------------------------------------------------------------------------------------------
+// stationary multigrid: u <- u + Cycle(f - A u), from the iterate in u
+// ------------------------------------------------------------------------------------------
+// sum of squares of level vector v into ctx->d_result[0] (all ranks), no host read
+static int k_sumsq(tgpu_hier *h, const double *v, size_t n)
+{
+	tgpu_ctx *ctx = h->ctx;
+	const int nb  = std::min(MAX_PARTIAL, grid_for(ctx, n, 256, 8));
+	Tag       tg(ctx, "reduce", 0);
+	TRY(launch(ctx, reduce_stage1<0>, dim3(nb), dim3(256), 0, n, v, v, ctx->d_partial));
+	TRY(launch(ctx, reduce_stage2<0>, dim3(1), dim3(256), 0, nb, (const double *) ctx->d_partial, ctx->d_result));
+	if (ctx->nranks > 1 && h->levels[0].distributed) NC(g_nccl.AllReduce(ctx->d_result, ctx->d_result, 1, ncclDouble, ncclSum, ctx->comm, ctx->stream));
+	return TGPU_OK;
+}
+// ||f - A u||^2 of the full residual (r: work vector) into ctx->d_result[0]
+static int k_residual_sumsq(tgpu_hier *h, const double *f, const double *u, double *r)
+{
+	LevelDev &L = h->levels[0];
+	TRY(k_extract_faces(h, 0, u, L.Fa));
+	TRY(k_exchange(h, 0, L.Fa, nullptr));
+	TRY(k_apply(h, 0, 1, u, f, L.Fa, r, nullptr));
+	TRY(k_exchange_done(h, 0));
+	return k_sumsq(h, r, L.ncells);
+}
+// ||f - A u||^2 into ctx->d_result[0] right after a cycle that emitted the slices of its result u and kept those of the
+// input of its last sweep (h->cycle_faces, h->cycle_faces_old, h->cycle_uc): face_residual_norm_kernel.  Reads S x M
+// values of two face buffers per patch; neither u nor f.  The neighbours' new slices reach the halo slots first.
+static int k_face_residual_norm(tgpu_hier *h)
+{
+	LevelDev &L   = h->levels[0];
+	tgpu_ctx *ctx = h->ctx;
+	double *  Fnew = h->cycle_faces;
+	const double *Fold = h->cycle_faces_old, *uc = h->cycle_uc;
+	if (!Fnew || !Fold) return fail(TGPU_ERR_ARG, "k_face_residual_norm: the cycle kept no boundary slices");
+	TRY(k_exchange(h, 0, Fnew, nullptr));
+	const int nb = std::max(1, std::min({L.P, ctx->sm_count * 8, MAX_PARTIAL}));
+	{
+		Tag tg(ctx, "face_residual_norm", 0);
+		DISPATCH_DN_ALL(h->D, h->N, {
+			const dim3   block(frn_threads<DD, NN>());
+			const size_t sm = frn_smem_bytes<DD, NN>();
+			if (uc) TRY(launch(ctx, face_residual_norm_kernel<DD, NN, FV_PROLONG_DIFF>, dim3(nb), block, sm, (const PatchMeta *) L.meta, L.P, (const double *) Fnew, Fold, uc, ctx->d_partial));
+			else TRY(launch(ctx, face_residual_norm_kernel<DD, NN, FV_DIFF>, dim3(nb), block, sm, (const PatchMeta *) L.meta, L.P, (const double *) Fnew, Fold, uc, ctx->d_partial));
+		});
+		TRY(launch(ctx, reduce_stage2<0>, dim3(1), dim3(256), 0, nb, (const double *) ctx->d_partial, ctx->d_result));
+	}
+	TRY(k_exchange_done(h, 0));
+	if (ctx->nranks > 1 && L.distributed) NC(g_nccl.AllReduce(ctx->d_result, ctx->d_result, 1, ncclDouble, ncclSum, ctx->comm, ctx->stream));
+	return TGPU_OK;
+}
+// host read of ctx->d_result[0 .. n)
+static int read_result(tgpu_ctx *ctx, double *out, int n = 1)
+{
+	CU(cudaMemcpyAsync(ctx->h_result, ctx->d_result, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+	CU(cudaStreamSynchronize(ctx->stream));
+	for (int i = 0; i < n; i++) out[i] = ctx->h_result[i];
+	return check_comm(ctx);
+}
+static int check_stationary_args(tgpu_hier *h, const tgpu_vec *f, const tgpu_vec *u, const char *what)
+{
+	TRY(check_level_vec(h, 0, f, what));
+	TRY(check_level_vec(h, 0, u, what));
+	if (f == u) return fail(TGPU_ERR_ARG, std::string(what) + ": f must not alias u");
+	return TGPU_OK;
+}
+static int ensure_gmg_ws(tgpu_hier *h)
+{
+	while (h->gmg_ws.size() < 2) {
+		tgpu_vec *v = nullptr;
+		TRY(tgpu_vec_create(h, 0, &v));
+		h->gmg_ws.push_back(v);
+	}
+	return TGPU_OK;
+}
+// one update u <- u + Cycle(f - A u); want_norm: ||f - A u_new||^2 in ctx->d_result[0] afterwards.  The fused schedule
+// starts from u (guess_schedule) and takes the norm from the faces; every other schedule runs the loop it replaces:
+// residual into a work vector, the cycle from zero, add, and (want_norm) a full residual of the result.
+static int update_once(tgpu_hier *h, const TgpuCycleOpts *opts, const TgpuCycleOpts &o, const tgpu_vec *f, tgpu_vec *u, bool want_norm)
+{
+	if (guess_schedule(h, o)) {
+		TRY(cycle_ptr(h, opts, f->d, u->d, want_norm, true));
+		return want_norm ? k_face_residual_norm(h) : TGPU_OK;
+	}
+	TRY(ensure_gmg_ws(h));
+	tgpu_vec *r = h->gmg_ws[0], *e = h->gmg_ws[1];
+	TRY(tgpu_residual(h, 0, f, u, r));
+	TRY(cycle_ptr(h, opts, r->d, e->d));
+	TRY(tgpu_vec_add(u, e));
+	return want_norm ? k_residual_sumsq(h, f->d, u->d, r->d) : TGPU_OK;
+}
+extern "C" int tgpu_vcycle_update(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu_vec *u, double *rel_residual)
+{
+	API_BEGIN
+	TRY(check_stationary_args(h, f, u, "tgpu_vcycle_update"));
+	TgpuCycleOpts o;
+	TRY(cycle_opts(h, opts, o));
+	TRY(update_once(h, opts, o, f, u, rel_residual != nullptr));
+	if (!rel_residual) return TGPU_OK;
+	double rr[2];
+	CU(cudaMemcpyAsync(h->ctx->d_result + 1, h->ctx->d_result, sizeof(double), cudaMemcpyDeviceToDevice, h->ctx->stream));
+	TRY(k_sumsq(h, f->d, f->n));
+	TRY(read_result(h->ctx, rr, 2)); // ||f||^2, ||f - A u||^2
+	*rel_residual = rr[0] > 0.0 ? sqrt(rr[1] / rr[0]) : sqrt(rr[1]);
+	return TGPU_OK;
+	API_END
+}
+// Stationary iteration of update_once.  The fused schedule iterates on the face norm and reports convergence only after a
+// full residual confirms it (the face norm leaves out the patch solve's rounding noise, ~1e-16 relative); one host read of
+// one double per cycle.
+extern "C" int tgpu_gmg_solve(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu_vec *u, double tol, int max_it,
+                              int *iterations, double *rel_residual, double *history)
+{
+	API_BEGIN
+	TRY(check_stationary_args(h, f, u, "tgpu_gmg_solve"));
+	if (!(tol >= 0.0) || max_it < 0) return fail(TGPU_ERR_ARG, "tgpu_gmg_solve: tol and max_it must not be negative");
+	TgpuCycleOpts o;
+	TRY(cycle_opts(h, opts, o));
+	tgpu_ctx *ctx = h->ctx;
+	TRY(ensure_gmg_ws(h));
+	double *r = h->gmg_ws[0]->d;
+	double  fsq, rsq;
+	TRY(k_sumsq(h, f->d, f->n));
+	TRY(read_result(ctx, &fsq));
+	const double scale = fsq > 0.0 ? 1.0 / sqrt(fsq) : 1.0; // f = 0: absolute residuals
+	TRY(k_residual_sumsq(h, f->d, u->d, r));
+	TRY(read_result(ctx, &rsq));
+	double rel = sqrt(rsq) * scale;
+	if (history) history[0] = rel;
+	bool converged = rel <= tol;
+	int  its       = 0;
+	const bool fused = guess_schedule(h, o);
+	while (!converged && its < max_it) {
+		if (fused) {
+			TRY(update_once(h, opts, o, f, u, true));
+			TRY(read_result(ctx, &rsq));
+			rel = sqrt(rsq) * scale;
+			if (rel <= tol) { // confirmation by the full residual
+				TRY(k_residual_sumsq(h, f->d, u->d, r));
+				TRY(read_result(ctx, &rsq));
+				rel = sqrt(rsq) * scale;
+			}
+		} else { // the loop: cycle from zero on the residual in gmg_ws[0], add, residual (also the convergence test)
+			tgpu_vec *rv = h->gmg_ws[0], *e = h->gmg_ws[1];
+			TRY(cycle_ptr(h, opts, rv->d, e->d));
+			TRY(tgpu_vec_add(u, e));
+			TRY(k_residual_sumsq(h, f->d, u->d, rv->d));
+			TRY(read_result(ctx, &rsq));
+			rel = sqrt(rsq) * scale;
+		}
+		its++;
+		if (history) history[its] = rel;
+		converged = rel <= tol;
+	}
+	if (iterations) *iterations = its;
+	if (rel_residual) *rel_residual = rel;
 	return TGPU_OK;
 	API_END
 }

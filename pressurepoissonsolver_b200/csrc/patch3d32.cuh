@@ -12,6 +12,7 @@
 // The operator apply for 32^3 patches is apply3d32_tma_kernel (apply_tma.cuh).
 // Reference functions replaced: same as smooth_kernel / face_residual_restrict_kernel.
 #pragma once
+#include <vector>
 
 namespace tgpu
 {
@@ -161,18 +162,67 @@ template <bool PROLONG> struct SideGamma32 {
 //   of six face terms.  The patch solve is linear, so each face term can enter smooth3d32c_kernel where it is uniform over the
 //   sweep's threads: the y faces before the y transform (as they are), the x faces at x = 0 / 31 of the rows of the x
 //   transform (transformed along y), the z faces at elimination step 0 (transformed along y, then x - the sweep's order).
-//   This kernel forms those terms once per patch, in the face-buffer shape G[p][6][1024]:
+//   This kernel forms those terms in the face shape G[slot][1024] (slots: IfaceSlots32 below):
 //     s = 0, 1 (x faces): Dst2_y(c(., z))[k_y]       at k_y + 32 z
 //     s = 2, 3 (y faces): c(x, z)                    at x + 32 z
 //     s = 4, 5 (z faces): Dst2_x(Dst2_y(c))[k_x, k_y] at k_x + 32 k_y
 //   with c = (2/h^2) gamma from the gathers of GDesc32 / SideGamma32 (gamma_entry32 on sides with coarse / fine neighbours),
 //   so the values of c are those the sweep subtracted when it gathered them itself; only where they enter moved.
-//   One warp per patch side, one patch per CTA at a time, a padded 32 x 33 tile per warp for the transposes.  On several
-//   GPUs this kernel is the consumer of the halo hand-over of the first post-sweep (halo_push / halo_wait_cta / halo_finish,
-//   as face_residual_restrict_big_kernel): the sweep after it reads no face data.
+//   One warp per slot, the warps of a CTA independent of each other, a padded 32 x 33 tile per warp for the transposes.  On
+//   several GPUs this kernel is the consumer of the halo hand-over of the first post-sweep (halo_push / halo_wait_warp /
+//   halo_finish, as face_residual_restrict_big_kernel): the sweep after it reads no face data.
 // ---------------------------------------------------------------------------------------------
-constexpr int    IR32_THREADS = 192, IR32_CTAS_PER_SM = 2, IR32_TP = 33;
-constexpr size_t iface_rhs32_smem_bytes() { return sizeof(double) * 6 * 32 * IR32_TP; }
+constexpr int    IR32_THREADS = 192, IR32_WARPS = IR32_THREADS / 32, IR32_CTAS_PER_SM = 2, IR32_TP = 33;
+constexpr size_t iface_rhs32_smem_bytes() { return sizeof(double) * IR32_WARPS * 32 * IR32_TP; }
+
+// Interface slots of a 32^3 level: where G holds the term of each patch side.  Two same-level neighbours p, q see the same
+// term on their common interface: c = 2/h^2 is the same for both, the gather of p's side s loads the four values of q's side
+// s ^ 1 with the halves swapped (c (0.5 (a0 + a1) + 0.5 (b0 + b1)), the sum is commutative), and x, y and z terms use the same
+// layout on both sides.  Such an interface gets one slot, gathered for the lower patch index (its owner), when
+//   - p's side s is NBR_NORMAL to q != p and q's side s ^ 1 is NBR_NORMAL back to p,
+//   - both are owned (index < P: no halo neighbour, so GD_WB stays set on both sides), neither has Neumann sides and both
+//     have the same h.
+// Every other side with a neighbour (coarse / fine / halo / not mutual) has a slot of its own; domain-boundary sides (the term
+// is zero) and patches with Neumann sides (smooth3d32n_kernel gathers for itself) have none.  Slots are numbered in the
+// order of their owner, so the patches [p0, p1) own the slots [begin[p0], begin[p1]); with the lower index as owner, a launch
+// over [p0, p1) after one over [0, p0) (interior patches first, then the ones with halo neighbours) reads only slots written
+// by itself or before.
+struct IfaceSlots32 {
+	std::vector<int32_t> gslot; // [P][6]: slot of side s of patch p, -1: no term
+	std::vector<int32_t> owner; // [nslots]: 6 p + s of the side whose gather produces the slot
+	std::vector<int32_t> begin; // [P + 1]
+};
+inline bool iface_shared32(const PatchMeta *meta, int P, int p, int s)
+{
+	const PatchMeta &a = meta[p];
+	if (a.neumann || a.nbr_type[s] != NBR_NORMAL) return false;
+	const int q = a.nbr_idx[s][0];
+	if (q == p || q < 0 || q >= P) return false;
+	const PatchMeta &b = meta[q];
+	return !b.neumann && b.nbr_type[s ^ 1] == NBR_NORMAL && b.nbr_idx[s ^ 1][0] == p && a.inv_h2 == b.inv_h2;
+}
+inline IfaceSlots32 build_iface_slots32(const PatchMeta *meta, int P)
+{
+	IfaceSlots32 t;
+	t.gslot.assign((size_t) P * 6, -1);
+	t.begin.resize((size_t) P + 1);
+	for (int p = 0; p < P; p++) {
+		t.begin[p] = (int32_t) t.owner.size();
+		if (meta[p].neumann) continue;
+		for (int s = 0; s < 6; s++) {
+			if (meta[p].nbr_type[s] == NBR_NONE) continue;
+			const bool shared = iface_shared32(meta, P, p, s);
+			const int  q      = meta[p].nbr_idx[s][0];
+			if (shared && q < p) continue; // q's slot, set when q was visited
+			const int32_t k = (int32_t) t.owner.size();
+			t.owner.push_back(p * 6 + s);
+			t.gslot[(size_t) p * 6 + s] = k;
+			if (shared) t.gslot[(size_t) q * 6 + (s ^ 1)] = k;
+		}
+	}
+	t.begin[P] = (int32_t) t.owner.size();
+	return t;
+}
 // c of side s of patch p: entry m = lane + 32 i to out[i * stride + lane]; AX = face-normal axis.  Sides with coarse / fine
 // neighbours go entry by entry through the out-of-line gamma_entry32 (SideGamma32::finish); the others keep IR32_BATCH entries'
 // loads in flight per lane and need no call, so that no in-flight load is held across one.
@@ -200,31 +250,30 @@ __device__ __forceinline__ void side_gamma32(const GDesc32 &d, const PatchMeta *
 		for (int j = 0; j < B; j++) out[(i0 + j) * stride + lane] = sg[j].combine(d);
 	}
 }
+// slots [k0, k1) of owner (6 p + s, IfaceSlots32::owner) into G[k]
 template <bool PROLONG, bool HALO>
 __global__ void __launch_bounds__(IR32_THREADS, IR32_CTAS_PER_SM)
-iface_rhs32_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *__restrict__ Fin, const double *__restrict__ uc,
-                   double *__restrict__ Gout, HaloSync hs = HaloSync{}, int skip_neumann = 0)
+iface_rhs32_kernel(const PatchMeta *__restrict__ meta, const int32_t *__restrict__ owner, int k0, int k1, const double *__restrict__ Fin,
+                   const double *__restrict__ uc, double *__restrict__ Gout, HaloSync hs = HaloSync{})
 {
-	// skip_neumann != 0: patches with Neumann domain sides are left out (smooth3d32n_kernel gathers its own interface values)
 	constexpr int N = 32, M = N * N, TP = IR32_TP;
-	extern __shared__ __align__(16) double T[]; // [6 warps][32][TP]
-	__shared__ GPatch32 GD;                     // GD.d[s]: written and read by warp s only
-	const int lane = threadIdx.x & 31, s = threadIdx.x >> 5;
-	double *  tw   = T + s * N * TP;
+	extern __shared__ __align__(16) double T[]; // [IR32_WARPS][32][TP]
+	__shared__ GPatch32 GD[IR32_WARPS];         // GD[w].d[s]: written and read by warp w only
+	const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+	double *  tw   = T + w * N * TP;
 	Mags<N>   mg;
 	mg.load();
 	pdl_launch_dependents();
 	pdl_wait();
 	if (HALO) halo_push<3, 32>(hs, meta);
 	bool halo_ok = false;
-	for (int g = blockIdx.x; g < P - p0; g += gridDim.x) {
-		const int p = p0 + g;
-		if (skip_neumann && meta[p].neumann) continue; // CTA-uniform
-		if (HALO) halo_wait_cta(hs, p, halo_ok);
-		if (lane == 0) make_gdesc32<PROLONG>(meta[p], p, s, GD);
+	for (int k = k0 + blockIdx.x * IR32_WARPS + w; k < k1; k += gridDim.x * IR32_WARPS) {
+		const int ps = __ldg(owner + k), p = ps / 6, s = ps - 6 * p;
+		if (HALO) halo_wait_warp(hs, p, halo_ok);
+		if (lane == 0) make_gdesc32<PROLONG>(meta[p], p, s, GD[w]);
 		__syncwarp();
-		const GDesc32 &d  = GD.d[s];
-		double *       Gp = Gout + ((size_t) p * 6 + s) * M;
+		const GDesc32 &d  = GD[w].d[s];
+		double *       Gp = Gout + (size_t) k * M;
 		double         v[N];
 		if (s < 2) { // x faces: entry (y, z) = (lane, i) -> tile row z; transform along y, pencil z = lane
 			side_gamma32<PROLONG, 0>(d, meta, p, s, lane, Fin, uc, tw, TP);
@@ -257,17 +306,19 @@ iface_rhs32_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 #pragma unroll
 			for (int i = 0; i < N; i++) Gp[lane + N * i] = tw[i * TP + lane];
 		}
-		__syncwarp(); // GD.d[s] and the tile are rewritten for the next patch
+		__syncwarp(); // GD[w] and the tile are rewritten for the next slot
 	}
 	if (HALO) halo_finish(hs);
 }
 
 // Sweeps that do not start from zero take the interface part of the right-hand side from G (iface_rhs32_kernel, launched
-// right before over the same patches): six coalesced loads per thread and patch, issued with the loads of f.
+// right before over the same patches or, for slots owned by a lower patch, earlier): up to six coalesced loads per thread and
+// patch, G[gslot[p][s]], issued with the loads of f; sides without a slot (domain boundary) load and subtract nothing.
 template <bool ZERO_GUESS, bool EMIT, bool WRITE_U>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(C32_THREADS, 1)
 smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *__restrict__ f, double *__restrict__ u,
-                   const double *__restrict__ G, double *__restrict__ Fout, const double *__restrict__ tri, int skip_neumann = 0)
+                   const double *__restrict__ G, double *__restrict__ Fout, const double *__restrict__ tri, int skip_neumann = 0,
+                   const int32_t *__restrict__ gslot = nullptr)
 {
 	// skip_neumann != 0: patches with Neumann domain sides are left to smooth3d32n_kernel (launched over the same range
 	// with only_neumann); both CTAs of the cluster skip together
@@ -301,14 +352,18 @@ smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 		// interface terms (see iface_rhs32_kernel): y faces of pencil (x, z) = (lane, z), x faces of row (k_y, z) = (lane, z),
 		// this half's z face at pencils (k_x, k_y) = (lane, w), (lane, w + 16)
 		double gy0 = 0.0, gy1 = 0.0, gx0 = 0.0, gx1 = 0.0, gz0 = 0.0, gz1 = 0.0;
-		if (!ZERO_GUESS) {
-			const double *Gp = G + (size_t) p * 6 * M;
-			gy0              = __ldcs(Gp + 2 * M + mf);
-			gy1              = __ldcs(Gp + 3 * M + mf);
-			gx0              = __ldcs(Gp + 0 * M + mf);
-			gx1              = __ldcs(Gp + 1 * M + mf);
-			gz0              = __ldcs(Gp + sz * M + lane + N * w);
-			gz1              = __ldcs(Gp + sz * M + lane + N * (w + 16));
+		if (!ZERO_GUESS) { // slot conditions are uniform over the cluster
+			const int2 *gs = reinterpret_cast<const int2 *>(gslot + (size_t) p * 6);
+			const int2  kx = __ldg(gs), ky = __ldg(gs + 1), kz = __ldg(gs + 2);
+			const int   ks = rank == 0 ? kz.x : kz.y;
+			if (ky.x >= 0) gy0 = __ldcs(G + (size_t) ky.x * M + mf);
+			if (ky.y >= 0) gy1 = __ldcs(G + (size_t) ky.y * M + mf);
+			if (kx.x >= 0) gx0 = __ldcs(G + (size_t) kx.x * M + mf);
+			if (kx.y >= 0) gx1 = __ldcs(G + (size_t) kx.y * M + mf);
+			if (ks >= 0) {
+				gz0 = __ldcs(G + (size_t) ks * M + lane + N * w);
+				gz1 = __ldcs(G + (size_t) ks * M + lane + N * (w + 16));
+			}
 		}
 		{ // y forward: pencil (x, z) = (lane, z), straight from memory
 			const double *fp = f + (size_t) p * NC + (size_t) z * M + lane;
@@ -319,8 +374,11 @@ smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 				prefetch_l2(fn);
 				prefetch_l2(fn + 16);
 				if (!ZERO_GUESS && lane < 12) {
-					const double *Gn = G + (size_t) pn * 6 * M + 16 * (lane & 1);
-					prefetch_l2(lane < 8 ? Gn + (lane >> 1) * M + N * z : Gn + sz * M + N * (w + 16 * ((lane >> 1) & 1)));
+					const int kn = __ldg(gslot + (size_t) pn * 6 + (lane < 8 ? lane >> 1 : sz));
+					if (kn >= 0) {
+						const double *Gn = G + (size_t) kn * M + 16 * (lane & 1);
+						prefetch_l2(lane < 8 ? Gn + N * z : Gn + N * (w + 16 * ((lane >> 1) & 1)));
+					}
 				}
 			}
 			if (!ZERO_GUESS) {

@@ -199,7 +199,9 @@ struct LevelDev {
 	double *   starts  = nullptr;
 	double *   spacing = nullptr;
 	double *   Fa = nullptr, *Fb = nullptr; // face buffers
-	double *   G  = nullptr; // 32^3 levels: [P][6][M] interface terms of the sweeps that do not start from zero (iface_rhs32_kernel)
+	double *   G  = nullptr; // 32^3 levels: [nslots][M] interface terms of the sweeps that do not start from zero (iface_rhs32_kernel)
+	int32_t *  gslot = nullptr, *gowner = nullptr; // with G: the slot table (IfaceSlots32), device [P][6] and [nslots]
+	std::vector<int32_t> gbegin;                   // with G: IfaceSlots32::begin on the host (slot range of a patch range)
 	double *   u = nullptr, *f = nullptr, *r = nullptr; // cycle work vectors (lazily allocated)
 	bool       has_neumann = false;
 	int32_t *  neu_list = nullptr;          // device: owned patches with Neumann domain sides, ascending (smooth3d16_kernel<.., NEU>)
@@ -413,17 +415,30 @@ template <bool Z, bool E, bool W> static int set_smem_attr_3d32()
 }
 // G of the 32^3 levels whose sweeps can reach smooth3d32c_kernel from a non-zero guess (iface_rhs32_kernel): lambda = 0 (a
 // shifted patch solve sends every patch through smooth3d32n_kernel) and at least one owned patch without Neumann sides.
-// Called at creation and when lambda changes (never during a graph capture); the graphs are freed before G is.
+template <typename T> static int dev_upload(T **dst, const T *src, size_t count);
+// G holds one term per interface slot (IfaceSlots32, built from the owned patches' metadata with the table).  Called at
+// creation and when lambda changes (never during a graph capture); the graphs are freed before G is.
 static int update_iface_buffers(tgpu_hier *h)
 {
 	if (!is_3d32(h)) return TGPU_OK;
 	for (LevelDev &L : h->levels) {
 		const bool want = h->lambda == 0.0 && L.neu_host.size() < (size_t) L.P;
-		if (want && !L.G) CU(cudaMalloc(&L.G, (size_t) L.P * 6 * 1024 * sizeof(double)));
+		if (want && !L.G) {
+			std::vector<PatchMeta> meta(L.P);
+			CU(cudaMemcpy(meta.data(), L.meta, meta.size() * sizeof(PatchMeta), cudaMemcpyDeviceToHost));
+			const IfaceSlots32 t = build_iface_slots32(meta.data(), L.P);
+			TRY(dev_upload(&L.gslot, t.gslot.data(), t.gslot.size()));
+			TRY(dev_upload(&L.gowner, t.owner.data(), t.owner.size()));
+			CU(cudaMalloc(&L.G, std::max<size_t>(t.owner.size(), 1) * 1024 * sizeof(double)));
+			L.gbegin = t.begin;
+		}
 		if (!want && L.G) {
 			CU(cudaDeviceSynchronize());
 			cudaFree(L.G);
-			L.G = nullptr;
+			cudaFree(L.gslot);
+			cudaFree(L.gowner);
+			L.G = nullptr, L.gslot = L.gowner = nullptr;
+			L.gbegin.clear();
 		}
 	}
 	return TGPU_OK;
@@ -1243,6 +1258,8 @@ extern "C" int tgpu_hierarchy_destroy(tgpu_hier *h)
 			cudaFree(L.Fb);
 		}
 		cudaFree(L.G);
+		cudaFree(L.gslot);
+		cudaFree(L.gowner);
 		cudaFree(L.send_peer);
 		cudaFree(L.send_ridx);
 		cudaFree(L.peer_rank);
@@ -1710,13 +1727,17 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 		if (!zero_guess) {
 			// the interface part of the right-hand side, transformed for the sweep (and the halo hand-over, which it consumes)
 			if (!L.G) return fail(TGPU_ERR_ARG, "k_smooth: interface-term buffer of the 32^3 level missing");
+			// over the slots the patches [p0, p1) own (IfaceSlots32), one warp per slot; at least one CTA, which does the
+			// hand-over when the range owns none
 			Tag          ti(h->ctx, "iface_rhs", l);
-			const dim3   gi(std::min(p1 - p0, h->ctx->sm_count * IR32_CTAS_PER_SM)), bi(IR32_THREADS);
+			const int    k0 = L.gbegin[p0], k1 = L.gbegin[p1];
+			const dim3   gi(std::max(1, std::min((k1 - k0 + IR32_WARPS - 1) / IR32_WARPS, h->ctx->sm_count * IR32_CTAS_PER_SM))), bi(IR32_THREADS);
 			const size_t si = iface_rhs32_smem_bytes();
-			if (hs.enabled && prolong) TRY(launch(h->ctx, iface_rhs32_kernel<true, true>, gi, bi, si, meta, p0, p1, Fin, uc, L.G, hs, skipn));
-			else if (hs.enabled) TRY(launch(h->ctx, iface_rhs32_kernel<false, true>, gi, bi, si, meta, p0, p1, Fin, uc, L.G, hs, skipn));
-			else if (prolong) TRY(launch(h->ctx, iface_rhs32_kernel<true, false>, gi, bi, si, meta, p0, p1, Fin, uc, L.G, hs, skipn));
-			else TRY(launch(h->ctx, iface_rhs32_kernel<false, false>, gi, bi, si, meta, p0, p1, Fin, uc, L.G, hs, skipn));
+			const int32_t *own = L.gowner;
+			if (hs.enabled && prolong) TRY(launch(h->ctx, iface_rhs32_kernel<true, true>, gi, bi, si, meta, own, k0, k1, Fin, uc, L.G, hs));
+			else if (hs.enabled) TRY(launch(h->ctx, iface_rhs32_kernel<false, true>, gi, bi, si, meta, own, k0, k1, Fin, uc, L.G, hs));
+			else if (prolong) TRY(launch(h->ctx, iface_rhs32_kernel<true, false>, gi, bi, si, meta, own, k0, k1, Fin, uc, L.G, hs));
+			else TRY(launch(h->ctx, iface_rhs32_kernel<false, false>, gi, bi, si, meta, own, k0, k1, Fin, uc, L.G, hs));
 		} else if (hs.enabled) {
 			return fail(TGPU_ERR_ARG, "smooth3d32c: no halo hand-over in a zero-guess sweep");
 		}
@@ -1724,7 +1745,7 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 		const dim3 grid(2 * std::min(p1 - p0, h->ctx->sm_count / 2)), block(C32_THREADS);
 		return smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto, auto W) {
 			return launch(h->ctx, smooth3d32c_kernel<Z, E, W>, grid, block, smooth3d32c_smem_bytes<Z>(), meta, p0, p1, f, u,
-			              (const double *) L.G, Fout, (const double *) h->tri, skipn);
+			              (const double *) L.G, Fout, (const double *) h->tri, skipn, (const int32_t *) L.gslot);
 		});
 	}
 	// 16^3 levels that contain patches with Neumann domain sides: the specialised kernel sweeps the Dirichlet patches of the

@@ -57,7 +57,7 @@ template <typename F> static float time_it(const char *name, int reps, double by
 	float ms;
 	cudaEventElapsedTime(&ms, e0, e1);
 	ms /= reps;
-	printf("%-40s %8.2f us   %7.1f GB/s (algorithmic)\n", name, ms * 1e3, bytes / ms / 1e6);
+	printf("%-52s %8.2f us   %7.1f GB/s (algorithmic)\n", name, ms * 1e3, bytes / ms / 1e6);
 	return ms;
 }
 
@@ -99,37 +99,73 @@ int main(int argc, char **argv)
 		CK(cudaMemcpyToSymbol(c_mag32, mag.data(), 33 * 8));
 	}
 	const size_t smZ = smooth3d32c_smem_bytes<true>(), smC = smooth3d32c_smem_bytes<false>(), smI = iface_rhs32_smem_bytes();
-	const int    gridC = 2 * std::min(P, sms / 2), gridI = std::min(P, sms * IR32_CTAS_PER_SM);
-	printf("G=%d P=%d cells=%zu cluster grid=%d smem %zu / %zu (zero guess / not), iface_rhs32 grid=%d smem %zu\n", G, P, nc, gridC, smZ, smC, gridI, smI);
+	const int    gridC = 2 * std::min(P, sms / 2);
+	printf("G=%d P=%d cells=%zu cluster grid=%d smem %zu / %zu (zero guess / not), iface_rhs32 smem %zu\n", G, P, nc, gridC, smZ, smC, smI);
 	const double b16 = 16.0 * nc;
+	// interface slots: the library's table (one term per same-level interface, none on domain-boundary sides) and, for
+	// comparison, one slot per side with a neighbour
+	const IfaceSlots32 ts = build_iface_slots32(hm.data(), P);
+	IfaceSlots32       tu;
+	tu.gslot.assign((size_t) P * 6, -1);
+	for (int p = 0; p < P; p++)
+		for (int s = 0; s < 6; s++)
+			if (hm[p].nbr_type[s] != NBR_NONE) tu.gslot[(size_t) p * 6 + s] = (int32_t) tu.owner.size(), tu.owner.push_back(p * 6 + s);
+	const int nsh = (int) ts.owner.size(), nun = (int) tu.owner.size();
+	printf("interface slots: %d shared, %d one per side (%d sides)\n", nsh, nun, 6 * P);
+	int32_t *gslot_s, *gslot_u, *own_s, *own_u;
+	CK(cudaMalloc(&gslot_s, ts.gslot.size() * 4)); CK(cudaMalloc(&gslot_u, tu.gslot.size() * 4));
+	CK(cudaMalloc(&own_s, std::max(nsh, 1) * 4)); CK(cudaMalloc(&own_u, std::max(nun, 1) * 4));
+	CK(cudaMemcpy(gslot_s, ts.gslot.data(), ts.gslot.size() * 4, cudaMemcpyHostToDevice));
+	CK(cudaMemcpy(gslot_u, tu.gslot.data(), tu.gslot.size() * 4, cudaMemcpyHostToDevice));
+	CK(cudaMemcpy(own_s, ts.owner.data(), nsh * 4, cudaMemcpyHostToDevice));
+	CK(cudaMemcpy(own_u, tu.owner.data(), nun * 4, cudaMemcpyHostToDevice));
 	double *Gv;
-	CK(cudaMalloc(&Gv, nf * 8));
+	CK(cudaMalloc(&Gv, std::max<size_t>(nun, 1) * M * 8));
 	CK(cudaFuncSetAttribute(iface_rhs32_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smI));
 	CK(cudaFuncSetAttribute(iface_rhs32_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smI));
+	bool          shared = true; // which table iface() and the sweeps use
+	const int32_t *gslot = gslot_s;
 	auto iface = [&](bool prolong) {
-		if (prolong) iface_rhs32_kernel<true, false><<<gridI, IR32_THREADS, smI>>>(meta, 0, P, Fa, uc, Gv);
-		else iface_rhs32_kernel<false, false><<<gridI, IR32_THREADS, smI>>>(meta, 0, P, Fa, uc, Gv);
+		const int      n     = shared ? nsh : nun;
+		const int32_t *own   = shared ? own_s : own_u;
+		const int      gridI = std::max(1, std::min((n + IR32_WARPS - 1) / IR32_WARPS, sms * IR32_CTAS_PER_SM));
+		if (prolong) iface_rhs32_kernel<true, false><<<gridI, IR32_THREADS, smI>>>(meta, own, 0, n, Fa, uc, Gv);
+		else iface_rhs32_kernel<false, false><<<gridI, IR32_THREADS, smI>>>(meta, own, 0, n, Fa, uc, Gv);
 	};
 #define VARIANT(NAME, Z, E, W, PRE)                                                                                              \
 	{                                                                                                                            \
 		const size_t sm_ = smooth3d32c_smem_bytes<Z>();                                                                          \
 		CK(cudaFuncSetAttribute(smooth3d32c_kernel<Z, E, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sm_));            \
 		CK(cudaMemset(u, 0, nc * 8)); CK(cudaMemset(Fb, 0, nf * 8));                                                             \
-		time_it(NAME, reps, b16, [&] { PRE; smooth3d32c_kernel<Z, E, W><<<gridC, C32_THREADS, sm_>>>(meta, 0, P, f, u, Gv, Fb, tri); }); \
+		time_it(NAME, reps, b16, [&] { PRE; smooth3d32c_kernel<Z, E, W><<<gridC, C32_THREADS, sm_>>>(meta, 0, P, f, u, Gv, Fb, tri, 0, gslot); }); \
 		CK(cudaGetLastError());                                                                                                  \
 	}
 	VARIANT("zero_guess faces-only", true, true, false, )
 	VARIANT("zero_guess write_u", true, false, true, )
 	VARIANT("zero_guess write_u+faces", true, true, true, )
 	// sweeps that do not start from zero: the interface terms (iface_rhs32_kernel) alone, the sweep alone (reading the terms
-	// left by the previous launch), and the two back to back as the library launches them
-	time_it("iface_rhs32 plain", reps, 8.0 * nf, [&] { iface(false); });
-	VARIANT("sweep write_u+faces", false, true, true, )
-	VARIANT("iface_rhs32 plain + sweep write_u+faces", false, true, true, iface(false))
-	if (G > 1) {
-		time_it("iface_rhs32 prolong", reps, 8.0 * nf, [&] { iface(true); });
-		VARIANT("sweep write_u", false, false, true, )
-		VARIANT("iface_rhs32 prolong + sweep write_u", false, false, true, iface(true))
+	// left by the previous launch), and the two back to back as the library launches them; with the shared slots, then with
+	// one slot per side
+	for (int sh = 1; sh >= 0; sh--) {
+		shared = sh != 0;
+		gslot  = shared ? gslot_s : gslot_u;
+		const char *tag = shared ? "[shared]  " : "[per side]";
+		char        name[96];
+		const double bi = 8.0 * M * (shared ? nsh : nun);
+		snprintf(name, sizeof name, "%s iface_rhs32 plain", tag);
+		time_it(name, reps, bi, [&] { iface(false); });
+		snprintf(name, sizeof name, "%s sweep write_u+faces", tag);
+		VARIANT(name, false, true, true, )
+		snprintf(name, sizeof name, "%s iface_rhs32 plain + sweep write_u+faces", tag);
+		VARIANT(name, false, true, true, iface(false))
+		if (G > 1) {
+			snprintf(name, sizeof name, "%s iface_rhs32 prolong", tag);
+			time_it(name, reps, bi, [&] { iface(true); });
+			snprintf(name, sizeof name, "%s sweep write_u", tag);
+			VARIANT(name, false, false, true, )
+			snprintf(name, sizeof name, "%s iface_rhs32 prolong + sweep write_u", tag);
+			VARIANT(name, false, false, true, iface(true))
+		}
 	}
 	return 0;
 }

@@ -382,7 +382,7 @@ template <int D, int N> __device__ __forceinline__ int parent_cell(int orth, con
 // push_faces_kernel) into the peers' halo slots; the last CTA to finish publishes DATA.  The stores then overlap the
 // launch's work on the patches without off-rank neighbours and no separate push launch sits on the critical path.
 // Needs every CTA of the grid to become resident without waiting for another CTA of the same grid to retire (the
-// host clamps the grid to the occupancy, see clamp_resident in launch(), tgpu.cu): CTAs poll for the peers' faces later on, and the
+// host clamps the grid to the occupancy, see halo_launch, tgpu.cu): CTAs poll for the peers' faces later on, and the
 // peers' faces are published by the last of THEIR CTAs.
 // Lives in device memory, one per (level, face buffer, with / without prolongation); written once at set-up.
 // ---------------------------------------------------------------------------------------------

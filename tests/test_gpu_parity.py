@@ -6,7 +6,6 @@ Tolerance: north_star asks for 1e-10 relative L2; fp re-association is all that 
 tests hold the kernels to 1e-12 (1e-10 only for Krylov trajectories)."""
 import os
 import subprocess
-import sys
 import tempfile
 
 import numpy as np
@@ -332,35 +331,26 @@ def test_neumann_rhs_initialiser_vs_reference(ctx):
     mesh.close()
 
 
-@pytest.mark.parametrize("switch", ["TGPU_NEUMANN_FAST", "TGPU_NEUMANN_SPLIT"])
-def test_neumann_alternative_paths(switch):
-    """the paths behind the diagnostic switches - TGPU_NEUMANN_FAST=0: patches with Neumann sides through the size-generic
-    kernel's general path instead of the Neumann instantiation of smooth3d16_kernel; TGPU_NEUMANN_SPLIT=0: whole levels on
-    the general path - give the oracle's cycle too (fresh process: the switches are read once)"""
-    code = (
-        "import os, sys, numpy as np\n"
-        "sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
-        "import pressurepoissonsolver_b200 as pps, gmg_oracle as go\n"
-        "ctx = pps.Context(0)\n"
-        "for mesh_file, n, divide in (('3uni.bin', 16, 1), ('2refine.bin', 16, 0), ('3uni.bin', 32, 0)):\n"
-        "    path = os.path.join(%r, mesh_file)\n"
-        "    mesh = pps.Mesh.load(path, 3).set_neumann(True)\n"
-        "    mesh.refine_leaves(divide)\n"
-        "    h = pps.Hierarchy.from_mesh(ctx, mesh, n)\n"
-        "    levels = go.build_hierarchy(path, 3, n, divide, neumann=True)\n"
-        "    fn = np.random.default_rng(5).standard_normal(levels[0].shape)\n"
-        "    fn -= fn.mean()\n"
-        "    f, u = h.new_vec(0, fn), h.new_vec(0)\n"
-        "    ref = go.vcycle(levels, fn, pre=2, post=2, coarse_sweeps=2)\n"
-        "    for graph in (0, 1):\n"
-        "        h.vcycle(f, u, pps.CycleOpts.default(use_graph=graph, pre_sweeps=2, post_sweeps=2, coarse_sweeps=2))\n"
-        "        err = np.linalg.norm(u.download() - ref.ravel()) / np.linalg.norm(ref)\n"
-        "        assert err < 1e-10, (mesh_file, graph, err)\n"
-        "print('ok', ctx.kernel_launches())\n"
-    ) % (ROOT, os.path.join(ROOT, "oracle"), MESHES)
-    env = dict(os.environ, **{switch: "0"})
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0 and out.stdout.startswith("ok"), out.stdout + out.stderr
+def test_neumann_generic_kernels_vs_oracle(ctx):
+    """16^3 Neumann levels with the size-generic kernels forced: every patch of a level through smooth_kernel's general path
+    instead of the split between the Neumann instantiation and the plain one of smooth3d16_kernel - gives the oracle's cycle too"""
+    for mesh_file, divide in (("3uni.bin", 1), ("2refine.bin", 0)):
+        path = os.path.join(MESHES, mesh_file)
+        mesh = pps.Mesh.load(path, 3).set_neumann(True)
+        mesh.refine_leaves(divide)
+        h = pps.Hierarchy.from_mesh(ctx, mesh, 16)
+        h.force_generic_kernels(True)
+        levels = go.build_hierarchy(path, 3, 16, divide, neumann=True)
+        fn = np.random.default_rng(5).standard_normal(levels[0].shape)
+        fn -= fn.mean()
+        f, u = h.new_vec(0, fn), h.new_vec(0)
+        ref = go.vcycle(levels, fn, pre=2, post=2, coarse_sweeps=2)
+        for graph in (0, 1):
+            h.vcycle(f, u, pps.CycleOpts.default(use_graph=graph, pre_sweeps=2, post_sweeps=2, coarse_sweeps=2))
+            err = np.linalg.norm(u.download() - ref.ravel()) / np.linalg.norm(ref)
+            assert err < 1e-10, (mesh_file, graph, err)
+        h.close()
+        mesh.close()
 
 
 def test_blas1_and_reductions(ctx):

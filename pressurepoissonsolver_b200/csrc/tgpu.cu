@@ -20,7 +20,6 @@
 
 using namespace tgpu;
 
-extern "C" int tgpu_hierarchy_destroy(tgpu_hier *h);
 // ------------------------------------------------------------------------------------------
 // errors
 // ------------------------------------------------------------------------------------------
@@ -112,15 +111,62 @@ int     load_nccl()
 // ------------------------------------------------------------------------------------------
 // objects
 // ------------------------------------------------------------------------------------------
+// Owners of what the library creates, one deleter per release call: every allocation, stream, event, graph and IPC
+// mapping is stored in one of these as it is created, so an error return releases it.  Kernels take .get().
+struct CudaFree { void operator()(void *p) const { cudaFree(p); } };
+struct CudaFreeHost { void operator()(const volatile void *p) const { cudaFreeHost((void *) p); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct GraphDestroy { void operator()(cudaGraph_t g) const { cudaGraphDestroy(g); } };
+struct GraphExecDestroy { void operator()(cudaGraphExec_t g) const { cudaGraphExecDestroy(g); } };
+struct IpcClose { void operator()(void *p) const { cudaIpcCloseMemHandle(p); } };
+struct VecDestroy { void operator()(tgpu_vec *v) const { tgpu_vec_destroy(v); } };
+template <typename T> using DevPtr  = std::unique_ptr<T, CudaFree>;
+template <typename T> using HostPtr = std::unique_ptr<T, CudaFreeHost>;
+using EventPtr     = std::unique_ptr<CUevent_st, EventDestroy>;
+using StreamPtr    = std::unique_ptr<CUstream_st, StreamDestroy>;
+using GraphPtr     = std::unique_ptr<CUgraph_st, GraphDestroy>;
+using GraphExecPtr = std::unique_ptr<CUgraphExec_st, GraphExecDestroy>;
+using IpcPtr       = std::unique_ptr<void, IpcClose>;
+using VecPtr       = std::unique_ptr<tgpu_vec, VecDestroy>;
+template <typename T> static cudaError_t dev_malloc(DevPtr<T> &p, size_t bytes)
+{
+	T *raw = nullptr;
+	const cudaError_t e = cudaMalloc(&raw, bytes);
+	if (e == cudaSuccess) p.reset(raw);
+	return e;
+}
+template <typename T> static cudaError_t host_alloc(HostPtr<T> &p, size_t bytes, unsigned flags = cudaHostAllocDefault)
+{
+	T *raw = nullptr;
+	const cudaError_t e = cudaHostAlloc(&raw, bytes, flags);
+	if (e == cudaSuccess) p.reset(raw);
+	return e;
+}
+static cudaError_t event_create(EventPtr &p, unsigned flags = cudaEventDefault)
+{
+	cudaEvent_t raw = nullptr;
+	const cudaError_t e = cudaEventCreateWithFlags(&raw, flags);
+	if (e == cudaSuccess) p.reset(raw);
+	return e;
+}
+static cudaError_t stream_create(StreamPtr &p)
+{
+	cudaStream_t raw = nullptr;
+	const cudaError_t e = cudaStreamCreateWithFlags(&raw, cudaStreamNonBlocking);
+	if (e == cudaSuccess) p.reset(raw);
+	return e;
+}
+
 struct tgpu_ctx {
 	int          device     = 0;
 	cudaStream_t stream     = nullptr;
-	bool         own_stream = false;
+	StreamPtr    own_stream;           // the stream tgpu_init created, until tgpu_set_stream replaces it
 	int          sm_count   = 148;
-	double *     d_partial  = nullptr; // [MAX_PARTIAL]
-	double *     d_result   = nullptr; // [8]
-	double *     h_result   = nullptr; // pinned [8]
-	cudaEvent_t  ev0 = nullptr, ev1 = nullptr;
+	DevPtr<double>  d_partial; // [MAX_PARTIAL]
+	DevPtr<double>  d_result;  // [8]
+	HostPtr<double> h_result;  // pinned [8]
+	EventPtr     ev0, ev1;
 	int64_t      launches  = 0;
 	bool         capturing = false;
 	bool         last_small = false;
@@ -129,16 +175,22 @@ struct tgpu_ctx {
 	ncclComm_t   comm        = nullptr;
 	int          rank        = 0;
 	int          nranks      = 1;
-	cudaStream_t comm_stream = nullptr; // halo exchanges run here, concurrently with interior sweeps
+	StreamPtr    comm_stream; // halo exchanges run here, concurrently with interior sweeps
 	// set by p2p_wait_kernel when a peer's flag never arrives (pinned, mapped host memory: the kernel writes it, the host
 	// reads it after every synchronisation point, see check_comm)
-	volatile int *p2p_err = nullptr;
+	HostPtr<volatile int> p2p_err;
 	// per-launch profiling
 	bool                          profiling = false;
 	const char *                  tag_name  = "kernel";
 	int                           tag_level = -1;
-	std::vector<cudaEvent_t>      prof_events;
+	std::vector<EventPtr>         prof_events;
 	std::vector<TgpuProfileEntry> prof_entries;
+	~tgpu_ctx()
+	{
+		cudaSetDevice(device);
+		cudaStreamSynchronize(stream);
+		if (comm && g_nccl.CommDestroy) g_nccl.CommDestroy(comm);
+	}
 };
 struct Tag {
 	tgpu_ctx *  ctx;
@@ -187,32 +239,33 @@ struct LevelDev {
 	int        slots  = 0; // owned + halo face slots
 	bool       distributed = false;
 	int        n_interior  = 0;
-	cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr}; // fork/join points of the overlapped exchange
+	EventPtr   ev[4]; // fork/join points of the overlapped exchange
 	std::vector<PeerDev> peers;
-	int32_t *  send_patch = nullptr, *send_side = nullptr, *recv_slot = nullptr, *recv_side = nullptr;
-	double *   sendbuf = nullptr, *recvbuf = nullptr;
+	DevPtr<int32_t> send_patch, send_side, recv_slot, recv_side;
+	DevPtr<double>  sendbuf, recvbuf;
 	size_t     nsend = 0, nrecv = 0;
 	size_t     ncells = 0, nface = 0;
-	PatchMeta *meta    = nullptr;
-	double *   starts  = nullptr;
-	double *   spacing = nullptr;
-	double *   Fa = nullptr, *Fb = nullptr; // face buffers
-	double *   G  = nullptr; // 32^3 levels: [nslots][M] interface terms of the sweeps that do not start from zero (iface_rhs32_kernel)
-	int32_t *  gslot = nullptr, *gowner = nullptr; // with G: the slot table (IfaceSlots32), device [P][6] and [nslots]
+	DevPtr<PatchMeta> meta;
+	DevPtr<double>    starts;
+	DevPtr<double>    spacing;
+	double *   Fa = nullptr, *Fb = nullptr; // face buffers: Fa_own / Fb_own, or views into the peer-to-peer arena (setup_p2p)
+	DevPtr<double> Fa_own, Fb_own;
+	DevPtr<double> G; // 32^3 levels: [nslots][M] interface terms of the sweeps that do not start from zero (iface_rhs32_kernel)
+	DevPtr<int32_t> gslot, gowner;                 // with G: the slot table (IfaceSlots32), device [P][6] and [nslots]
 	std::vector<int32_t> gbegin;                   // with G: IfaceSlots32::begin on the host (slot range of a patch range)
-	double *   u = nullptr, *f = nullptr, *r = nullptr; // cycle work vectors (lazily allocated)
+	DevPtr<double> u, f, r; // cycle work vectors (lazily allocated)
 	bool       has_neumann = false;
-	int32_t *  neu_list = nullptr;          // device: owned patches with Neumann domain sides, ascending (smooth3d16_kernel<.., NEU>)
+	DevPtr<int32_t> neu_list;               // device: owned patches with Neumann domain sides, ascending (smooth3d16_kernel<.., NEU>)
 	std::vector<int32_t> neu_host;          // the same list on the host (sub-ranges are found by binary search)
 	// peer-to-peer halo exchange: peers' face buffers and flags mapped with CUDA IPC (see setup_p2p)
 	bool       p2p = false;
-	int32_t *  send_peer = nullptr, *send_ridx = nullptr, *peer_rank = nullptr; // device: per send face / per peer
-	double **  peerFa = nullptr, **peerFb = nullptr;             // device [npeers]: the peers' Fa / Fb
-	uint64_t **peer_data_flag = nullptr, **peer_ack_flag = nullptr; // device [npeers]: my entry of the peers' flag rows
+	DevPtr<int32_t> send_peer, send_ridx, peer_rank;             // device: per send face / per peer
+	DevPtr<double *> peerFa, peerFb;                             // device [npeers]: the peers' Fa / Fb
+	DevPtr<uint64_t *> peer_data_flag, peer_ack_flag;            // device [npeers]: my entry of the peers' flag rows
 	uint64_t * data_flags = nullptr, *ack_flags = nullptr;       // my flag rows [nranks] (in the arena, written by peers)
-	uint64_t * cnt = nullptr;                                    // generation counters: data sent / awaited, ack sent / awaited
-	unsigned * tickets = nullptr;                                // [2] finished-CTA counters of the fused push / consumer kernels
-	PushDesc * push_desc = nullptr;                              // device [4]: (Fa | Fb) x (plain | + prolonged correction), see ensure_push_desc
+	DevPtr<uint64_t> cnt;                                        // generation counters: data sent / awaited, ack sent / awaited
+	DevPtr<unsigned> tickets;                                    // [2] finished-CTA counters of the fused push / consumer kernels
+	DevPtr<PushDesc> push_desc;                                  // device [4]: (Fa | Fb) x (plain | + prolonged correction), see ensure_push_desc
 	const double *push_uc = nullptr;                             // the coarse vector the descriptors were built with
 };
 
@@ -224,7 +277,7 @@ struct GraphEntry {
 	const double *  f;
 	double *        u;
 	TgpuCycleOpts   opts;
-	cudaGraphExec_t exec;
+	GraphExecPtr    exec;
 	int64_t         kernels;
 };
 
@@ -232,30 +285,48 @@ struct tgpu_hier {
 	tgpu_ctx *            ctx = nullptr;
 	int                   D = 0, N = 0;
 	std::vector<LevelDev> levels;
-	double *              scratch32 = nullptr; // smooth3d32n_kernel (32^3 levels with Neumann sides): one 256 KB block per CTA
+	DevPtr<double>        scratch32; // smooth3d32n_kernel (32^3 levels with Neumann sides): one 256 KB block per CTA
 	double *              cycle_faces = nullptr; // boundary slices of the last cycle's result (level 0), if it was asked to emit them
 	// ... and of the iterate before its last sweep: cycle_faces_old, plus P cycle_uc on the boundary cells if that sweep was
 	// the first post-sweep (cycle_uc == nullptr otherwise); see k_face_residual_norm
 	const double *        cycle_faces_old = nullptr, *cycle_uc = nullptr;
-	double *              tri = nullptr; // [N/2 + 1][N^(D-1)] tridiagonal multipliers (TriSolve)
-	double *              mats = nullptr, *lam = nullptr; // Neumann patches: transform matrices [6][N][N], 1-D eigenvalues [3][N]
+	DevPtr<double>        tri; // [N/2 + 1][N^(D-1)] tridiagonal multipliers (TriSolve)
+	DevPtr<double>        mats, lam; // Neumann patches: transform matrices [6][N][N], 1-D eigenvalues [3][N]
 	std::vector<GraphEntry> graphs;
-	std::vector<tgpu_vec *> krylov_ws;
-	std::vector<tgpu_vec *> gmg_ws; // stationary solve: residual and correction of the schedules without a start from a guess
-	double *              krylov_sc = nullptr; // BiCGStab scalars on the device
-	tgpu_vec *            host_f = nullptr, *host_u = nullptr;
+	std::vector<VecPtr>   krylov_ws;
+	std::vector<VecPtr>   gmg_ws; // stationary solve: residual and correction of the schedules without a start from a guess
+	DevPtr<double>        krylov_sc; // BiCGStab scalars on the device
+	VecPtr                host_f, host_u;
 	// pipelined host-buffer path (tgpu_vcycle_host_async): two slots, copy-in / copy-out streams
-	tgpu_vec *            pipe_f[2] = {nullptr, nullptr}, *pipe_u[2] = {nullptr, nullptr};
-	cudaStream_t          s_in = nullptr, s_out = nullptr;
-	cudaEvent_t           ev_in[2] = {nullptr, nullptr}, ev_cyc[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
+	VecPtr                pipe_f[2], pipe_u[2];
+	StreamPtr             s_in, s_out;
+	EventPtr              ev_in[2], ev_cyc[2], ev_out[2];
 	uint64_t              pipe_count = 0;
 	bool                  generic_kernels = false; // test hook: force the size-generic smoother
 	double                lambda = 0.0;            // the patch solver's shift (tgpu_hierarchy_set_lambda)
 	int                   last_level = 0;          // coarsest level the running cycle visits (CycleOpts max_levels / patches_per_proc)
 	// peer-to-peer arena: flag rows + the face buffers of the distributed levels, one IPC-exported allocation
-	void *                arena = nullptr;
-	std::vector<void *>   ipc_opened;
-	int *                 p2p_abort = nullptr; // device flag: a wait of this hierarchy has timed out (p2p_wait_kernel)
+	DevPtr<void>          arena;
+	std::vector<IpcPtr>   ipc_opened;
+	DevPtr<int>           p2p_abort; // device flag: a wait of this hierarchy has timed out (p2p_wait_kernel)
+
+	// the cached graphs and the vectors the hierarchy created for itself; tgpu_vec_destroy needs the hierarchy intact
+	void release_workspace()
+	{
+		graphs.clear();
+		krylov_ws.clear();
+		gmg_ws.clear();
+		host_f.reset(), host_u.reset();
+		for (int k = 0; k < 2; k++) pipe_f[k].reset(), pipe_u[k].reset();
+	}
+	~tgpu_hier()
+	{
+		cudaSetDevice(ctx->device);
+		if (s_in) cudaStreamSynchronize(s_in.get()); // pending copies of the pipelined host path still use the slot vectors
+		if (s_out) cudaStreamSynchronize(s_out.get());
+		cudaStreamSynchronize(ctx->stream);
+		release_workspace();
+	}
 };
 
 struct tgpu_vec {
@@ -268,15 +339,28 @@ struct tgpu_vec {
 // ------------------------------------------------------------------------------------------
 // launch helpers
 // ------------------------------------------------------------------------------------------
+// brackets stream work (a kernel launch, NCCL calls) with profiling events
+struct ProfSpan {
+	tgpu_ctx *ctx;
+	ProfSpan(tgpu_ctx *c, const char *name, int level) : ctx(c)
+	{
+		if (!c->profiling) return;
+		EventPtr e0, e1;
+		event_create(e0);
+		event_create(e1);
+		cudaEventRecord(e0.get(), c->stream);
+		c->prof_events.push_back(std::move(e0));
+		c->prof_events.push_back(std::move(e1));
+		c->prof_entries.push_back(TgpuProfileEntry{name, level, 0.f});
+	}
+	~ProfSpan()
+	{
+		if (ctx->profiling) cudaEventRecord(ctx->prof_events.back().get(), ctx->stream);
+	}
+};
 template <typename... KArgs, typename... Args>
 static int launch(tgpu_ctx *ctx, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, Args... args)
 {
-	cudaEvent_t e0 = nullptr, e1 = nullptr;
-	if (ctx->profiling) {
-		cudaEventCreate(&e0);
-		cudaEventCreate(&e1);
-		cudaEventRecord(e0, ctx->stream);
-	}
 	cudaLaunchConfig_t  cfg = {};
 	cudaLaunchAttribute at[1];
 	cfg.gridDim          = grid;
@@ -293,12 +377,9 @@ static int launch(tgpu_ctx *ctx, void (*kernel)(KArgs...), dim3 grid, dim3 block
 	const bool small = (int) (grid.x * grid.y) <= ctx->sm_count;
 	cfg.numAttrs     = small && ctx->last_small ? 1 : 0;
 	ctx->last_small  = small;
-	cudaLaunchKernelEx(&cfg, kernel, args...);
-	if (ctx->profiling) {
-		cudaEventRecord(e1, ctx->stream);
-		ctx->prof_events.push_back(e0);
-		ctx->prof_events.push_back(e1);
-		ctx->prof_entries.push_back(TgpuProfileEntry{ctx->tag_name, ctx->tag_level, 0.f});
+	{
+		ProfSpan span(ctx, ctx->tag_name, ctx->tag_level);
+		cudaLaunchKernelEx(&cfg, kernel, args...);
 	}
 	cudaError_t e = cudaGetLastError();
 	if (e != cudaSuccess) return fail(TGPU_ERR_CUDA, std::string("kernel launch: ") + cudaGetErrorString(e));
@@ -321,25 +402,6 @@ static int halo_launch(tgpu_ctx *ctx, const HaloSync &hs, void (*kernel)(KArgs..
 	}
 	return launch(ctx, kernel, grid, block, smem, args...);
 }
-// brackets non-kernel stream work (NCCL calls) with profiling events
-struct ProfSpan {
-	tgpu_ctx *ctx;
-	ProfSpan(tgpu_ctx *c, const char *name, int level) : ctx(c)
-	{
-		if (!c->profiling) return;
-		cudaEvent_t e0, e1;
-		cudaEventCreate(&e0);
-		cudaEventCreate(&e1);
-		cudaEventRecord(e0, c->stream);
-		c->prof_events.push_back(e0);
-		c->prof_events.push_back(e1);
-		c->prof_entries.push_back(TgpuProfileEntry{name, level, 0.f});
-	}
-	~ProfSpan()
-	{
-		if (ctx->profiling) cudaEventRecord(ctx->prof_events.back(), ctx->stream);
-	}
-};
 static int grid_for(tgpu_ctx *ctx, size_t n, int block = 256, int per_sm = 8)
 {
 	size_t want = (n + block - 1) / block;
@@ -407,7 +469,7 @@ template <class Fn> static int each_smooth_variant(Fn &&fn)
 }
 // G of the 32^3 levels whose sweeps can reach smooth3d32c_kernel from a non-zero guess (iface_rhs32_kernel): lambda = 0 (a
 // shifted patch solve sends every patch through smooth3d32n_kernel) and at least one owned patch without Neumann sides.
-template <typename T> static int dev_upload(T **dst, const T *src, size_t count);
+template <typename T> static int dev_upload(DevPtr<T> &dst, const T *src, size_t count);
 // G holds one term per interface slot (IfaceSlots32, built from the owned patches' metadata with the table).  Called at
 // creation and when lambda changes (never during a graph capture); the graphs are freed before G is.
 static int update_iface_buffers(tgpu_hier *h)
@@ -417,19 +479,16 @@ static int update_iface_buffers(tgpu_hier *h)
 		const bool want = h->lambda == 0.0 && L.neu_host.size() < (size_t) L.P;
 		if (want && !L.G) {
 			std::vector<PatchMeta> meta(L.P);
-			CU(cudaMemcpy(meta.data(), L.meta, meta.size() * sizeof(PatchMeta), cudaMemcpyDeviceToHost));
+			CU(cudaMemcpy(meta.data(), L.meta.get(), meta.size() * sizeof(PatchMeta), cudaMemcpyDeviceToHost));
 			const IfaceSlots32 t = build_iface_slots32(meta.data(), L.P);
-			TRY(dev_upload(&L.gslot, t.gslot.data(), t.gslot.size()));
-			TRY(dev_upload(&L.gowner, t.owner.data(), t.owner.size()));
-			CU(cudaMalloc(&L.G, std::max<size_t>(t.owner.size(), 1) * 1024 * sizeof(double)));
+			TRY(dev_upload(L.gslot, t.gslot.data(), t.gslot.size()));
+			TRY(dev_upload(L.gowner, t.owner.data(), t.owner.size()));
+			CU(dev_malloc(L.G, std::max<size_t>(t.owner.size(), 1) * 1024 * sizeof(double)));
 			L.gbegin = t.begin;
 		}
 		if (!want && L.G) {
 			CU(cudaDeviceSynchronize());
-			cudaFree(L.G);
-			cudaFree(L.gslot);
-			cudaFree(L.gowner);
-			L.G = nullptr, L.gslot = L.gowner = nullptr;
+			L.G.reset(), L.gslot.reset(), L.gowner.reset();
 			L.gbegin.clear();
 		}
 	}
@@ -441,7 +500,7 @@ static int ensure_scratch32(tgpu_hier *h)
 {
 	bool want = h->lambda != 0.0;
 	for (const LevelDev &L : h->levels) want = want || L.has_neumann;
-	if (is_3d32(h) && want && !h->scratch32) CU(cudaMalloc(&h->scratch32, (size_t) h->ctx->sm_count * 2 * 32768 * sizeof(double)));
+	if (is_3d32(h) && want && !h->scratch32) CU(dev_malloc(h->scratch32, (size_t) h->ctx->sm_count * 2 * 32768 * sizeof(double)));
 	return TGPU_OK;
 }
 static constexpr size_t FRR32_SMEM = 6 * 1024 * 8; // face_residual_restrict_big_kernel<3, 32>: dynamic shared memory
@@ -542,13 +601,13 @@ extern "C" int tgpu_init(int device, tgpu_ctx **out)
 	cudaDeviceProp prop;
 	CU(cudaGetDeviceProperties(&prop, device));
 	ctx->sm_count = prop.multiProcessorCount;
-	CU(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
-	ctx->own_stream = true;
-	CU(cudaMalloc(&ctx->d_partial, MAX_PARTIAL * sizeof(double)));
-	CU(cudaMalloc(&ctx->d_result, 8 * sizeof(double)));
-	CU(cudaMallocHost(&ctx->h_result, 8 * sizeof(double)));
-	CU(cudaEventCreate(&ctx->ev0));
-	CU(cudaEventCreate(&ctx->ev1));
+	CU(stream_create(ctx->own_stream));
+	ctx->stream = ctx->own_stream.get();
+	CU(dev_malloc(ctx->d_partial, MAX_PARTIAL * sizeof(double)));
+	CU(dev_malloc(ctx->d_result, 8 * sizeof(double)));
+	CU(host_alloc(ctx->h_result, 8 * sizeof(double)));
+	CU(event_create(ctx->ev0));
+	CU(event_create(ctx->ev1));
 	{ // vector storage pool (tgpu_vec_create): keep freed blocks across synchronisations; tgpu_hierarchy_trim releases them
 		cudaMemPool_t pool = nullptr;
 		CU(cudaDeviceGetDefaultMemPool(&pool, device));
@@ -562,18 +621,6 @@ extern "C" int tgpu_init(int device, tgpu_ctx **out)
 }
 extern "C" int tgpu_finalize(tgpu_ctx *ctx)
 {
-	if (!ctx) return TGPU_OK;
-	cudaSetDevice(ctx->device);
-	cudaStreamSynchronize(ctx->stream);
-	if (ctx->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(ctx->comm);
-	if (ctx->comm_stream) cudaStreamDestroy(ctx->comm_stream);
-	if (ctx->p2p_err) cudaFreeHost((void *) ctx->p2p_err);
-	cudaFree(ctx->d_partial);
-	cudaFree(ctx->d_result);
-	cudaFreeHost(ctx->h_result);
-	cudaEventDestroy(ctx->ev0);
-	cudaEventDestroy(ctx->ev1);
-	if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
 	delete ctx;
 	return TGPU_OK;
 }
@@ -581,9 +628,8 @@ extern "C" int tgpu_set_stream(tgpu_ctx *ctx, void *s)
 {
 	if (!ctx) return fail(TGPU_ERR_ARG, "null context");
 	CU(cudaStreamSynchronize(ctx->stream));
-	if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
-	ctx->stream     = (cudaStream_t) s;
-	ctx->own_stream = false;
+	ctx->own_stream.reset();
+	ctx->stream = (cudaStream_t) s;
 	return TGPU_OK;
 }
 extern "C" int tgpu_sync(tgpu_ctx *ctx)
@@ -601,16 +647,16 @@ extern "C" int tgpu_kernel_launches(tgpu_ctx *ctx, int64_t *count)
 extern "C" int tgpu_timer_start(tgpu_ctx *ctx)
 {
 	if (!ctx) return fail(TGPU_ERR_ARG, "null context");
-	CU(cudaEventRecord(ctx->ev0, ctx->stream));
+	CU(cudaEventRecord(ctx->ev0.get(), ctx->stream));
 	return TGPU_OK;
 }
 extern "C" int tgpu_timer_stop(tgpu_ctx *ctx, double *ms)
 {
 	if (!ctx || !ms) return fail(TGPU_ERR_ARG, "null argument");
-	CU(cudaEventRecord(ctx->ev1, ctx->stream));
-	CU(cudaEventSynchronize(ctx->ev1));
+	CU(cudaEventRecord(ctx->ev1.get(), ctx->stream));
+	CU(cudaEventSynchronize(ctx->ev1.get()));
 	float f = 0;
-	CU(cudaEventElapsedTime(&f, ctx->ev0, ctx->ev1));
+	CU(cudaEventElapsedTime(&f, ctx->ev0.get(), ctx->ev1.get()));
 	*ms = f;
 	return check_comm(ctx);
 }
@@ -619,7 +665,6 @@ extern "C" int tgpu_profile_begin(tgpu_ctx *ctx)
 {
 	if (!ctx) return fail(TGPU_ERR_ARG, "null context");
 	CU(cudaStreamSynchronize(ctx->stream));
-	for (cudaEvent_t e : ctx->prof_events) cudaEventDestroy(e);
 	ctx->prof_events.clear();
 	ctx->prof_entries.clear();
 	ctx->profiling = true;
@@ -631,7 +676,7 @@ extern "C" int tgpu_profile_end(tgpu_ctx *ctx, int *n, const TgpuProfileEntry **
 	ctx->profiling = false;
 	CU(cudaStreamSynchronize(ctx->stream));
 	for (size_t i = 0; i < ctx->prof_entries.size(); i++)
-		CU(cudaEventElapsedTime(&ctx->prof_entries[i].ms, ctx->prof_events[2 * i], ctx->prof_events[2 * i + 1]));
+		CU(cudaEventElapsedTime(&ctx->prof_entries[i].ms, ctx->prof_events[2 * i].get(), ctx->prof_events[2 * i + 1].get()));
 	*n       = (int) ctx->prof_entries.size();
 	*entries = ctx->prof_entries.data();
 	return TGPU_OK;
@@ -725,20 +770,20 @@ extern "C" int tgpu_mesh_level_ids(const tgpu_mesh *m, int level, const int32_t 
 // ------------------------------------------------------------------------------------------
 // hierarchy
 // ------------------------------------------------------------------------------------------
-template <typename T> static int dev_upload(T **dst, const T *src, size_t count)
+template <typename T> static int dev_upload(DevPtr<T> &dst, const T *src, size_t count)
 {
-	CU(cudaMalloc(dst, std::max<size_t>(1, count) * sizeof(T)));
-	if (count) CU(cudaMemcpy(*dst, src, count * sizeof(T), cudaMemcpyHostToDevice));
+	CU(dev_malloc(dst, std::max<size_t>(1, count) * sizeof(T)));
+	if (count) CU(cudaMemcpy(dst.get(), src, count * sizeof(T), cudaMemcpyHostToDevice));
 	return TGPU_OK;
 }
 
 // n_owned == nullptr: every patch of every level is owned (single GPU).  Otherwise level l has n_owned[l]
 // owned patches followed by halo face slots (multi-GPU, see tgpu_hierarchy_create_distributed).
 static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const TgpuLevelDesc *levels, const int32_t *n_owned,
-                                 tgpu_hier **out)
+                                 std::unique_ptr<tgpu_hier> &out)
 {
 	API_BEGIN
-	if (!ctx || !levels || !out || nlevels < 1) return fail(TGPU_ERR_ARG, "tgpu_hierarchy_create: bad argument");
+	if (!ctx || !levels || nlevels < 1) return fail(TGPU_ERR_ARG, "tgpu_hierarchy_create: bad argument");
 	if (!supported_dn(D, n))
 		return fail(TGPU_ERR_UNSUPPORTED, "tgpu_hierarchy_create: (D, n) must be one of 2D n=4/8/16/32, 3D n=4/8/16/32");
 	CU(cudaSetDevice(ctx->device));
@@ -811,13 +856,14 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 				}
 			}
 		}
-		TRY(dev_upload(&L.meta, meta.data(), meta.size()));
-		if (!L.neu_host.empty()) TRY(dev_upload(&L.neu_list, L.neu_host.data(), L.neu_host.size()));
-		TRY(dev_upload(&L.spacing, d.spacing, (size_t) d.npatch * D));
-		if (d.starts) TRY(dev_upload(&L.starts, d.starts, (size_t) d.npatch * D));
-		CU(cudaMalloc(&L.Fa, L.nface * sizeof(double)));
-		CU(cudaMalloc(&L.Fb, L.nface * sizeof(double)));
-		h->levels.push_back(L);
+		TRY(dev_upload(L.meta, meta.data(), meta.size()));
+		if (!L.neu_host.empty()) TRY(dev_upload(L.neu_list, L.neu_host.data(), L.neu_host.size()));
+		TRY(dev_upload(L.spacing, d.spacing, (size_t) d.npatch * D));
+		if (d.starts) TRY(dev_upload(L.starts, d.starts, (size_t) d.npatch * D));
+		CU(dev_malloc(L.Fa_own, L.nface * sizeof(double)));
+		CU(dev_malloc(L.Fb_own, L.nface * sizeof(double)));
+		L.Fa = L.Fa_own.get(), L.Fb = L.Fb_own.get();
+		h->levels.push_back(std::move(L));
 	}
 	// multipliers of the two-sided tridiagonal elimination along the axis that is not transformed, for every
 	// pencil of the other axes' transform indices (TriSolve, kernels.cuh): [n/2 + 1][n^(D-1)]
@@ -839,7 +885,7 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 			}
 			tri[(size_t) H * M + m] = (double) (1.0L / (1.0L - a * a));
 		}
-		TRY(dev_upload(&h->tri, tri.data(), tri.size()));
+		TRY(dev_upload(h->tri, tri.data(), tri.size()));
 	}
 	// general transform path (patches with Neumann domain sides): the six matrices of DftPatchSolver.h:237-289,
 	// M[k][j] such that y_k = sum_j M[k][j] x_j, order TK_*; 1-D eigenvalues -4 sin^2((k + shift) pi / 2n), shift 1, 0, 1/2
@@ -858,19 +904,23 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 		const double shift[3] = {1.0, 0.0, 0.5};
 		for (int t = 0; t < 3; t++)
 			for (int k = 0; k < n; k++) lam[(size_t) t * n + k] = -4.0 * pow(sin((k + shift[t]) * M_PI / (2 * n)), 2);
-		TRY(dev_upload(&h->mats, mats.data(), mats.size()));
-		TRY(dev_upload(&h->lam, lam.data(), lam.size()));
+		TRY(dev_upload(h->mats, mats.data(), mats.size()));
+		TRY(dev_upload(h->lam, lam.data(), lam.size()));
 	}
 	TRY(set_kernel_attrs(h.get()));
 	TRY(ensure_scratch32(h.get()));
 	TRY(update_iface_buffers(h.get()));
-	*out = h.release();
+	out = std::move(h);
 	return TGPU_OK;
 	API_END
 }
 extern "C" int tgpu_hierarchy_create(tgpu_ctx *ctx, int D, int n, int nlevels, const TgpuLevelDesc *levels, tgpu_hier **out)
 {
-	return hierarchy_create_impl(ctx, D, n, nlevels, levels, nullptr, out);
+	if (!out) return fail(TGPU_ERR_ARG, "tgpu_hierarchy_create: bad argument");
+	std::unique_ptr<tgpu_hier> h;
+	TRY(hierarchy_create_impl(ctx, D, n, nlevels, levels, nullptr, h));
+	*out = h.release();
+	return TGPU_OK;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -960,12 +1010,10 @@ extern "C" int tgpu_comm_init(tgpu_ctx *ctx, const void *id128, int rank, int nr
 	ncclUniqueId id;
 	memcpy(&id, id128, sizeof(id));
 	NC(g_nccl.CommInitRank(&ctx->comm, nranks, id, rank));
-	if (!ctx->comm_stream) CU(cudaStreamCreateWithFlags(&ctx->comm_stream, cudaStreamNonBlocking));
+	if (!ctx->comm_stream) CU(stream_create(ctx->comm_stream));
 	if (!ctx->p2p_err) {
-		int *e = nullptr;
-		CU(cudaHostAlloc(&e, sizeof(int), cudaHostAllocMapped | cudaHostAllocPortable));
-		*e           = 0;
-		ctx->p2p_err = e;
+		CU(host_alloc(ctx->p2p_err, sizeof(int), cudaHostAllocMapped | cudaHostAllocPortable));
+		*ctx->p2p_err = 0;
 	}
 	ctx->rank   = rank;
 	ctx->nranks = nranks;
@@ -1031,13 +1079,13 @@ static int setup_p2p(tgpu_hier *h, const Partition &pt)
             cudaGetLastError();
         }
 	};
-	soft(cudaMalloc(&h->arena, off), "cudaMalloc(arena)");
-	if (ok) soft(cudaMemset(h->arena, 0, off), "cudaMemset(arena)");
+	soft(dev_malloc(h->arena, off), "cudaMalloc(arena)");
+	if (ok) soft(cudaMemset(h->arena.get(), 0, off), "cudaMemset(arena)");
 	if (ok) {
 		void *base = nullptr;
-		if (alloc_base_of(h->arena, &base) != TGPU_OK) ok = 0, why = "cuMemGetAddressRange failed";
+		if (alloc_base_of(h->arena.get(), &base) != TGPU_OK) ok = 0, why = "cuMemGetAddressRange failed";
 		else {
-			mine.base_off = (uint64_t) ((char *) h->arena - (char *) base);
+			mine.base_off = (uint64_t) ((char *) h->arena.get() - (char *) base);
 			soft(cudaIpcGetMemHandle(&mine.handle, base), "cudaIpcGetMemHandle");
 		}
 	}
@@ -1045,50 +1093,44 @@ static int setup_p2p(tgpu_hier *h, const Partition &pt)
 	// ---- all-gather the packs ----
 	std::vector<P2PPack> all(nr);
 	{
-		P2PPack *d_mine = nullptr, *d_all = nullptr;
-		CU(cudaMalloc(&d_mine, sizeof(P2PPack)));
-		CU(cudaMalloc(&d_all, sizeof(P2PPack) * nr));
-		CU(cudaMemcpy(d_mine, &mine, sizeof(P2PPack), cudaMemcpyHostToDevice));
-		NC(g_nccl.AllGather(d_mine, d_all, sizeof(P2PPack), ncclChar, ctx->comm, ctx->stream));
+		DevPtr<P2PPack> d_mine, d_all;
+		CU(dev_malloc(d_mine, sizeof(P2PPack)));
+		CU(dev_malloc(d_all, sizeof(P2PPack) * nr));
+		CU(cudaMemcpy(d_mine.get(), &mine, sizeof(P2PPack), cudaMemcpyHostToDevice));
+		NC(g_nccl.AllGather(d_mine.get(), d_all.get(), sizeof(P2PPack), ncclChar, ctx->comm, ctx->stream));
 		CU(cudaStreamSynchronize(ctx->stream));
-		CU(cudaMemcpy(all.data(), d_all, sizeof(P2PPack) * nr, cudaMemcpyDeviceToHost));
-		cudaFree(d_mine);
-		cudaFree(d_all);
+		CU(cudaMemcpy(all.data(), d_all.get(), sizeof(P2PPack) * nr, cudaMemcpyDeviceToHost));
 	}
 	for (int r = 0; r < nr; r++)
 		if (!all[r].ok && ok) ok = 0, why = "rank " + std::to_string(r) + " could not export its arena";
 	// ---- map the arenas of the ranks I exchange with ----
 	std::vector<char *> rarena(nr, nullptr);
-	rarena[me] = (char *) h->arena;
+	rarena[me] = (char *) h->arena.get();
 	for (int l = 0; l < nl && ok; l++)
 		for (const PeerDev &pd : h->levels[l].peers) {
 			if (rarena[pd.peer] || !ok) continue;
 			void *rb = nullptr;
 			soft(cudaIpcOpenMemHandle(&rb, all[pd.peer].handle, cudaIpcMemLazyEnablePeerAccess), "cudaIpcOpenMemHandle");
 			if (!ok) break;
-			h->ipc_opened.push_back(rb);
+			h->ipc_opened.emplace_back(rb);
 			rarena[pd.peer] = (char *) rb + all[pd.peer].base_off;
 		}
-	if (ok) soft(cudaMalloc(&h->p2p_abort, sizeof(int)), "cudaMalloc(abort flag)");
-	if (ok) soft(cudaMemset(h->p2p_abort, 0, sizeof(int)), "cudaMemset(abort flag)");
+	if (ok) soft(dev_malloc(h->p2p_abort, sizeof(int)), "cudaMalloc(abort flag)");
+	if (ok) soft(cudaMemset(h->p2p_abort.get(), 0, sizeof(int)), "cudaMemset(abort flag)");
 	{ // agreement: peer-to-peer only if every rank mapped everything it needs
-		int *d = nullptr;
-		CU(cudaMalloc(&d, sizeof(int)));
-		CU(cudaMemcpy(d, &ok, sizeof(int), cudaMemcpyHostToDevice));
-		NC(g_nccl.AllReduce(d, d, 1, ncclInt32, ncclMin, ctx->comm, ctx->stream));
+		DevPtr<int> d;
+		CU(dev_malloc(d, sizeof(int)));
+		CU(cudaMemcpy(d.get(), &ok, sizeof(int), cudaMemcpyHostToDevice));
+		NC(g_nccl.AllReduce(d.get(), d.get(), 1, ncclInt32, ncclMin, ctx->comm, ctx->stream));
 		CU(cudaStreamSynchronize(ctx->stream));
 		int all_ok = 0;
-		CU(cudaMemcpy(&all_ok, d, sizeof(int), cudaMemcpyDeviceToHost));
-		cudaFree(d);
+		CU(cudaMemcpy(&all_ok, d.get(), sizeof(int), cudaMemcpyDeviceToHost));
 		if (!all_ok) {
 			if (!ok) fprintf(stderr, "tgpu: rank %d cannot use the peer-to-peer halo exchange (%s)\n", me, why.c_str());
 			if (me == 0) fprintf(stderr, "tgpu: peer-to-peer mapping unavailable on at least one rank: using the NCCL send/recv halo exchange\n");
-			for (void *b : h->ipc_opened) cudaIpcCloseMemHandle(b);
 			h->ipc_opened.clear();
-			cudaFree(h->arena);
-			cudaFree(h->p2p_abort);
-			h->arena     = nullptr;
-			h->p2p_abort = nullptr;
+			h->arena.reset();
+			h->p2p_abort.reset();
 			return TGPU_OK; // L.p2p stays false on every level
 		}
 	}
@@ -1097,30 +1139,28 @@ static int setup_p2p(tgpu_hier *h, const Partition &pt)
 		LevelDev &       L  = h->levels[l];
 		const PartLevel &PL = pt.levels[l];
 		if (!L.distributed || (L.nsend == 0 && L.nrecv == 0)) continue;
-		cudaFree(L.Fa);
-		cudaFree(L.Fb);
-		L.Fa         = (double *) ((char *) h->arena + mine.fa_off[l]);
-		L.Fb         = (double *) ((char *) h->arena + mine.fb_off[l]);
-		L.data_flags = (uint64_t *) ((char *) h->arena + mine.flags_off) + ((size_t) l * 2 + 0) * nr;
-		L.ack_flags  = (uint64_t *) ((char *) h->arena + mine.flags_off) + ((size_t) l * 2 + 1) * nr;
-		CU(cudaMalloc(&L.cnt, 4 * sizeof(uint64_t)));
-		CU(cudaMemset(L.cnt, 0, 4 * sizeof(uint64_t)));
-		CU(cudaMalloc(&L.tickets, 2 * sizeof(unsigned)));
-		CU(cudaMemset(L.tickets, 0, 2 * sizeof(unsigned)));
+		L.Fa_own.reset(), L.Fb_own.reset();
+		L.Fa         = (double *) ((char *) h->arena.get() + mine.fa_off[l]);
+		L.Fb         = (double *) ((char *) h->arena.get() + mine.fb_off[l]);
+		L.data_flags = (uint64_t *) ((char *) h->arena.get() + mine.flags_off) + ((size_t) l * 2 + 0) * nr;
+		L.ack_flags  = (uint64_t *) ((char *) h->arena.get() + mine.flags_off) + ((size_t) l * 2 + 1) * nr;
+		CU(dev_malloc(L.cnt, 4 * sizeof(uint64_t)));
+		CU(cudaMemset(L.cnt.get(), 0, 4 * sizeof(uint64_t)));
+		CU(dev_malloc(L.tickets, 2 * sizeof(unsigned)));
+		CU(cudaMemset(L.tickets.get(), 0, 2 * sizeof(unsigned)));
 		const int np = (int) L.peers.size();
 		// my halo slots as the peers see them: they send (slot, side) lists in the agreed order
-		int32_t *d_rslot = nullptr;
-		CU(cudaMalloc(&d_rslot, std::max<size_t>(1, L.nsend) * sizeof(int32_t)));
+		DevPtr<int32_t> d_rslot;
+		CU(dev_malloc(d_rslot, std::max<size_t>(1, L.nsend) * sizeof(int32_t)));
 		NC(g_nccl.GroupStart());
 		for (const PeerDev &pd : L.peers) {
-			if (pd.recv_n) NC(g_nccl.Send(L.recv_slot + pd.recv_off, pd.recv_n, ncclInt32, pd.peer, ctx->comm, ctx->stream));
-			if (pd.send_n) NC(g_nccl.Recv(d_rslot + pd.send_off, pd.send_n, ncclInt32, pd.peer, ctx->comm, ctx->stream));
+			if (pd.recv_n) NC(g_nccl.Send(L.recv_slot.get() + pd.recv_off, pd.recv_n, ncclInt32, pd.peer, ctx->comm, ctx->stream));
+			if (pd.send_n) NC(g_nccl.Recv(d_rslot.get() + pd.send_off, pd.send_n, ncclInt32, pd.peer, ctx->comm, ctx->stream));
 		}
 		NC(g_nccl.GroupEnd());
 		CU(cudaStreamSynchronize(ctx->stream));
 		std::vector<int32_t> rslot(L.nsend), ridx(L.nsend), speer(L.nsend), prank(np);
-		if (L.nsend) CU(cudaMemcpy(rslot.data(), d_rslot, L.nsend * sizeof(int32_t), cudaMemcpyDeviceToHost));
-		cudaFree(d_rslot);
+		if (L.nsend) CU(cudaMemcpy(rslot.data(), d_rslot.get(), L.nsend * sizeof(int32_t), cudaMemcpyDeviceToHost));
 		std::vector<double *>   pfa(np), pfb(np);
 		std::vector<uint64_t *> pdf(np), paf(np);
 		size_t                  k = 0;
@@ -1139,23 +1179,22 @@ static int setup_p2p(tgpu_hier *h, const Partition &pt)
 				ridx[k]  = rslot[k] * S + x.send_side[j];
 			}
 		}
-		TRY(dev_upload(&L.send_peer, speer.data(), speer.size()));
-		TRY(dev_upload(&L.send_ridx, ridx.data(), ridx.size()));
-		TRY(dev_upload(&L.peer_rank, prank.data(), prank.size()));
-		TRY(dev_upload(&L.peerFa, pfa.data(), pfa.size()));
-		TRY(dev_upload(&L.peerFb, pfb.data(), pfb.size()));
-		TRY(dev_upload(&L.peer_data_flag, pdf.data(), pdf.size()));
-		TRY(dev_upload(&L.peer_ack_flag, paf.data(), paf.size()));
+		TRY(dev_upload(L.send_peer, speer.data(), speer.size()));
+		TRY(dev_upload(L.send_ridx, ridx.data(), ridx.size()));
+		TRY(dev_upload(L.peer_rank, prank.data(), prank.size()));
+		TRY(dev_upload(L.peerFa, pfa.data(), pfa.size()));
+		TRY(dev_upload(L.peerFb, pfb.data(), pfb.size()));
+		TRY(dev_upload(L.peer_data_flag, pdf.data(), pdf.size()));
+		TRY(dev_upload(L.peer_ack_flag, paf.data(), paf.size()));
 		L.p2p = true;
 	}
 	// nobody may push before everybody has finished mapping
 	{
-		int *d = nullptr;
-		CU(cudaMalloc(&d, sizeof(int)));
-		CU(cudaMemset(d, 0, sizeof(int)));
-		NC(g_nccl.AllReduce(d, d, 1, ncclInt32, ncclSum, ctx->comm, ctx->stream));
+		DevPtr<int> d;
+		CU(dev_malloc(d, sizeof(int)));
+		CU(cudaMemset(d.get(), 0, sizeof(int)));
+		NC(g_nccl.AllReduce(d.get(), d.get(), 1, ncclInt32, ncclSum, ctx->comm, ctx->stream));
 		CU(cudaStreamSynchronize(ctx->stream));
-		cudaFree(d);
 	}
 	return TGPU_OK;
 }
@@ -1168,8 +1207,8 @@ extern "C" int tgpu_hierarchy_create_distributed(tgpu_ctx *ctx, const tgpu_part 
 		return fail(TGPU_ERR_ARG, "tgpu_hierarchy_create_distributed: call tgpu_comm_init with the partition's rank/nranks first");
 	std::vector<int32_t> owned;
 	for (const PartLevel &L : pt.levels) owned.push_back(L.n_owned);
-	tgpu_hier *h = nullptr;
-	TRY(hierarchy_create_impl(ctx, pt.D, pt.n, (int) pt.levels.size(), part->descs.data(), owned.data(), &h));
+	std::unique_ptr<tgpu_hier> h;
+	TRY(hierarchy_create_impl(ctx, pt.D, pt.n, (int) pt.levels.size(), part->descs.data(), owned.data(), h));
 	size_t M = 1;
 	for (int i = 0; i < pt.D - 1; i++) M *= pt.n;
 	for (size_t l = 0; l < pt.levels.size(); l++) {
@@ -1178,7 +1217,7 @@ extern "C" int tgpu_hierarchy_create_distributed(tgpu_ctx *ctx, const tgpu_part 
 		L.distributed       = PL.distributed;
 		L.n_interior        = PL.n_interior;
 		if (PL.distributed && l < pt.owner.size()) L.global_P = (int64_t) pt.owner[l].size();
-		for (int e = 0; e < 4; e++) CU(cudaEventCreateWithFlags(&L.ev[e], cudaEventDisableTiming));
+		for (int e = 0; e < 4; e++) CU(event_create(L.ev[e], cudaEventDisableTiming));
 		std::vector<int32_t> sp, ss, rs, rsd;
 		for (const PeerExchange &x : PL.peers) {
 			PeerDev pd;
@@ -1193,14 +1232,14 @@ extern "C" int tgpu_hierarchy_create_distributed(tgpu_ctx *ctx, const tgpu_part 
 		}
 		L.nsend = sp.size(), L.nrecv = rs.size();
 		if (L.nsend) {
-			TRY(dev_upload(&L.send_patch, sp.data(), sp.size()));
-			TRY(dev_upload(&L.send_side, ss.data(), ss.size()));
-			CU(cudaMalloc(&L.sendbuf, L.nsend * M * sizeof(double)));
+			TRY(dev_upload(L.send_patch, sp.data(), sp.size()));
+			TRY(dev_upload(L.send_side, ss.data(), ss.size()));
+			CU(dev_malloc(L.sendbuf, L.nsend * M * sizeof(double)));
 		}
 		if (L.nrecv) {
-			TRY(dev_upload(&L.recv_slot, rs.data(), rs.size()));
-			TRY(dev_upload(&L.recv_side, rsd.data(), rsd.size()));
-			CU(cudaMalloc(&L.recvbuf, L.nrecv * M * sizeof(double)));
+			TRY(dev_upload(L.recv_slot, rs.data(), rs.size()));
+			TRY(dev_upload(L.recv_side, rsd.data(), rsd.size()));
+			CU(dev_malloc(L.recvbuf, L.nrecv * M * sizeof(double)));
 		}
 		// halo slots must never hold NaN garbage before the first exchange
 		CU(cudaMemset(L.Fa, 0, L.nface * sizeof(double)));
@@ -1208,87 +1247,14 @@ extern "C" int tgpu_hierarchy_create_distributed(tgpu_ctx *ctx, const tgpu_part 
 	}
 	// TGPU_P2P=0 keeps the NCCL send/recv exchange (pack, ncclSend/ncclRecv, unpack)
 	const char *e = getenv("TGPU_P2P");
-	if (pt.nranks > 1 && !(e && atoi(e) == 0)) {
-		int rc = setup_p2p(h, pt);
-		if (rc != TGPU_OK) {
-			tgpu_hierarchy_destroy(h);
-			return rc;
-		}
-	}
-	*out = h;
+	if (pt.nranks > 1 && !(e && atoi(e) == 0)) TRY(setup_p2p(h.get(), pt));
+	*out = h.release();
 	return TGPU_OK;
 	API_END
 }
 
-static void free_graphs(tgpu_hier *h)
-{
-	for (GraphEntry &g : h->graphs) cudaGraphExecDestroy(g.exec);
-	h->graphs.clear();
-}
-extern "C" int tgpu_vec_destroy(tgpu_vec *v);
 extern "C" int tgpu_hierarchy_destroy(tgpu_hier *h)
 {
-	if (!h) return TGPU_OK;
-	cudaSetDevice(h->ctx->device);
-	if (h->s_in) cudaStreamSynchronize(h->s_in); // pending copies of the pipelined host path still use the slot vectors
-	if (h->s_out) cudaStreamSynchronize(h->s_out);
-	cudaStreamSynchronize(h->ctx->stream);
-	free_graphs(h);
-	for (tgpu_vec *v : h->krylov_ws) tgpu_vec_destroy(v);
-	for (tgpu_vec *v : h->gmg_ws) tgpu_vec_destroy(v);
-	tgpu_vec_destroy(h->host_f);
-	tgpu_vec_destroy(h->host_u);
-	for (int k = 0; k < 2; k++) {
-		tgpu_vec_destroy(h->pipe_f[k]);
-		tgpu_vec_destroy(h->pipe_u[k]);
-		if (h->ev_in[k]) cudaEventDestroy(h->ev_in[k]);
-		if (h->ev_cyc[k]) cudaEventDestroy(h->ev_cyc[k]);
-		if (h->ev_out[k]) cudaEventDestroy(h->ev_out[k]);
-	}
-	if (h->s_in) cudaStreamDestroy(h->s_in);
-	if (h->s_out) cudaStreamDestroy(h->s_out);
-	for (LevelDev &L : h->levels) {
-		cudaFree(L.meta);
-		cudaFree(L.neu_list);
-		cudaFree(L.starts);
-		cudaFree(L.spacing);
-		if (!L.p2p) { // otherwise they live in the arena
-			cudaFree(L.Fa);
-			cudaFree(L.Fb);
-		}
-		cudaFree(L.G);
-		cudaFree(L.gslot);
-		cudaFree(L.gowner);
-		cudaFree(L.send_peer);
-		cudaFree(L.send_ridx);
-		cudaFree(L.peer_rank);
-		cudaFree(L.peerFa);
-		cudaFree(L.peerFb);
-		cudaFree(L.peer_data_flag);
-		cudaFree(L.peer_ack_flag);
-		cudaFree(L.cnt);
-		cudaFree(L.tickets);
-		cudaFree(L.push_desc);
-		for (int e = 0; e < 4; e++)
-			if (L.ev[e]) cudaEventDestroy(L.ev[e]);
-		cudaFree(L.send_patch);
-		cudaFree(L.send_side);
-		cudaFree(L.recv_slot);
-		cudaFree(L.recv_side);
-		cudaFree(L.sendbuf);
-		cudaFree(L.recvbuf);
-		cudaFree(L.u);
-		cudaFree(L.f);
-		cudaFree(L.r);
-	}
-	for (void *b : h->ipc_opened) cudaIpcCloseMemHandle(b);
-	cudaFree(h->arena);
-	cudaFree(h->p2p_abort);
-	cudaFree(h->krylov_sc);
-	cudaFree(h->mats);
-	cudaFree(h->lam);
-	cudaFree(h->scratch32);
-	cudaFree(h->tri);
 	delete h;
 	return TGPU_OK;
 }
@@ -1301,20 +1267,10 @@ extern "C" int tgpu_hierarchy_trim(tgpu_hier *h)
 	if (!h) return fail(TGPU_ERR_ARG, "null hierarchy");
 	tgpu_ctx *ctx = h->ctx;
 	CU(cudaSetDevice(ctx->device));
-	if (h->s_in) CU(cudaStreamSynchronize(h->s_in));
-	if (h->s_out) CU(cudaStreamSynchronize(h->s_out));
+	if (h->s_in) CU(cudaStreamSynchronize(h->s_in.get()));
+	if (h->s_out) CU(cudaStreamSynchronize(h->s_out.get()));
 	CU(cudaStreamSynchronize(ctx->stream));
-	free_graphs(h);
-	for (tgpu_vec *v : h->krylov_ws) tgpu_vec_destroy(v);
-	h->krylov_ws.clear();
-	for (tgpu_vec *v : h->gmg_ws) tgpu_vec_destroy(v);
-	h->gmg_ws.clear();
-	tgpu_vec_destroy(h->host_f), h->host_f = nullptr;
-	tgpu_vec_destroy(h->host_u), h->host_u = nullptr;
-	for (int k = 0; k < 2; k++) {
-		tgpu_vec_destroy(h->pipe_f[k]), h->pipe_f[k] = nullptr;
-		tgpu_vec_destroy(h->pipe_u[k]), h->pipe_u[k] = nullptr;
-	}
+	h->release_workspace();
 	h->pipe_count = 0;
 	CU(cudaStreamSynchronize(ctx->stream));
 	cudaMemPool_t pool = nullptr;
@@ -1340,7 +1296,7 @@ extern "C" int tgpu_hierarchy_set_lambda(tgpu_hier *h, double lambda)
 	if (!(lambda == lambda)) return fail(TGPU_ERR_ARG, "tgpu_hierarchy_set_lambda: lambda is NaN");
 	h->lambda = lambda;
 	TRY(ensure_scratch32(h));
-	free_graphs(h);
+	h->graphs.clear();
 	TRY(update_iface_buffers(h));
 	return TGPU_OK;
 }
@@ -1348,7 +1304,7 @@ extern "C" int tgpu_hierarchy_force_generic_kernels(tgpu_hier *h, int on)
 {
 	if (!h) return fail(TGPU_ERR_ARG, "null argument");
 	h->generic_kernels = on != 0;
-	free_graphs(h);
+	h->graphs.clear();
 	return TGPU_OK;
 }
 extern "C" int tgpu_level_npatch(const tgpu_hier *h, int level, int64_t *npatch, int64_t *ncells)
@@ -1379,18 +1335,22 @@ extern "C" int tgpu_vec_create(tgpu_hier *h, int level, tgpu_vec **out)
 	*out = v.release();
 	return TGPU_OK;
 }
+// tgpu_vec_create into an owner: the work vectors a hierarchy keeps for itself
+static int vec_create(tgpu_hier *h, int level, VecPtr &v)
+{
+	tgpu_vec *raw = nullptr;
+	TRY(tgpu_vec_create(h, level, &raw));
+	v.reset(raw);
+	return TGPU_OK;
+}
 extern "C" int tgpu_vec_destroy(tgpu_vec *v)
 {
 	if (!v) return TGPU_OK;
 	tgpu_hier *h = v->h;
 	// cached cycle graphs that were captured on this storage are dropped; graphs of other vectors stay
 	for (size_t i = 0; i < h->graphs.size();) {
-		if (h->graphs[i].f == v->d || h->graphs[i].u == v->d) {
-			cudaGraphExecDestroy(h->graphs[i].exec);
-			h->graphs.erase(h->graphs.begin() + i);
-		} else {
-			i++;
-		}
+		if (h->graphs[i].f == v->d || h->graphs[i].u == v->d) h->graphs.erase(h->graphs.begin() + i);
+		else i++;
 	}
 	cudaFreeAsync(v->d, h->ctx->stream); // stream-ordered: work already queued on the vector completes first
 	delete v;
@@ -1493,13 +1453,13 @@ template <int OP> static int reduce(const tgpu_vec *a, const tgpu_vec *b, double
 	tgpu_ctx *ctx = a->h->ctx;
 	const int nb  = std::min(MAX_PARTIAL, grid_for(ctx, a->n, 256, 8));
 	Tag       tg(ctx, "reduce", a->level);
-	TRY(launch(ctx, reduce_stage1<OP>, dim3(nb), dim3(256), 0, a->n, (const double *) a->d, (const double *) b->d, ctx->d_partial));
-	TRY(launch(ctx, reduce_stage2<OP>, dim3(1), dim3(256), 0, nb, (const double *) ctx->d_partial, ctx->d_result));
+	TRY(launch(ctx, reduce_stage1<OP>, dim3(nb), dim3(256), 0, a->n, (const double *) a->d, (const double *) b->d, ctx->d_partial.get()));
+	TRY(launch(ctx, reduce_stage2<OP>, dim3(1), dim3(256), 0, nb, (const double *) ctx->d_partial.get(), ctx->d_result.get()));
 	if (ctx->nranks > 1 && a->h->levels[a->level].distributed)
-		NC(g_nccl.AllReduce(ctx->d_result, ctx->d_result, 1, ncclDouble, OP == 0 ? ncclSum : ncclMax, ctx->comm, ctx->stream));
-	CU(cudaMemcpyAsync(ctx->h_result, ctx->d_result, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+		NC(g_nccl.AllReduce(ctx->d_result.get(), ctx->d_result.get(), 1, ncclDouble, OP == 0 ? ncclSum : ncclMax, ctx->comm, ctx->stream));
+	CU(cudaMemcpyAsync(ctx->h_result.get(), ctx->d_result.get(), sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
 	CU(cudaStreamSynchronize(ctx->stream));
-	*result = ctx->h_result[0];
+	*result = ctx->h_result.get()[0];
 	return check_comm(ctx);
 }
 extern "C" int tgpu_vec_dot(const tgpu_vec *v, const tgpu_vec *b, double *result) { return reduce<0>(v, b, result); }
@@ -1540,29 +1500,29 @@ static bool push_in_kernel(const tgpu_hier *h, int l)
 static int ensure_push_desc(tgpu_hier *h, int l)
 {
 	LevelDev &L = h->levels[l];
-	const double *ucv = l + 1 < (int) h->levels.size() ? h->levels[l + 1].u : nullptr;
+	const double *ucv = l + 1 < (int) h->levels.size() ? h->levels[l + 1].u.get() : nullptr;
 	if (!L.p2p || (L.push_desc && L.push_uc == ucv)) return TGPU_OK;
 	PushDesc d[4];
 	for (int i = 0; i < 4; i++) {
-		d[i].patch          = L.send_patch;
-		d[i].side           = L.send_side;
-		d[i].peer_of        = L.send_peer;
-		d[i].ridx           = L.send_ridx;
+		d[i].patch          = L.send_patch.get();
+		d[i].side           = L.send_side.get();
+		d[i].peer_of        = L.send_peer.get();
+		d[i].ridx           = L.send_ridx.get();
 		d[i].F              = (i & 2) ? L.Fb : L.Fa;
 		d[i].uc             = (i & 1) ? ucv : nullptr;
-		d[i].peerF          = (i & 2) ? L.peerFb : L.peerFa;
+		d[i].peerF          = (i & 2) ? L.peerFb.get() : L.peerFa.get();
 		d[i].ack_flags      = L.ack_flags;
-		d[i].peer_rank      = L.peer_rank;
-		d[i].peer_data_flag = L.peer_data_flag;
-		d[i].cnt            = L.cnt;
-		d[i].ticket         = L.tickets;
-		d[i].abort          = h->p2p_abort;
-		d[i].host_err       = (int *) h->ctx->p2p_err;
+		d[i].peer_rank      = L.peer_rank.get();
+		d[i].peer_data_flag = L.peer_data_flag.get();
+		d[i].cnt            = L.cnt.get();
+		d[i].ticket         = L.tickets.get();
+		d[i].abort          = h->p2p_abort.get();
+		d[i].host_err       = (int *) h->ctx->p2p_err.get();
 		d[i].nfaces         = (int) L.nsend;
 		d[i].npeers         = (int) L.peers.size();
 	}
-	if (!L.push_desc) CU(cudaMalloc(&L.push_desc, sizeof(d)));
-	CU(cudaMemcpy(L.push_desc, d, sizeof(d), cudaMemcpyHostToDevice));
+	if (!L.push_desc) CU(dev_malloc(L.push_desc, sizeof(d)));
+	CU(cudaMemcpy(L.push_desc.get(), d, sizeof(d), cudaMemcpyHostToDevice));
 	L.push_uc = ucv;
 	return TGPU_OK;
 }
@@ -1571,14 +1531,14 @@ static HaloSync halo_sync(tgpu_hier *h, int l, const double *pushF = nullptr, bo
 {
 	LevelDev &L = h->levels[l];
 	HaloSync  hs;
-	if (pushF && L.push_desc) hs.push = L.push_desc + ((pushF == L.Fb ? 2 : 0) + (with_uc ? 1 : 0));
+	if (pushF && L.push_desc) hs.push = L.push_desc.get() + ((pushF == L.Fb ? 2 : 0) + (with_uc ? 1 : 0));
 	hs.data_flags       = L.data_flags;
-	hs.peer_rank        = L.peer_rank;
-	hs.peer_ack_flag    = L.peer_ack_flag;
-	hs.cnt              = L.cnt;
-	hs.ticket           = L.tickets + 1;
-	hs.abort            = h->p2p_abort;
-	hs.host_err         = (int *) h->ctx->p2p_err;
+	hs.peer_rank        = L.peer_rank.get();
+	hs.peer_ack_flag    = L.peer_ack_flag.get();
+	hs.cnt              = L.cnt.get();
+	hs.ticket           = L.tickets.get() + 1;
+	hs.abort            = h->p2p_abort.get();
+	hs.host_err         = (int *) h->ctx->p2p_err.get();
 	hs.npeers           = (int) L.peers.size();
 	hs.first_halo_patch = L.n_interior;
 	hs.enabled          = 1;
@@ -1591,7 +1551,7 @@ static int k_extract_faces(tgpu_hier *h, int l, const double *u, double *F)
 	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, extract_faces_kernel<DD, NN>, dim3(grid_for(h->ctx, L.nface)), dim3(256), 0, L.P, u, F));
 }
 // mode 0: out = A u; 1: out = f - A u; 2: coarse = R (f - A u).  F must hold the faces of u.
-// mode 3: out = A u with the block partial sums of out . f and out . out written to ctx->d_partial ([0..nb),
+// mode 3: out = A u with the block partial sums of out . f and out . out written to ctx->d_partial.get() ([0..nb),
 // [MAX_PARTIAL / 2 ..)); *nb_out = number of partials
 static int k_apply(tgpu_hier *h, int l, int mode, const double *u, const double *f, const double *F, double *out, double *coarse,
                    int p0 = 0, int p1 = -1, int *nb_out = nullptr)
@@ -1600,20 +1560,20 @@ static int k_apply(tgpu_hier *h, int l, int mode, const double *u, const double 
 	if (p1 < 0) p1 = L.P;
 	if (p1 <= p0) return TGPU_OK;
 	Tag       tg(h->ctx, mode == 0 ? "apply" : (mode == 1 ? "residual" : (mode == 2 ? "residual_restrict" : "apply_dots")), l);
-	double *const  part    = h->ctx->d_partial;
+	double *const  part    = h->ctx->d_partial.get();
 	constexpr int  pstride = MAX_PARTIAL / 2;
-	if (is_3d32(h)) { // mode 2: f - A u into L.r, then the restriction
+	if (is_3d32(h)) { // mode 2: f - A u into L.r.get(), then the restriction
 		if (mode == 2 && (p0 != 0 || p1 != L.P)) return fail(TGPU_ERR_UNSUPPORTED, "residual+restrict on a patch range is not available for 32^3 patches");
 		const dim3 grid(std::min((p1 - p0) * 4, h->ctx->sm_count * 2));
 		if (nb_out) *nb_out = (int) grid.x;
 		auto go = [&](auto kernel, double *o) {
-			return launch(h->ctx, kernel, grid, dim3(TGPU_THREADS), apply3d32_tma_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, u, f, F, o, part, pstride);
+			return launch(h->ctx, kernel, grid, dim3(TGPU_THREADS), apply3d32_tma_smem_bytes(), (const PatchMeta *) L.meta.get(), p0, p1, u, f, F, o, part, pstride);
 		};
 		if (mode == 0) return go(apply3d32_tma_kernel<0>, out);
 		if (mode == 3) return go(apply3d32_tma_kernel<3>, out);
 		if (mode == 1) return go(apply3d32_tma_kernel<1>, out);
-		TRY(go(apply3d32_tma_kernel<1>, L.r));
-		return launch(h->ctx, restrict_kernel<3, 32>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta, L.P, (const double *) L.r, coarse);
+		TRY(go(apply3d32_tma_kernel<1>, L.r.get()));
+		return launch(h->ctx, restrict_kernel<3, 32>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, (const double *) L.r.get(), coarse);
 	}
 	DISPATCH_DN(h->D, h->N, {
 		using G        = Geo<DD, NN>;
@@ -1621,7 +1581,7 @@ static int k_apply(tgpu_hier *h, int l, int mode, const double *u, const double 
 		const int grid = std::min(nblk, h->ctx->sm_count * 2);
 		if (nb_out) *nb_out = grid;
 		auto go = [&](auto kernel) {
-			return launch(h->ctx, kernel, dim3(grid), dim3(TGPU_THREADS), apply_tma_smem_bytes<DD, NN>(), (const PatchMeta *) L.meta, p0, p1, u, f, F, out, coarse, part, pstride);
+			return launch(h->ctx, kernel, dim3(grid), dim3(TGPU_THREADS), apply_tma_smem_bytes<DD, NN>(), (const PatchMeta *) L.meta.get(), p0, p1, u, f, F, out, coarse, part, pstride);
 		};
 		if (mode == 0) return go(apply_tma_kernel<DD, NN, 0>);
 		if (mode == 1) return go(apply_tma_kernel<DD, NN, 1>);
@@ -1644,17 +1604,17 @@ static int launch_smooth3d16(tgpu_hier *h, const LevelDev &L, int p0, int p1, co
 		const int  nn = (int) (b1 - b0);
 		if (nn == 0) return TGPU_OK;
 		const dim3 gridn(std::min(nn, h->ctx->sm_count * s16_ctas_per_sm(Z, true))), blockn(S16_BLOCK);
-		return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W, false, true>, gridn, blockn, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta, p0,
-		              p1, f, u, Fin, Fout, (const double *) h->tri, uc, HaloSync{}, 0, NeuTabs{h->mats, h->lam, L.neu_list + (b0 - L.neu_host.begin()), nn});
+		return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W, false, true>, gridn, blockn, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta.get(), p0,
+		              p1, f, u, Fin, Fout, (const double *) h->tri.get(), uc, HaloSync{}, 0, NeuTabs{h->mats.get(), h->lam.get(), L.neu_list.get() + (b0 - L.neu_host.begin()), nn});
 	}
 	const dim3 grid(std::min(p1 - p0, h->ctx->sm_count * s16_ctas_per_sm(Z))), block(S16_BLOCK);
 	if (hs.enabled) {
 		if (Z) return fail(TGPU_ERR_ARG, "smooth3d16: no halo hand-over in a zero-guess sweep");
-		return halo_launch(h->ctx, hs, smooth3d16_kernel<Z, E, PR, W, !Z>, grid, block, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta, p0, p1,
-		                   f, u, Fin, Fout, (const double *) h->tri, uc, hs, skip_neumann, NeuTabs{});
+		return halo_launch(h->ctx, hs, smooth3d16_kernel<Z, E, PR, W, !Z>, grid, block, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta.get(), p0, p1,
+		                   f, u, Fin, Fout, (const double *) h->tri.get(), uc, hs, skip_neumann, NeuTabs{});
 	}
-	return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W>, grid, block, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta, p0, p1, f, u, Fin,
-	              Fout, (const double *) h->tri, uc, hs, skip_neumann, NeuTabs{});
+	return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W>, grid, block, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta.get(), p0, p1, f, u, Fin,
+	              Fout, (const double *) h->tri.get(), uc, hs, skip_neumann, NeuTabs{});
 }
 // hsp != nullptr (multi-GPU, kernels that support it: halo_in_kernel): the launch covers interior and boundary patches and
 // does the halo hand-over itself
@@ -1671,7 +1631,7 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 	                          : (uc ? (write_u ? "smooth_prolong" : "smooth_prolong_faces") : (write_u ? "smooth" : "smooth_faces")),
 	       l);
 	const bool prolong = uc != nullptr;
-	const PatchMeta *meta = L.meta;
+	const PatchMeta *meta = L.meta.get();
 	// A mixed level: the general path sweeps the patches of the range with Neumann domain sides, the specialised kernel skips
 	// them and sweeps the others (two launches, disjoint patches).  lambda != 0 sends every patch through the general path.
 	const bool mixed = specialised(h) && L.has_neumann && h->lambda == 0.0 && !hsp;
@@ -1679,8 +1639,8 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 		if (is_3d32(h)) { // general transform path through an L2-resident scratch block
 			const int nblk = std::min(p1 - p0, h->ctx->sm_count * 2);
 			if (!h->scratch32) return fail(TGPU_ERR_ARG, "k_smooth: scratch for the general 32^3 patch solve missing");
-			TRY(launch(h->ctx, smooth3d32n_kernel, dim3(nblk), dim3(TGPU_THREADS), 0, meta, p0, p1, f, u, Fin, Fout, uc, (const double *) h->mats,
-			           (const double *) h->lam, h->scratch32, (int) zero_guess, (int) emit, (int) prolong, (int) write_u, h->lambda, (int) mixed));
+			TRY(launch(h->ctx, smooth3d32n_kernel, dim3(nblk), dim3(TGPU_THREADS), 0, meta, p0, p1, f, u, Fin, Fout, uc, (const double *) h->mats.get(),
+			           (const double *) h->lam.get(), h->scratch32.get(), (int) zero_guess, (int) emit, (int) prolong, (int) write_u, h->lambda, (int) mixed));
 		} else if (mixed && h->D == 3 && h->N == 16) { // the Neumann instantiation of the specialised kernel
 			TRY(smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto W) {
 				return launch_smooth3d16<Z, E, PR, W>(h, L, p0, p1, f, u, Fin, Fout, uc, HaloSync{}, 0, true);
@@ -1692,8 +1652,8 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 				const dim3   grid(std::min(nblk, h->ctx->sm_count * smooth_min_blocks<NN>())), block(TGPU_THREADS);
 				const size_t sm = smooth_smem_bytes<DD, NN, true>();
 				TRY(smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto) {
-					return launch(h->ctx, smooth_kernel<DD, NN, Z, E, PR>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri, uc,
-					              (const double *) h->mats, (const double *) h->lam, h->lambda, (int) mixed);
+					return launch(h->ctx, smooth_kernel<DD, NN, Z, E, PR>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri.get(), uc,
+					              (const double *) h->mats.get(), (const double *) h->lam.get(), h->lambda, (int) mixed);
 				}));
 			});
 		}
@@ -1710,9 +1670,9 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 			Tag          ti(h->ctx, "iface_rhs", l);
 			const int    k0 = L.gbegin[p0], k1 = L.gbegin[p1];
 			const dim3   gi(std::max(1, std::min((k1 - k0 + IR32_WARPS - 1) / IR32_WARPS, h->ctx->sm_count * IR32_CTAS_PER_SM))), bi(IR32_THREADS);
-			const int32_t *own = L.gowner;
+			const int32_t *own = L.gowner.get();
 			TRY(flag_variant(prolong, hs.enabled, [&](auto PR, auto HALO) {
-				return halo_launch(h->ctx, hs, iface_rhs32_kernel<PR, HALO>, gi, bi, iface_rhs32_smem_bytes(), meta, own, k0, k1, Fin, uc, L.G, hs);
+				return halo_launch(h->ctx, hs, iface_rhs32_kernel<PR, HALO>, gi, bi, iface_rhs32_smem_bytes(), meta, own, k0, k1, Fin, uc, L.G.get(), hs);
 			}));
 		} else if (hs.enabled) {
 			return fail(TGPU_ERR_ARG, "smooth3d32c: no halo hand-over in a zero-guess sweep");
@@ -1721,7 +1681,7 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 		const dim3 grid(2 * std::min(p1 - p0, h->ctx->sm_count / 2)), block(C32_THREADS);
 		return smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto, auto W) {
 			return launch(h->ctx, smooth3d32c_kernel<Z, E, W>, grid, block, smooth3d32c_smem_bytes<Z>(), meta, p0, p1, f, u,
-			              (const double *) L.G, Fout, (const double *) h->tri, skipn, (const int32_t *) L.gslot);
+			              (const double *) L.G.get(), Fout, (const double *) h->tri.get(), skipn, (const int32_t *) L.gslot.get());
 		});
 	}
 	if (h->D == 3)
@@ -1734,7 +1694,7 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 	return smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto W) {
 		return flag_variant(mixed || hs.enabled, [&](auto EXTRA) {
 			return halo_launch(h->ctx, hs, smooth2d32_kernel<Z, E, PR, W, EXTRA>, grid, block, smooth2d32_smem_bytes(), meta, p0, p1, f, u, Fin, Fout,
-			                   (const double *) h->tri, uc, hs, skipn);
+			                   (const double *) h->tri.get(), uc, hs, skipn);
 		});
 	});
 }
@@ -1749,7 +1709,7 @@ static int k_face_residual_restrict(tgpu_hier *h, int l, const double *Fnew, con
 	if (p1 < 0) p1 = L.P;
 	if (p1 <= p0) return hs.push ? fail(TGPU_ERR_ARG, "k_face_residual_restrict: a launch that pushes faces needs patches") : TGPU_OK;
 	Tag tg(h->ctx, "face_residual_restrict", l);
-	const PatchMeta *meta = L.meta;
+	const PatchMeta *meta = L.meta.get();
 	if (is_3d32(h)) {
 		const dim3 grid(std::min(p1 - p0, h->ctx->sm_count * 4)), block(TGPU_THREADS);
 		return flag_variant(Fold != nullptr, hs.enabled, [&](auto FOLD, auto HALO) {
@@ -1778,25 +1738,25 @@ static int k_restrict(tgpu_hier *h, int l, const double *fine, double *coarse)
 {
 	LevelDev &L = h->levels[l];
 	Tag       tg(h->ctx, "restrict", l);
-	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, restrict_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta, L.P, fine, coarse));
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, restrict_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, fine, coarse));
 }
 static int k_prolong_add(tgpu_hier *h, int l, const double *coarse, double *fine)
 {
 	LevelDev &L = h->levels[l];
 	Tag       tg(h->ctx, "prolong_add", l);
-	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, prolong_add_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta, L.P, coarse, fine));
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, prolong_add_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, coarse, fine));
 }
 static int k_prolong_linear_add(tgpu_hier *h, int l, const double *coarse, double *fine)
 {
 	LevelDev &L = h->levels[l];
 	Tag       tg(h->ctx, "prolong_linear_add", l);
-	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, prolong_linear_add_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta, L.P, coarse, fine));
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, prolong_linear_add_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, coarse, fine));
 }
 static int k_prolong_faces(tgpu_hier *h, int l, const double *coarse, double *F)
 {
 	LevelDev &L = h->levels[l];
 	Tag       tg(h->ctx, "prolong_faces", l);
-	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, prolong_faces_kernel<DD, NN>, dim3(grid_for(h->ctx, L.nface)), dim3(256), 0, (const PatchMeta *) L.meta, L.P, coarse, F));
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, prolong_faces_kernel<DD, NN>, dim3(grid_for(h->ctx, L.nface)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, coarse, F));
 }
 static int k_set(tgpu_hier *h, double *v, size_t n, double alpha)
 {
@@ -1814,15 +1774,15 @@ static int p2p_signal(tgpu_hier *h, int l, int kind)
 {
 	LevelDev &L = h->levels[l];
 	Tag       tg(h->ctx, kind == P2P_DATA ? "p2p_signal_data" : "p2p_signal_ack", l);
-	return launch(h->ctx, p2p_signal_kernel, dim3(1), dim3(32), 0, (uint64_t *const *) (kind == P2P_DATA ? L.peer_data_flag : L.peer_ack_flag),
-	              (int) L.peers.size(), L.cnt + (kind == P2P_DATA ? 0 : 2));
+	return launch(h->ctx, p2p_signal_kernel, dim3(1), dim3(32), 0, (uint64_t *const *) (kind == P2P_DATA ? L.peer_data_flag.get() : L.peer_ack_flag.get()),
+	              (int) L.peers.size(), L.cnt.get() + (kind == P2P_DATA ? 0 : 2));
 }
 static int p2p_wait(tgpu_hier *h, int l, int kind, int lag)
 {
 	LevelDev &L = h->levels[l];
 	Tag       tg(h->ctx, kind == P2P_DATA ? "p2p_wait_data" : "p2p_wait_ack", l);
 	return launch(h->ctx, p2p_wait_kernel, dim3(1), dim3(32), 0, (const uint64_t *) (kind == P2P_DATA ? L.data_flags : L.ack_flags),
-	              (const int32_t *) L.peer_rank, (int) L.peers.size(), L.cnt + (kind == P2P_DATA ? 1 : 3), lag, h->p2p_abort, (int *) h->ctx->p2p_err);
+	              (const int32_t *) L.peer_rank.get(), (int) L.peers.size(), L.cnt.get() + (kind == P2P_DATA ? 1 : 3), lag, h->p2p_abort.get(), (int *) h->ctx->p2p_err.get());
 }
 // store my boundary faces (F, or F + P uc on the boundary cells) into the peers' halo slots and publish them: one kernel
 // that waits for the peers' ACK of the previous generation, pushes, and signals DATA from its last block (PushSync)
@@ -1839,18 +1799,18 @@ static int p2p_push(tgpu_hier *h, int l, double *F, const double *uc)
 	}
 	PushSync ps;
 	ps.ack_flags      = L.ack_flags;
-	ps.peer_rank      = L.peer_rank;
-	ps.peer_data_flag = L.peer_data_flag;
-	ps.cnt            = L.cnt;
-	ps.ticket         = L.tickets;
-	ps.abort          = h->p2p_abort;
-	ps.host_err       = (int *) ctx->p2p_err;
+	ps.peer_rank      = L.peer_rank.get();
+	ps.peer_data_flag = L.peer_data_flag.get();
+	ps.cnt            = L.cnt.get();
+	ps.ticket         = L.tickets.get();
+	ps.abort          = h->p2p_abort.get();
+	ps.host_err       = (int *) ctx->p2p_err.get();
 	ps.npeers         = (int) L.peers.size();
 	ps.enabled        = 1;
 	Tag             tg(ctx, "p2p_push_faces", l);
-	double *const *pf = (F == L.Fa) ? L.peerFa : L.peerFb;
+	double *const *pf = (F == L.Fa) ? L.peerFa.get() : L.peerFb.get();
 	DISPATCH_DN_ALL(h->D, h->N, return flag_variant(uc != nullptr, [&](auto PR) {
-		return launch(ctx, push_faces_kernel<DD, NN, PR>, dim3(grid_for(ctx, L.nsend * M)), dim3(256), 0, (const PatchMeta *) L.meta, (int) L.nsend, (const int32_t *) L.send_patch, (const int32_t *) L.send_side, (const int32_t *) L.send_peer, (const int32_t *) L.send_ridx, (const double *) F, uc, pf, ps);
+		return launch(ctx, push_faces_kernel<DD, NN, PR>, dim3(grid_for(ctx, L.nsend * M)), dim3(256), 0, (const PatchMeta *) L.meta.get(), (int) L.nsend, (const int32_t *) L.send_patch.get(), (const int32_t *) L.send_side.get(), (const int32_t *) L.send_peer.get(), (const int32_t *) L.send_ridx.get(), (const double *) F, uc, pf, ps);
 	}));
 }
 static bool exchanges(const tgpu_hier *h, int l)
@@ -1877,20 +1837,20 @@ static int k_exchange(tgpu_hier *h, int l, double *F, const double *uc)
 	Tag tg(ctx, "halo_exchange", l);
 	if (L.nsend) {
 		DISPATCH_DN_ALL(h->D, h->N, TRY(flag_variant(uc != nullptr, [&](auto PR) {
-			return launch(ctx, pack_faces_kernel<DD, NN, PR>, dim3(grid_for(ctx, L.nsend * M)), dim3(256), 0, (const PatchMeta *) L.meta, (int) L.nsend, (const int32_t *) L.send_patch, (const int32_t *) L.send_side, (const double *) F, uc, L.sendbuf);
+			return launch(ctx, pack_faces_kernel<DD, NN, PR>, dim3(grid_for(ctx, L.nsend * M)), dim3(256), 0, (const PatchMeta *) L.meta.get(), (int) L.nsend, (const int32_t *) L.send_patch.get(), (const int32_t *) L.send_side.get(), (const double *) F, uc, L.sendbuf.get());
 		})));
 	}
 	{
 	ProfSpan span(ctx, "nccl_sendrecv", l);
 	NC(g_nccl.GroupStart());
 	for (const PeerDev &pd : L.peers) {
-		if (pd.send_n) NC(g_nccl.Send(L.sendbuf + pd.send_off * M, pd.send_n * M, ncclDouble, pd.peer, ctx->comm, ctx->stream));
-		if (pd.recv_n) NC(g_nccl.Recv(L.recvbuf + pd.recv_off * M, pd.recv_n * M, ncclDouble, pd.peer, ctx->comm, ctx->stream));
+		if (pd.send_n) NC(g_nccl.Send(L.sendbuf.get() + pd.send_off * M, pd.send_n * M, ncclDouble, pd.peer, ctx->comm, ctx->stream));
+		if (pd.recv_n) NC(g_nccl.Recv(L.recvbuf.get() + pd.recv_off * M, pd.recv_n * M, ncclDouble, pd.peer, ctx->comm, ctx->stream));
 	}
 	NC(g_nccl.GroupEnd());
 	}
 	if (L.nrecv) {
-		DISPATCH_DN_ALL(h->D, h->N, TRY(launch(ctx, unpack_faces_kernel<DD, NN>, dim3(grid_for(ctx, L.nrecv * M)), dim3(256), 0, (int) L.nrecv, (const int32_t *) L.recv_slot, (const int32_t *) L.recv_side, (const double *) L.recvbuf, F)));
+		DISPATCH_DN_ALL(h->D, h->N, TRY(launch(ctx, unpack_faces_kernel<DD, NN>, dim3(grid_for(ctx, L.nrecv * M)), dim3(256), 0, (int) L.nrecv, (const int32_t *) L.recv_slot.get(), (const int32_t *) L.recv_side.get(), (const double *) L.recvbuf.get(), F)));
 	}
 	return TGPU_OK;
 }
@@ -1956,9 +1916,9 @@ static int ensure_work(tgpu_hier *h, int l, bool need_r)
 {
 	LevelDev &L = h->levels[l];
 	// the finest level works on the caller's f and u; r only exists for the API-granular schedule (GMG/Cycle.h:59)
-	if (l > 0 && !L.u) CU(cudaMalloc(&L.u, L.ncells * sizeof(double)));
-	if (l > 0 && !L.f) CU(cudaMalloc(&L.f, L.ncells * sizeof(double)));
-	if (need_r && !L.r) CU(cudaMalloc(&L.r, L.ncells * sizeof(double)));
+	if (l > 0 && !L.u) CU(dev_malloc(L.u, L.ncells * sizeof(double)));
+	if (l > 0 && !L.f) CU(dev_malloc(L.f, L.ncells * sizeof(double)));
+	if (need_r && !L.r) CU(dev_malloc(L.r, L.ncells * sizeof(double)));
 	return TGPU_OK;
 }
 extern "C" int tgpu_smooth_jacobi(tgpu_hier *h, int level, const tgpu_vec *f, tgpu_vec *u, double omega)
@@ -1970,9 +1930,9 @@ extern "C" int tgpu_smooth_jacobi(tgpu_hier *h, int level, const tgpu_vec *f, tg
 	LevelDev &L = h->levels[level];
 	TRY(k_extract_faces(h, level, u->d, L.Fa));
 	TRY(k_exchange(h, level, L.Fa, nullptr));
-	TRY(k_apply(h, level, 1, u->d, f->d, L.Fa, L.r, nullptr));
+	TRY(k_apply(h, level, 1, u->d, f->d, L.Fa, L.r.get(), nullptr));
 	TRY(k_exchange_done(h, level));
-	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, jacobi_update_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta, L.P, (const double *) L.r, u->d, omega));
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, jacobi_update_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, (const double *) L.r.get(), u->d, omega));
 	API_END
 }
 extern "C" int tgpu_restrict(tgpu_hier *h, int fine_level, const tgpu_vec *fine, tgpu_vec *coarse)
@@ -2051,12 +2011,12 @@ static int generic_prep_coarser(tgpu_hier *h, int l, const double *f, const doub
 	LevelDev &L = h->levels[l], &C = h->levels[l + 1];
 	TRY(k_extract_faces(h, l, u, L.Fa));
 	TRY(k_exchange(h, l, L.Fa, nullptr));
-	TRY(k_apply(h, l, 1, u, f, L.Fa, L.r, nullptr)); // r = A u; r = -r + f
+	TRY(k_apply(h, l, 1, u, f, L.Fa, L.r.get(), nullptr)); // r = A u; r = -r + f
 	TRY(k_exchange_done(h, l));
-	TRY(k_set(h, C.u, C.ncells, 0.0));               // new_u (zero-initialised Vec)
-	if (crosses_replication(h, l)) TRY(k_set(h, C.f, C.ncells, 0.0));
-	TRY(k_restrict(h, l, L.r, C.f));                 // new_f = R r
-	if (crosses_replication(h, l)) TRY(k_allreduce_sum(h, C.f, C.ncells));
+	TRY(k_set(h, C.u.get(), C.ncells, 0.0));               // new_u (zero-initialised Vec)
+	if (crosses_replication(h, l)) TRY(k_set(h, C.f.get(), C.ncells, 0.0));
+	TRY(k_restrict(h, l, L.r.get(), C.f.get()));                 // new_f = R r
+	if (crosses_replication(h, l)) TRY(k_allreduce_sum(h, C.f.get(), C.ncells));
 	return TGPU_OK;
 }
 static int generic_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double *f, double *u)
@@ -2068,13 +2028,13 @@ static int generic_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const doub
 		LevelDev &C = h->levels[l + 1];
 		for (int i = 0; i < o.pre_sweeps; i++) TRY(generic_smooth(h, l, f, u));
 		TRY(generic_prep_coarser(h, l, f, u));
-		auto prolong = [&]() { return o.interpolator == 1 ? k_prolong_linear_add(h, l, C.u, u) : k_prolong_add(h, l, C.u, u); };
-		TRY(generic_visit(h, o, l + 1, C.f, C.u));
+		auto prolong = [&]() { return o.interpolator == 1 ? k_prolong_linear_add(h, l, C.u.get(), u) : k_prolong_add(h, l, C.u.get(), u); };
+		TRY(generic_visit(h, o, l + 1, C.f.get(), C.u.get()));
 		TRY(prolong());
 		if (o.cycle_type == 1) {
 			for (int i = 0; i < o.mid_sweeps; i++) TRY(generic_smooth(h, l, f, u));
 			TRY(generic_prep_coarser(h, l, f, u));
-			TRY(generic_visit(h, o, l + 1, C.f, C.u));
+			TRY(generic_visit(h, o, l + 1, C.f.get(), C.u.get()));
 			TRY(prolong());
 		}
 		for (int i = 0; i < o.post_sweeps; i++) TRY(generic_smooth(h, l, f, u));
@@ -2088,12 +2048,12 @@ static int exchange_async(tgpu_hier *h, int l, double *F, const double *uc, cuda
 	tgpu_ctx *   ctx  = h->ctx;
 	cudaStream_t main = ctx->stream;
 	CU(cudaEventRecord(fork, main));
-	CU(cudaStreamWaitEvent(ctx->comm_stream, fork, 0));
-	ctx->stream = ctx->comm_stream;
+	CU(cudaStreamWaitEvent(ctx->comm_stream.get(), fork, 0));
+	ctx->stream = ctx->comm_stream.get();
 	int rc      = k_exchange(h, l, F, uc);
 	ctx->stream = main;
 	TRY(rc);
-	CU(cudaEventRecord(done, ctx->comm_stream));
+	CU(cudaEventRecord(done, ctx->comm_stream.get()));
 	return TGPU_OK;
 }
 // Fused schedule for V cycles with >= 1 pre and post sweep.  Per level visit:
@@ -2137,10 +2097,10 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 	const double *Fold    = (guess || o.pre_sweeps > 1) ? Falt : nullptr;
 	const bool    overlap = exchanges(h, l);
 	auto residual_restrict = [&](int p0, int p1) {
-		if (from_faces) return k_face_residual_restrict(h, l, Fcur, Fold, C.f, p0, p1);
-		return k_apply(h, l, 2, u, f, Fcur, nullptr, C.f, p0, p1);
+		if (from_faces) return k_face_residual_restrict(h, l, Fcur, Fold, C.f.get(), p0, p1);
+		return k_apply(h, l, 2, u, f, Fcur, nullptr, C.f.get(), p0, p1);
 	};
-	if (crosses_replication(h, l)) TRY(k_set(h, C.f, C.ncells, 0.0));
+	if (crosses_replication(h, l)) TRY(k_set(h, C.f.get(), C.ncells, 0.0));
 	if (overlap && L.p2p && from_faces && halo_in_kernel(h, l)) {
 		// the faces of the pre-smoothed u go straight into the neighbours' halo slots; theirs arrive while the patches
 		// without off-rank neighbours are swept: ONE launch over all owned patches whose CTAs poll the peers' flags
@@ -2148,7 +2108,7 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 		// (push_in_kernel: the same launch pushes this rank's faces first, halo_push_cta)
 		const HaloSync hs = halo_sync(h, l, push_in_kernel(h, l) ? Fcur : nullptr, false);
 		if (!hs.push) TRY(p2p_push(h, l, Fcur, nullptr));
-		TRY(k_face_residual_restrict(h, l, Fcur, Fold, C.f, 0, L.P, &hs));
+		TRY(k_face_residual_restrict(h, l, Fcur, Fold, C.f.get(), 0, L.P, &hs));
 	} else if (overlap && L.p2p) {
 		TRY(p2p_push(h, l, Fcur, nullptr));
 		TRY(residual_restrict(0, L.n_interior));
@@ -2157,34 +2117,34 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 		TRY(k_exchange_done(h, l));
 	} else if (overlap) {
 		// faces of the pre-smoothed u travel on the comm stream while the interior patches are swept
-		TRY(exchange_async(h, l, Fcur, nullptr, L.ev[0], L.ev[1]));
+		TRY(exchange_async(h, l, Fcur, nullptr, L.ev[0].get(), L.ev[1].get()));
 		TRY(residual_restrict(0, L.n_interior));
-		CU(cudaStreamWaitEvent(h->ctx->stream, L.ev[1], 0));
+		CU(cudaStreamWaitEvent(h->ctx->stream, L.ev[1].get(), 0));
 		TRY(residual_restrict(L.n_interior, L.P));
 	} else {
 		TRY(residual_restrict(0, L.P));
 	}
-	if (crosses_replication(h, l)) TRY(k_allreduce_sum(h, C.f, C.ncells));
-	TRY(fused_visit(h, o, l + 1, C.f, C.u, false));
+	if (crosses_replication(h, l)) TRY(k_allreduce_sum(h, C.f.get(), C.ncells));
+	TRY(fused_visit(h, o, l + 1, C.f.get(), C.u.get(), false));
 	if (o.cycle_type == 1) {
 		// W cycle (GMG/WCycle.h:57-63; one GPU, mid_sweeps >= 1): the second coarse-grid correction.  The iterate before the
 		// mid sweeps is u_pre + P u_c, seen only through its boundary slices: Fcur += (P u_c) on the boundary cells; every
 		// mid sweep emits the slices of its result, and the residual after the last one is again supported on the faces
 		// (old slices - new slices), so neither u_pre + P u_c nor the mid-smoothed u is ever written.
-		TRY(k_prolong_faces(h, l, C.u, Fcur));
+		TRY(k_prolong_faces(h, l, C.u.get(), Fcur));
 		for (int i = 0; i < o.mid_sweeps; i++) {
 			TRY(k_smooth(h, l, false, true, f, u, Fcur, Falt, nullptr, 0, -1, !from_faces));
 			std::swap(Fcur, Falt);
 		}
 		Fold = Falt;
 		TRY(residual_restrict(0, L.P));
-		TRY(fused_visit(h, o, l + 1, C.f, C.u, false));
+		TRY(fused_visit(h, o, l + 1, C.f.get(), C.u.get(), false));
 	}
 	// same faces + prolonged correction for the neighbours on other GPUs (owned faces add it on the fly)
-	const bool push_folded = overlap && L.p2p && o.post_sweeps >= 1 && push_in_kernel(h, l) && L.push_desc && L.push_uc == C.u;
+	const bool push_folded = overlap && L.p2p && o.post_sweeps >= 1 && push_in_kernel(h, l) && L.push_desc && L.push_uc == C.u.get();
 	if (push_folded) {} // the first post-sweep's launch pushes them itself
-	else if (overlap && L.p2p) TRY(p2p_push(h, l, Fcur, C.u));
-	else if (overlap) TRY(exchange_async(h, l, Fcur, C.u, L.ev[2], L.ev[3]));
+	else if (overlap && L.p2p) TRY(p2p_push(h, l, Fcur, C.u.get()));
+	else if (overlap) TRY(exchange_async(h, l, Fcur, C.u.get(), L.ev[2].get(), L.ev[3].get()));
 	for (int i = 0; i < o.post_sweeps; i++) {
 		const bool lastsweep = (i + 1 == o.post_sweeps);
 		const bool emit      = !lastsweep || want_faces;
@@ -2192,15 +2152,15 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 		if (i > 0) TRY(k_exchange(h, l, Fcur, nullptr));
 		if (i == 0 && overlap && L.p2p && halo_in_kernel(h, l)) {
 			const HaloSync hs = halo_sync(h, l, push_folded ? Fcur : nullptr, true);
-			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, C.u, 0, L.P, lastsweep, &hs));
+			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, C.u.get(), 0, L.P, lastsweep, &hs));
 		} else if (i == 0 && overlap) {
-			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, C.u, 0, L.n_interior, lastsweep));
+			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, C.u.get(), 0, L.n_interior, lastsweep));
 			if (L.p2p) TRY(p2p_wait(h, l, P2P_DATA, 0));
-			else CU(cudaStreamWaitEvent(h->ctx->stream, L.ev[3], 0));
-			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, C.u, L.n_interior, L.P, lastsweep));
+			else CU(cudaStreamWaitEvent(h->ctx->stream, L.ev[3].get(), 0));
+			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, C.u.get(), L.n_interior, L.P, lastsweep));
 			TRY(k_exchange_done(h, l));
 		} else {
-			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, i == 0 ? C.u : nullptr, 0, -1, lastsweep));
+			TRY(k_smooth(h, l, false, emit, f, u, Fcur, Falt, i == 0 ? C.u.get() : nullptr, 0, -1, lastsweep));
 			if (i > 0) TRY(k_exchange_done(h, l));
 		}
 		std::swap(Fcur, Falt);
@@ -2208,7 +2168,7 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 	if (l == 0 && want_faces) { // the last sweep emitted the slices of u here; Falt holds those of its input
 		h->cycle_faces     = Fcur;
 		h->cycle_faces_old = Falt;
-		h->cycle_uc        = o.post_sweeps == 1 ? C.u : nullptr;
+		h->cycle_uc        = o.post_sweeps == 1 ? C.u.get() : nullptr;
 	}
 	return TGPU_OK;
 }
@@ -2280,36 +2240,32 @@ static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, d
 			h->cycle_faces     = g.faces;
 			h->cycle_faces_old = g.faces_old;
 			h->cycle_uc        = g.faces_uc;
-			CU(cudaGraphLaunch(g.exec, ctx->stream));
+			CU(cudaGraphLaunch(g.exec.get(), ctx->stream));
 			ctx->launches += g.kernels;
 			return TGPU_OK;
 		}
 	// capture
-	cudaGraph_t graph = nullptr;
-	ctx->capturing    = true;
-	ctx->captured     = 0;
+	ctx->capturing = true;
+	ctx->captured  = 0;
 	CU(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-	int         rc = run_cycle(h, o, f, u, want_faces, guess);
-	cudaError_t e  = cudaStreamEndCapture(ctx->stream, &graph);
+	int         rc  = run_cycle(h, o, f, u, want_faces, guess);
+	cudaGraph_t raw = nullptr;
+	cudaError_t e   = cudaStreamEndCapture(ctx->stream, &raw);
+	GraphPtr    graph(raw);
 	ctx->capturing = false;
-	if (rc != TGPU_OK) {
-		if (graph) cudaGraphDestroy(graph);
-		return rc;
-	}
+	TRY(rc);
 	if (e != cudaSuccess) return fail(TGPU_ERR_CUDA, std::string("cudaStreamEndCapture: ") + cudaGetErrorString(e));
 	GraphEntry g;
 	g.f = f, g.u = u, g.opts = o, g.kernels = ctx->captured;
 	g.want_faces = want_faces, g.faces = h->cycle_faces;
 	g.guess = guess, g.faces_old = h->cycle_faces_old, g.faces_uc = h->cycle_uc;
-	CU(cudaGraphInstantiate(&g.exec, graph, 0));
-	cudaGraphDestroy(graph);
-	if (h->graphs.size() >= 8) {
-		cudaGraphExecDestroy(h->graphs.front().exec);
-		h->graphs.erase(h->graphs.begin());
-	}
-	h->graphs.push_back(g);
-	CU(cudaGraphLaunch(g.exec, ctx->stream));
-	ctx->launches += g.kernels;
+	cudaGraphExec_t exec = nullptr;
+	CU(cudaGraphInstantiate(&exec, graph.get(), 0));
+	g.exec.reset(exec);
+	if (h->graphs.size() >= 8) h->graphs.erase(h->graphs.begin());
+	h->graphs.push_back(std::move(g));
+	CU(cudaGraphLaunch(h->graphs.back().exec.get(), ctx->stream));
+	ctx->launches += h->graphs.back().kernels;
 	return TGPU_OK;
 }
 extern "C" int tgpu_vcycle(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu_vec *u)
@@ -2325,16 +2281,26 @@ extern "C" int tgpu_vcycle_host(tgpu_hier *h, const TgpuCycleOpts *opts, const d
 {
 	API_BEGIN
 	if (!h || !f_host || !u_host) return fail(TGPU_ERR_ARG, "tgpu_vcycle_host: null argument");
-	if (!h->host_f) TRY(tgpu_vec_create(h, 0, &h->host_f));
-	if (!h->host_u) TRY(tgpu_vec_create(h, 0, &h->host_u));
-	TRY(tgpu_vec_upload_async(h->host_f, f_host));
+	if (!h->host_f) TRY(vec_create(h, 0, h->host_f));
+	if (!h->host_u) TRY(vec_create(h, 0, h->host_u));
+	TRY(tgpu_vec_upload_async(h->host_f.get(), f_host));
 	TRY(cycle_ptr(h, opts, h->host_f->d, h->host_u->d));
-	TRY(tgpu_vec_download_async(h->host_u, u_host));
+	TRY(tgpu_vec_download_async(h->host_u.get(), u_host));
 	CU(cudaStreamSynchronize(h->ctx->stream));
 	return check_comm(h->ctx);
 	API_END
 }
 
+// the copy-in / copy-out streams of the pipelined host path and their events, created on first use
+static int ensure_pipe_streams(tgpu_hier *h)
+{
+	for (StreamPtr *s : {&h->s_in, &h->s_out})
+		if (!*s) CU(stream_create(*s));
+	for (int k = 0; k < 2; k++)
+		for (EventPtr *e : {&h->ev_in[k], &h->ev_cyc[k], &h->ev_out[k]})
+			if (!*e) CU(event_create(*e, cudaEventDisableTiming));
+	return TGPU_OK;
+}
 // Pipelined form of tgpu_vcycle_host for a stream of independent right-hand sides: the upload of call k + 1
 // runs on a copy-in stream while cycle k is on the main stream and result k - 1 travels back on a copy-out
 // stream (PCIe is full duplex), with two device slots.  The caller owns the pinned buffers; u_pinned of call k
@@ -2344,19 +2310,11 @@ extern "C" int tgpu_vcycle_host_async(tgpu_hier *h, const TgpuCycleOpts *opts, c
 	API_BEGIN
 	if (!h || !f_host || !u_host) return fail(TGPU_ERR_ARG, "tgpu_vcycle_host_async: null argument");
 	tgpu_ctx *ctx = h->ctx;
-	if (!h->s_in) {
-		CU(cudaStreamCreateWithFlags(&h->s_in, cudaStreamNonBlocking));
-		CU(cudaStreamCreateWithFlags(&h->s_out, cudaStreamNonBlocking));
-		for (int k = 0; k < 2; k++) {
-			CU(cudaEventCreateWithFlags(&h->ev_in[k], cudaEventDisableTiming));
-			CU(cudaEventCreateWithFlags(&h->ev_cyc[k], cudaEventDisableTiming));
-			CU(cudaEventCreateWithFlags(&h->ev_out[k], cudaEventDisableTiming));
-		}
-	}
+	TRY(ensure_pipe_streams(h));
 	if (!h->pipe_f[0]) { // first call, or the first one after tgpu_hierarchy_trim
 		for (int k = 0; k < 2; k++) {
-			TRY(tgpu_vec_create(h, 0, &h->pipe_f[k]));
-			TRY(tgpu_vec_create(h, 0, &h->pipe_u[k]));
+			TRY(vec_create(h, 0, h->pipe_f[k]));
+			TRY(vec_create(h, 0, h->pipe_u[k]));
 		}
 		CU(cudaStreamSynchronize(ctx->stream)); // the zero fills of the new vectors
 	}
@@ -2365,18 +2323,18 @@ extern "C" int tgpu_vcycle_host_async(tgpu_hier *h, const TgpuCycleOpts *opts, c
 	const size_t bytes = h->pipe_f[k]->n * sizeof(double);
 	h->pipe_count++;
 	// copy-in: the cycle that last read this slot's f must be done
-	if (!first) CU(cudaStreamWaitEvent(h->s_in, h->ev_cyc[k], 0));
-	CU(cudaMemcpyAsync(h->pipe_f[k]->d, f_host, bytes, cudaMemcpyHostToDevice, h->s_in));
-	CU(cudaEventRecord(h->ev_in[k], h->s_in));
+	if (!first) CU(cudaStreamWaitEvent(h->s_in.get(), h->ev_cyc[k].get(), 0));
+	CU(cudaMemcpyAsync(h->pipe_f[k]->d, f_host, bytes, cudaMemcpyHostToDevice, h->s_in.get()));
+	CU(cudaEventRecord(h->ev_in[k].get(), h->s_in.get()));
 	// cycle: needs this slot's f, and its u must have left for the host
-	CU(cudaStreamWaitEvent(ctx->stream, h->ev_in[k], 0));
-	if (!first) CU(cudaStreamWaitEvent(ctx->stream, h->ev_out[k], 0));
+	CU(cudaStreamWaitEvent(ctx->stream, h->ev_in[k].get(), 0));
+	if (!first) CU(cudaStreamWaitEvent(ctx->stream, h->ev_out[k].get(), 0));
 	TRY(cycle_ptr(h, opts, h->pipe_f[k]->d, h->pipe_u[k]->d));
-	CU(cudaEventRecord(h->ev_cyc[k], ctx->stream));
+	CU(cudaEventRecord(h->ev_cyc[k].get(), ctx->stream));
 	// copy-out
-	CU(cudaStreamWaitEvent(h->s_out, h->ev_cyc[k], 0));
-	CU(cudaMemcpyAsync(u_host, h->pipe_u[k]->d, bytes, cudaMemcpyDeviceToHost, h->s_out));
-	CU(cudaEventRecord(h->ev_out[k], h->s_out));
+	CU(cudaStreamWaitEvent(h->s_out.get(), h->ev_cyc[k].get(), 0));
+	CU(cudaMemcpyAsync(u_host, h->pipe_u[k]->d, bytes, cudaMemcpyDeviceToHost, h->s_out.get()));
+	CU(cudaEventRecord(h->ev_out[k].get(), h->s_out.get()));
 	return TGPU_OK;
 	API_END
 }
@@ -2388,20 +2346,12 @@ extern "C" int tgpu_vec_transfer_pair(tgpu_hier *h, tgpu_vec *dst_dev, const dou
 	TRY(check_level_vec(h, 0, dst_dev, "tgpu_vec_transfer_pair"));
 	TRY(check_level_vec(h, 0, src_dev, "tgpu_vec_transfer_pair"));
 	if (!src_pinned || !dst_pinned) return fail(TGPU_ERR_ARG, "tgpu_vec_transfer_pair: null host buffer");
-	if (!h->s_in) {
-		CU(cudaStreamCreateWithFlags(&h->s_in, cudaStreamNonBlocking));
-		CU(cudaStreamCreateWithFlags(&h->s_out, cudaStreamNonBlocking));
-		for (int k = 0; k < 2; k++) {
-			CU(cudaEventCreateWithFlags(&h->ev_in[k], cudaEventDisableTiming));
-			CU(cudaEventCreateWithFlags(&h->ev_cyc[k], cudaEventDisableTiming));
-			CU(cudaEventCreateWithFlags(&h->ev_out[k], cudaEventDisableTiming));
-		}
-	}
+	TRY(ensure_pipe_streams(h));
 	CU(cudaStreamSynchronize(h->ctx->stream));
-	CU(cudaMemcpyAsync(dst_dev->d, src_pinned, dst_dev->n * sizeof(double), cudaMemcpyHostToDevice, h->s_in));
-	CU(cudaMemcpyAsync(dst_pinned, src_dev->d, src_dev->n * sizeof(double), cudaMemcpyDeviceToHost, h->s_out));
-	CU(cudaStreamSynchronize(h->s_in));
-	CU(cudaStreamSynchronize(h->s_out));
+	CU(cudaMemcpyAsync(dst_dev->d, src_pinned, dst_dev->n * sizeof(double), cudaMemcpyHostToDevice, h->s_in.get()));
+	CU(cudaMemcpyAsync(dst_pinned, src_dev->d, src_dev->n * sizeof(double), cudaMemcpyDeviceToHost, h->s_out.get()));
+	CU(cudaStreamSynchronize(h->s_in.get()));
+	CU(cudaStreamSynchronize(h->s_out.get()));
 	return TGPU_OK;
 	API_END
 }
@@ -2409,7 +2359,7 @@ extern "C" int tgpu_vcycle_host_wait(tgpu_hier *h)
 {
 	API_BEGIN
 	if (!h) return fail(TGPU_ERR_ARG, "null hierarchy");
-	if (h->s_out) CU(cudaStreamSynchronize(h->s_out));
+	if (h->s_out) CU(cudaStreamSynchronize(h->s_out.get()));
 	CU(cudaStreamSynchronize(h->ctx->stream));
 	return check_comm(h->ctx);
 	API_END
@@ -2423,24 +2373,24 @@ static int bicgstab_fused(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_ve
 {
 	tgpu_ctx *ctx = h->ctx;
 	while (h->krylov_ws.size() < 8) {
-		tgpu_vec *v = nullptr;
-		TRY(tgpu_vec_create(h, 0, &v));
-		h->krylov_ws.push_back(v);
+		VecPtr v;
+		TRY(vec_create(h, 0, v));
+		h->krylov_ws.push_back(std::move(v));
 	}
-	if (!h->krylov_sc) CU(cudaMalloc(&h->krylov_sc, 8 * sizeof(double)));
-	tgpu_vec *resid = h->krylov_ws[0], *rhat = h->krylov_ws[1], *p = h->krylov_ws[2], *ap = h->krylov_ws[3];
-	tgpu_vec *as = h->krylov_ws[4], *s = h->krylov_ws[5], *ms = h->krylov_ws[6], *mp = h->krylov_ws[7];
+	if (!h->krylov_sc) CU(dev_malloc(h->krylov_sc, 8 * sizeof(double)));
+	tgpu_vec *resid = h->krylov_ws[0].get(), *rhat = h->krylov_ws[1].get(), *p = h->krylov_ws[2].get(), *ap = h->krylov_ws[3].get();
+	tgpu_vec *as = h->krylov_ws[4].get(), *s = h->krylov_ws[5].get(), *ms = h->krylov_ws[6].get(), *mp = h->krylov_ws[7].get();
 	const bool   prec   = opts != nullptr;
 	const bool   dist   = ctx->nranks > 1 && h->levels[0].distributed;
 	const size_t n      = resid->n;
 	const int    stride = MAX_PARTIAL / 2;
 	const int    nb     = std::min(stride, grid_for(ctx, n, 256, 8));
-	double *     sc     = h->krylov_sc;
+	double *     sc     = h->krylov_sc.get();
 	auto A = [&](const tgpu_vec *in, tgpu_vec *out) { return tgpu_apply(h, 0, in, out); };
 	// the preconditioner's last sweep emits the boundary slices of its result, which is all A needs besides the result
 	auto M = [&](const tgpu_vec *in, tgpu_vec *out) { return cycle_ptr(h, opts, in->d, out->d, true); };
 	// out = A in for in = the vector M has just produced (its boundary slices are in h->cycle_faces), with the dot products the
-	// iteration needs next (out . dotv, out . out) formed by the same kernel: *nbp block partials in ctx->d_partial
+	// iteration needs next (out . dotv, out . out) formed by the same kernel: *nbp block partials in ctx->d_partial.get()
 	auto AM = [&](const tgpu_vec *in, tgpu_vec *out, const tgpu_vec *dotv, int *nbp) {
 		double *F = h->cycle_faces;
 		if (!F) {
@@ -2453,7 +2403,7 @@ static int bicgstab_fused(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_ve
 	};
 	auto finish = [&](int step, int nparts) {
 		Tag tg(ctx, "bicg_scalars", 0);
-		TRY(launch(ctx, bicg_finish_kernel, dim3(1), dim3(256), 0, nparts, stride, (const double *) ctx->d_partial, sc, step, dist ? 0 : 1));
+		TRY(launch(ctx, bicg_finish_kernel, dim3(1), dim3(256), 0, nparts, stride, (const double *) ctx->d_partial.get(), sc, step, dist ? 0 : 1));
 		if (dist) {
 			NC(g_nccl.AllReduce(sc + SC_SUM0, sc + SC_SUM0, 2, ncclDouble, ncclSum, ctx->comm, ctx->stream));
 			TRY(launch(ctx, bicg_scalars_kernel, dim3(1), dim3(32), 0, sc, step));
@@ -2462,13 +2412,13 @@ static int bicgstab_fused(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_ve
 	};
 	auto dots = [&](const tgpu_vec *a, const tgpu_vec *c, int step) {
 		Tag tg(ctx, "bicg_dots", 0);
-		TRY(launch(ctx, bicg_dots_kernel, dim3(nb), dim3(256), 0, n, (const double *) a->d, (const double *) c->d, ctx->d_partial, stride));
+		TRY(launch(ctx, bicg_dots_kernel, dim3(nb), dim3(256), 0, n, (const double *) a->d, (const double *) c->d, ctx->d_partial.get(), stride));
 		return finish(step, nb);
 	};
 	auto read_rnorm = [&](double *out) {
-		CU(cudaMemcpyAsync(ctx->h_result, sc + SC_RNORM, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+		CU(cudaMemcpyAsync(ctx->h_result.get(), sc + SC_RNORM, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
 		CU(cudaStreamSynchronize(ctx->stream));
-		*out = ctx->h_result[0];
+		*out = ctx->h_result.get()[0];
 		return check_comm(ctx);
 	};
 	TRY(A(x, resid));
@@ -2507,7 +2457,7 @@ static int bicgstab_fused(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_ve
 		}
 		{
 			Tag tg(ctx, "bicg_xr", 0);
-			TRY(launch(ctx, bicg_xr_kernel, dim3(nb), dim3(256), 0, n, x->d, (const double *) pp->d, (const double *) ss->d, resid->d, (const double *) ap->d, (const double *) as->d, (const double *) rhat->d, (const double *) sc, ctx->d_partial, stride));
+			TRY(launch(ctx, bicg_xr_kernel, dim3(nb), dim3(256), 0, n, x->d, (const double *) pp->d, (const double *) ss->d, resid->d, (const double *) ap->d, (const double *) as->d, (const double *) rhat->d, (const double *) sc, ctx->d_partial.get(), stride));
 		}
 		TRY(finish(3, nb)); // rho, beta, |r|
 		{
@@ -2535,18 +2485,18 @@ extern "C" int tgpu_bicgstab(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu
 // ------------------------------------------------------------------------------------------
 // stationary multigrid: u <- u + Cycle(f - A u), from the iterate in u
 // ------------------------------------------------------------------------------------------
-// sum of squares of level vector v into ctx->d_result[0] (all ranks), no host read
+// sum of squares of level vector v into ctx->d_result.get()[0] (all ranks), no host read
 static int k_sumsq(tgpu_hier *h, const double *v, size_t n)
 {
 	tgpu_ctx *ctx = h->ctx;
 	const int nb  = std::min(MAX_PARTIAL, grid_for(ctx, n, 256, 8));
 	Tag       tg(ctx, "reduce", 0);
-	TRY(launch(ctx, reduce_stage1<0>, dim3(nb), dim3(256), 0, n, v, v, ctx->d_partial));
-	TRY(launch(ctx, reduce_stage2<0>, dim3(1), dim3(256), 0, nb, (const double *) ctx->d_partial, ctx->d_result));
-	if (ctx->nranks > 1 && h->levels[0].distributed) NC(g_nccl.AllReduce(ctx->d_result, ctx->d_result, 1, ncclDouble, ncclSum, ctx->comm, ctx->stream));
+	TRY(launch(ctx, reduce_stage1<0>, dim3(nb), dim3(256), 0, n, v, v, ctx->d_partial.get()));
+	TRY(launch(ctx, reduce_stage2<0>, dim3(1), dim3(256), 0, nb, (const double *) ctx->d_partial.get(), ctx->d_result.get()));
+	if (ctx->nranks > 1 && h->levels[0].distributed) NC(g_nccl.AllReduce(ctx->d_result.get(), ctx->d_result.get(), 1, ncclDouble, ncclSum, ctx->comm, ctx->stream));
 	return TGPU_OK;
 }
-// ||f - A u||^2 of the full residual (r: work vector) into ctx->d_result[0]
+// ||f - A u||^2 of the full residual (r: work vector) into ctx->d_result.get()[0]
 static int k_residual_sumsq(tgpu_hier *h, const double *f, const double *u, double *r)
 {
 	LevelDev &L = h->levels[0];
@@ -2556,7 +2506,7 @@ static int k_residual_sumsq(tgpu_hier *h, const double *f, const double *u, doub
 	TRY(k_exchange_done(h, 0));
 	return k_sumsq(h, r, L.ncells);
 }
-// ||f - A u||^2 into ctx->d_result[0] right after a cycle that emitted the slices of its result u and kept those of the
+// ||f - A u||^2 into ctx->d_result.get()[0] right after a cycle that emitted the slices of its result u and kept those of the
 // input of its last sweep (h->cycle_faces, h->cycle_faces_old, h->cycle_uc): face_residual_norm_kernel.  Reads S x M
 // values of two face buffers per patch; neither u nor f.  The neighbours' new slices reach the halo slots first.
 static int k_face_residual_norm(tgpu_hier *h)
@@ -2574,21 +2524,21 @@ static int k_face_residual_norm(tgpu_hier *h)
 			const dim3   block(frn_threads<DD, NN>());
 			const size_t sm = frn_smem_bytes<DD, NN>();
 			TRY(flag_variant(uc != nullptr, [&](auto UC) {
-				return launch(ctx, face_residual_norm_kernel<DD, NN, UC ? FV_PROLONG_DIFF : FV_DIFF>, dim3(nb), block, sm, (const PatchMeta *) L.meta, L.P, (const double *) Fnew, Fold, uc, ctx->d_partial);
+				return launch(ctx, face_residual_norm_kernel<DD, NN, UC ? FV_PROLONG_DIFF : FV_DIFF>, dim3(nb), block, sm, (const PatchMeta *) L.meta.get(), L.P, (const double *) Fnew, Fold, uc, ctx->d_partial.get());
 			}));
 		});
-		TRY(launch(ctx, reduce_stage2<0>, dim3(1), dim3(256), 0, nb, (const double *) ctx->d_partial, ctx->d_result));
+		TRY(launch(ctx, reduce_stage2<0>, dim3(1), dim3(256), 0, nb, (const double *) ctx->d_partial.get(), ctx->d_result.get()));
 	}
 	TRY(k_exchange_done(h, 0));
-	if (ctx->nranks > 1 && L.distributed) NC(g_nccl.AllReduce(ctx->d_result, ctx->d_result, 1, ncclDouble, ncclSum, ctx->comm, ctx->stream));
+	if (ctx->nranks > 1 && L.distributed) NC(g_nccl.AllReduce(ctx->d_result.get(), ctx->d_result.get(), 1, ncclDouble, ncclSum, ctx->comm, ctx->stream));
 	return TGPU_OK;
 }
-// host read of ctx->d_result[0 .. n)
+// host read of ctx->d_result.get()[0 .. n)
 static int read_result(tgpu_ctx *ctx, double *out, int n = 1)
 {
-	CU(cudaMemcpyAsync(ctx->h_result, ctx->d_result, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+	CU(cudaMemcpyAsync(ctx->h_result.get(), ctx->d_result.get(), n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
 	CU(cudaStreamSynchronize(ctx->stream));
-	for (int i = 0; i < n; i++) out[i] = ctx->h_result[i];
+	for (int i = 0; i < n; i++) out[i] = ctx->h_result.get()[i];
 	return check_comm(ctx);
 }
 static int check_stationary_args(tgpu_hier *h, const tgpu_vec *f, const tgpu_vec *u, const char *what)
@@ -2601,13 +2551,13 @@ static int check_stationary_args(tgpu_hier *h, const tgpu_vec *f, const tgpu_vec
 static int ensure_gmg_ws(tgpu_hier *h)
 {
 	while (h->gmg_ws.size() < 2) {
-		tgpu_vec *v = nullptr;
-		TRY(tgpu_vec_create(h, 0, &v));
-		h->gmg_ws.push_back(v);
+		VecPtr v;
+		TRY(vec_create(h, 0, v));
+		h->gmg_ws.push_back(std::move(v));
 	}
 	return TGPU_OK;
 }
-// one update u <- u + Cycle(f - A u); want_norm: ||f - A u_new||^2 in ctx->d_result[0] afterwards.  The fused schedule
+// one update u <- u + Cycle(f - A u); want_norm: ||f - A u_new||^2 in ctx->d_result.get()[0] afterwards.  The fused schedule
 // starts from u (guess_schedule) and takes the norm from the faces; every other schedule runs the loop it replaces:
 // residual into a work vector, the cycle from zero, add, and (want_norm) a full residual of the result.
 static int update_once(tgpu_hier *h, const TgpuCycleOpts *opts, const TgpuCycleOpts &o, const tgpu_vec *f, tgpu_vec *u, bool want_norm)
@@ -2617,7 +2567,7 @@ static int update_once(tgpu_hier *h, const TgpuCycleOpts *opts, const TgpuCycleO
 		return want_norm ? k_face_residual_norm(h) : TGPU_OK;
 	}
 	TRY(ensure_gmg_ws(h));
-	tgpu_vec *r = h->gmg_ws[0], *e = h->gmg_ws[1];
+	tgpu_vec *r = h->gmg_ws[0].get(), *e = h->gmg_ws[1].get();
 	TRY(tgpu_residual(h, 0, f, u, r));
 	TRY(cycle_ptr(h, opts, r->d, e->d));
 	TRY(tgpu_vec_add(u, e));
@@ -2632,7 +2582,7 @@ extern "C" int tgpu_vcycle_update(tgpu_hier *h, const TgpuCycleOpts *opts, const
 	TRY(update_once(h, opts, o, f, u, rel_residual != nullptr));
 	if (!rel_residual) return TGPU_OK;
 	double rr[2];
-	CU(cudaMemcpyAsync(h->ctx->d_result + 1, h->ctx->d_result, sizeof(double), cudaMemcpyDeviceToDevice, h->ctx->stream));
+	CU(cudaMemcpyAsync(h->ctx->d_result.get() + 1, h->ctx->d_result.get(), sizeof(double), cudaMemcpyDeviceToDevice, h->ctx->stream));
 	TRY(k_sumsq(h, f->d, f->n));
 	TRY(read_result(h->ctx, rr, 2)); // ||f||^2, ||f - A u||^2
 	*rel_residual = rr[0] > 0.0 ? sqrt(rr[1] / rr[0]) : sqrt(rr[1]);
@@ -2675,7 +2625,7 @@ extern "C" int tgpu_gmg_solve(tgpu_hier *h, const TgpuCycleOpts *opts, const tgp
 				rel = sqrt(rsq) * scale;
 			}
 		} else { // the loop: cycle from zero on the residual in gmg_ws[0], add, residual (also the convergence test)
-			tgpu_vec *rv = h->gmg_ws[0], *e = h->gmg_ws[1];
+			tgpu_vec *rv = h->gmg_ws[0].get(), *e = h->gmg_ws[1].get();
 			TRY(cycle_ptr(h, opts, rv->d, e->d));
 			TRY(tgpu_vec_add(u, e));
 			TRY(k_residual_sumsq(h, f->d, u->d, rv->d));
@@ -2701,7 +2651,7 @@ extern "C" int tgpu_init_neumann_rhs(tgpu_hier *h, int problem, tgpu_vec *f, tgp
 	if (h->D == 2 && problem != 0) return fail(TGPU_ERR_UNSUPPORTED, "tgpu_init_neumann_rhs: 2D has the trig problem only");
 	LevelDev &L = h->levels[0];
 	if (!L.starts) return fail(TGPU_ERR_ARG, "tgpu_init_neumann_rhs: hierarchy was created without patch starts");
-	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, init_neumann_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta, L.P, (const double *) L.starts, (const double *) L.spacing, f->d, exact ? exact->d : (double *) nullptr, problem));
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, init_neumann_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, (const double *) L.starts.get(), (const double *) L.spacing.get(), f->d, exact ? exact->d : (double *) nullptr, problem));
 	API_END
 }
 extern "C" int tgpu_vec_integrate(tgpu_hier *h, const tgpu_vec *v, double *integral, double *volume)
@@ -2711,19 +2661,16 @@ extern "C" int tgpu_vec_integrate(tgpu_hier *h, const tgpu_vec *v, double *integ
 	if (!integral && !volume) return fail(TGPU_ERR_ARG, "tgpu_vec_integrate: nothing asked for");
 	LevelDev &L      = h->levels[0];
 	const int owned  = L.P; // owned patches come first
-	double *  d_part = nullptr;
-	CU(cudaMalloc(&d_part, sizeof(double) * (size_t) std::max(owned, 1)));
-	int rc = TGPU_OK;
+	DevPtr<double> d_part;
+	CU(dev_malloc(d_part, sizeof(double) * (size_t) std::max(owned, 1)));
 	{
 		Tag tg(h->ctx, "patch_integrals", 0);
-		DISPATCH_DN_ALL(h->D, h->N, rc = launch(h->ctx, patch_integrals_kernel<DD, NN>, dim3(std::min(std::max(owned, 1), h->ctx->sm_count * 8)), dim3(256), 0, owned, (const double *) L.spacing, (const double *) v->d, d_part));
+		DISPATCH_DN_ALL(h->D, h->N, TRY(launch(h->ctx, patch_integrals_kernel<DD, NN>, dim3(std::min(std::max(owned, 1), h->ctx->sm_count * 8)), dim3(256), 0, owned, (const double *) L.spacing.get(), (const double *) v->d, d_part.get())));
 	}
 	std::vector<double> part((size_t) owned), sp((size_t) owned * h->D);
-	if (rc == TGPU_OK && cudaMemcpyAsync(part.data(), d_part, sizeof(double) * owned, cudaMemcpyDeviceToHost, h->ctx->stream) != cudaSuccess) rc = TGPU_ERR_CUDA;
-	if (rc == TGPU_OK && cudaMemcpyAsync(sp.data(), L.spacing, sizeof(double) * owned * h->D, cudaMemcpyDeviceToHost, h->ctx->stream) != cudaSuccess) rc = TGPU_ERR_CUDA;
-	if (rc == TGPU_OK && cudaStreamSynchronize(h->ctx->stream) != cudaSuccess) rc = TGPU_ERR_CUDA;
-	cudaFree(d_part);
-	if (rc != TGPU_OK) return rc == TGPU_ERR_CUDA ? fail(TGPU_ERR_CUDA, "tgpu_vec_integrate: copy failed") : rc;
+	CU(cudaMemcpyAsync(part.data(), d_part.get(), sizeof(double) * owned, cudaMemcpyDeviceToHost, h->ctx->stream));
+	CU(cudaMemcpyAsync(sp.data(), L.spacing.get(), sizeof(double) * owned * h->D, cudaMemcpyDeviceToHost, h->ctx->stream));
+	CU(cudaStreamSynchronize(h->ctx->stream));
 	double res[2] = {0.0, 0.0};
 	for (int p = 0; p < owned; p++) {
 		res[0] += part[p];
@@ -2732,16 +2679,12 @@ extern "C" int tgpu_vec_integrate(tgpu_hier *h, const tgpu_vec *v, double *integ
 		res[1] += vol;
 	}
 	if (h->ctx->nranks > 1 && h->levels[0].distributed) { // a replicated level: every rank already holds the global sums
-		double *d2 = nullptr;
-		CU(cudaMalloc(&d2, 2 * sizeof(double)));
-		CU(cudaMemcpyAsync(d2, res, 2 * sizeof(double), cudaMemcpyHostToDevice, h->ctx->stream));
-		rc = k_allreduce_sum(h, d2, 2);
-		if (rc == TGPU_OK) {
-			CU(cudaMemcpyAsync(res, d2, 2 * sizeof(double), cudaMemcpyDeviceToHost, h->ctx->stream));
-			CU(cudaStreamSynchronize(h->ctx->stream));
-		}
-		cudaFree(d2);
-		TRY(rc);
+		DevPtr<double> d2;
+		CU(dev_malloc(d2, 2 * sizeof(double)));
+		CU(cudaMemcpyAsync(d2.get(), res, 2 * sizeof(double), cudaMemcpyHostToDevice, h->ctx->stream));
+		TRY(k_allreduce_sum(h, d2.get(), 2));
+		CU(cudaMemcpyAsync(res, d2.get(), 2 * sizeof(double), cudaMemcpyDeviceToHost, h->ctx->stream));
+		CU(cudaStreamSynchronize(h->ctx->stream));
 	}
 	if (integral) *integral = res[0];
 	if (volume) *volume = res[1];
@@ -2755,6 +2698,6 @@ extern "C" int tgpu_init_trig_rhs(tgpu_hier *h, tgpu_vec *f, tgpu_vec *exact)
 	if (exact) TRY(check_level_vec(h, 0, exact, "tgpu_init_trig_rhs"));
 	LevelDev &L = h->levels[0];
 	if (!L.starts) return fail(TGPU_ERR_ARG, "tgpu_init_trig_rhs: hierarchy was created without patch starts");
-	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, init_trig_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta, L.P, (const double *) L.starts, (const double *) L.spacing, f->d, exact ? exact->d : (double *) nullptr));
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, init_trig_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, (const double *) L.starts.get(), (const double *) L.spacing.get(), f->d, exact ? exact->d : (double *) nullptr));
 	API_END
 }

@@ -116,8 +116,8 @@ int tgpu_mesh_level_ids(const tgpu_mesh *mesh, int level, const int32_t **ids, c
 int tgpu_hierarchy_create(tgpu_ctx *ctx, int D, int n, int nlevels, const TgpuLevelDesc *levels, tgpu_hier **h);
 int tgpu_hierarchy_destroy(tgpu_hier *h);
 int tgpu_hierarchy_info(const tgpu_hier *h, int *D, int *n, int *nlevels);
-/* frees what earlier calls allocated lazily (Krylov work vectors, host-buffer slots, cached cycle graphs, pooled vector
- * storage); tables, face buffers and per-level cycle vectors stay */
+/* frees what earlier calls allocated lazily (Krylov and full-multigrid work vectors, full-multigrid boundary data,
+ * host-buffer slots, cached cycle graphs, pooled vector storage); tables, face buffers and per-level cycle vectors stay */
 int tgpu_hierarchy_trim(tgpu_hier *h);
 int tgpu_level_npatch(const tgpu_hier *h, int level, int64_t *npatch, int64_t *ncells);
 /* the patch solver's shift, FftwPatchSolver(domain, lambda) (PatchSolvers/FftwPatchSolver.h:66,170): block-Jacobi patch
@@ -182,6 +182,27 @@ int tgpu_vcycle_update(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *
  * doubles): the relative residual before the first cycle and after each one (iterations + 1 entries are written). */
 int tgpu_gmg_solve(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu_vec *u, double tol, int max_it,
                    int *iterations, double *rel_residual, double *history);
+/* ---- boundary data (level 0) ----
+ * The domain-boundary sides of level 0 (nbr_type TGPU_NBR_NONE) of the owned patches, in ascending (patch, side) order.
+ * patch, side (nullable): host arrays of count entries, owned by the hierarchy. */
+int tgpu_boundary_sides(const tgpu_hier *h, int64_t *count, const int32_t **patch, const int8_t **side);
+/* A zero-initialised vector of count * n^(D-1) doubles: side k's values in the library's face order (the two or one
+ * remaining axes, lower axis fastest).  upload / download / device_ptr / set / scale / copy / add / norms / destroy work
+ * as for any vector; no level operation accepts it. */
+int tgpu_boundary_vec_create(tgpu_hier *h, tgpu_vec **b);
+/* f (level 0) -= the boundary terms of b: 2 b / h^2 on Dirichlet sides (b = the boundary value on the face), b / h on
+ * Neumann sides (b = the outward normal derivative).  Edge and corner cells take every side's term, as
+ * tgpu_init_trig_rhs and tgpu_init_neumann_rhs fold their data. */
+int tgpu_fold_boundary(tgpu_hier *h, const tgpu_vec *b, tgpu_vec *f);
+/* Full multigrid: u <- FMG(f).  f is level 0 with boundary data folded in, as for every other solver.  b (nullable)
+ * holds the Dirichlet values folded into f (tgpu_boundary_vec_create layout); NULL means homogeneous Dirichlet data.
+ * Neumann entries of b are not read: R f already carries Neumann folds consistently.  opts as tgpu_vcycle
+ * (NULL = defaults); FMG starts on the coarsest level the options select (max_levels / patches_per_proc) with
+ * coarse_sweeps sweeps from zero, interpolates each level's result linearly to the next finer level and runs
+ * cycles >= 1 cycles from it there (one level: the coarse sweeps only).  u is overwritten.  f aliasing u, vectors of
+ * another level or hierarchy, a b that is not a boundary vector of h, cycles < 1 or bad options give TGPU_ERR_ARG and
+ * leave u untouched. */
+int tgpu_fmg(tgpu_hier *h, const TgpuCycleOpts *opts, int cycles, const tgpu_vec *f, const tgpu_vec *b, tgpu_vec *u);
 /* host-buffer convenience (the e2e path): f_host -> device, one cycle, u -> u_host */
 int tgpu_vcycle_host(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f_pinned, double *u_pinned);
 /* pipelined form for a stream of independent right-hand sides: returns once the work is enqueued; upload of

@@ -9,7 +9,8 @@ The class names mirror the reference's plugin surface (src/Thunderegg/GMG/*.h, V
 ``Hierarchy`` ~ the Level list built by GMG::CycleFactory, ``Vec`` ~ Vector<D>,
 ``Hierarchy.apply/smooth/restrict/prolong_add/vcycle`` ~ Operator/Smoother/Restrictor/
 Interpolator/Cycle, ``Hierarchy.bicgstab`` ~ BiCGStab<D>::solve, ``Hierarchy.vcycle_update/gmg_solve`` ~ stationary
-multigrid from an initial guess.
+multigrid from an initial guess, ``Hierarchy.fmg`` ~ full multigrid (with ``new_boundary_vec/fold_boundary`` for the
+caller's boundary data).
 """
 import ctypes as C
 import os
@@ -80,7 +81,8 @@ ABI_SYMBOLS = [
     "tgpu_comm_unique_id", "tgpu_comm_init", "tgpu_hierarchy_create_distributed",
     "tgpu_hierarchy_force_generic_kernels", "tgpu_mesh_set_neumann", "tgpu_vcycle_host_async", "tgpu_vcycle_host_wait",
     "tgpu_hierarchy_trim", "tgpu_hierarchy_set_lambda", "tgpu_prolong_add_linear", "tgpu_vec_transfer_pair",
-    "tgpu_vcycle_update", "tgpu_gmg_solve",
+    "tgpu_vcycle_update", "tgpu_gmg_solve", "tgpu_boundary_sides", "tgpu_boundary_vec_create", "tgpu_fold_boundary",
+    "tgpu_fmg",
 ]
 
 lib.tgpu_last_error.restype = C.c_char_p
@@ -126,6 +128,9 @@ for _name, _args in {
     "tgpu_vcycle_update": [_vp, C.POINTER(CycleOpts), _vp, _vp, C.POINTER(C.c_double)],
     "tgpu_gmg_solve": [_vp, C.POINTER(CycleOpts), _vp, _vp, C.c_double, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_double),
                        C.POINTER(C.c_double)],
+    "tgpu_boundary_sides": [_vp, C.POINTER(C.c_int64), C.POINTER(C.POINTER(C.c_int32)), C.POINTER(C.POINTER(C.c_int8))],
+    "tgpu_boundary_vec_create": [_vp, C.POINTER(_vp)], "tgpu_fold_boundary": [_vp, _vp, _vp],
+    "tgpu_fmg": [_vp, C.POINTER(CycleOpts), C.c_int, _vp, _vp, _vp],
     "tgpu_init_trig_rhs": [_vp, _vp, _vp],
     "tgpu_init_neumann_rhs": [_vp, C.c_int, _vp, _vp],
     "tgpu_vec_integrate": [_vp, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double)],
@@ -496,6 +501,35 @@ class Hierarchy:
         if history:
             return its.value, rel.value, list(hist[:its.value + 1])
         return its.value, rel.value
+
+    def boundary_sides(self):
+        """-> (patch, side): the domain-boundary sides of level 0's owned patches, ascending; row k of a boundary vector
+        holds side k's n^(D-1) values in face order"""
+        cnt, pa, sa = C.c_int64(), C.POINTER(C.c_int32)(), C.POINTER(C.c_int8)()
+        check(lib.tgpu_boundary_sides(self._p, C.byref(cnt), C.byref(pa), C.byref(sa)))
+        if cnt.value == 0:
+            return np.zeros(0, np.int32), np.zeros(0, np.int8)
+        return (np.ctypeslib.as_array(pa, shape=(cnt.value,)).copy(), np.ctypeslib.as_array(sa, shape=(cnt.value,)).copy())
+
+    def new_boundary_vec(self, data=None):
+        """boundary data of level 0: Dirichlet values / outward normal derivatives, one row per boundary_sides() entry"""
+        v = Vec.__new__(Vec)
+        v.hier, v.level, v._p = self, -1, _vp()
+        check(lib.tgpu_boundary_vec_create(self._p, C.byref(v._p)))
+        n = C.c_int64()
+        check(lib.tgpu_vec_device_ptr(v._p, None, C.byref(n)))
+        v.ncells = n.value
+        if data is not None:
+            v.upload(data)
+        return v
+
+    def fold_boundary(self, b, f):
+        """f -= 2 b / h^2 (Dirichlet sides), b / h (Neumann sides) on the boundary cells of level 0"""
+        check(lib.tgpu_fold_boundary(self._p, b._p, f._p))
+
+    def fmg(self, f, u, b=None, opts=None, cycles=2):
+        """full multigrid u <- FMG(f); b: the Dirichlet values folded into f (None: homogeneous)"""
+        check(lib.tgpu_fmg(self._p, C.byref(opts) if opts is not None else None, cycles, f._p, b._p if b is not None else None, u._p))
 
     def init_trig_rhs(self, f, exact=None):
         check(lib.tgpu_init_trig_rhs(self._p, f._p, exact._p if exact is not None else None))

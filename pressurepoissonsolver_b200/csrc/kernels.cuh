@@ -1745,6 +1745,158 @@ __global__ void bicg_scalars_kernel(double *__restrict__ sc, int step)
 	if (threadIdx.x == 0) bicg_scalars(step, sc);
 }
 
+// ---------------------------------------------------------------------------------------------
+// boundary data and full multigrid (tgpu_fold_boundary, tgpu_fmg)
+// ---------------------------------------------------------------------------------------------
+// Level-0 boundary data: one slice of M values per domain-boundary side (nbr_type NBR_NONE) of an owned patch, in the
+// order of the list (patch[k], side[k]); bidx[p * S + s] = k, or -1 where side s of patch p is not a boundary side.
+// f -= 2 b / h^2 on Dirichlet sides, f -= b / h on Neumann sides (b = outward normal derivative), every side's term in
+// side order on edge and corner cells, with the arithmetic of init_trig_kernel / init_neumann_kernel.  One thread per
+// boundary face entry; a cell on several boundary sides is folded by the thread of the lowest of them.
+template <int D, int N>
+__global__ void fold_boundary_kernel(const PatchMeta *__restrict__ meta, int nsides, const int32_t *__restrict__ patch,
+                                     const int8_t *__restrict__ side, const int32_t *__restrict__ bidx, const double *__restrict__ spacing,
+                                     const double *__restrict__ b, double *__restrict__ f)
+{
+	pdl_launch_dependents();
+	pdl_wait();
+	using G            = Geo<D, N>;
+	const size_t total = (size_t) nsides * G::M;
+	for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < total; i += (size_t) gridDim.x * blockDim.x) {
+		const int        m = (int) (i % G::M), k = (int) (i / G::M);
+		const int        p = patch[k], s = side[k];
+		const PatchMeta &pm = meta[p];
+		int              c[3];
+		face_cell<D, N>(s, m, c);
+		auto on = [&](int t) { return pm.nbr_type[t] == NBR_NONE && c[t >> 1] == ((t & 1) ? N - 1 : 0); };
+		bool mine = true;
+		for (int t = 0; t < s; t++) mine = mine && !on(t);
+		if (!mine) continue;
+		double *const dst = f + (size_t) p * G::NC + (c[2] * N + c[1]) * N + c[0];
+		double        val = *dst;
+		for (int t = 0; t < G::S; t++) {
+			if (!on(t)) continue;
+			const double bv = b[(size_t) bidx[p * G::S + t] * G::M + face_index<D, N>(t, c)];
+			const double h  = spacing[(size_t) p * D + (t >> 1)];
+			if ((pm.neumann >> t) & 1) val -= bv / h;
+			else val -= 2 * bv / (h * h);
+		}
+		*dst = val;
+	}
+}
+// coarse = R fine (restrict_kernel's arithmetic), and with boundary data (bc != nullptr) the Dirichlet folds re-posed for
+// the coarse spacing on the coarse boundary cells: + R (2 b_f / h_f^2) - 2 b_c / h_c^2, b_c = mean of the 2^(D-1) fine
+// face values over the coarse face cell, written to bc ([slot][side][M], the face-buffer layout of the coarse level).
+// A patch present on both levels copies f and b.  bf: the fine level's boundary data, in the face-buffer layout
+// (bidx == nullptr) or in the level-0 list layout (bidx, see fold_boundary_kernel).  Neumann folds restrict consistently
+// (R (b / h_f) = b / h_c) and are left as R made them.
+template <int D, int N>
+__global__ void restrict_rhs_kernel(const PatchMeta *__restrict__ meta, int P, const double *__restrict__ fine, double *__restrict__ coarse,
+                                    const double *__restrict__ bf, const int32_t *__restrict__ bidx, double *__restrict__ bc)
+{
+	pdl_launch_dependents();
+	pdl_wait();
+	using G            = Geo<D, N>;
+	constexpr int H    = N / 2;
+	constexpr int CC   = G::NC >> D;
+	constexpr int Q    = 1 << (D - 1);
+	const size_t total = (size_t) P * G::NC;
+	for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < total; i += (size_t) gridDim.x * blockDim.x) {
+		const int        c = (int) (i % G::NC);
+		const size_t     p = i / G::NC;
+		const PatchMeta &pm = meta[p];
+		const int        orth = pm.orth_on_parent;
+		double *         dst  = coarse + (size_t) pm.parent_idx * G::NC;
+		const double *   src  = fine + p * G::NC;
+		auto dirichlet = [&](int s) { return pm.nbr_type[s] == NBR_NONE && !((pm.neumann >> s) & 1); };
+		auto fine_b    = [&](int s, const int (&fc)[3]) {
+            const size_t row = bidx ? (size_t) bidx[p * G::S + s] : p * G::S + s;
+            return bf[row * G::M + face_index<D, N>(s, fc)];
+		};
+		if (orth < 0) {
+			dst[c] = src[c];
+			if (!bc) continue;
+			const int cc[3] = {c % N, (c / N) % N, (D == 2) ? 0 : c / (N * N)};
+			for (int s = 0; s < G::S; s++)
+				if (dirichlet(s) && cc[s >> 1] == ((s & 1) ? N - 1 : 0))
+					bc[((size_t) pm.parent_idx * G::S + s) * G::M + face_index<D, N>(s, cc)] = fine_b(s, cc);
+		} else if (c < CC) {
+			const int cx = c % H, cy = (c / H) % H, cz = (D == 2) ? 0 : c / (H * H);
+			double    acc = 0.0;
+			for (int dz = 0; dz < (D == 2 ? 1 : 2); dz++)
+				for (int dy = 0; dy < 2; dy++)
+					for (int dx = 0; dx < 2; dx++)
+						acc += src[((2 * cz + dz) * N + (2 * cy + dy)) * N + (2 * cx + dx)] / (1 << D);
+			const int ox = (orth & 1) * H, oy = ((orth >> 1) & 1) * H, oz = (D == 2) ? 0 : ((orth >> 2) & 1) * H;
+			const int pc[3] = {cx + ox, cy + oy, cz + oz};
+			if (bc) {
+				const int hc[3] = {cx, cy, cz};
+				for (int s = 0; s < G::S; s++) {
+					const int ax = s >> 1;
+					if (!dirichlet(s) || hc[ax] != ((s & 1) ? H - 1 : 0)) continue;
+					double sum = 0.0;
+					for (int q = 0; q < Q; q++) { // the fine face cells over this coarse face cell, lower axis fastest
+						int fc[3] = {0, 0, 0}, bit = 0;
+						for (int a = 0; a < D; a++) {
+							if (a == ax) fc[a] = (s & 1) ? N - 1 : 0;
+							else fc[a] = 2 * hc[a] + ((q >> bit++) & 1);
+						}
+						sum += fine_b(s, fc);
+					}
+					const double mean = sum / Q;
+					acc += 2 * sum / pm.h2 / (1 << D);
+					acc -= 2 * mean / (4 * pm.h2);
+					bc[((size_t) pm.parent_idx * G::S + s) * G::M + face_index<D, N>(s, pc)] = mean;
+				}
+			}
+			dst[(pc[2] * N + pc[1]) * N + pc[0]] = acc;
+		}
+	}
+}
+// uf = P_linear uc (prolong_linear_add_kernel's arithmetic, assigned instead of added), and the boundary-cell slices of uf
+// into the face buffer F (what extract_faces_kernel would read back): the guess of a full-multigrid level and the faces
+// its first cycle starts from
+template <int D, int N>
+__global__ void fmg_interp_kernel(const PatchMeta *__restrict__ meta, int P, const double *__restrict__ uc, double *__restrict__ uf,
+                                  double *__restrict__ F)
+{
+	pdl_launch_dependents();
+	pdl_wait();
+	using G            = Geo<D, N>;
+	const size_t total = (size_t) P * G::NC;
+	for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < total; i += (size_t) gridDim.x * blockDim.x) {
+		const int        ci = (int) (i % G::NC);
+		const size_t     p  = i / G::NC;
+		const PatchMeta &pm = meta[p];
+		const double *   src = uc + (size_t) pm.parent_idx * G::NC;
+		const int        orth = pm.orth_on_parent;
+		const int        c[3] = {ci % N, (ci / N) % N, (D == 2) ? 0 : ci / (N * N)};
+		double           val;
+		if (orth < 0) {
+			val = __ldg(src + ci);
+		} else {
+			int    cc[3] = {0, 0, 0}, cq[3] = {0, 0, 0};
+			double wc[3] = {1, 1, 1}, wq[3] = {0, 0, 0};
+			for (int a = 0; a < D; a++) {
+				const int  off = ((orth >> a) & 1) * (N / 2), k = off + c[a] / 2, odd = c[a] & 1;
+				const int  nb = odd ? k + 1 : k - 1;
+				const bool in = nb >= 0 && nb < N;
+				cc[a] = k;
+				cq[a] = in ? nb : (odd ? k - 1 : k + 1);
+				wc[a] = in ? 0.75 : 1.25;
+				wq[a] = in ? 0.25 : -0.25;
+			}
+			auto at = [&](int x, int y, int z) { return __ldg(src + (z * N + y) * N + x); };
+			auto line = [&](int y, int z) { return at(cc[0], y, z) * wc[0] + at(cq[0], y, z) * wq[0]; };
+			auto plane = [&](int z) { return line(cc[1], z) * wc[1] + line(cq[1], z) * wq[1]; };
+			val = (D == 2) ? plane(0) : plane(cc[2]) * wc[2] + plane(cq[2]) * wq[2];
+		}
+		uf[i] = val;
+		for (int s = 0; s < G::S; s++)
+			if (c[s >> 1] == ((s & 1) ? N - 1 : 0)) F[(p * G::S + s) * G::M + face_index<D, N>(s, c)] = val;
+	}
+}
+
 // manufactured trig problem (apps/3d/steady.cpp:253-265, apps/2d/steady.cpp:314-316) with the
 // Dirichlet data folded into f on domain-boundary cells (apps/shared/Init.cpp:183-241,329-357)
 template <int D> __device__ __forceinline__ double trig_exact(double x, double y, double z)

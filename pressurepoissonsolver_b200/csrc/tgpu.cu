@@ -254,6 +254,7 @@ struct LevelDev {
 	DevPtr<int32_t> gslot, gowner;                 // with G: the slot table (IfaceSlots32), device [P][6] and [nslots]
 	std::vector<int32_t> gbegin;                   // with G: IfaceSlots32::begin on the host (slot range of a patch range)
 	DevPtr<double> u, f, r; // cycle work vectors (lazily allocated)
+	DevPtr<double> bnd;     // levels >= 1: Dirichlet data of the full-multigrid right-hand side, [slot][side][M] (lazily allocated)
 	bool       has_neumann = false;
 	DevPtr<int32_t> neu_list;               // device: owned patches with Neumann domain sides, ascending (smooth3d16_kernel<.., NEU>)
 	std::vector<int32_t> neu_host;          // the same list on the host (sub-ranges are found by binary search)
@@ -276,6 +277,8 @@ struct GraphEntry {
 	const double *faces_old = nullptr, *faces_uc = nullptr;
 	const double *  f;
 	double *        u;
+	const double *  b          = nullptr; // full multigrid: the boundary data
+	int             fmg_cycles = 0;       // full multigrid: cycles per level (0: a cycle)
 	TgpuCycleOpts   opts;
 	GraphExecPtr    exec;
 	int64_t         kernels;
@@ -290,11 +293,19 @@ struct tgpu_hier {
 	// ... and of the iterate before its last sweep: cycle_faces_old, plus P cycle_uc on the boundary cells if that sweep was
 	// the first post-sweep (cycle_uc == nullptr otherwise); see k_face_residual_norm
 	const double *        cycle_faces_old = nullptr, *cycle_uc = nullptr;
+	double *              visit_faces = nullptr; // the slices of the result of the last fused_visit that was asked to emit them
 	DevPtr<double>        tri; // [N/2 + 1][N^(D-1)] tridiagonal multipliers (TriSolve)
 	DevPtr<double>        mats, lam; // Neumann patches: transform matrices [6][N][N], 1-D eigenvalues [3][N]
 	std::vector<GraphEntry> graphs;
 	std::vector<VecPtr>   krylov_ws;
 	std::vector<VecPtr>   gmg_ws; // stationary solve: residual and correction of the schedules without a start from a guess
+	std::vector<VecPtr>   fmg_ws; // full multigrid, schedules without a start from a guess: residual and correction of each level
+	// domain-boundary sides of level 0's owned patches, ascending (patch, side) (tgpu_boundary_sides), and on the device the
+	// same list with bnd_index [P][2D]: position in the list, -1 for the other sides
+	std::vector<int32_t>  bnd_patch;
+	std::vector<int8_t>   bnd_side;
+	DevPtr<int32_t>       bnd_patch_d, bnd_index;
+	DevPtr<int8_t>        bnd_side_d;
 	DevPtr<double>        krylov_sc; // BiCGStab scalars on the device
 	VecPtr                host_f, host_u;
 	// pipelined host-buffer path (tgpu_vcycle_host_async): two slots, copy-in / copy-out streams
@@ -316,6 +327,8 @@ struct tgpu_hier {
 		graphs.clear();
 		krylov_ws.clear();
 		gmg_ws.clear();
+		fmg_ws.clear();
+		for (LevelDev &L : levels) L.bnd.reset();
 		host_f.reset(), host_u.reset();
 		for (int k = 0; k < 2; k++) pipe_f[k].reset(), pipe_u[k].reset();
 	}
@@ -329,6 +342,8 @@ struct tgpu_hier {
 	}
 };
 
+// level of a boundary-data vector (tgpu_boundary_vec_create): no level operation accepts it
+static constexpr int BOUNDARY_LEVEL = -1;
 struct tgpu_vec {
 	tgpu_hier *h     = nullptr;
 	int        level = 0;
@@ -907,6 +922,20 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 		TRY(dev_upload(h->mats, mats.data(), mats.size()));
 		TRY(dev_upload(h->lam, lam.data(), lam.size()));
 	}
+	{ // the domain-boundary sides of level 0 (tgpu_boundary_sides)
+		const int            P0 = h->levels[0].P;
+		std::vector<int32_t> index((size_t) P0 * S, -1);
+		for (int p = 0; p < P0; p++)
+			for (int s = 0; s < S; s++)
+				if (levels[0].nbr_type[(size_t) p * S + s] == NBR_NONE) {
+					index[(size_t) p * S + s] = (int32_t) h->bnd_patch.size();
+					h->bnd_patch.push_back(p);
+					h->bnd_side.push_back((int8_t) s);
+				}
+		TRY(dev_upload(h->bnd_patch_d, h->bnd_patch.data(), h->bnd_patch.size()));
+		TRY(dev_upload(h->bnd_side_d, h->bnd_side.data(), h->bnd_side.size()));
+		TRY(dev_upload(h->bnd_index, index.data(), index.size()));
+	}
 	TRY(set_kernel_attrs(h.get()));
 	TRY(ensure_scratch32(h.get()));
 	TRY(update_iface_buffers(h.get()));
@@ -1349,7 +1378,7 @@ extern "C" int tgpu_vec_destroy(tgpu_vec *v)
 	tgpu_hier *h = v->h;
 	// cached cycle graphs that were captured on this storage are dropped; graphs of other vectors stay
 	for (size_t i = 0; i < h->graphs.size();) {
-		if (h->graphs[i].f == v->d || h->graphs[i].u == v->d) h->graphs.erase(h->graphs.begin() + i);
+		if (h->graphs[i].f == v->d || h->graphs[i].u == v->d || h->graphs[i].b == v->d) h->graphs.erase(h->graphs.begin() + i);
 		else i++;
 	}
 	cudaFreeAsync(v->d, h->ctx->stream); // stream-ordered: work already queued on the vector completes first
@@ -1455,7 +1484,8 @@ template <int OP> static int reduce(const tgpu_vec *a, const tgpu_vec *b, double
 	Tag       tg(ctx, "reduce", a->level);
 	TRY(launch(ctx, reduce_stage1<OP>, dim3(nb), dim3(256), 0, a->n, (const double *) a->d, (const double *) b->d, ctx->d_partial.get()));
 	TRY(launch(ctx, reduce_stage2<OP>, dim3(1), dim3(256), 0, nb, (const double *) ctx->d_partial.get(), ctx->d_result.get()));
-	if (ctx->nranks > 1 && a->h->levels[a->level].distributed)
+	// (boundary data is split over the ranks like level 0)
+	if (ctx->nranks > 1 && a->h->levels[std::max(a->level, 0)].distributed)
 		NC(g_nccl.AllReduce(ctx->d_result.get(), ctx->d_result.get(), 1, ncclDouble, OP == 0 ? ncclSum : ncclMax, ctx->comm, ctx->stream));
 	CU(cudaMemcpyAsync(ctx->h_result.get(), ctx->d_result.get(), sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
 	CU(cudaStreamSynchronize(ctx->stream));
@@ -2068,11 +2098,16 @@ static int exchange_async(tgpu_hier *h, int l, double *F, const double *uc, cuda
 // guess (level 0 of a cycle with coarser levels): start from the iterate in u instead of zero.  The first pre-sweep needs
 // only u's boundary slices, extracted into Fcur; from there every pre-sweep is the non-zero-guess sweep of i > 0, so
 // one cycle computes u + Cycle(f - A u) (the smoother is linear and stationary).  Coarser levels start from zero.
-static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double *f, double *u, bool want_faces, bool guess = false)
+// faces (with guess): L.Fa or L.Fb already holds u's boundary slices, no extraction (full multigrid: fmg_interp_kernel or
+// the previous cycle's last sweep wrote them).  want_faces on a level above the coarsest: h->visit_faces is the face buffer
+// that holds the slices of the result afterwards.
+static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double *f, double *u, bool want_faces, bool guess = false,
+                       const double *faces = nullptr)
 {
 	const int last = h->last_level;
 	LevelDev &L    = h->levels[l];
 	double *  Fcur = L.Fa, *Falt = L.Fb;
+	if (faces == L.Fb) std::swap(Fcur, Falt);
 	if (l == last) {
 		for (int i = 0; i < o.coarse_sweeps; i++) {
 			const bool emit = (i + 1 < o.coarse_sweeps);
@@ -2085,7 +2120,7 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 	}
 	const bool from_faces = (o.fused != 2);
 	LevelDev & C          = h->levels[l + 1];
-	if (guess) TRY(k_extract_faces(h, l, u, Fcur));
+	if (guess && !faces) TRY(k_extract_faces(h, l, u, Fcur));
 	for (int i = 0; i < o.pre_sweeps; i++) {
 		const bool nonzero = guess || i > 0;
 		if (nonzero) TRY(k_exchange(h, l, Fcur, nullptr));
@@ -2165,6 +2200,7 @@ static int fused_visit(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double
 		}
 		std::swap(Fcur, Falt);
 	}
+	if (want_faces) h->visit_faces = Fcur;
 	if (l == 0 && want_faces) { // the last sweep emitted the slices of u here; Falt holds those of its input
 		h->cycle_faces     = Fcur;
 		h->cycle_faces_old = Falt;
@@ -2223,20 +2259,16 @@ static bool guess_schedule(const tgpu_hier *h, const TgpuCycleOpts &o)
 {
 	return fused_schedule(o, h->ctx->nranks) && h->lambda == 0.0 && h->last_level > 0;
 }
-static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, double *u, bool want_faces = false, bool guess = false)
+// Runs run() once, through the hierarchy's cached CUDA graph of key (its f, u, b, fmg_cycles, want_faces, guess and opts):
+// replayed when one was captured before, captured and launched otherwise.  o.use_graph = 0, profiling and several GPUs
+// (unless use_graph >= 2) run it directly.
+template <class Fn> static int graph_run(tgpu_hier *h, const TgpuCycleOpts &o, GraphEntry key, Fn &&run)
 {
-	TgpuCycleOpts o;
-	TRY(cycle_opts(h, opts, o));
 	tgpu_ctx *ctx = h->ctx;
-	if (guess && !guess_schedule(h, o)) return fail(TGPU_ERR_ARG, "cycle_ptr: this schedule cannot start from a guess");
-	for (size_t l = 0; l <= (size_t) h->last_level; l++) {
-		const bool fused_sched = fused_schedule(o, ctx->nranks);
-		TRY(ensure_work(h, (int) l, !fused_sched || (o.fused == 2 && is_3d32(h))));
-	}
-	for (int l = 0; l <= h->last_level; l++) TRY(ensure_push_desc(h, l));
-	if (!o.use_graph || ctx->profiling || (ctx->nranks > 1 && o.use_graph < 2)) return run_cycle(h, o, f, u, want_faces, guess);
+	if (!o.use_graph || ctx->profiling || (ctx->nranks > 1 && o.use_graph < 2)) return run();
 	for (GraphEntry &g : h->graphs)
-		if (g.f == f && g.u == u && g.want_faces == want_faces && g.guess == guess && same_opts(g.opts, o)) {
+		if (g.f == key.f && g.u == key.u && g.b == key.b && g.fmg_cycles == key.fmg_cycles && g.want_faces == key.want_faces
+		    && g.guess == key.guess && same_opts(g.opts, o)) {
 			h->cycle_faces     = g.faces;
 			h->cycle_faces_old = g.faces_old;
 			h->cycle_uc        = g.faces_uc;
@@ -2248,17 +2280,16 @@ static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, d
 	ctx->capturing = true;
 	ctx->captured  = 0;
 	CU(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-	int         rc  = run_cycle(h, o, f, u, want_faces, guess);
+	int         rc  = run();
 	cudaGraph_t raw = nullptr;
 	cudaError_t e   = cudaStreamEndCapture(ctx->stream, &raw);
 	GraphPtr    graph(raw);
 	ctx->capturing = false;
 	TRY(rc);
 	if (e != cudaSuccess) return fail(TGPU_ERR_CUDA, std::string("cudaStreamEndCapture: ") + cudaGetErrorString(e));
-	GraphEntry g;
-	g.f = f, g.u = u, g.opts = o, g.kernels = ctx->captured;
-	g.want_faces = want_faces, g.faces = h->cycle_faces;
-	g.guess = guess, g.faces_old = h->cycle_faces_old, g.faces_uc = h->cycle_uc;
+	GraphEntry &g = key;
+	g.opts = o, g.kernels = ctx->captured;
+	g.faces = h->cycle_faces, g.faces_old = h->cycle_faces_old, g.faces_uc = h->cycle_uc;
 	cudaGraphExec_t exec = nullptr;
 	CU(cudaGraphInstantiate(&exec, graph.get(), 0));
 	g.exec.reset(exec);
@@ -2267,6 +2298,21 @@ static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, d
 	CU(cudaGraphLaunch(h->graphs.back().exec.get(), ctx->stream));
 	ctx->launches += h->graphs.back().kernels;
 	return TGPU_OK;
+}
+static int cycle_ptr(tgpu_hier *h, const TgpuCycleOpts *opts, const double *f, double *u, bool want_faces = false, bool guess = false)
+{
+	TgpuCycleOpts o;
+	TRY(cycle_opts(h, opts, o));
+	tgpu_ctx *ctx = h->ctx;
+	if (guess && !guess_schedule(h, o)) return fail(TGPU_ERR_ARG, "cycle_ptr: this schedule cannot start from a guess");
+	for (size_t l = 0; l <= (size_t) h->last_level; l++) {
+		const bool fused_sched = fused_schedule(o, ctx->nranks);
+		TRY(ensure_work(h, (int) l, !fused_sched || (o.fused == 2 && is_3d32(h))));
+	}
+	for (int l = 0; l <= h->last_level; l++) TRY(ensure_push_desc(h, l));
+	GraphEntry key;
+	key.f = f, key.u = u, key.want_faces = want_faces, key.guess = guess;
+	return graph_run(h, o, std::move(key), [&] { return run_cycle(h, o, f, u, want_faces, guess); });
 }
 extern "C" int tgpu_vcycle(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu_vec *u)
 {
@@ -2639,6 +2685,158 @@ extern "C" int tgpu_gmg_solve(tgpu_hier *h, const TgpuCycleOpts *opts, const tgp
 	if (iterations) *iterations = its;
 	if (rel_residual) *rel_residual = rel;
 	return TGPU_OK;
+	API_END
+}
+
+// ------------------------------------------------------------------------------------------
+// boundary data and full multigrid
+// ------------------------------------------------------------------------------------------
+extern "C" int tgpu_boundary_sides(const tgpu_hier *h, int64_t *count, const int32_t **patch, const int8_t **side)
+{
+	if (!h || !count) return fail(TGPU_ERR_ARG, "tgpu_boundary_sides: null argument");
+	*count = (int64_t) h->bnd_patch.size();
+	if (patch) *patch = h->bnd_patch.data();
+	if (side) *side = h->bnd_side.data();
+	return TGPU_OK;
+}
+static size_t face_size(const tgpu_hier *h)
+{
+	size_t M = 1;
+	for (int i = 0; i < h->D - 1; i++) M *= h->N;
+	return M;
+}
+extern "C" int tgpu_boundary_vec_create(tgpu_hier *h, tgpu_vec **out)
+{
+	if (!h || !out) return fail(TGPU_ERR_ARG, "tgpu_boundary_vec_create: null argument");
+	CU(cudaSetDevice(h->ctx->device));
+	std::unique_ptr<tgpu_vec> v(new tgpu_vec());
+	v->h     = h;
+	v->level = BOUNDARY_LEVEL;
+	v->n     = h->bnd_patch.size() * face_size(h);
+	CU(cudaMallocAsync(&v->d, std::max<size_t>(1, v->n) * sizeof(double), h->ctx->stream));
+	CU(cudaMemsetAsync(v->d, 0, v->n * sizeof(double), h->ctx->stream));
+	*out = v.release();
+	return TGPU_OK;
+}
+static int check_boundary_vec(const tgpu_hier *h, const tgpu_vec *b, const char *what)
+{
+	if (!b || b->h != h || b->level != BOUNDARY_LEVEL || b->n != h->bnd_patch.size() * face_size(h))
+		return fail(TGPU_ERR_ARG, std::string(what) + ": not a boundary-data vector of this hierarchy");
+	return TGPU_OK;
+}
+extern "C" int tgpu_fold_boundary(tgpu_hier *h, const tgpu_vec *b, tgpu_vec *f)
+{
+	API_BEGIN
+	TRY(check_level_vec(h, 0, f, "tgpu_fold_boundary"));
+	TRY(check_boundary_vec(h, b, "tgpu_fold_boundary"));
+	if (b->n == 0) return TGPU_OK;
+	LevelDev &L = h->levels[0];
+	Tag       tg(h->ctx, "fold_boundary", 0);
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, fold_boundary_kernel<DD, NN>, dim3(grid_for(h->ctx, b->n)), dim3(256), 0, (const PatchMeta *) L.meta.get(), (int) h->bnd_patch.size(), (const int32_t *) h->bnd_patch_d.get(), (const int8_t *) h->bnd_side_d.get(), (const int32_t *) h->bnd_index.get(), (const double *) L.spacing.get(), (const double *) b->d, f->d));
+	API_END
+}
+// level l + 1's right-hand side from level l's: coarse = R fine, and with boundary data bf (level 0: the caller's list
+// layout, else level l's bnd) the Dirichlet folds re-posed for the coarse spacing, the coarse data into level l + 1's bnd
+static int k_restrict_rhs(tgpu_hier *h, int l, const double *fine, const double *bf, double *coarse)
+{
+	LevelDev &L = h->levels[l], &C = h->levels[l + 1];
+	double *  bc = bf ? C.bnd.get() : nullptr;
+	const bool cross = crosses_replication(h, l);
+	if (cross) {
+		TRY(k_set(h, coarse, C.ncells, 0.0));
+		if (bc) TRY(k_set(h, bc, C.nface, 0.0));
+	}
+	{
+		Tag tg(h->ctx, "restrict_rhs", l);
+		DISPATCH_DN_ALL(h->D, h->N, TRY(launch(h->ctx, restrict_rhs_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, fine, coarse, bf, l == 0 ? (const int32_t *) h->bnd_index.get() : (const int32_t *) nullptr, bc)));
+	}
+	if (cross) {
+		TRY(k_allreduce_sum(h, coarse, C.ncells));
+		if (bc) TRY(k_allreduce_sum(h, bc, C.nface));
+	}
+	return TGPU_OK;
+}
+static int k_fmg_interp(tgpu_hier *h, int l, const double *coarse, double *fine, double *F)
+{
+	LevelDev &L = h->levels[l];
+	Tag       tg(h->ctx, "fmg_interp", l);
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, fmg_interp_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, coarse, fine, F));
+}
+// u = Cycle(f) from zero, starting on level l (run_cycle's schedules)
+static int visit_from_zero(tgpu_hier *h, const TgpuCycleOpts &o, int l, const double *f, double *u)
+{
+	if (fused_schedule(o, h->ctx->nranks)) return fused_visit(h, o, l, f, u, false);
+	TRY(k_set(h, u, h->levels[l].ncells, 0.0));
+	return generic_visit(h, o, l, f, u);
+}
+// Full multigrid over levels 0 .. last_level: the right-hand sides restricted down (levels[l].f), the coarsest level's
+// sweeps from zero, then per level the linear interpolation of the coarser solution as the guess (levels[l].u; level 0:
+// the caller's f and u) and `cycles` cycles from it.  A cycle from level l uses only levels[k], k > l, as work space, whose
+// right-hand sides and solutions have been consumed by then.  The fused schedule starts the first cycle of a level from
+// the slices fmg_interp_kernel wrote; the others compute r = f - A u, a cycle from zero on r and the sum (update_once).
+static int fmg_run(tgpu_hier *h, const TgpuCycleOpts &o, int cycles, const double *f, const double *b, double *u)
+{
+	const int last = h->last_level;
+	auto fl = [&](int l) { return l == 0 ? f : (const double *) h->levels[l].f.get(); };
+	auto ul = [&](int l) { return l == 0 ? u : h->levels[l].u.get(); };
+	for (int l = 0; l < last; l++) TRY(k_restrict_rhs(h, l, fl(l), b ? (l == 0 ? b : (const double *) h->levels[l].bnd.get()) : nullptr, h->levels[l + 1].f.get()));
+	TRY(visit_from_zero(h, o, last, fl(last), ul(last)));
+	const bool guess = guess_schedule(h, o);
+	for (int l = last - 1; l >= 0; l--) {
+		LevelDev &L = h->levels[l];
+		TRY(k_fmg_interp(h, l, ul(l + 1), ul(l), L.Fa));
+		const double *faces = L.Fa;
+		for (int c = 0; c < cycles; c++) {
+			if (guess) { // every cycle but the last emits its result's slices for the next one
+				const bool emit = c + 1 < cycles;
+				TRY(fused_visit(h, o, l, fl(l), ul(l), emit, true, faces));
+				faces = h->visit_faces;
+				continue;
+			}
+			double *r = h->fmg_ws[2 * l]->d, *e = h->fmg_ws[2 * l + 1]->d;
+			TRY(k_extract_faces(h, l, ul(l), L.Fa));
+			TRY(k_exchange(h, l, L.Fa, nullptr));
+			TRY(k_apply(h, l, 1, ul(l), fl(l), L.Fa, r, nullptr));
+			TRY(k_exchange_done(h, l));
+			TRY(visit_from_zero(h, o, l, r, e));
+			Tag tg(h->ctx, "blas1", l);
+			TRY(launch(h->ctx, blas1_kernel<B_ADD>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, L.ncells, ul(l), (const double *) e, (const double *) nullptr, 0.0, 0.0, 0.0));
+		}
+	}
+	return TGPU_OK;
+}
+extern "C" int tgpu_fmg(tgpu_hier *h, const TgpuCycleOpts *opts, int cycles, const tgpu_vec *f, const tgpu_vec *b, tgpu_vec *u)
+{
+	API_BEGIN
+	TRY(check_stationary_args(h, f, u, "tgpu_fmg"));
+	if (b) TRY(check_boundary_vec(h, b, "tgpu_fmg"));
+	if (cycles < 1) return fail(TGPU_ERR_ARG, "tgpu_fmg: cycles must be at least 1");
+	TgpuCycleOpts o;
+	TRY(cycle_opts(h, opts, o));
+	tgpu_ctx * ctx   = h->ctx;
+	const bool fused = fused_schedule(o, ctx->nranks);
+	for (int l = 0; l <= h->last_level; l++) {
+		TRY(ensure_work(h, l, !fused || (o.fused == 2 && is_3d32(h))));
+		TRY(ensure_push_desc(h, l));
+		if (b && l > 0 && !h->levels[l].bnd) CU(dev_malloc(h->levels[l].bnd, h->levels[l].nface * sizeof(double)));
+	}
+	if (!guess_schedule(h, o))
+		for (int l = (int) h->fmg_ws.size() / 2; l < h->last_level; l++)
+			for (int k = 0; k < 2; k++) {
+				VecPtr v;
+				TRY(vec_create(h, l, v));
+				h->fmg_ws.push_back(std::move(v));
+			}
+	GraphEntry key;
+	key.f = f->d, key.u = u->d, key.b = b ? b->d : nullptr, key.fmg_cycles = cycles;
+	return graph_run(h, o, std::move(key), [&] {
+		h->cycle_faces     = nullptr;
+		h->cycle_faces_old = h->cycle_uc = nullptr;
+		const int rc       = fmg_run(h, o, cycles, f->d, b ? b->d : nullptr, u->d);
+		h->cycle_faces     = nullptr; // (a cycle of level 0 may have recorded its slices; FMG reports none)
+		h->cycle_faces_old = h->cycle_uc = nullptr;
+		return rc;
+	});
 	API_END
 }
 

@@ -42,7 +42,9 @@ typedef struct TgpuLevelDesc {
 	int32_t        npatch;
 	const double  *spacing;        /* [npatch][D]   cell size h; patches must be cubic/isotropic */
 	const double  *starts;         /* [npatch][D]   lower corner (only used for the manufactured RHS) */
-	const uint8_t *neumann_bits;   /* [npatch]      bit s set: side s is a Neumann domain boundary */
+	const uint8_t *neumann_bits;   /* [npatch]      bit s set: side s is a Neumann domain boundary (a cleared bit on such a
+	                                  side: Dirichlet).  An owned patch with a bit on a side that has a neighbour, or a
+	                                  bit s >= 2D, makes tgpu_hierarchy_create return TGPU_ERR_ARG */
 	const int8_t  *nbr_type;       /* [npatch][2D]  TGPU_NBR_* */
 	const int32_t *nbr_idx;        /* [npatch][2D][Q] local index of the neighbour patch(es): normal/coarse use
 	                                  slot 0, fine uses all Q slots ordered by Orthant<D-1> on the face */

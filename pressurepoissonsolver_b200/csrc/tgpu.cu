@@ -870,6 +870,14 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 					pm.orth_on_coarse[s] = (int8_t) o;
 				}
 			}
+			// a Neumann bit means a domain side: on a side with a neighbour the smoother would pick a Neumann transform that
+			// the operator (which reads the neighbour) does not match, and bits past side 2D - 1 name no side
+			if (p < L.P) {
+				if (pm.neumann >> S) return fail(TGPU_ERR_ARG, "neumann_bits: bit set past side 2D - 1");
+				for (int s = 0; s < S; s++)
+					if (((pm.neumann >> s) & 1) && pm.nbr_type[s] != NBR_NONE)
+						return fail(TGPU_ERR_ARG, "neumann_bits: Neumann bit on a side with a neighbour");
+			}
 		}
 		TRY(dev_upload(L.meta, meta.data(), meta.size()));
 		if (!L.neu_host.empty()) TRY(dev_upload(L.neu_list, L.neu_host.data(), L.neu_host.size()));

@@ -123,8 +123,22 @@ int tgpu_hierarchy_info(const tgpu_hier *h, int *D, int *n, int *nlevels);
 int tgpu_hierarchy_trim(tgpu_hier *h);
 int tgpu_level_npatch(const tgpu_hier *h, int level, int64_t *npatch, int64_t *ncells);
 /* the patch solver's shift, FftwPatchSolver(domain, lambda) (PatchSolvers/FftwPatchSolver.h:66,170): block-Jacobi patch
- * problems (Laplacian + lambda) u = rhs; default 0.  Non-zero values take the general (dense-transform) patch solve. */
+ * problems (Laplacian + lambda) u = rhs; default 0.  The operator keeps its own shift (tgpu_hierarchy_set_helmholtz, 0 by
+ * default).  While the two differ, every cycle computes its residuals in full passes (the fused schedule's face-only
+ * residuals need equal shifts); a non-zero patch solver shift then also takes the general (dense-transform) patch
+ * solve, while lambda = 0 keeps the specialised sweeps with unshifted tables. */
 int tgpu_hierarchy_set_lambda(tgpu_hier *h, double lambda);
+/* Helmholtz problems: afterwards the operator of every level is A_l + lambda I (tgpu_apply, tgpu_residual,
+ * tgpu_residual_restrict, tgpu_smooth_jacobi's diagonal, every cycle and solver), and the patch solver's shift is lambda too,
+ * so the sweeps solve the shifted patch problems exactly and run on the same kernels and schedules as lambda = 0.
+ * lambda must be finite and <= 0 (an implicit diffusion step (I - nu dt Laplacian) u = g is lambda = -1 / (nu dt) with
+ * right-hand side -g / (nu dt)); otherwise TGPU_ERR_ARG and the hierarchy is unchanged.  lambda = 0 restores the Poisson
+ * problem, bit for bit.  A later tgpu_hierarchy_set_lambda(mu) changes the patch solver's shift only, as without this call;
+ * setting it back to lambda restores the fast paths.  Boundary folds (tgpu_fold_boundary, tgpu_init_*) come from the
+ * Laplacian part and do not change.  Drops the cached cycle graphs and rebuilds the patch solve tables (one per cell size;
+ * sizes within a relative 1e-12 share one).  A hierarchy with more than 256 cell sizes takes lambda = 0 only:
+ * TGPU_ERR_UNSUPPORTED otherwise, hierarchy unchanged. */
+int tgpu_hierarchy_set_helmholtz(tgpu_hier *h, double lambda);
 /* test hook: on != 0 routes every smoother launch through the size-generic kernel even where a
  * specialised one exists (D = 3, n = 16), so that the two can be compared */
 int tgpu_hierarchy_force_generic_kernels(tgpu_hier *h, int on);
@@ -176,7 +190,8 @@ int tgpu_bicgstab(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tg
  * another level or hierarchy, tol < 0 or max_it < 0 give TGPU_ERR_ARG and leave u untouched.
  * u <- u + Cycle(f - A u): one cycle from the guess u (opts as tgpu_vcycle; NULL = defaults).  The fused schedule
  * starts the finest level's pre-sweep from u's boundary slices; the others (fused = 0, interpolator = 1, W cycles on
- * several GPUs, no post-sweep, one level, lambda != 0) compute the residual, a cycle from zero and the sum.
+ * several GPUs, no post-sweep, one level, a patch solver shift the operator does not carry) compute the residual, a
+ * cycle from zero and the sum.
  * rel_residual (nullable): ||f - A u_new||_2 / ||f||_2 of the result (fused: from the boundary slices, see DESIGN). */
 int tgpu_vcycle_update(tgpu_hier *h, const TgpuCycleOpts *opts, const tgpu_vec *f, tgpu_vec *u, double *rel_residual);
 /* cycles of tgpu_vcycle_update until ||f - A u||_2 <= tol ||f||_2 (confirmed by a full residual) or max_it cycles.

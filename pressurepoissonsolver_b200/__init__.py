@@ -80,7 +80,7 @@ ABI_SYMBOLS = [
     "tgpu_init_trig_rhs", "tgpu_init_neumann_rhs", "tgpu_vec_integrate", "tgpu_mesh_partition", "tgpu_part_destroy", "tgpu_part_info", "tgpu_part_level", "tgpu_part_peer", "tgpu_part_level_interior",
     "tgpu_comm_unique_id", "tgpu_comm_init", "tgpu_hierarchy_create_distributed",
     "tgpu_hierarchy_force_generic_kernels", "tgpu_mesh_set_neumann", "tgpu_vcycle_host_async", "tgpu_vcycle_host_wait",
-    "tgpu_hierarchy_trim", "tgpu_hierarchy_set_lambda", "tgpu_prolong_add_linear", "tgpu_vec_transfer_pair",
+    "tgpu_hierarchy_trim", "tgpu_hierarchy_set_lambda", "tgpu_hierarchy_set_helmholtz", "tgpu_prolong_add_linear", "tgpu_vec_transfer_pair",
     "tgpu_vcycle_update", "tgpu_gmg_solve", "tgpu_boundary_sides", "tgpu_boundary_vec_create", "tgpu_fold_boundary",
     "tgpu_fmg",
 ]
@@ -146,6 +146,7 @@ for _name, _args in {
     "tgpu_comm_unique_id": [_vp], "tgpu_comm_init": [_vp, _vp, C.c_int, C.c_int],
     "tgpu_hierarchy_create_distributed": [_vp, _vp, C.POINTER(_vp)],
     "tgpu_hierarchy_force_generic_kernels": [_vp, C.c_int], "tgpu_hierarchy_set_lambda": [_vp, C.c_double],
+    "tgpu_hierarchy_set_helmholtz": [_vp, C.c_double],
     "tgpu_mesh_set_neumann": [_vp, C.c_int],
     "tgpu_vcycle_host_async": [_vp, C.POINTER(CycleOpts), _vp, _vp], "tgpu_vcycle_host_wait": [_vp],
     "tgpu_vec_transfer_pair": [_vp, _vp, _vp, _vp, _vp],
@@ -427,6 +428,10 @@ class Hierarchy:
     def set_lambda(self, lam):
         """the patch solver's shift (FftwPatchSolver(domain, lambda), PatchSolvers/FftwPatchSolver.h:66,170)"""
         check(lib.tgpu_hierarchy_set_lambda(self._p, lam))
+
+    def set_helmholtz(self, lam):
+        """operator A + lam I on every level, with the patch solver's shift lam too (lam finite and <= 0; 0: Poisson)"""
+        check(lib.tgpu_hierarchy_set_helmholtz(self._p, lam))
 
     def force_generic_kernels(self, on=True):
         check(lib.tgpu_hierarchy_force_generic_kernels(self._p, 1 if on else 0))

@@ -52,11 +52,13 @@ __device__ __forceinline__ void tma_load_1d(void *smem_dst, const void *gsrc, un
 // MODE 0: out = A u, 1: out = f - A u, 2: coarse = AvgRstr(f - A u) (GMG/AvgRstr.h:88-107; the fine residual is never written),
 // 3: out = A u and, riding along, the block partial sums of out . f and out . out (f = the vector the Krylov iteration dots A u
 //    with next, BiCGStab.h:77,89: one pass over memory less per operator application; partial[b], partial[pstride + b])
+// shift != 0: A is the Helmholtz operator Laplacian + shift (tgpu_hierarchy_set_helmholtz), the term shift h^2 u joins the
+// stencil sum before the 1/h^2 (a launch-uniform branch: shift = 0 runs the plain stencil's arithmetic)
 template <int D, int N, int MODE>
 __global__ void __launch_bounds__(TGPU_THREADS, 2)
 apply_tma_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *__restrict__ u, const double *__restrict__ f,
                  const double *__restrict__ F, double *__restrict__ out, double *__restrict__ coarse, double *__restrict__ partial = nullptr,
-                 int pstride = 0)
+                 int pstride = 0, double shift = 0.0)
 {
 	using G = Geo<D, N>;
 	pdl_launch_dependents();
@@ -106,11 +108,12 @@ apply_tma_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double
 			for (int k = 0; k < N; k++) r[k] = valid ? __ldg(f + (size_t) p * G::NC + k * G::M + m) : 0.0;
 		}
 		// ---- ghost faces of this patch: entry m of every side (independent of the tile, overlaps the bulk copy) ----
-		double inv_h2 = 0.0;
+		double inv_h2 = 0.0, sh2 = 0.0;
 		int    orth = -1, parent = 0;
 		if (valid) {
 			const PatchMeta &pm = meta[p];
 			inv_h2              = pm.inv_h2;
+			sh2                 = shift * pm.h2;
 			orth                = pm.orth_on_parent;
 			parent              = pm.parent_idx;
 			int    ty[G::S];
@@ -154,6 +157,7 @@ apply_tma_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double
 				double       acc;
 				if (D == 2) acc = (wp[k * ws] - 2 * ce + ep[k * es]) + (lo - 2 * ce + hi);
 				else acc = (wp[k * ws] - 2 * ce + ep[k * es]) + (sp[k * ss] - 2 * ce + np_[k * ns]) + (lo - 2 * ce + hi);
+				if (shift != 0.0) acc = fma(sh2, ce, acc);
 				if (MODE == 3) {
 					const double o = acc * inv_h2;
 					d0             = fma(o, r[k], d0);
@@ -219,7 +223,8 @@ constexpr size_t apply3d32_tma_smem_bytes() { return sizeof(double) * (10 * 1024
 template <int MODE>
 __global__ void __launch_bounds__(TGPU_THREADS, 2)
 apply3d32_tma_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *__restrict__ u, const double *__restrict__ f,
-                     const double *__restrict__ F, double *__restrict__ out, double *__restrict__ partial = nullptr, int pstride = 0)
+                     const double *__restrict__ F, double *__restrict__ out, double *__restrict__ partial = nullptr, int pstride = 0,
+                     double shift = 0.0)
 {
 	constexpr int N = 32, M = N * N, NC = N * N * N;
 	extern __shared__ __align__(16) double U[]; // [10][32][32], then GX[2][256], GY[2][256]
@@ -271,7 +276,7 @@ apply3d32_tma_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const do
 		}
 		__syncthreads();
 		mbar_wait(&bar, n & 1);
-		const double inv_h2 = pm.inv_h2;
+		const double inv_h2 = pm.inv_h2, sh2 = shift * pm.h2; // (shift: see apply_tma_kernel)
 #pragma unroll
 		for (int j = 0; j < 4; j++) {
 			const int     x = lo, y = hi + 8 * j;
@@ -284,7 +289,8 @@ apply3d32_tma_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const do
 #pragma unroll
 			for (int k = 0; k < 8; k++) {
 				const double hi_v = cp[(k + 1) * M];
-				const double acc  = (wp[k * ws] - 2 * ce + ep[k * es]) + (sp[k * ss] - 2 * ce + np_[k * ns]) + (lo_v - 2 * ce + hi_v);
+				double       acc  = (wp[k * ws] - 2 * ce + ep[k * es]) + (sp[k * ss] - 2 * ce + np_[k * ns]) + (lo_v - 2 * ce + hi_v);
+				if (shift != 0.0) acc = fma(sh2, ce, acc);
 				const size_t o    = (size_t) p * NC + (size_t) (zs * 8 + k) * M + y * N + x;
 				if (MODE == 3) {
 					const double v = acc * inv_h2;

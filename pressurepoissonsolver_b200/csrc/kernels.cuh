@@ -43,7 +43,8 @@ struct __align__(16) PatchMeta {
 	uint8_t neumann;
 	int8_t  nbr_type[6];
 	int8_t  orth_on_coarse[6];
-	int8_t  pad_[2];
+	uint8_t tab;    // the patch's elimination multiplier table (one per distinct h, see TriSolve)
+	int8_t  pad_[1];
 	int32_t nbr_idx[6][4];
 	int32_t nbr_parent[6]; // parent_idx of nbr_idx[s][0] (normal neighbours; lets the post-smoother fold the
 	int8_t  nbr_orth[6];   // prolongation into its face reads without a dependent table lookup)
@@ -298,8 +299,10 @@ template <int NT> struct Dst3<NT, 1> {
 // pairs + one Thomas solve instead of three transform pairs; same patch solve as FftwPatchSolver.h:174-206 /
 // DftPatchSolver.h:173-216 in exact arithmetic, 56 fp64 operations per pencil instead of 248).
 // For the pencil with transform indices (k_a, k_b) the remaining system is  M y = h^2 r,
-//   M = tridiag(1, d_j, 1),  d_j = mu - 2 (mu - 3 at both ends: the Dirichlet closure of StarPatchOp.h:46-64),
-//   mu = -4 sin^2((k_a+1) pi/2n) - 4 sin^2((k_b+1) pi/2n).
+//   M = tridiag(1, d_j, 1),  d_j = mu - 2 + lambda h^2 (mu - 3 + lambda h^2 at both ends: the Dirichlet closure of
+//   StarPatchOp.h:46-64),  mu = -4 sin^2((k_a+1) pi/2n) - 4 sin^2((k_b+1) pi/2n),
+// lambda = the shift of a Helmholtz operator (tgpu_hierarchy_set_helmholtz), 0 otherwise.  With lambda != 0 the multipliers
+// depend on h: the hierarchy keeps one table per distinct cell size, PatchMeta::tab names a patch's.
 // M is symmetric under j -> n-1-j, so it is eliminated from both ends towards the middle with ONE set of
 // multipliers a_0 = 1/d_0, a_j = 1/(d_j - a_{j-1}) (two independent dependency chains of n/2), leaving
 //   y_j + a_j y_{j+1} = rho_j (j < n/2),  y_{n-1-j} + a_j y_{n-2-j} = rho'_j,  and a 2 x 2 system in the middle.
@@ -704,13 +707,14 @@ __global__ void __launch_bounds__(TGPU_THREADS, smooth_min_blocks<N>())
 smooth_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *__restrict__ f, double *__restrict__ u,
               const double *__restrict__ Fin, double *__restrict__ Fout, const double *__restrict__ tri,
               const double *__restrict__ uc, const double *__restrict__ mats, const double *__restrict__ lam, double lam_shift,
-              int only_neumann = 0)
+              int only_neumann = 0, int helm = 0)
 {
 	// only_neumann != 0: only patches with Neumann domain sides are swept - the others of the range belong to a specialised
 	// kernel launched over the same range (smooth3d16_kernel / smooth2d32_kernel with skip_neumann)
 	// lam_shift: the patch solver's "lambda" (FftwPatchSolver.h:66,170, DftPatchSolver.h:78,168): the patch problems are
 	// (Laplacian + lambda) u = rhs; != 0 sends every patch through the general transform path, whose eigenvalue sums are
-	// formed on the fly
+	// formed on the fly, unless helm != 0: the operator carries the same shift (tgpu_hierarchy_set_helmholtz), the Dirichlet
+	// patches take the tridiagonal solve with their shifted table tri[pm.tab], and an all-Neumann patch keeps its zero mode
 	// works on patches [p0, P) (multi-GPU: interior and boundary patches are separate launches)
 	// Persistent CTAs: each loops over groups of PPB patches (group g = blockIdx.x + k gridDim.x).
 	// The right-hand side of the NEXT group streams into the second shared-memory buffer with
@@ -770,6 +774,7 @@ smooth_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *_
 
 		double *S = Sall + pp * G::SP;
 		double  cfac = 0.0, h2 = 0.0;
+		int     tab  = 0;
 		int     neu  = 0; // Neumann domain sides of this patch: != 0 takes the general transform path
 		bool    general = false;
 		int8_t  ntype[6] = {-1, -1, -1, -1, -1, -1};
@@ -778,8 +783,9 @@ smooth_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *_
 			const PatchMeta &pm = meta[p];
 			cfac                = 2.0 * pm.inv_h2;
 			h2                  = pm.h2;
+			tab                 = pm.tab;
 			neu                 = pm.neumann;
-			general             = neu != 0 || lam_shift != 0.0;
+			general             = neu != 0 || (lam_shift != 0.0 && !helm);
 			if (!ZERO_GUESS) {
 				// entry m of every side is both produced and consumed by thread m: no staging needed
 				int    ty[G::S];
@@ -855,7 +861,7 @@ smooth_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *_
 				double       scale = h2;
 #pragma unroll
 				for (int a = 0; a < D; a++) scale *= 2.0 / N;
-				const bool singular = neu == (1 << (2 * D)) - 1;
+				const bool singular = neu == (1 << (2 * D)) - 1 && !helm;
 #pragma unroll
 				for (int k = 0; k < N; k++) {
 					const double sum = __ldg(lam + kx.lam * N + k) + rest + lam_shift * h2;
@@ -864,8 +870,9 @@ smooth_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *_
 				general_transform<N>(mats, kx.inv, v, S + m * G::ROW, 1, mg);
 			} else {
 				// the other axes are diagonalised: row m is a tridiagonal system along x (TriSolve)
-				TriSolve<N, G::M>::forward(v, tri + m, h2 * ((D == 2) ? 2.0 / N : 4.0 / (N * N)));
-				TriSolve<N, G::M>::backward(v, tri + m);
+				const double *tb = tri + (size_t) tab * ((N / 2 + 1) * G::M) + m;
+				TriSolve<N, G::M>::forward(v, tb, h2 * ((D == 2) ? 2.0 / N : 4.0 / (N * N)));
+				TriSolve<N, G::M>::backward(v, tb);
 #pragma unroll
 				for (int k = 0; k < N; k++) S[m * G::ROW + k] = v[k];
 			}
@@ -1262,10 +1269,11 @@ __global__ void restrict_kernel(const PatchMeta *__restrict__ meta, int P, const
 // diagonal of the ghost-eliminated composite operator: -(2 D)/h^2 per cell plus, per patch side the cell touches, the
 // cell's own coefficient in the ghost value 2 gamma - u (StarPatchOp.h:46-64, interface weights SURVEY App. A.2):
 // domain side -1 (Dirichlet) / +1 (Neumann), same-level neighbour 0, coarse neighbour 5/6 (3D) or 2/3 (2D), fine
-// neighbours -1/3.  The "weighted-Jacobi option" of the north star (no reference counterpart; oracle: gmg_oracle.jacobi).
+// neighbours -1/3, plus the operator's shift (tgpu_hierarchy_set_helmholtz).  The "weighted-Jacobi option" of the north
+// star (no reference counterpart; oracle: gmg_oracle.jacobi).
 template <int D, int N>
 __global__ void jacobi_update_kernel(const PatchMeta *__restrict__ meta, int P, const double *__restrict__ r,
-                                     double *__restrict__ u, double omega)
+                                     double *__restrict__ u, double omega, double shift)
 {
 	pdl_launch_dependents();
 	pdl_wait();
@@ -1288,7 +1296,7 @@ __global__ void jacobi_update_kernel(const PatchMeta *__restrict__ meta, int P, 
 			if (c[a] == 0) diag += side(2 * a);
 			if (c[a] == N - 1) diag += side(2 * a + 1);
 		}
-		u[i] += omega * r[i] / (diag * pm.inv_h2);
+		u[i] += omega * r[i] / (diag * pm.inv_h2 + shift);
 	}
 }
 

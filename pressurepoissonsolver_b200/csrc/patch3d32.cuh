@@ -344,6 +344,7 @@ smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 		const bool   next = g + ncl < npatch;
 		const int    pn   = p + ncl;
 		const double h2   = meta[p].h2;
+		const double *tp  = tri + (size_t) meta[p].tab * (17 * M); // the patch's multiplier table [17][M] (TriSolve)
 		double       v[N];
 		if (skip_neumann && meta[p].neumann) { // cluster-uniform: this patch belongs to the general path
 			cluster_sync_all(); // keeps the pair in step: the exchange planes alternate by iteration parity
@@ -415,7 +416,7 @@ smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 		for (int q = 0; q < 2; q++) {
 			const int     ky = w + 16 * q;
 			const double *zp = S + ky * ROW + lane;
-			const double *tb = tri + ky * N + lane;
+			const double *tb = tp + ky * N + lane;
 			double        rho = 0.0;
 #pragma unroll
 			for (int j = 0; j < 16; j++) {
@@ -432,7 +433,7 @@ smooth3d32c_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 		for (int q = 0; q < 2; q++) {
 			const int     ky = w + 16 * q;
 			double *      zp = S + ky * ROW + lane;
-			const double *tb = tri + ky * N + lane;
+			const double *tb = tp + ky * N + lane;
 			const double  a15 = __ldg(tb + 15 * M), kap = __ldg(tb + 16 * M);
 			double        y   = kap * fma(-a15, ld_dsmem(Xo + ky * N + lane, rank ^ 1), zp[15 * PL]);
 			zp[15 * PL]       = y;
@@ -547,7 +548,7 @@ __global__ void __launch_bounds__(TGPU_THREADS)
 smooth3d32n_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const double *__restrict__ f, double *__restrict__ u,
                    const double *__restrict__ Fin, double *__restrict__ Fout, const double *__restrict__ uc,
                    const double *__restrict__ mats, const double *__restrict__ lam, double *__restrict__ scratch, int zero_guess,
-                   int emit, int prolong, int write_u, double lam_shift, int only_neumann = 0)
+                   int emit, int prolong, int write_u, double lam_shift, int only_neumann = 0, int helm = 0)
 {
 	// only_neumann != 0: only patches with Neumann domain sides are swept (the others of the range belong to
 	// smooth3d32c_kernel, skip_neumann)
@@ -588,7 +589,7 @@ smooth3d32n_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doub
 			if (pass == 3) {
 				const AxisKind kx = axis_kind(neu, 0), ky = axis_kind(neu, 1), kz = axis_kind(neu, 2);
 				const double   scale = h2 * (2.0 / N) * (2.0 / N) * (2.0 / N);
-				const bool     singular = neu == 63;
+				const bool     singular = neu == 63 && !helm; // (helm: a Helmholtz operator, the zero mode is solved for)
 				for (int i = t; i < NC; i += TGPU_THREADS) {
 					const double sum = __ldg(lam + kx.lam * N + i % N) + (__ldg(lam + ky.lam * N + (i / N) % N) + __ldg(lam + kz.lam * N + i / M)) + lam_shift * h2;
 					W[i]             = (singular && i == 0) ? 0.0 : W[i] * scale / sum;

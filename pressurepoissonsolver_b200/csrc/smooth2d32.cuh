@@ -105,6 +105,7 @@ smooth2d32_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 		const bool   next = g + nw < npatch;
 		const int    pn   = p + nw;
 		const double h2   = meta[p].h2;
+		const double *tb  = tri + (size_t) meta[p].tab * (17 * 32) + lane; // the patch's table [17][32] (TriSolve)
 		double       v[N];
 		if (EXTRA && !ZERO_GUESS && next) halo_wait_warp(hs, pn, halo_ok); // gamma of patch pn is gathered during this iteration
 		if (EXTRA && skip_neumann && meta[p].neumann) { // warp-uniform
@@ -164,8 +165,8 @@ smooth2d32_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 				v[2 * j]        = d.x;
 				v[2 * j + 1]    = d.y;
 			}
-			TriSolve<N, N>::forward(v, tri + lane, h2 * (2.0 / N));
-			TriSolve<N, N>::backward(v, tri + lane);
+			TriSolve<N, N>::forward(v, tb, h2 * (2.0 / N));
+			TriSolve<N, N>::backward(v, tb);
 #pragma unroll
 			for (int j = 0; j < N / 2; j++) rowp[j] = make_double2(v[2 * j], v[2 * j + 1]);
 		}

@@ -67,7 +67,8 @@ enum { GD_SA = 1, GD_SB = 2, GD_WB = 4, GD_SLOW = 8 };
 struct GPatch16 {
 	GDesc16 d[6];
 	double  h2;
-	int     neu, pad; // Neumann bits of the patch (a level with Neumann patches: this kernel skips them, see skip_neumann)
+	int     neu;      // Neumann bits of the patch (a level with Neumann patches: this kernel skips them, see skip_neumann)
+	int     tab;      // the patch's multiplier table (PatchMeta::tab)
 };
 template <bool PROLONG>
 __device__ __forceinline__ void make_gdesc16(const PatchMeta &pm, int p, int s, GPatch16 &out)
@@ -128,11 +129,14 @@ template <bool PROLONG> struct SideGamma16 {
 	}
 };
 
-// tables of the general patch solve (smooth_kernel's): dense transform matrices by kind and the eigenvalue rows
+// tables of the general patch solve (smooth_kernel's): dense transform matrices by kind and the eigenvalue rows, and the
+// shift of a Helmholtz operator (tgpu_hierarchy_set_helmholtz; helm != 0: an all-Neumann patch keeps its zero mode)
 struct NeuTabs {
 	const double * mats = nullptr, *lam = nullptr;
 	const int32_t *list = nullptr; // the patches the launch sweeps (those of the range with Neumann sides), ascending
 	int            n    = 0;
+	int            helm = 0;
+	double         shift = 0.0;
 };
 // HALO = false compiles the multi-GPU hand-over (HaloSync / halo_push_cta) out: the single-GPU instantiations carry none of it
 // NEU = true: the instantiation for the patches WITH Neumann domain sides of a level (it sweeps exactly those of the range,
@@ -176,7 +180,7 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 	// one thread per side (lane 31 of warps 0-5) resolves the descriptors of patch q into GD[slot]
 	auto describe = [&](const PatchMeta &pm, int q, int slot) {
 		if ((t & 31) == 31 && t < 6 * 32) make_gdesc16<PROLONG>(pm, q, t >> 5, GD[slot]);
-		if (t == 6 * 32 + 31) GD[slot].h2 = pm.h2, GD[slot].neu = pm.neumann;
+		if (t == 6 * 32 + 31) GD[slot].h2 = pm.h2, GD[slot].neu = pm.neumann, GD[slot].tab = pm.tab;
 	};
 
 	int g = blockIdx.x;
@@ -226,6 +230,7 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 		__syncthreads();
 		if (HALO && !ZERO_GUESS && next) halo_wait_cta(hs, pn, halo_ok); // gamma of patch pn is gathered during this iteration
 		const double h2 = ZERO_GUESS ? meta[p].h2 : GD[b].h2;
+		const int    tab = NEU ? 0 : (ZERO_GUESS ? meta[p].tab : GD[b].tab);
 		// table entry of the patch after the next -> metaS (read by describe() after the next barrier but one)
 		if (!ZERO_GUESS && t < MW && gn + (int) gridDim.x < npatch)
 			cp_async8(&metaS[t], reinterpret_cast<const double *>(meta + pnn) + t, true);
@@ -319,14 +324,14 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 				// transform along y as well and divide by the eigenvalue sum of (k_x, k_y, k_z) = (lo, k, hi)
 				const AxisKind kx = axis_kind(neu_p, 0), ky = axis_kind(neu_p, 1), kz = axis_kind(neu_p, 2);
 				general_transform<N>(nt.mats, ky.fwd, v, q, ROW, mg);
-				const double rest     = __ldg(nt.lam + kx.lam * N + lo) + __ldg(nt.lam + kz.lam * N + hi);
+				const double rest     = __ldg(nt.lam + kx.lam * N + lo) + __ldg(nt.lam + kz.lam * N + hi) + nt.shift * h2;
 				const double scale    = h2 * (8.0 / (N * N * N));
-				const bool   singular = neu_p == 63 && t == 0; // all-Neumann patch: the constant mode is left out
+				const bool   singular = neu_p == 63 && t == 0 && !nt.helm; // all-Neumann patch: the constant mode is left out
 #pragma unroll
 				for (int k = 0; k < N; k++) v[k] = (singular && k == 0) ? 0.0 : q[k * ROW] * scale / (__ldg(nt.lam + ky.lam * N + k) + rest);
 			} else {
 				// z and x are diagonalised: what is left per (k_x, k_z) is a tridiagonal system along y
-				TriSolve<N>::forward(v, tri + t, h2 * (4.0 / (N * N)));
+				TriSolve<N>::forward(v, tri + (size_t) tab * (9 * 256) + t, h2 * (4.0 / (N * N)));
 			}
 			double gx0 = 0.0, gx1 = 0.0;
 			if (!ZERO_GUESS && next) {
@@ -336,7 +341,7 @@ smooth3d16_kernel(const PatchMeta *__restrict__ meta, int p0, int P, const doubl
 			if (NEU) {
 				general_transform<N>(nt.mats, axis_kind(neu_p, 1).inv, v, q, ROW, mg);
 			} else {
-				TriSolve<N>::backward(v, tri + t);
+				TriSolve<N>::backward(v, tri + (size_t) tab * (9 * 256) + t);
 #pragma unroll
 				for (int k = 0; k < N; k++) q[k * ROW] = v[k];
 			}

@@ -294,7 +294,10 @@ struct tgpu_hier {
 	// the first post-sweep (cycle_uc == nullptr otherwise); see k_face_residual_norm
 	const double *        cycle_faces_old = nullptr, *cycle_uc = nullptr;
 	double *              visit_faces = nullptr; // the slices of the result of the last fused_visit that was asked to emit them
-	DevPtr<double>        tri; // [N/2 + 1][N^(D-1)] tridiagonal multipliers (TriSolve)
+	DevPtr<double>        tri; // [table][N/2 + 1][N^(D-1)] tridiagonal multipliers (TriSolve), one table per distinct h
+	std::vector<double>   tab_h2;          // h^2 of each table (PatchMeta::tab)
+	bool                  tab_overflow = false; // more than 256 cell sizes: one table index cannot name them all
+	double                tab_shift = 0.0; // the shift the tables were built with (upload_tri)
 	DevPtr<double>        mats, lam; // Neumann patches: transform matrices [6][N][N], 1-D eigenvalues [3][N]
 	std::vector<GraphEntry> graphs;
 	std::vector<VecPtr>   krylov_ws;
@@ -314,7 +317,8 @@ struct tgpu_hier {
 	EventPtr              ev_in[2], ev_cyc[2], ev_out[2];
 	uint64_t              pipe_count = 0;
 	bool                  generic_kernels = false; // test hook: force the size-generic smoother
-	double                lambda = 0.0;            // the patch solver's shift (tgpu_hierarchy_set_lambda)
+	double                lambda = 0.0;            // the patch solver's shift (tgpu_hierarchy_set_lambda / _set_helmholtz)
+	double                op_shift = 0.0;          // the operator's shift: A + op_shift I (tgpu_hierarchy_set_helmholtz)
 	int                   last_level = 0;          // coarsest level the running cycle visits (CycleOpts max_levels / patches_per_proc)
 	// peer-to-peer arena: flag rows + the face buffers of the distributed levels, one IPC-exported allocation
 	DevPtr<void>          arena;
@@ -455,6 +459,14 @@ static bool specialised(const tgpu_hier *h)
 {
 	return is_3d32(h) || (((h->D == 3 && h->N == 16) || (h->D == 2 && h->N == 32)) && !h->generic_kernels);
 }
+// The operator carries the patch solver's shift, so the face identity of DESIGN §3 holds after a sweep: the schedules and
+// kernels that work from face buffers apply.  Always so without a shift.
+static bool consistent(const tgpu_hier *h) { return h->op_shift == h->lambda; }
+// A smoother-only shift (tgpu_hierarchy_set_lambda): every patch takes the general transform path
+static bool shifted_smoother(const tgpu_hier *h) { return h->lambda != 0.0 && !consistent(h); }
+// A Helmholtz problem (tgpu_hierarchy_set_helmholtz): the Dirichlet patch solves read shifted multiplier tables, and the
+// general path solves the shifted problem of an all-Neumann patch with its zero mode
+static int helmholtz(const tgpu_hier *h) { return consistent(h) && h->lambda != 0.0; }
 
 // Calls fn with one std::integral_constant<bool, ...> argument per run-time template flag.
 template <class Fn> static int flag_variant(bool a, Fn &&fn) { return a ? fn(std::true_type{}) : fn(std::false_type{}); }
@@ -482,8 +494,8 @@ template <class Fn> static int each_smooth_variant(Fn &&fn)
 		if (is_sweep_variant(v & 8, v & 4, v & 2, v & 1)) TRY(smooth_variant(v & 8, v & 4, v & 2, v & 1, fn));
 	return TGPU_OK;
 }
-// G of the 32^3 levels whose sweeps can reach smooth3d32c_kernel from a non-zero guess (iface_rhs32_kernel): lambda = 0 (a
-// shifted patch solve sends every patch through smooth3d32n_kernel) and at least one owned patch without Neumann sides.
+// G of the 32^3 levels whose sweeps can reach smooth3d32c_kernel from a non-zero guess (iface_rhs32_kernel): no smoother-only
+// shift (it sends every patch through smooth3d32n_kernel) and at least one owned patch without Neumann sides.
 template <typename T> static int dev_upload(DevPtr<T> &dst, const T *src, size_t count);
 // G holds one term per interface slot (IfaceSlots32, built from the owned patches' metadata with the table).  Called at
 // creation and when lambda changes (never during a graph capture); the graphs are freed before G is.
@@ -491,7 +503,7 @@ static int update_iface_buffers(tgpu_hier *h)
 {
 	if (!is_3d32(h)) return TGPU_OK;
 	for (LevelDev &L : h->levels) {
-		const bool want = h->lambda == 0.0 && L.neu_host.size() < (size_t) L.P;
+		const bool want = !shifted_smoother(h) && L.neu_host.size() < (size_t) L.P;
 		if (want && !L.G) {
 			std::vector<PatchMeta> meta(L.P);
 			CU(cudaMemcpy(meta.data(), L.meta.get(), meta.size() * sizeof(PatchMeta), cudaMemcpyDeviceToHost));
@@ -510,10 +522,10 @@ static int update_iface_buffers(tgpu_hier *h)
 	return TGPU_OK;
 }
 // smooth3d32n_kernel's scratch, one 256 KB block per CTA: 32^3 hierarchies whose sweeps take the general patch solve (a level
-// with Neumann sides, or lambda != 0)
+// with Neumann sides, or a smoother-only shift)
 static int ensure_scratch32(tgpu_hier *h)
 {
-	bool want = h->lambda != 0.0;
+	bool want = shifted_smoother(h);
 	for (const LevelDev &L : h->levels) want = want || L.has_neumann;
 	if (is_3d32(h) && want && !h->scratch32) CU(dev_malloc(h->scratch32, (size_t) h->ctx->sm_count * 2 * 32768 * sizeof(double)));
 	return TGPU_OK;
@@ -792,6 +804,45 @@ template <typename T> static int dev_upload(DevPtr<T> &dst, const T *src, size_t
 	return TGPU_OK;
 }
 
+// Multipliers of the two-sided tridiagonal elimination along the axis that is not transformed, for every pencil of the other
+// axes' transform indices (TriSolve, kernels.cuh): one table [n/2 + 1][n^(D-1)] per cell size h of the hierarchy (h->tab_h2),
+// with the diagonal shifted by lambda h^2 in the Helmholtz state and unshifted otherwise.  Unshifted tables are all equal.
+// Rebuilt when the shift changes; the caller has dropped the graphs that could still be reading them.
+static int upload_tri(tgpu_hier *h)
+{
+	const double shift = helmholtz(h) ? h->lambda : 0.0;
+	if (h->tri && shift == h->tab_shift) return TGPU_OK;
+	const int    D = h->D, n = h->N, H = n / 2;
+	const size_t M = D == 2 ? n : (size_t) n * n, T = (size_t) (H + 1) * M;
+	std::vector<double>      tri(T * h->tab_h2.size());
+	std::vector<long double> ll(n);
+	for (int k = 0; k < n; k++) {
+		const long double sn = sinl((k + 1) * 3.141592653589793238462643383279502884L / (2 * n));
+		ll[k]                = -4.0L * sn * sn;
+	}
+	for (size_t t = 0; t < h->tab_h2.size(); t++) {
+		const long double lh2 = (long double) shift * h->tab_h2[t];
+		double *const     tab = tri.data() + t * T;
+		for (size_t m = 0; m < M; m++) {
+			const long double mu = (D == 2) ? ll[m] : ll[m % n] + ll[m / n];
+			long double       a  = 0.0L;
+			for (int j = 0; j < H; j++) {
+				const long double d = mu - (j == 0 ? 3.0L : 2.0L) + lh2;
+				a                   = 1.0L / (d - (j == 0 ? 0.0L : a));
+				tab[(size_t) j * M + m] = (double) a;
+			}
+			tab[(size_t) H * M + m] = (double) (1.0L / (1.0L - a * a));
+		}
+	}
+	if (!h->tri) TRY(dev_upload(h->tri, tri.data(), tri.size()));
+	else {
+		CU(cudaStreamSynchronize(h->ctx->stream)); // sweeps still in flight read the old tables
+		CU(cudaMemcpy(h->tri.get(), tri.data(), tri.size() * sizeof(double), cudaMemcpyHostToDevice));
+	}
+	h->tab_shift = shift;
+	return TGPU_OK;
+}
+
 // n_owned == nullptr: every patch of every level is owned (single GPU).  Otherwise level l has n_owned[l]
 // owned patches followed by halo face slots (multi-GPU, see tgpu_hierarchy_create_distributed).
 static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const TgpuLevelDesc *levels, const int32_t *n_owned,
@@ -810,6 +861,10 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 	size_t    M = 1;
 	for (int i = 0; i < D - 1; i++) M *= n;
 	const size_t NC = M * n;
+	// h^2 -> multiplier table (PatchMeta::tab).  Sizes within the isotropy check's relative 1e-12 share a table.  Past 256
+	// sizes the extra ones point at table 0: unshifted tables are all equal, and tgpu_hierarchy_set_helmholtz refuses a
+	// shift on such a hierarchy.
+	std::map<double, int> tab_of;
 	for (int l = 0; l < nlevels; l++) {
 		const TgpuLevelDesc &d = levels[l];
 		if (d.npatch < 1) return fail(TGPU_ERR_ARG, "level without patches");
@@ -835,6 +890,16 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 					return fail(TGPU_ERR_UNSUPPORTED, "patches must be cubic with isotropic spacing (SURVEY App. A.1)");
 			pm.h2             = hx * hx;
 			pm.inv_h2         = 1.0 / (hx * hx);
+			{
+				const auto near = tab_of.lower_bound(pm.h2 * (1.0 - 1e-12));
+				int        tab  = (int) tab_of.size();
+				if (near != tab_of.end() && near->first <= pm.h2 * (1.0 + 1e-12)) tab = near->second;
+				else {
+					tab_of.emplace(pm.h2, tab);
+					if (tab < 256) h->tab_h2.push_back(pm.h2);
+				}
+				pm.tab = (uint8_t) (tab < 256 ? tab : 0);
+			}
 			pm.neumann        = d.neumann_bits ? d.neumann_bits[p] : 0;
 			if (pm.neumann) L.has_neumann = true;
 			if (pm.neumann && p < L.P) L.neu_host.push_back(p);
@@ -888,28 +953,8 @@ static int hierarchy_create_impl(tgpu_ctx *ctx, int D, int n, int nlevels, const
 		L.Fa = L.Fa_own.get(), L.Fb = L.Fb_own.get();
 		h->levels.push_back(std::move(L));
 	}
-	// multipliers of the two-sided tridiagonal elimination along the axis that is not transformed, for every
-	// pencil of the other axes' transform indices (TriSolve, kernels.cuh): [n/2 + 1][n^(D-1)]
-	{
-		const int                H = n / 2;
-		std::vector<double>      tri((size_t) (H + 1) * M);
-		std::vector<long double> ll(n);
-		for (int k = 0; k < n; k++) {
-			const long double sn = sinl((k + 1) * 3.141592653589793238462643383279502884L / (2 * n));
-			ll[k]                = -4.0L * sn * sn;
-		}
-		for (size_t m = 0; m < M; m++) {
-			const long double mu = (D == 2) ? ll[m] : ll[m % n] + ll[m / n];
-			long double       a  = 0.0L;
-			for (int j = 0; j < H; j++) {
-				const long double d = mu - (j == 0 ? 3.0L : 2.0L);
-				a                   = 1.0L / (d - (j == 0 ? 0.0L : a));
-				tri[(size_t) j * M + m] = (double) a;
-			}
-			tri[(size_t) H * M + m] = (double) (1.0L / (1.0L - a * a));
-		}
-		TRY(dev_upload(h->tri, tri.data(), tri.size()));
-	}
+	h->tab_overflow = tab_of.size() > 256;
+	TRY(upload_tri(h.get()));
 	// general transform path (patches with Neumann domain sides): the six matrices of DftPatchSolver.h:237-289,
 	// M[k][j] such that y_k = sum_j M[k][j] x_j, order TK_*; 1-D eigenvalues -4 sin^2((k + shift) pi / 2n), shift 1, 0, 1/2
 	{
@@ -1324,18 +1369,36 @@ extern "C" int tgpu_hierarchy_info(const tgpu_hier *h, int *D, int *n, int *nlev
 	if (nlevels) *nlevels = (int) h->levels.size();
 	return TGPU_OK;
 }
+// After either call: the cached graphs are dropped, the multiplier tables follow the Helmholtz state (upload_tri), and the
+// buffers of the patch solve paths the new state takes exist.
+static int shifts_changed(tgpu_hier *h)
+{
+	h->graphs.clear();
+	TRY(ensure_scratch32(h));
+	TRY(upload_tri(h));
+	return update_iface_buffers(h);
+}
 // FftwPatchSolver(domain, lambda) / DftPatchSolver(domain, lambda) (PatchSolvers/FftwPatchSolver.h:66,170,
 // DftPatchSolver.h:78,168): the block-Jacobi patch problems become (Laplacian + lambda) u = rhs.  As in the reference the
-// shift lives in the patch solver only; the operator (StarPatchOp) is unchanged.
+// shift lives in the patch solver only; the operator (StarPatchOp) keeps the shift of tgpu_hierarchy_set_helmholtz.
 extern "C" int tgpu_hierarchy_set_lambda(tgpu_hier *h, double lambda)
 {
 	if (!h) return fail(TGPU_ERR_ARG, "null argument");
 	if (!(lambda == lambda)) return fail(TGPU_ERR_ARG, "tgpu_hierarchy_set_lambda: lambda is NaN");
 	h->lambda = lambda;
-	TRY(ensure_scratch32(h));
-	h->graphs.clear();
-	TRY(update_iface_buffers(h));
-	return TGPU_OK;
+	return shifts_changed(h);
+}
+// Helmholtz operator A + lambda I on every level, with the same patch solver shift: the sweeps solve the shifted patch
+// problems exactly, so every kernel and schedule of the Poisson problem applies (DESIGN §3.8).
+extern "C" int tgpu_hierarchy_set_helmholtz(tgpu_hier *h, double lambda)
+{
+	if (!std::isfinite(lambda) || lambda > 0.0)
+		return fail(TGPU_ERR_ARG, "tgpu_hierarchy_set_helmholtz: lambda must be finite and <= 0");
+	if (!h) return fail(TGPU_ERR_ARG, "null argument");
+	if (lambda != 0.0 && h->tab_overflow)
+		return fail(TGPU_ERR_UNSUPPORTED, "tgpu_hierarchy_set_helmholtz: the hierarchy has more than 256 distinct cell sizes");
+	h->op_shift = h->lambda = lambda;
+	return shifts_changed(h);
 }
 extern "C" int tgpu_hierarchy_force_generic_kernels(tgpu_hier *h, int on)
 {
@@ -1526,7 +1589,7 @@ static bool halo_in_kernel(const tgpu_hier *h, int l)
 {
 	static const bool off = getenv("TGPU_HALO_IN_KERNEL") && atoi(getenv("TGPU_HALO_IN_KERNEL")) == 0;
 	const LevelDev &  L   = h->levels[l];
-	return !off && L.p2p && specialised(h) && !h->generic_kernels && !L.has_neumann && h->lambda == 0.0;
+	return !off && L.p2p && specialised(h) && !h->generic_kernels && !L.has_neumann && consistent(h);
 }
 // producer side folded into the consumer kernel as well (halo_push_cta): no separate push launch
 static bool push_in_kernel(const tgpu_hier *h, int l)
@@ -1605,7 +1668,7 @@ static int k_apply(tgpu_hier *h, int l, int mode, const double *u, const double 
 		const dim3 grid(std::min((p1 - p0) * 4, h->ctx->sm_count * 2));
 		if (nb_out) *nb_out = (int) grid.x;
 		auto go = [&](auto kernel, double *o) {
-			return launch(h->ctx, kernel, grid, dim3(TGPU_THREADS), apply3d32_tma_smem_bytes(), (const PatchMeta *) L.meta.get(), p0, p1, u, f, F, o, part, pstride);
+			return launch(h->ctx, kernel, grid, dim3(TGPU_THREADS), apply3d32_tma_smem_bytes(), (const PatchMeta *) L.meta.get(), p0, p1, u, f, F, o, part, pstride, h->op_shift);
 		};
 		if (mode == 0) return go(apply3d32_tma_kernel<0>, out);
 		if (mode == 3) return go(apply3d32_tma_kernel<3>, out);
@@ -1619,7 +1682,7 @@ static int k_apply(tgpu_hier *h, int l, int mode, const double *u, const double 
 		const int grid = std::min(nblk, h->ctx->sm_count * 2);
 		if (nb_out) *nb_out = grid;
 		auto go = [&](auto kernel) {
-			return launch(h->ctx, kernel, dim3(grid), dim3(TGPU_THREADS), apply_tma_smem_bytes<DD, NN>(), (const PatchMeta *) L.meta.get(), p0, p1, u, f, F, out, coarse, part, pstride);
+			return launch(h->ctx, kernel, dim3(grid), dim3(TGPU_THREADS), apply_tma_smem_bytes<DD, NN>(), (const PatchMeta *) L.meta.get(), p0, p1, u, f, F, out, coarse, part, pstride, h->op_shift);
 		};
 		if (mode == 0) return go(apply_tma_kernel<DD, NN, 0>);
 		if (mode == 1) return go(apply_tma_kernel<DD, NN, 1>);
@@ -1643,7 +1706,8 @@ static int launch_smooth3d16(tgpu_hier *h, const LevelDev &L, int p0, int p1, co
 		if (nn == 0) return TGPU_OK;
 		const dim3 gridn(std::min(nn, h->ctx->sm_count * s16_ctas_per_sm(Z, true))), blockn(S16_BLOCK);
 		return launch(h->ctx, smooth3d16_kernel<Z, E, PR, W, false, true>, gridn, blockn, smooth3d16_smem_bytes(), (const PatchMeta *) L.meta.get(), p0,
-		              p1, f, u, Fin, Fout, (const double *) h->tri.get(), uc, HaloSync{}, 0, NeuTabs{h->mats.get(), h->lam.get(), L.neu_list.get() + (b0 - L.neu_host.begin()), nn});
+		              p1, f, u, Fin, Fout, (const double *) h->tri.get(), uc, HaloSync{}, 0,
+		              NeuTabs{h->mats.get(), h->lam.get(), L.neu_list.get() + (b0 - L.neu_host.begin()), nn, helmholtz(h), h->lambda});
 	}
 	const dim3 grid(std::min(p1 - p0, h->ctx->sm_count * s16_ctas_per_sm(Z))), block(S16_BLOCK);
 	if (hs.enabled) {
@@ -1671,14 +1735,16 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 	const bool prolong = uc != nullptr;
 	const PatchMeta *meta = L.meta.get();
 	// A mixed level: the general path sweeps the patches of the range with Neumann domain sides, the specialised kernel skips
-	// them and sweeps the others (two launches, disjoint patches).  lambda != 0 sends every patch through the general path.
-	const bool mixed = specialised(h) && L.has_neumann && h->lambda == 0.0 && !hsp;
-	if (!specialised(h) || L.has_neumann || h->lambda != 0.0) { // the size's general path: the whole range, or its Neumann patches
+	// them and sweeps the others (two launches, disjoint patches).  A smoother-only shift sends every patch through the general
+	// path; in the Helmholtz state the Dirichlet patches read their shifted tables.
+	const bool mixed = specialised(h) && L.has_neumann && !shifted_smoother(h) && !hsp;
+	if (!specialised(h) || L.has_neumann || shifted_smoother(h)) { // the size's general path: the whole range, or its Neumann patches
 		if (is_3d32(h)) { // general transform path through an L2-resident scratch block
 			const int nblk = std::min(p1 - p0, h->ctx->sm_count * 2);
 			if (!h->scratch32) return fail(TGPU_ERR_ARG, "k_smooth: scratch for the general 32^3 patch solve missing");
 			TRY(launch(h->ctx, smooth3d32n_kernel, dim3(nblk), dim3(TGPU_THREADS), 0, meta, p0, p1, f, u, Fin, Fout, uc, (const double *) h->mats.get(),
-			           (const double *) h->lam.get(), h->scratch32.get(), (int) zero_guess, (int) emit, (int) prolong, (int) write_u, h->lambda, (int) mixed));
+			           (const double *) h->lam.get(), h->scratch32.get(), (int) zero_guess, (int) emit, (int) prolong, (int) write_u, h->lambda, (int) mixed,
+			           helmholtz(h)));
 		} else if (mixed && h->D == 3 && h->N == 16) { // the Neumann instantiation of the specialised kernel
 			TRY(smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto W) {
 				return launch_smooth3d16<Z, E, PR, W>(h, L, p0, p1, f, u, Fin, Fout, uc, HaloSync{}, 0, true);
@@ -1691,7 +1757,7 @@ static int k_smooth(tgpu_hier *h, int l, bool zero_guess, bool emit, const doubl
 				const size_t sm = smooth_smem_bytes<DD, NN, true>();
 				TRY(smooth_variant(zero_guess, emit, prolong, write_u, [&](auto Z, auto E, auto PR, auto) {
 					return launch(h->ctx, smooth_kernel<DD, NN, Z, E, PR>, grid, block, sm, meta, p0, p1, f, u, Fin, Fout, (const double *) h->tri.get(), uc,
-					              (const double *) h->mats.get(), (const double *) h->lam.get(), h->lambda, (int) mixed);
+					              (const double *) h->mats.get(), (const double *) h->lam.get(), h->lambda, (int) mixed, helmholtz(h));
 				}));
 			});
 		}
@@ -1970,7 +2036,7 @@ extern "C" int tgpu_smooth_jacobi(tgpu_hier *h, int level, const tgpu_vec *f, tg
 	TRY(k_exchange(h, level, L.Fa, nullptr));
 	TRY(k_apply(h, level, 1, u->d, f->d, L.Fa, L.r.get(), nullptr));
 	TRY(k_exchange_done(h, level));
-	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, jacobi_update_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, (const double *) L.r.get(), u->d, omega));
+	DISPATCH_DN_ALL(h->D, h->N, return launch(h->ctx, jacobi_update_kernel<DD, NN>, dim3(grid_for(h->ctx, L.ncells)), dim3(256), 0, (const PatchMeta *) L.meta.get(), L.P, (const double *) L.r.get(), u->d, omega, h->op_shift));
 	API_END
 }
 extern "C" int tgpu_restrict(tgpu_hier *h, int fine_level, const tgpu_vec *fine, tgpu_vec *coarse)
@@ -2244,9 +2310,9 @@ static int cycle_opts(tgpu_hier *h, const TgpuCycleOpts *opts, TgpuCycleOpts &o)
 	if (opts) o = *opts;
 	else tgpu_cycle_opts_default(&o);
 	o.reserved_ = 0;
-	// With a shifted patch solver the sweep solves (A_p + lambda) u = ..., so the residual of the unshifted operator
-	// right after a sweep is no longer supported on the patch boundaries: the face-only residual schedule does not apply
-	if (h->lambda != 0.0 && o.fused == 1) o.fused = 2;
+	// With a patch solver shift the operator does not carry, the sweep solves (A_p + lambda) u = ..., so the residual of the
+	// operator right after a sweep is no longer supported on the patch boundaries: the face-only residual schedule does not apply
+	if (!consistent(h) && o.fused == 1) o.fused = 2;
 	if (o.pre_sweeps < 0 || o.post_sweeps < 0 || o.coarse_sweeps < 0 || o.mid_sweeps < 0 || (o.cycle_type != 0 && o.cycle_type != 1)
 	    || (o.interpolator != 0 && o.interpolator != 1))
 		return fail(TGPU_ERR_ARG, "tgpu_vcycle: bad cycle options"); /* reference: throw 3, GMG/CycleFactory3d.cpp:131 */
@@ -2261,11 +2327,11 @@ static int cycle_opts(tgpu_hier *h, const TgpuCycleOpts *opts, TgpuCycleOpts &o)
 	}
 	return TGPU_OK;
 }
-// the fused schedule starts from a guess on level 0 when the face identity holds for its sweeps (no shifted patch solve)
+// the fused schedule starts from a guess on level 0 when the face identity holds for its sweeps (consistent shifts)
 // and there is a coarser level; cycle_opts must have run
 static bool guess_schedule(const tgpu_hier *h, const TgpuCycleOpts &o)
 {
-	return fused_schedule(o, h->ctx->nranks) && h->lambda == 0.0 && h->last_level > 0;
+	return fused_schedule(o, h->ctx->nranks) && consistent(h) && h->last_level > 0;
 }
 // Runs run() once, through the hierarchy's cached CUDA graph of key (its f, u, b, fmg_cycles, want_faces, guess and opts):
 // replayed when one was captured before, captured and launched otherwise.  o.use_graph = 0, profiling and several GPUs
